@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] ...    # the reference's CPU learner
+    python bench.py [--gpus N] ... --dump-outputs DIR              # CUDA path: also the last timed step's results as .npy
 
 A "step" is one pass of the learner hot path over one batch of synthetic trajectories: ring
 gather -> MLP actor-critic forward -> fused V-trace loss head -> backward -> (gradient
@@ -30,6 +31,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the source tree: it imports modules the build never
+                                 # imported (freeimpala_b200.dp), whose bytecode caches would otherwise land there
 
 METRIC = "learner_transitions_per_s"
 UNIT = "transitions/s"
@@ -58,7 +61,15 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU work budget of the cpu_baseline leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="CUDA path (--impl b200) only: write what the last step of the headline timed pass computed (losses, "
+                         "parameters, gradients; rank 0) to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the CUDA path (--impl b200)")
+    return args
 
 
 def synth_slots(seed: int, m: int, t: int) -> np.ndarray:
@@ -289,10 +300,12 @@ class Job:
         return float(t.item())
 
 
-def measure(job: Job, args, workload: str, M: int, windows: list, *, with_e2e: bool, with_prof: bool):
+def measure(job: Job, args, workload: str, M: int, windows: list, *, with_e2e: bool, with_prof: bool,
+            with_outputs: bool = False):
     """One workload at M trajectories per GPU: `value` (inputs resident in HBM, EXACTLY K steps between two events on the
     learner's stream, max over ranks), the per-kernel profile of a second, instrumented pass, and `e2e` (host buffers through
-    SharedBuffer::write -> readBatch -> trainModel -> loss read-back, wall clock, max over ranks)."""
+    SharedBuffer::write -> readBatch -> trainModel -> loss read-back, wall clock, max over ranks). `with_outputs` keeps
+    what the last step of the headline pass computed in res["outputs"]."""
     import freeimpala_b200 as fi
     from freeimpala_b200 import dp
     from freeimpala_b200._lib import FiBatch
@@ -365,6 +378,10 @@ def measure(job: Job, args, workload: str, M: int, windows: list, *, with_e2e: b
     ms_total, launches, _ = timed_pass(False)
     res = {"M": M, "ms_per_step": ms_total / K, "value": world * M * T / (ms_total / K / 1e3), "launches": int(launches),
            "per_rank_ms": per_rank_ms[0], "param_count": L.param_count, "ring_cap": ring_cap, "prof": None, "e2e": None}
+    if with_outputs:
+        # what a caller of the step receives after step W + K: its losses and the updated weights, with the gradients that
+        # produced them; read before the instrumented pass moves the weights on
+        res["outputs"] = {"losses": L.last_losses(0), "params": L.get_params(0), "grads": L.get_grads(0)}
     if with_prof:
         ms_prof_total, _, prof = timed_pass(True)
         res["prof"], res["ms_per_step_prof"] = prof, ms_prof_total / K
@@ -535,7 +552,8 @@ def run_b200_arm(args):
     windows = []
     if rank == 0:
         sampler.start()
-    main = measure(job, args, args.workload, M, windows, with_e2e=not args.no_e2e, with_prof=True)
+    main = measure(job, args, args.workload, M, windows, with_e2e=not args.no_e2e, with_prof=True,
+                   with_outputs=bool(args.dump_outputs) and rank == 0)
     # the reference's own learner step (FarmerLstm / MSE / Adam) at the same batch x seq, in the same run: the like-for-like
     # partner of `bench.py --impl reference` (VERDICT r1: the headline V-trace step has no counterpart in the reference)
     ref_wl = None
@@ -629,8 +647,19 @@ def run_b200_arm(args):
                "strong_scaling": wl_block(strong_wl, f"vtrace_mlp_actor_critic learner step, GLOBAL batch {args.batch} x T={T} sharded over "
                                                      f"{world} GPUs (SURVEY.md 8d config 4)")}
         print(json.dumps(out), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, main["outputs"])
     if world > 1:
         job.dist.destroy_process_group()
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """DIR/<name>.npy: losses (float64), params and grads (float32, the whole arena: 4.6 MB each for the actor-critic,
+    6.1 MB for FarmerLstm). Inputs and initial weights are seeded, so two builds run with the same arguments can be
+    compared array by array."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 if __name__ == "__main__":

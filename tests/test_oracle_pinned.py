@@ -95,7 +95,7 @@ def test_checkpoint_format_golden():
 
 
 # ---------------------------------------------------------------- live against oracle/_ref
-needs_ref = pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref not built (no /root/reference)")
+needs_ref = pytest.mark.skipif(not po.ref_available(), reason="oracle/_ref is not in this tree (built from the reference's sources)")
 
 
 @needs_ref
