@@ -204,6 +204,7 @@ constexpr int kWDiscount = 180;
 constexpr int kWAux = 181;
 constexpr int kWX = 192;
 constexpr int kXPerRec = 64;
+constexpr int kFarmerMinEntry = (kXDim + kXPerRec - 1) / kXPerRec;   // 8 records carry x: the shortest FarmerLstm trajectory
 constexpr int kHid = 512;                    // trunk width (reference main.cpp:17-21)
 constexpr int kHead = kNumActions + 1;       // fused policy/value head rows
 constexpr int kLstmH = 128;                  // reference main.cpp:16

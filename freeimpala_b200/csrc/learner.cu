@@ -345,6 +345,11 @@ fi_learner* fi_learner_create(const fi_learner_config* cfg) {
         set_error(FI_ERR_ARG, "fi_learner_create: model %d does not support loss %d", cfg->model, cfg->loss);
         return nullptr;
     }
+    if (farmer && cfg->entry_size < fi::kFarmerMinEntry) {   // a shorter trajectory would train on a truncated x
+        set_error(FI_ERR_ARG, "fi_learner_create: the FarmerLstm model needs entry_size >= %d (x[484] spans records 0..%d), got %zu",
+                  fi::kFarmerMinEntry, fi::kFarmerMinEntry - 1, cfg->entry_size);
+        return nullptr;
+    }
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
         cudaGetLastError();
@@ -1115,7 +1120,7 @@ int fi_learner_debug_relu_masks(fi_learner* l, int player, unsigned char* host, 
     FI_CUDA_OK(cudaMalloc((void**)&dev, n));
     int rc = FI_OK;
     for (int layer = 0; layer < 5 && rc == FI_OK; layer++) {
-        if (const uint32_t* bits = farmer ? nullptr : fi::ac_relu_bits(p, layer)) {
+        if (const uint32_t* bits = farmer ? fi::farmer_relu_bits(p, layer) : fi::ac_relu_bits(p, layer)) {
             // the tensor-core path keeps the decisions its backward pass used as bit masks
             fi::LaunchScope ls("relu_bits_expand_kernel", p->stream, 1.125 * per_layer, fi::kWorkBytes);
             relu_bits_expand_kernel<<<fi::kNumSMs * 4, 256, 0, p->stream>>>(bits, per_layer, dev + layer * per_layer);

@@ -148,6 +148,7 @@ int ac_infer(fi_learner* l, Player* p, const float* params, const float* obs_dev
 const uint32_t* ac_relu_bits(Player* p, int layer);
 int ac_activation(Player* p, int layer, const float** a, const float** lo);
 int farmer_activation(Player* p, int layer, const float** a, const float** lo);
+const uint32_t* farmer_relu_bits(Player* p, int layer);
 // model_farmer.cu
 int farmer_alloc(fi_learner* l, Player* p);
 void farmer_free(Player* p);

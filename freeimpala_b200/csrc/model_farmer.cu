@@ -64,6 +64,7 @@ struct FarmerWs {
     float* colsum_scratch[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     void* slab_ws[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     size_t slab_bytes[6] = {0, 0, 0, 0, 0, 0};
+    bool last_dense_tc = false;                    // the last step's dense stack ran here (relu_bits), not on fp32 act[]
 };
 constexpr int kFeatLdH = 640;   // 612 feature columns padded to whole 128-byte lines of fp16
 constexpr int kDyLd = 32;
@@ -737,6 +738,7 @@ int farmer_forward_backward(fi_learner* l, Player* p, const float* batch, int m,
     float* d = w->d_a;
     int ldd = kHid;
     const bool dense_tc = farmer_dense_tc(l, w, m);
+    w->last_dense_tc = dense_tc;
     if (dense_tc) {
         // As model_ac.cu's backward: every dgrad epilogue applies the ReLU bit mask, writes the next gradient as fp16 pairs and
         // leaves per-32-row column sums (the bias gradient); wgrad split-K slabs and those sums are reduced by two launches.
@@ -852,10 +854,17 @@ int farmer_forward_backward(fi_learner* l, Player* p, const float* batch, int m,
     return FI_OK;
 }
 
+// Bit-packed ReLU decisions of hidden layer `layer` ([rows, 16] words) when the last step ran the dense stack on the tensor
+// cores (they are what its backward pass used), else null: the fp32 activations of farmer_activation hold them.
+const uint32_t* farmer_relu_bits(Player* p, int layer) {
+    const FarmerWs* w = static_cast<const FarmerWs*>(p->farmer_ws);
+    return (w && w->last_dense_tc && layer >= 0 && layer < 5) ? w->relu_bits[layer] : nullptr;
+}
+
 int farmer_activation(Player* p, int layer, const float** a, const float** lo) {
     FarmerWs* w = static_cast<FarmerWs*>(p->farmer_ws);
     if (!w || layer < 0 || layer >= 5) return set_error(FI_ERR_ARG, "no such hidden layer %d", layer);
-    if (w->dhs) return set_error(FI_ERR_STATE, "the dense stack may have run on fp16 pairs: no fp32 activations to read back");
+    if (w->last_dense_tc) return set_error(FI_ERR_STATE, "the dense stack ran on fp16 pairs: no fp32 activations to read back");
     *a = w->act[layer];
     *lo = nullptr;
     return FI_OK;

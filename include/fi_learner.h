@@ -157,7 +157,8 @@ typedef struct fi_learner_config {
     int device;               /* CUDA ordinal */
     int num_players;          /* p  (learner.h ctor) */
     size_t buffer_capacity;   /* B */
-    size_t entry_size;        /* S: records (FI_ELEMENT_SIZE bytes each) per trajectory = T */
+    size_t entry_size;        /* S: records (FI_ELEMENT_SIZE bytes each) per trajectory = T; FarmerLstm needs S >= 8
+                                 (x[484] spans records 0..7) */
     size_t batch_size;        /* M: trajectories per step on THIS rank */
     int model;                /* fi_model_kind */
     int loss;                 /* fi_loss_kind */

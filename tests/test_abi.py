@@ -59,6 +59,14 @@ def test_no_cpu_fallback_without_a_device(fi):
         fi.Learner(1, 4, 5, 2)
 
 
+@pytest.mark.parametrize("s", [1, 4, 7])
+def test_farmer_learner_rejects_trajectories_too_short_for_x(fi, s):
+    """x[484] is carried in words 192..255 of records 0..7 (DESIGN.md, record layout): with fewer than 8 records a farmer
+    learner would train on an x whose tail is zero. Creation refuses, before it looks for a device, so this runs anywhere."""
+    with pytest.raises(fi.FiError, match=r"entry_size >= 8 \(x\[484\] spans records 0\.\.7\), got %d" % s):
+        fi.Learner(1, 4, s, 2, model="farmer_lstm")
+
+
 def test_defaults_follow_the_reference_cli(fi):
     from freeimpala_b200 import _lib
     cfg = _lib.FiLearnerConfig()

@@ -501,12 +501,19 @@ def test_full_size_step_vs_oracle(fi, oracle):
     L.close()
 
 
-@pytest.mark.parametrize("model", ["mlp_actor_critic", "farmer_lstm"])
-def test_graph_replayed_steps_equal_stream_launched_steps(fi, model, monkeypatch):
+@pytest.mark.parametrize("model,partial", [
+    pytest.param("mlp_actor_critic", False, id="mlp_actor_critic"),
+    pytest.param("farmer_lstm", False, id="farmer_lstm"),
+    pytest.param("mlp_actor_critic", True, id="mlp_actor_critic-partial"),
+    pytest.param("farmer_lstm", True, id="farmer_lstm-partial"),
+])
+def test_graph_replayed_steps_equal_stream_launched_steps(fi, model, partial, monkeypatch):
     """fi_learner_step replays the step as one CUDA graph from the third step on (only the optimiser node is re-parameterised:
     step count, snapshot and loss slots). Ten steps through the graph path must give the same bits as ten steps enqueued launch
     by launch (FI_GRAPH=0 is read once per process, so the reference run uses forward_backward + apply_update, which never
-    use the graph), with the batch alternating between two buffers so that the graph is re-captured on the way."""
+    use the graph), with the batch alternating between two buffers so that the graph is re-captured on the way. `partial`:
+    steps 5, 6 and 9 stage m/2 trajectories into the SAME staged buffer as the full batches around them, so only the batch
+    size changes between captures (a graph replayed for the wrong m would read the stale second half of the buffer)."""
     m, t = 16, 20
     farmer = model == "farmer_lstm"
     mk = (lambda: _farmer_learner(fi, m, t, gemm_mode="auto")) if farmer else (lambda: _ac_learner(fi, m, t, gemm_mode="auto"))
@@ -523,12 +530,13 @@ def test_graph_replayed_steps_equal_stream_launched_steps(fi, model, monkeypatch
     n0 = fi.kernel_launch_count()
     ring = A.getSharedBuffers()[0]
     for s in range(10):
+        n = m // 2 if partial and s in (5, 6, 9) else m
         if s % 4 == 3:                       # through the ring now and then: another batch buffer -> re-capture
             assert ring.write_many(slots[s % 3]) == m
             A.trainModel(0, ring.readBatch(m))
         else:
-            A.trainModel(0, A.stage_batch(0, slots[s % 3]))
-        B.forward_backward(0, B.stage_batch(0, slots[s % 3]))
+            A.trainModel(0, A.stage_batch(0, slots[s % 3][:n]))
+        B.forward_backward(0, B.stage_batch(0, slots[s % 3][:n]))
         B.apply_update(0)
         np.testing.assert_allclose(A.last_losses(0), B.last_losses(0), rtol=1e-6)   # loss sums: double atomics, order varies
     assert np.array_equal(A.get_params(0), B.get_params(0))
