@@ -18,7 +18,7 @@ ELEMENT_SIZE = 1024
 DP_ID_BYTES = 128
 MODEL = {"farmer_lstm": 0, "mlp_actor_critic": 1}
 LOSS = {"mse": 0, "mae": 1, "huber": 2, "vtrace": 3}
-OPT = {"adam": 0, "sgd": 1, "adamw": 2}
+OPT = {"adam": 0, "sgd": 1, "adamw": 2, "rmsprop": 3}
 GEMM = {"auto": 0, "simt": 1, "tcgen05": 2, "tcgen05_f16": 3}
 
 
@@ -33,7 +33,9 @@ class FiLearnerConfig(C.Structure):
                 ("optimizer", c_int), ("lr", c_double), ("seed", c_u64),
                 ("rho_bar", c_float), ("c_bar", c_float), ("pg_rho_bar", c_float), ("lambda_", c_float),
                 ("baseline_cost", c_float), ("entropy_cost", c_float),
-                ("gemm_mode", c_int), ("publish_every", c_int), ("checkpoint_location", c_char_p)]
+                ("gemm_mode", c_int), ("publish_every", c_int), ("checkpoint_location", c_char_p),
+                ("max_grad_norm", c_double), ("rmsprop_alpha", c_double), ("rmsprop_eps", c_double),
+                ("rmsprop_momentum", c_double)]
 
 
 class FiProfEntry(C.Structure):
@@ -78,6 +80,8 @@ SIGNATURES = {
     "fi_learner_last_losses": (c_int, [_P, c_int, C.POINTER(c_float)]),
     "fi_learner_last_losses_f64": (c_int, [_P, c_int, C.POINTER(c_double)]),
     "fi_learner_losses_at": (c_int, [_P, c_int, c_u64, C.POINTER(c_float)]),
+    "fi_learner_grad_norm_at": (c_int, [_P, c_int, c_u64, C.POINTER(c_double)]),
+    "fi_learner_set_lr": (c_int, [_P, c_int, c_double]),
     "fi_learner_sync": (c_int, [_P, c_int]),
     "fi_learner_steps_done": (c_u64, [_P, c_int]),
     "fi_learner_debug_relu_masks": (c_int, [_P, c_int, _P, c_size_t]),
@@ -108,6 +112,8 @@ SIGNATURES = {
     "fi_op_vtrace": (c_int, [c_int, c_int] + [_P] * 5 + [c_float] * 4 + [_P, _P, _P]),
     "fi_op_vtrace_loss_head": (c_int, [_P, c_int, c_int, _P, c_int] + [c_float] * 6 + [_P] * 5),
     "fi_op_adam": (c_int, [c_int, c_double, c_i64, c_size_t, _P, _P, _P, _P, c_float, _P]),
+    "fi_op_grad_norm_clip": (c_int, [c_size_t, _P, c_double, _P, _P, _P]),
+    "fi_op_rmsprop": (c_int, [c_double] * 4 + [c_size_t] + [_P] * 6),
     "fi_op_gemm_workspace_bytes": (c_size_t, [c_int] * 5),
     "fi_op_gemm": (c_int, [c_int] * 4 + [_P, c_int, _P, c_int, _P, c_int, _P, c_int, c_int, _P, c_size_t, _P]),
 }

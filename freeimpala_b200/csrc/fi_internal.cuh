@@ -9,8 +9,17 @@ int launch_gather(const void* ring_base, size_t capacity, size_t slot_bytes, siz
 // ring.cu: the consumer of a gathered batch tells the owning ring (looked up by the batch pointer; no-op for other pointers)
 // that every read of it has been enqueued on `consumer`, so that the ring's next gather is ordered behind them
 int ring_note_consumed(const void* dev_ptr, cudaStream_t consumer);
-int launch_opt(int opt_kind, double lr, int64_t step, size_t n, float* p, const float* g, float* m, float* v,
-               float grad_scale, cudaStream_t stream, float* snapshot = nullptr, const double* losses_src = nullptr,
+// The learner's device loss slots: {total, pg, baseline, entropy} of the step, then the pre-clip gradient norm that
+// grad_norm_clip_kernel writes. The optimiser kernel copies all of them into the pinned read-back ring.
+constexpr int kLossWords = 5;
+struct OptConfig {       // what the fused optimiser kernel computes (adam.cu)
+    int kind = FI_OPT_ADAM;  // fi_opt_kind
+    double lr = 0.0;
+    double rms_alpha = 0.99, rms_eps = 1e-8, rms_momentum = 0.0;   // FI_OPT_RMSPROP only
+};
+// coef: device float, the clip coefficient grad_norm_clip_kernel wrote (null = no clipping)
+int launch_opt(const OptConfig& o, int64_t step, size_t n, float* p, const float* g, float* m, float* v, float grad_scale,
+               cudaStream_t stream, const float* coef = nullptr, float* snapshot = nullptr, const double* losses_src = nullptr,
                double* losses_dst = nullptr);
 struct OptLaunchDesc {   // a launch of the fused optimiser kernel, by value (adam.cu)
     const void* func;
@@ -21,8 +30,13 @@ struct OptLaunchDesc {   // a launch of the fused optimiser kernel, by value (ad
     void* args[7];
     double work_bytes;
 };
-int opt_launch_desc(int opt_kind, double lr, int64_t step, size_t n, float* p, const float* g, float* m, float* v, float grad_scale,
-                    float* snapshot, const double* losses_src, double* losses_dst, OptLaunchDesc* d);
+int opt_launch_desc(const OptConfig& o, int64_t step, size_t n, float* p, const float* g, float* m, float* v, float grad_scale,
+                    const float* coef, float* snapshot, const double* losses_src, double* losses_dst, OptLaunchDesc* d);
+// grad_norm.cu: *norm = ||g||_2 (squares and sums in double, deterministic order), *coef = min(1, max_norm / (*norm + 1e-6)).
+// `scratch` holds grad_norm_scratch_bytes() of device memory, zeroed once; the kernel leaves it ready for the next launch,
+// so a captured launch can be replayed.
+size_t grad_norm_scratch_bytes();
+int launch_grad_norm_clip(size_t n, const float* g, double max_norm, double* norm, float* coef, void* scratch, cudaStream_t stream);
 int launch_vtrace_scan(int m, int t, const float* log_rho, const float* discount, const float* reward,
                        const float* value, const float* bootstrap, float rho_bar, float c_bar, float pg_rho_bar,
                        float lambda_, float* vs, float* pg_adv, cudaStream_t stream);

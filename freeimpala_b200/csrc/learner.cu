@@ -220,7 +220,7 @@ void free_player(fi_learner* l, Player* p) {
         if (d) cudaFree(d);
     for (float* d : p->store.dev_snap)
         if (d) cudaFree(d);
-    void* devv[] = {p->d_losses, p->gemm_ws, p->colsum_ws, p->model_ws, p->stage_dev, p->inf_model_ws};
+    void* devv[] = {p->d_losses, p->gemm_ws, p->colsum_ws, p->model_ws, p->stage_dev, p->inf_model_ws, p->clip_coef, p->norm_ws};
     for (void* d : devv)
         if (d) cudaFree(d);
     void* pinned[] = {p->h_losses, p->stage_host, p->inf_host_in, p->inf_host_x, p->inf_host_out,
@@ -253,10 +253,18 @@ int create_player(fi_learner* l, int index) {
         FI_CUDA_OK(cudaMalloc((void**)a, abytes));
         FI_CUDA_OK(cudaMemset(*a, 0, abytes));
     }
-    FI_CUDA_OK(cudaMalloc((void**)&p->d_losses, 4 * sizeof(double)));
-    FI_CUDA_OK(cudaMemset(p->d_losses, 0, 4 * sizeof(double)));
-    FI_CUDA_OK(cudaHostAlloc((void**)&p->h_losses, (Player::kLossRing + 1) * 4 * sizeof(double), cudaHostAllocPortable | cudaHostAllocMapped));
-    memset(p->h_losses, 0, (Player::kLossRing + 1) * 4 * sizeof(double));
+    FI_CUDA_OK(cudaMalloc((void**)&p->d_losses, fi::kLossWords * sizeof(double)));
+    FI_CUDA_OK(cudaMemset(p->d_losses, 0, fi::kLossWords * sizeof(double)));
+    const size_t ring_bytes = (Player::kLossRing + 1) * fi::kLossWords * sizeof(double);
+    FI_CUDA_OK(cudaHostAlloc((void**)&p->h_losses, ring_bytes, cudaHostAllocPortable | cudaHostAllocMapped));
+    memset(p->h_losses, 0, ring_bytes);
+    if (l->cfg.max_grad_norm > 0.0) {
+        FI_CUDA_OK(cudaMalloc((void**)&p->clip_coef, sizeof(float)));
+        FI_CUDA_OK(cudaMemset(p->clip_coef, 0, sizeof(float)));
+        FI_CUDA_OK(cudaMalloc(&p->norm_ws, fi::grad_norm_scratch_bytes()));
+        FI_CUDA_OK(cudaMemset(p->norm_ws, 0, fi::grad_norm_scratch_bytes()));
+    }
+    p->lr = l->cfg.lr;
     FI_CUDA_OK(cudaHostGetDevicePointer((void**)&p->h_losses_dev, p->h_losses, 0));
     for (cudaEvent_t& e : p->loss_ev) FI_CUDA_OK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     FI_CUDA_OK(cudaEventCreateWithFlags(&p->batch_ready, cudaEventDisableTiming));
@@ -303,7 +311,11 @@ bool file_exists(const std::string& path) {
     return stat(path.c_str(), &st) == 0;
 }
 
+// optimiser-state sections of a checkpoint: Adam / AdamW / SGD (m, v = the two Adam moments) and RMSProp (m = momentum
+// buffer, v = square average). The layouts are the same; the magic keeps one family's state out of the other's learner.
 const char kOptMagic[8] = {'F', 'I', 'O', 'P', 'T', '0', '0', '1'};
+const char kRmsMagic[8] = {'F', 'I', 'R', 'M', 'S', '0', '0', '1'};
+const char* opt_magic(const fi_learner* l) { return l->cfg.optimizer == FI_OPT_RMSPROP ? kRmsMagic : kOptMagic; }
 
 }  // namespace
 
@@ -331,6 +343,10 @@ void fi_learner_config_default(fi_learner_config* c) {
     c->gemm_mode = FI_GEMM_AUTO;
     c->publish_every = 1;
     c->checkpoint_location = nullptr;
+    c->max_grad_norm = 0.0;      // no clipping
+    c->rmsprop_alpha = 0.99;     // torch.optim.RMSprop defaults
+    c->rmsprop_eps = 1e-8;
+    c->rmsprop_momentum = 0.0;
 }
 
 fi_learner* fi_learner_create(const fi_learner_config* cfg) {
@@ -343,6 +359,20 @@ fi_learner* fi_learner_create(const fi_learner_config* cfg) {
     if ((farmer && cfg->loss == FI_LOSS_VTRACE) || (!farmer && cfg->loss != FI_LOSS_VTRACE) ||
         (cfg->model != FI_MODEL_FARMER_LSTM && cfg->model != FI_MODEL_MLP_ACTOR_CRITIC)) {
         set_error(FI_ERR_ARG, "fi_learner_create: model %d does not support loss %d", cfg->model, cfg->loss);
+        return nullptr;
+    }
+    if (cfg->optimizer < FI_OPT_ADAM || cfg->optimizer > FI_OPT_RMSPROP) {
+        set_error(FI_ERR_ARG, "fi_learner_create: unknown optimizer %d", cfg->optimizer);
+        return nullptr;
+    }
+    if (!(cfg->max_grad_norm >= 0.0) || !std::isfinite(cfg->max_grad_norm)) {
+        set_error(FI_ERR_ARG, "fi_learner_create: max_grad_norm must be finite and >= 0 (0 = no clipping), got %g", cfg->max_grad_norm);
+        return nullptr;
+    }
+    if (!(cfg->rmsprop_alpha > 0.0 && cfg->rmsprop_alpha < 1.0) || !(cfg->rmsprop_eps > 0.0) || !std::isfinite(cfg->rmsprop_eps) ||
+        !(cfg->rmsprop_momentum >= 0.0 && cfg->rmsprop_momentum < 1.0)) {
+        set_error(FI_ERR_ARG, "fi_learner_create: RMSProp options need 0 < rmsprop_alpha < 1, rmsprop_eps > 0 and 0 <= rmsprop_momentum < 1 "
+                              "(got %g, %g, %g)", cfg->rmsprop_alpha, cfg->rmsprop_eps, cfg->rmsprop_momentum);
         return nullptr;
     }
     if (farmer && cfg->entry_size < fi::kFarmerMinEntry) {   // a shorter trajectory would train on a truncated x
@@ -472,10 +502,31 @@ int begin_update(fi_learner* l, Player* p, UpdateTicket* u) {
     return FI_OK;
 }
 
-// one kernel: the update, the model store's device snapshot and the loss read-back (into mapped pinned memory)
+fi::OptConfig opt_config(const fi_learner* l, const Player* p) {
+    fi::OptConfig o;
+    o.kind = l->cfg.optimizer;
+    o.lr = p->lr;
+    o.rms_alpha = l->cfg.rmsprop_alpha;
+    o.rms_eps = l->cfg.rmsprop_eps;
+    o.rms_momentum = l->cfg.rmsprop_momentum;
+    return o;
+}
+
+// one kernel: the update, the model store's device snapshot and the loss + gradient-norm read-back (into mapped pinned memory)
 int opt_desc_for(fi_learner* l, Player* p, const UpdateTicket& u, fi::OptLaunchDesc* d) {
-    return fi::opt_launch_desc(l->cfg.optimizer, l->cfg.lr, p->opt_step, l->param_count, p->params, p->grads, p->adam_m, p->adam_v, 1.0f,
-                               u.publish ? p->store.dev_snap[u.sn] : nullptr, p->d_losses, p->h_losses_dev + 4 * u.slot, d);
+    return fi::opt_launch_desc(opt_config(l, p), p->opt_step, l->param_count, p->params, p->grads, p->adam_m, p->adam_v, 1.0f,
+                               p->clip_coef, u.publish ? p->store.dev_snap[u.sn] : nullptr, p->d_losses,
+                               p->h_losses_dev + fi::kLossWords * u.slot, d);
+}
+
+// Gradient clipping (max_grad_norm > 0): the global norm of the gradient arena and the clip coefficient, on the device, right
+// before the optimiser. It runs after the all-reduce, so every data-parallel rank derives the same coefficient from the same
+// reduced arena and the replicas stay identical; the optimiser applies the coefficient on the fly and leaves the arena as the
+// all-reduce left it (fi_learner_get_grads returns the unclipped gradient). The norm lands in d_losses[4] and travels with the
+// losses. Fixed for the learner, so the graph replays this launch unchanged.
+int enqueue_clip(fi_learner* l, Player* p) {
+    if (!(l->cfg.max_grad_norm > 0.0)) return FI_OK;
+    return fi::launch_grad_norm_clip(l->param_count, p->grads, l->cfg.max_grad_norm, p->d_losses + 4, p->clip_coef, p->norm_ws, p->stream);
 }
 
 int finish_update(fi_learner* l, Player* p, const UpdateTicket& u) {
@@ -559,6 +610,7 @@ int step_with_graph(fi_learner* l, Player* p, const fi_batch* b, bool* used) {
         int rc = e == cudaSuccess ? FI_OK : FI_ERR_CUDA;
         if (rc == FI_OK) rc = enqueue_forward_backward(l, p, b);
         if (rc == FI_OK) rc = enqueue_allreduce(l, p);
+        if (rc == FI_OK) rc = enqueue_clip(l, p);
         if (rc == FI_OK) {
             fi::LaunchScope ls("fused_opt_kernel", p->stream, d.work_bytes, fi::kWorkBytes);
             e = cudaLaunchKernel(d.func, dim3(d.grid), dim3(d.block), d.args, 0, p->stream);
@@ -599,6 +651,7 @@ int step_with_graph(fi_learner* l, Player* p, const fi_batch* b, bool* used) {
             fprintf(stderr, "[freeimpala_b200] step graph capture failed (player %d): continuing with stream launches\n", p->index);
             FI_TRY(enqueue_forward_backward(l, p, b));
             FI_TRY(enqueue_allreduce(l, p));
+            FI_TRY(enqueue_clip(l, p));
             fi::LaunchScope ls("fused_opt_kernel", p->stream, d.work_bytes, fi::kWorkBytes);
             if (cudaLaunchKernel(d.func, dim3(d.grid), dim3(d.block), d.args, 0, p->stream) != cudaSuccess)
                 return set_error(FI_ERR_CUDA, "launch of fused_opt_kernel failed");
@@ -648,9 +701,10 @@ int fi_learner_apply_update(fi_learner* l, int player) {
     FI_TRY(enqueue_allreduce(l, p));
     UpdateTicket u;
     FI_TRY(begin_update(l, p, &u));
-    FI_TRY(fi::launch_opt(l->cfg.optimizer, l->cfg.lr, p->opt_step, l->param_count, p->params, p->grads, p->adam_m,
-                          p->adam_v, 1.0f, p->stream, u.publish ? p->store.dev_snap[u.sn] : nullptr, p->d_losses,
-                          p->h_losses_dev + 4 * u.slot));
+    FI_TRY(enqueue_clip(l, p));
+    FI_TRY(fi::launch_opt(opt_config(l, p), p->opt_step, l->param_count, p->params, p->grads, p->adam_m, p->adam_v, 1.0f,
+                          p->stream, p->clip_coef, u.publish ? p->store.dev_snap[u.sn] : nullptr, p->d_losses,
+                          p->h_losses_dev + fi::kLossWords * u.slot));
     return finish_update(l, p, u);
 }
 
@@ -680,7 +734,7 @@ int fi_learner_last_losses(fi_learner* l, int player, float losses[4]) {
         FI_CUDA_OK(cudaEventRecord(p->loss_ev[0], p->stream));
     }
     FI_CUDA_OK(cudaEventSynchronize(p->loss_ev[slot]));
-    for (int i = 0; i < 4; i++) losses[i] = (float)p->h_losses[4 * slot + i];
+    for (int i = 0; i < 4; i++) losses[i] = (float)p->h_losses[fi::kLossWords * slot + i];
     return FI_OK;
 }
 int fi_learner_losses_at(fi_learner* l, int player, uint64_t step, float losses[4]) {
@@ -693,16 +747,39 @@ int fi_learner_losses_at(fi_learner* l, int player, uint64_t step, float losses[
     FI_CUDA_OK(cudaSetDevice(l->cfg.device));
     const int slot = (int)(step % Player::kLossRing);
     FI_CUDA_OK(cudaEventSynchronize(p->loss_ev[slot]));
-    for (int i = 0; i < 4; i++) losses[i] = (float)p->h_losses[4 * slot + i];
+    for (int i = 0; i < 4; i++) losses[i] = (float)p->h_losses[fi::kLossWords * slot + i];
     return FI_OK;
 }
 int fi_learner_last_losses_f64(fi_learner* l, int player, double losses[4]) {
     Player* p = get_player(l, player);
     if (!p || !losses) return set_error(FI_ERR_ARG, "fi_learner_last_losses_f64: null argument");
     FI_CUDA_OK(cudaSetDevice(l->cfg.device));
-    FI_CUDA_OK(cudaMemcpyAsync(p->h_losses + 4 * Player::kLossRing, p->d_losses, 4 * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+    double* scratch = p->h_losses + fi::kLossWords * Player::kLossRing;  // scratch slot behind the ring
+    FI_CUDA_OK(cudaMemcpyAsync(scratch, p->d_losses, 4 * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
     FI_CUDA_OK(cudaStreamSynchronize(p->stream));
-    for (int i = 0; i < 4; i++) losses[i] = p->h_losses[4 * Player::kLossRing + i];  // scratch slot behind the ring
+    for (int i = 0; i < 4; i++) losses[i] = scratch[i];
+    return FI_OK;
+}
+int fi_learner_grad_norm_at(fi_learner* l, int player, uint64_t step, double* norm) {
+    Player* p = get_player(l, player);
+    if (!p || !norm) return set_error(FI_ERR_ARG, "fi_learner_grad_norm_at: null argument");
+    if (!(l->cfg.max_grad_norm > 0.0)) return set_error(FI_ERR_STATE, "fi_learner_grad_norm_at: the learner does not clip (max_grad_norm = 0)");
+    const uint64_t done = p->steps_done.load(std::memory_order_acquire);
+    if (step == 0 || step > done || step + Player::kLossRing <= done)
+        return set_error(FI_ERR_ARG, "fi_learner_grad_norm_at: step %llu is not among the last %d of %llu", (unsigned long long)step,
+                         Player::kLossRing, (unsigned long long)done);
+    FI_CUDA_OK(cudaSetDevice(l->cfg.device));
+    const int slot = (int)(step % Player::kLossRing);
+    FI_CUDA_OK(cudaEventSynchronize(p->loss_ev[slot]));
+    *norm = p->h_losses[fi::kLossWords * slot + 4];
+    return FI_OK;
+}
+int fi_learner_set_lr(fi_learner* l, int player, double lr) {
+    Player* p = get_player(l, player);
+    if (!p) return FI_ERR_ARG;
+    if (!(lr >= 0.0) || !std::isfinite(lr)) return set_error(FI_ERR_ARG, "fi_learner_set_lr: lr must be finite and >= 0, got %g", lr);
+    std::lock_guard<std::mutex> step_lock(p->step_mu);   // the next update (graph or stream) reads it under the same lock
+    p->lr = lr;
     return FI_OK;
 }
 uint64_t fi_learner_steps_done(fi_learner* l, int player) {
@@ -968,7 +1045,7 @@ int fi_model_save(fi_learner* l, int player, uint64_t iteration, int with_optimi
         bool ok = fwrite(&version, sizeof(version), 1, f) == 1 && fwrite(blob.data(), 1, blob.size(), f) == blob.size();
         if (ok && with_optimizer_state) {
             const uint64_t n = l->param_count;
-            ok = fwrite(kOptMagic, 1, 8, f) == 8 && fwrite(&opt_step, 8, 1, f) == 1 && fwrite(&n, 8, 1, f) == 1 &&
+            ok = fwrite(opt_magic(l), 1, 8, f) == 8 && fwrite(&opt_step, 8, 1, f) == 1 && fwrite(&n, 8, 1, f) == 1 &&
                  fwrite(om.data(), 4, n, f) == n && fwrite(ov.data(), 4, n, f) == n;
         }
         ok = (fclose(f) == 0) && ok;
@@ -1026,7 +1103,12 @@ int fi_model_load(fi_learner* l, const char* dir) {
         char magic[8];
         uint64_t opt_step = 0, n = 0;
         std::vector<float> om, ov;
-        bool have_opt = fread(magic, 1, 8, f) == 8 && memcmp(magic, kOptMagic, 8) == 0 && fread(&opt_step, 8, 1, f) == 1 &&
+        const bool have_magic = fread(magic, 1, 8, f) == 8;
+        const char* other = opt_magic(l) == kOptMagic ? kRmsMagic : kOptMagic;
+        if (have_magic && memcmp(magic, other, 8) == 0)   // never read one optimiser family's state as the other's
+            fprintf(stderr, "[freeimpala_b200] %s: optimiser state written by %s, this learner runs %s: loaded the weights only\n",
+                    path.c_str(), other == kRmsMagic ? "RMSProp" : "Adam/AdamW/SGD", other == kRmsMagic ? "Adam/AdamW/SGD" : "RMSProp");
+        bool have_opt = have_magic && memcmp(magic, opt_magic(l), 8) == 0 && fread(&opt_step, 8, 1, f) == 1 &&
                         fread(&n, 8, 1, f) == 1 && n == l->param_count;
         if (have_opt) {
             om.resize(n);

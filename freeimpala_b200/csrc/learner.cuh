@@ -70,15 +70,18 @@ struct Player {
     int index = 0;
     std::mutex step_mu;         // serialises enqueueing on `stream` against checkpoint / arena access
     cudaStream_t stream = nullptr;
-    float *params = nullptr, *grads = nullptr, *adam_m = nullptr, *adam_v = nullptr;
+    float *params = nullptr, *grads = nullptr, *adam_m = nullptr, *adam_v = nullptr;  // RMSProp: m = momentum buffer, v = square average
     int64_t opt_step = 0;
+    double lr = 0.0;            // learning rate of the next optimiser step (fi_learner_set_lr), written under step_mu
+    float* clip_coef = nullptr; // device float: the clip coefficient of this step (max_grad_norm > 0 only)
+    void* norm_ws = nullptr;    // grad_norm_clip_kernel's block partials and ticket
     std::atomic<uint64_t> steps_done{0};  // written under step_mu (release), read without it by fi_learner_losses_at / steps_done
     uint64_t version = 1;       // version of the weights in `params` (Model ctor -> 1, :55-58,127)
-    double* d_losses = nullptr; // device double[4]
+    double* d_losses = nullptr; // device double[kLossWords]: the four loss sums, then the step's pre-clip gradient norm
     // loss read-back ring: step s (1-based) lands in slot s % kLossRing of the pinned array, so that a host loop can read
     // step s-1's losses while step s runs (fi_learner_losses_at) without stalling the stream
     static constexpr int kLossRing = 8;
-    double* h_losses = nullptr; // pinned double[kLossRing + 1][4]
+    double* h_losses = nullptr; // pinned double[kLossRing + 1][kLossWords]
     double* h_losses_dev = nullptr;  // the same memory as the device sees it (the optimiser kernel writes the losses there)
     cudaEvent_t loss_ev[kLossRing] = {};
     cudaEvent_t batch_ready = nullptr;

@@ -78,7 +78,9 @@ class Learner:
                  T: int = 0, *, device: int = 0, model: str = "mlp_actor_critic", loss: str | None = None,
                  optimizer: str = "adam", lr: float = 5e-4, seed: int = 0, gemm_mode: str = "auto",
                  publish_every: int = 1, rho_bar: float = 1.0, c_bar: float = 1.0, pg_rho_bar: float = 1.0,
-                 lambda_: float = 1.0, baseline_cost: float = 0.5, entropy_cost: float = 0.01):
+                 lambda_: float = 1.0, baseline_cost: float = 0.5, entropy_cost: float = 0.01,
+                 max_grad_norm: float = 0.0, rmsprop_alpha: float = 0.99, rmsprop_eps: float = 1e-8,
+                 rmsprop_momentum: float = 0.0):
         self._lib = _lib.load()
         self.num_players, self.buffer_capacity, self.entry_size, self.batch_size = p, B, S, M
         self.train_time_ms, self.checkpoint_frequency = r, c
@@ -92,6 +94,8 @@ class Learner:
         cfg.rho_bar, cfg.c_bar, cfg.pg_rho_bar, cfg.lambda_ = rho_bar, c_bar, pg_rho_bar, lambda_
         cfg.baseline_cost, cfg.entropy_cost = baseline_cost, entropy_cost
         cfg.gemm_mode, cfg.publish_every = _lib.GEMM[gemm_mode], publish_every
+        cfg.max_grad_norm = max_grad_norm   # global-norm gradient clipping; 0 = off
+        cfg.rmsprop_alpha, cfg.rmsprop_eps, cfg.rmsprop_momentum = rmsprop_alpha, rmsprop_eps, rmsprop_momentum
         self._ckpt = l.encode() if l else None
         cfg.checkpoint_location = self._ckpt
         self._h = self._lib.fi_learner_create(C.byref(cfg))
@@ -220,6 +224,16 @@ class Learner:
         out = (C.c_float * 4)()
         check(self._lib.fi_learner_losses_at(self._h, player_index, step, out), "fi_learner_losses_at")
         return np.array(list(out), dtype=np.float64)
+
+    def grad_norm_at(self, player_index: int, step: int) -> float:
+        """Pre-clip gradient L2 norm of optimiser step `step` (one of the last 8; needs max_grad_norm > 0)."""
+        out = C.c_double()
+        check(self._lib.fi_learner_grad_norm_at(self._h, player_index, step, C.byref(out)), "fi_learner_grad_norm_at")
+        return out.value
+
+    def set_lr(self, player_index: int, lr: float) -> None:
+        """Learning rate of this player's optimiser from its next update on (e.g. a linear decay, one call per step)."""
+        check(self._lib.fi_learner_set_lr(self._h, player_index, lr), "fi_learner_set_lr")
 
     def debug_relu_masks(self, player_index: int, rows: int) -> np.ndarray:
         out = np.empty((5, rows * 512), np.uint8)

@@ -30,6 +30,17 @@ def adam(kind: str, lr: float, step: int, n: int, p: int, g: int, m: int, v: int
     check(_lib.load().fi_op_adam(_lib.OPT[kind], lr, step, n, p, g, m, v, grad_scale, stream), "fi_op_adam")
 
 
+def rmsprop(lr: float, n: int, p: int, g: int, square_avg: int, momentum_buf: int = None, alpha=0.99, eps=1e-8,
+            momentum=0.0, coef: int = None, stream=None) -> None:
+    """torch.optim.RMSprop (centered=False, weight_decay=0) over n fp32 values; `coef` (device float) multiplies g first."""
+    check(_lib.load().fi_op_rmsprop(lr, alpha, eps, momentum, n, p, g, square_avg, momentum_buf, coef, stream), "fi_op_rmsprop")
+
+
+def grad_norm_clip(n: int, g: int, max_norm: float, norm: int, coef: int, stream=None) -> None:
+    """*norm (device double) = ||g||_2, *coef (device float) = min(1, max_norm / (norm + 1e-6))."""
+    check(_lib.load().fi_op_grad_norm_clip(n, g, max_norm, norm, coef, stream), "fi_op_grad_norm_clip")
+
+
 TRANS = {"NT": 0, "NN": 1, "TN": 2}
 
 
