@@ -213,14 +213,14 @@ void free_player(fi_learner* l, Player* p) {
     p->graph_exec = p->graph = nullptr;
     if (p->nccl_comm && nccl().ok) nccl().CommDestroy((ncclComm_t)p->nccl_comm);
     if (l->cfg.model == FI_MODEL_FARMER_LSTM) fi::farmer_free(p);
-    else fi::ac_free(p);
-    float* dev[] = {p->params, p->grads, p->adam_m, p->adam_v, p->d_a, p->d_b, p->head, p->dhead,
-                    p->inf_in, p->inf_x, p->inf_out};
+    fi::dense_free(&p->dense);
+    fi::dense_free(&p->inf_dense);
+    float* dev[] = {p->params, p->grads, p->adam_m, p->adam_v, p->head, p->dhead, p->inf_in, p->inf_x, p->inf_out};
     for (float* d : dev)
         if (d) cudaFree(d);
     for (float* d : p->store.dev_snap)
         if (d) cudaFree(d);
-    void* devv[] = {p->d_losses, p->gemm_ws, p->colsum_ws, p->model_ws, p->stage_dev, p->inf_model_ws, p->clip_coef, p->norm_ws};
+    void* devv[] = {p->d_losses, p->gemm_ws, p->colsum_ws, p->stage_dev, p->clip_coef, p->norm_ws};
     for (void* d : devv)
         if (d) cudaFree(d);
     void* pinned[] = {p->h_losses, p->stage_host, p->inf_host_in, p->inf_host_x, p->inf_host_out,
@@ -1202,18 +1202,20 @@ int fi_learner_debug_relu_masks(fi_learner* l, int player, unsigned char* host, 
     FI_CUDA_OK(cudaMalloc((void**)&dev, n));
     int rc = FI_OK;
     for (int layer = 0; layer < 5 && rc == FI_OK; layer++) {
-        if (const uint32_t* bits = farmer ? fi::farmer_relu_bits(p, layer) : fi::ac_relu_bits(p, layer)) {
-            // the tensor-core path keeps the decisions its backward pass used as bit masks
+        if (const uint32_t* bits = fi::dense_relu_bits(p->dense, layer)) {
+            // the split-operand path keeps the decisions its backward pass used as bit masks
             fi::LaunchScope ls("relu_bits_expand_kernel", p->stream, 1.125 * per_layer, fi::kWorkBytes);
             relu_bits_expand_kernel<<<fi::kNumSMs * 4, 256, 0, p->stream>>>(bits, per_layer, dev + layer * per_layer);
             rc = ls.done();
             continue;
         }
-        const float *a = nullptr, *lo = nullptr;
-        rc = farmer ? fi::farmer_activation(p, layer, &a, &lo) : fi::ac_activation(p, layer, &a, &lo);
-        if (rc != FI_OK) break;
+        const float* a = fi::dense_activation(p->dense, layer);
+        if (!a) {
+            rc = set_error(FI_ERR_STATE, "fi_learner_debug_relu_masks: no activations of the last step to read back");
+            break;
+        }
         fi::LaunchScope ls("relu_mask_kernel", p->stream, 5.0 * per_layer, fi::kWorkBytes);
-        relu_mask_kernel<<<fi::kNumSMs * 4, 256, 0, p->stream>>>(a, lo, per_layer, dev + layer * per_layer);
+        relu_mask_kernel<<<fi::kNumSMs * 4, 256, 0, p->stream>>>(a, nullptr, per_layer, dev + layer * per_layer);
         rc = ls.done();
     }
     if (rc == FI_OK && cudaMemcpyAsync(host, dev, n, cudaMemcpyDeviceToHost, p->stream) != cudaSuccess) rc = FI_ERR_CUDA;

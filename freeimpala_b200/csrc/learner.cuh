@@ -1,5 +1,6 @@
 // Internal learner structures shared by learner.cu (host orchestration, model store, DP),
-// model_ac.cu (MLP actor-critic V-trace step) and model_farmer.cu (FarmerLstm step).
+// model_ac.cu (MLP actor-critic V-trace step), model_farmer.cu (FarmerLstm step) and
+// dense_stack.cu (the 5 x Linear(512) + ReLU stack and linear head both steps end in).
 #pragma once
 #include <atomic>
 #include <condition_variable>
@@ -56,6 +57,54 @@ struct PublishTicket {                      // argument of the publication host 
     uint64_t version;
 };
 
+// fp16 elements of a split observation row: 162 padded to 192 = three whole 128-byte lines per row, so that every TMA box row
+// (one 64-element k-block of one observation) is ONE aligned line; with the minimal 168 (336-byte rows) each box row straddled
+// two lines and layer 1's operand loads took 5800 clocks (profiles/r2_gemm_trace.md)
+constexpr int kObsLdH = 192;
+
+// The dense stack (dense_stack.cu): five Linear(512) + ReLU layers and a linear head. The actor-critic runs it as its whole
+// trunk (162 -> 512 x 5 -> 17), FarmerLstm after the LSTM (612 -> 512 x 5 -> 1); the shape is data, the code is one.
+struct DenseShape {
+    int in;       // input width
+    int in_ld;    // row stride of the split input pair and of dense1.w's re-laid-out copy (split-operand path)
+    int out;      // head width
+    int w0;       // tensor index of dense1.w: layer l's weight / bias are w0 + 2l / w0 + 2l + 1, the head's w0 + 10 / w0 + 11
+};
+// HScale slots of the split-operand path's 3xFP16 format (one per split tensor)
+enum { kHsW = 0, kHsIn = 1, kHsDout = 2, kHsAct0 = 3, kHsD0 = 8, kHsCount = 14 };
+constexpr int kDoutLd = 32;   // the output gradient pair [rows, 32]: `out` columns padded to one k-block, the rest stay zero
+enum DenseUse { kDenseNone = 0, kDenseForward = 1, kDenseTrain = 2 };   // which buffers dense_alloc provides for a path
+
+struct DenseStack {
+    DenseShape sh{};
+    size_t rows = 0;
+    bool last_split = false;                       // the last forward ran on split operands: relu_bits hold its ReLU decisions
+    // Split-operand path: every wgrad keeps its split-K slabs and every dgrad its column sums until the end of the backward
+    // pass, where two launches (grad_reduce.cu) sum them all into the gradient arena.
+    bool split = false, half = false;              // split buffers exist; 3xFP16 (fp16 pairs + HScales) instead of 3xTF32
+    size_t esz = 0;                                // bytes per element of the hi / lo arrays
+    HScale* hs = nullptr;                          // [kHsCount], 3xFP16 only
+    void *w_hi = nullptr, *w_lo = nullptr;         // split parameter arena (same element offsets as params)
+    void *w1_hi = nullptr, *w1_lo = nullptr;       // dense1.w re-laid out as [512, in_ld]
+    void *in_hi = nullptr, *in_lo = nullptr;       // [rows, in_ld]
+    // per-layer outputs [rows, 512]; forward-only stacks hold two buffers and alternate them (layer l writes buffer l % 2)
+    void* act_hi[5] = {};
+    void* act_lo[5] = {};
+    uint32_t* relu_bits[5] = {};                   // [rows, 16] words: act_l > 0, bit-packed (training only)
+    void* d_hi[2] = {};
+    void* d_lo[2] = {};                            // back-propagated gradient ping-pong [rows, 512]
+    void *dout_hi = nullptr, *dout_lo = nullptr;   // the loss gradient dL/dy [rows, kDoutLd]
+    float* colsum_part[5] = {};                    // [4 * ceil(rows/128), 512] left by the dgrad that produced d_l
+    float* colsum_scratch[6] = {};                 // row-block partials of the 5 layer biases + the head bias
+    void* slab[6] = {};                            // split-K slabs of the 5 layer wgrads + the head wgrad
+    size_t slab_bytes[6] = {};
+    // plain fp32 path
+    float* act[5] = {};                            // [rows, 512]
+    float* d[2] = {};                              // [rows, max(in, 512)]: the layer-0 dgrad writes all `in` columns
+};
+
+struct FarmerWs;   // model_farmer.cu
+
 struct InferReq {   // one caller of fi_learner_infer waiting for its rows
     const float* obs;
     const float* x;
@@ -87,15 +136,13 @@ struct Player {
     cudaEvent_t batch_ready = nullptr;
     size_t last_rows = 0;
     bool grads_valid = false;
-    // step workspaces (model specific, sized for batch_size x entry_size rows)
-    std::vector<float*> act;    // activations
-    float *d_a = nullptr, *d_b = nullptr, *head = nullptr, *dhead = nullptr;
-    void* gemm_ws = nullptr; size_t gemm_ws_bytes = 0;
-    void* colsum_ws = nullptr; size_t colsum_ws_bytes = 0;
-    void* model_ws = nullptr;
-    void* ac_tc = nullptr;          // AcTc (model_ac.cu): hi/lo activation pairs of the tensor-core path
-    void* farmer_ws = nullptr;      // FarmerWs (model_farmer.cu): training workspaces
-    void* farmer_inf_ws = nullptr;  // FarmerWs for batched inference
+    // step workspaces (sized for the step's rows: batch_size x entry_size for the actor-critic, batch_size for FarmerLstm)
+    DenseStack dense;               // the step's dense stack
+    float *head = nullptr, *dhead = nullptr;   // actor-critic: head output [rows, 17] and the loss head's fp32 gradient of it
+    void* gemm_ws = nullptr; size_t gemm_ws_bytes = 0;       // actor-critic FFMA path
+    void* colsum_ws = nullptr; size_t colsum_ws_bytes = 0;   // actor-critic
+    FarmerWs* farmer_ws = nullptr;      // FarmerLstm training workspaces
+    FarmerWs* farmer_inf_ws = nullptr;  // FarmerLstm workspaces for batched inference
     unsigned char* stage_dev = nullptr;  // staged batch (fi_learner_stage_batch)
     unsigned char* stage_host = nullptr; // pinned bounce buffer for pageable sources
     size_t stage_bytes = 0;
@@ -108,8 +155,7 @@ struct Player {
     cudaStream_t infer_stream = nullptr;
     float *inf_in = nullptr, *inf_x = nullptr, *inf_out = nullptr;
     float *inf_host_in = nullptr, *inf_host_x = nullptr, *inf_host_out = nullptr;  // pinned
-    std::vector<float*> inf_act;
-    void* inf_model_ws = nullptr;
+    DenseStack inf_dense;       // the dense stack of batched inference (forward only)
     size_t inf_rows_cap = 0, inf_t_cap = 0;
     // the step as one CUDA graph (learner.cu step_with_graph)
     void* graph_exec = nullptr;       // cudaGraphExec_t
@@ -139,19 +185,36 @@ struct fi_learner {
 };
 
 namespace fi {
+// dense_stack.cu. `rows` of a forward / backward call may be fewer than the stack was allocated for.
+// split / plain: the buffers of each path; a forward-only split stack keeps two activation pairs and no masks.
+int dense_alloc(DenseStack* s, const DenseShape& sh, size_t rows, size_t arena_elems, DenseUse split, bool half, DenseUse plain);
+void dense_free(DenseStack* s);   // frees every buffer and leaves an empty stack
+// Split-operand path. The parameter arena and dense1.w's re-laid-out copy as hi/lo pairs (3xFP16: hs[kHsW] must be zero; one
+// cooperative launch measures max |p| and writes both). The caller splits the input into in_hi / in_lo itself (scale
+// hs[kHsIn]) and, for the backward pass, the loss gradient into dout_hi / dout_lo (scale hs[kHsDout]).
+int dense_split_params(const fi_learner* l, DenseStack* s, const float* params, cudaStream_t st);
+int dense_forward_split(const fi_learner* l, DenseStack* s, const float* params, int rows, float* y, cudaStream_t st);
+// dout: the loss gradient in fp32 [rows, out] (3xFP16: the head bias gradient is its column sum; 3xTF32 sums the pair with
+// colsum_ws instead). din (may be null): the first din_cols columns of dL/d(input), [rows, din_cols].
+int dense_backward_split(const fi_learner* l, DenseStack* s, const float* dout, int rows, float* g, float* din, int din_cols,
+                         void* colsum_ws, size_t colsum_ws_bytes, cudaStream_t st);
+// Plain fp32 path through launch_gemm(mode): x [rows, in] with row stride ldx. din (may be null) receives dL/d(input)
+// [rows, in] (row stride in), which is one of the stack's d buffers.
+int dense_forward_plain(const fi_learner* l, DenseStack* s, int mode, const float* params, const float* x, int ldx, int rows, float* y,
+                        void* ws, size_t ws_bytes, cudaStream_t st);
+int dense_backward_plain(const fi_learner* l, DenseStack* s, int mode, const float* params, const float* x, int ldx, const float* dout,
+                         int rows, float* g, const float** din, void* ws, size_t ws_bytes, void* colsum_ws, size_t colsum_ws_bytes,
+                         cudaStream_t st);
+// ReLU decisions of hidden layer `layer` of the last forward: bit-packed [rows, 16] words when it ran on split operands, else
+// the fp32 activations [rows, 512]; the other accessor returns null
+const uint32_t* dense_relu_bits(const DenseStack& s, int layer);
+const float* dense_activation(const DenseStack& s, int layer);
 // model_ac.cu
 int ac_alloc(fi_learner* l, Player* p);
-void ac_free(Player* p);
 int ac_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int t, int global_m);
 int ac_infer_alloc(fi_learner* l, Player* p, size_t rows);
-void ac_infer_free(Player* p);
 int ac_infer(fi_learner* l, Player* p, const float* params, const float* obs_dev, size_t rows, float* out_dev,
              cudaStream_t stream);
-// ReLU outputs of hidden layer `layer` of the last forward: *a (+ *lo when stored as a hi/lo pair)
-const uint32_t* ac_relu_bits(Player* p, int layer);
-int ac_activation(Player* p, int layer, const float** a, const float** lo);
-int farmer_activation(Player* p, int layer, const float** a, const float** lo);
-const uint32_t* farmer_relu_bits(Player* p, int layer);
 // model_farmer.cu
 int farmer_alloc(fi_learner* l, Player* p);
 void farmer_free(Player* p);

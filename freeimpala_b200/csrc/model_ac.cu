@@ -3,48 +3,17 @@
 // transition to the 162-feature observation; one fused head [17, 512]: 16 policy logits + value.
 // Parameter order: dense1.w [512,162], dense1.b, dense2..5 .w [512,512], .b, head.w [17,512], head.b.
 //
-// Two execution paths, same math:
-//  * tensor-core path (gemm_mode auto / tcgen05): every GEMM is the tcgen05 3xTF32 kernel (gemm_tc.cu).
-//    Activations and back-propagated gradients live in HBM as exact hi/lo pairs written by the
-//    producing GEMM's epilogue, so no GEMM ever re-splits its big operand; only the observations
-//    (read out of the gathered batch, row stride 256 words) and the weights are split by a pre-pass.
-//  * SIMT path (gemm_mode simt): fp32 FFMA GEMMs (gemm_simt.cu); the first GEMM reads the
-//    observations straight out of the gathered batch.
+// The trunk and head are the dense stack (dense_stack.cu), on one of its two paths:
+//  * split operands (gemm_mode auto / tcgen05 / tcgen05_f16): the tcgen05 kernel (gemm_tc.cu) in the 3xFP16 format, or in
+//    3xTF32 for gemm_mode tcgen05 (and auto with FI_AC_FORMAT=tf32). The observations are split out of the gathered batch
+//    (row stride 256 words) by a pre-pass here.
+//  * plain fp32 (gemm_mode simt): FFMA GEMMs (gemm_simt.cu); the first GEMM reads the observations straight out of the
+//    gathered batch.
 #include "learner.cuh"
 
 namespace fi {
 
 constexpr int kObsLd = 164;     // 162 observation words padded to a 16-byte multiple (TMA row stride), 3xTF32 format
-constexpr int kObsLdH = 192;    // fp16 elements: 162 padded to 192 = three whole 128-byte lines per row, so that every TMA box row
-                                // (one 64-element k-block of one observation) is ONE aligned line; with the minimal 168 (336-byte
-                                // rows) each box row straddled two lines and layer 1's operand loads took 5800 clocks (profiles/r2_gemm_trace.md)
-constexpr int kDheadLd = 32;    // 17 head gradients padded to one TF32 k-block
-
-// HScale slots of the 3xFP16 format (one per split tensor)
-enum { kHsW = 0, kHsObs = 1, kHsDhead = 2, kHsAct0 = 3, kHsD0 = 8, kHsCount = 14 };
-
-struct AcTc {  // tensor-core path state, owned by the Player (Player::ac_tc)
-    bool half = false;                             // 3xFP16 (fp16 pairs + per-tensor scales) instead of 3xTF32
-    size_t esz = 4;                                // bytes per element of the hi / lo arrays
-    int obs_ld = kObsLd;
-    HScale* hs = nullptr;                          // [kHsCount], fp16 format only
-    void *w_hi = nullptr, *w_lo = nullptr;         // split parameter arena (same element offsets as params)
-    void *w1_hi = nullptr, *w1_lo = nullptr;       // dense1.w re-laid out as [512, obs_ld]
-    void *obs_hi = nullptr, *obs_lo = nullptr;     // [rows, obs_ld]
-    void* act_hi[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    void* act_lo[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    void* d_hi[2] = {nullptr, nullptr};
-    void* d_lo[2] = {nullptr, nullptr};
-    void *dhead_hi = nullptr, *dhead_lo = nullptr;   // [rows, 32], columns 17..31 stay zero
-    float* dhead = nullptr;                          // fp16 format: the loss head's plain fp32 output [rows, 17]
-    uint32_t* relu_bits[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};  // [rows, 16] words: act_l > 0, bit-packed
-    // Every wgrad product keeps its split-K slabs and every dgrad epilogue its per-32-row column sums until the end of the
-    // backward pass, where two launches (grad_reduce.cu) sum them all into the gradient arena.
-    float* colsum_part[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};  // [4 * ceil(rows/128), 512] left by the dgrad that produced d_l
-    float* colsum_scratch[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};  // row-block partials of the 5 layer biases + the head bias
-    void* ws[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // split-K slabs of the 5 layer wgrads + the head wgrad
-    size_t ws_bytes[6] = {0, 0, 0, 0, 0, 0};
-};
 
 static bool use_tc(const fi_learner* l) { return l->cfg.gemm_mode != FI_GEMM_SIMT && gemm_tc_available(); }
 
@@ -56,339 +25,89 @@ int ac_alloc(fi_learner* l, Player* p) {
     p->colsum_ws_bytes = colsum_workspace_bytes((int)rows, kHid);
     FI_CUDA_OK(cudaMalloc(&p->colsum_ws, p->colsum_ws_bytes));
     if (use_tc(l)) {
-        AcTc* t = new AcTc();
-        p->ac_tc = t;
         // AUTO picks the 3xFP16 format (twice the tensor-core rate of 3xTF32 at the same 22 significant bits);
         // FI_AC_FORMAT=tf32 keeps AUTO on 3xTF32 (A/B experiments)
         const char* fmt = getenv("FI_AC_FORMAT");
-        t->half = l->cfg.gemm_mode == FI_GEMM_TCGEN05_F16 || (l->cfg.gemm_mode == FI_GEMM_AUTO && !(fmt && fmt[0] == 't'));
-        t->esz = t->half ? 2 : 4;
-        t->obs_ld = t->half ? kObsLdH : kObsLd;
-        const size_t ab = ((l->arena_elems + 7) & ~(size_t)7) * t->esz, rb = rows * kHid * t->esz;
-        FI_CUDA_OK(cudaMalloc((void**)&t->w_hi, ab));
-        FI_CUDA_OK(cudaMalloc((void**)&t->w_lo, ab));
-        FI_CUDA_OK(cudaMalloc((void**)&t->w1_hi, (size_t)kHid * t->obs_ld * t->esz));
-        FI_CUDA_OK(cudaMalloc((void**)&t->w1_lo, (size_t)kHid * t->obs_ld * t->esz));
-        FI_CUDA_OK(cudaMalloc((void**)&t->obs_hi, rows * t->obs_ld * t->esz));
-        FI_CUDA_OK(cudaMalloc((void**)&t->obs_lo, rows * t->obs_ld * t->esz));
-        if (t->half) {
-            FI_CUDA_OK(cudaMalloc((void**)&t->hs, kHsCount * sizeof(HScale)));
-            FI_CUDA_OK(cudaMalloc((void**)&t->dhead, rows * kHead * sizeof(float)));
-        }
-        for (int i = 0; i < 5; i++) {
-            FI_CUDA_OK(cudaMalloc((void**)&t->act_hi[i], rb));
-            FI_CUDA_OK(cudaMalloc((void**)&t->act_lo[i], rb));
-            FI_CUDA_OK(cudaMalloc((void**)&t->relu_bits[i], rows * (kHid / 32) * sizeof(uint32_t)));
-        }
-        for (int i = 0; i < 2; i++) {
-            FI_CUDA_OK(cudaMalloc((void**)&t->d_hi[i], rb));
-            FI_CUDA_OK(cudaMalloc((void**)&t->d_lo[i], rb));
-        }
-        FI_CUDA_OK(cudaMalloc((void**)&t->dhead_hi, rows * kDheadLd * t->esz));
-        FI_CUDA_OK(cudaMalloc((void**)&t->dhead_lo, rows * kDheadLd * t->esz));
-        FI_CUDA_OK(cudaMemset(t->dhead_hi, 0, rows * kDheadLd * t->esz));
-        FI_CUDA_OK(cudaMemset(t->dhead_lo, 0, rows * kDheadLd * t->esz));
-        const int part_rows = 4 * (int)((rows + 127) / 128);
-        for (int i = 0; i < 5; i++) {
-            FI_CUDA_OK(cudaMalloc((void**)&t->colsum_part[i], (size_t)part_rows * kHid * sizeof(float)));
-            FI_CUDA_OK(cudaMalloc((void**)&t->colsum_scratch[i], grad_colsum_scratch_bytes(part_rows, kHid)));
-            t->ws_bytes[i] = gemm_tc_split_workspace_bytes(2, kHid, i == 0 ? kZDim : kHid, (int)rows);
-        }
-        FI_CUDA_OK(cudaMalloc((void**)&t->colsum_scratch[5], grad_colsum_scratch_bytes((int)rows, kHead)));
-        t->ws_bytes[5] = gemm_tc_split_workspace_bytes(2, kHid, kHead, (int)rows);
-        for (int i = 0; i < 6; i++)
-            if (t->ws_bytes[i]) FI_CUDA_OK(cudaMalloc(&t->ws[i], t->ws_bytes[i]));
+        const bool half = l->cfg.gemm_mode == FI_GEMM_TCGEN05_F16 || (l->cfg.gemm_mode == FI_GEMM_AUTO && !(fmt && fmt[0] == 't'));
+        FI_TRY(dense_alloc(&p->dense, DenseShape{kZDim, half ? kObsLdH : kObsLd, kHead, 0}, rows, l->arena_elems, kDenseTrain, half,
+                           kDenseNone));
+        // 3xFP16: the loss head writes plain fp32 rows (and their max |x|), split afterwards; 3xTF32: it writes the pair itself
+        if (half) FI_CUDA_OK(cudaMalloc((void**)&p->dhead, rows * kHead * sizeof(float)));
         return FI_OK;
     }
-    p->act.assign(5, nullptr);
-    for (int i = 0; i < 5; i++) FI_CUDA_OK(cudaMalloc((void**)&p->act[i], rows * kHid * sizeof(float)));
-    FI_CUDA_OK(cudaMalloc((void**)&p->d_a, rows * kHid * sizeof(float)));
-    FI_CUDA_OK(cudaMalloc((void**)&p->d_b, rows * kHid * sizeof(float)));
+    FI_TRY(dense_alloc(&p->dense, DenseShape{kZDim, 0, kHead, 0}, rows, l->arena_elems, kDenseNone, false, kDenseTrain));
     FI_CUDA_OK(cudaMalloc((void**)&p->dhead, rows * kHead * sizeof(float)));
     p->gemm_ws_bytes = gemm_simt_workspace_bytes(2, kHid, kHid, (int)rows);
     if (p->gemm_ws_bytes) FI_CUDA_OK(cudaMalloc(&p->gemm_ws, p->gemm_ws_bytes));
     return FI_OK;
 }
 
-void ac_infer_free(Player* p);
-
-void ac_free(Player* p) {
-    ac_infer_free(p);
-    for (auto a : p->act) if (a) cudaFree(a);
-    p->act.clear();
-    for (auto a : p->inf_act) if (a) cudaFree(a);
-    p->inf_act.clear();
-    if (AcTc* t = static_cast<AcTc*>(p->ac_tc)) {
-        void* f[] = {t->w_hi, t->w_lo, t->w1_hi, t->w1_lo, t->obs_hi, t->obs_lo, t->dhead_hi, t->dhead_lo, t->d_hi[0],
-                     t->d_hi[1], t->d_lo[0], t->d_lo[1], t->hs, t->dhead};
-        for (void* x : f) if (x) cudaFree(x);
-        for (int i = 0; i < 6; i++) {
-            if (i < 5 && t->colsum_part[i]) cudaFree(t->colsum_part[i]);
-            if (t->colsum_scratch[i]) cudaFree(t->colsum_scratch[i]);
-            if (t->ws[i]) cudaFree(t->ws[i]);
-        }
-        for (int i = 0; i < 5; i++) {
-            if (t->act_hi[i]) cudaFree(t->act_hi[i]);
-            if (t->act_lo[i]) cudaFree(t->act_lo[i]);
-            if (t->relu_bits[i]) cudaFree(t->relu_bits[i]);
-        }
-        delete t;
-        p->ac_tc = nullptr;
-    }
-}
-
-// Bit-packed ReLU decisions of hidden layer `layer` ([rows, 16] words) when the tensor-core path recorded them, else null.
-const uint32_t* ac_relu_bits(Player* p, int layer) {
-    AcTc* t = static_cast<AcTc*>(p->ac_tc);
-    return (t && layer >= 0 && layer < 5) ? t->relu_bits[layer] : nullptr;
-}
-
-int ac_activation(Player* p, int layer, const float** a, const float** lo) {
-    if (layer < 0 || layer >= 5) return set_error(FI_ERR_ARG, "no such hidden layer %d", layer);
-    if (AcTc* t = static_cast<AcTc*>(p->ac_tc)) {
-        if (t->half) return set_error(FI_ERR_STATE, "activations are fp16 pairs in this format: use the bit masks");
-        *a = static_cast<const float*>(t->act_hi[layer]);
-        *lo = static_cast<const float*>(t->act_lo[layer]);
-    } else {
-        *a = p->act[layer];
-        *lo = nullptr;
-    }
-    return FI_OK;
-}
-
-// ---------------------------------------------------------------- SIMT path ------------------
-static int ac_forward_simt(fi_learner* l, const float* params, const float* in, int ld_in, int rows,
-                           float* const* act, float* head, void* ws, size_t ws_bytes, cudaStream_t st) {
-    const auto& T = l->tensors;
-    const float* x = in;
-    int ldx = ld_in, k = kZDim;
-    for (int layer = 0; layer < 5; layer++) {
-        FI_TRY(launch_gemm_simt(0, rows, kHid, k, x, ldx, params + T[2 * layer].offset, k, act[layer], kHid,
-                                params + T[2 * layer + 1].offset, 1, nullptr, 0, ws, ws_bytes, st));
-        x = act[layer];
-        ldx = kHid;
-        k = kHid;
-    }
-    return launch_gemm_simt(0, rows, kHead, kHid, x, kHid, params + T[10].offset, kHid, head, kHead,
-                            params + T[11].offset, 0, nullptr, 0, ws, ws_bytes, st);
-}
-
-static int ac_forward_backward_simt(fi_learner* l, Player* p, const float* batch, int m, int t) {
-    const auto& T = l->tensors;
+int ac_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int t, int /*global_m*/) {
     const auto& c = l->cfg;
+    DenseStack* s = &p->dense;
     const int rows = m * t;
     cudaStream_t st = p->stream;
-    FI_TRY(ac_forward_simt(l, p->params, batch, kRecWords, rows, p->act.data(), p->head, p->gemm_ws, p->gemm_ws_bytes, st));
-    FI_TRY(launch_zero2(p->d_losses, 4 * sizeof(double), nullptr, 0, st));
-    FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
-                                   c.baseline_cost, c.entropy_cost, p->dhead, nullptr, nullptr, p->d_losses, st));
-    // head: dW = dhead^T act4, db = colsum(dhead), d4 = (dhead Wh) * relu'(act4)
-    float* g = p->grads;
-    FI_TRY(launch_colsum(p->dhead, kHead, rows, kHead, g + T[11].offset, p->colsum_ws, p->colsum_ws_bytes, st));
-    FI_TRY(launch_gemm_simt(2, kHead, kHid, rows, p->dhead, kHead, p->act[4], kHid, g + T[10].offset, kHid, nullptr,
-                            0, nullptr, 0, p->gemm_ws, p->gemm_ws_bytes, st));
-    float* d = p->d_a;
-    float* d_next = p->d_b;
-    FI_TRY(launch_gemm_simt(1, rows, kHid, kHead, p->dhead, kHead, p->params + T[10].offset, kHid, d, kHid, nullptr,
-                            0, p->act[4], kHid, p->gemm_ws, p->gemm_ws_bytes, st));
-    for (int layer = 4; layer >= 0; layer--) {
-        const float* in = layer == 0 ? batch : p->act[layer - 1];
-        const int ld_in = layer == 0 ? kRecWords : kHid, k = layer == 0 ? kZDim : kHid;
-        FI_TRY(launch_colsum(d, kHid, rows, kHid, g + T[2 * layer + 1].offset, p->colsum_ws, p->colsum_ws_bytes, st));
-        FI_TRY(launch_gemm_simt(2, kHid, k, rows, d, kHid, in, ld_in, g + T[2 * layer].offset, k, nullptr, 0, nullptr,
-                                0, p->gemm_ws, p->gemm_ws_bytes, st));
-        if (layer > 0) {
-            FI_TRY(launch_gemm_simt(1, rows, kHid, kHid, d, kHid, p->params + T[2 * layer].offset, kHid, d_next, kHid,
-                                    nullptr, 0, p->act[layer - 1], kHid, p->gemm_ws, p->gemm_ws_bytes, st));
-            float* tmp = d; d = d_next; d_next = tmp;
-        }
+    if (!s->split) {
+        FI_TRY(dense_forward_plain(l, s, FI_GEMM_SIMT, p->params, batch, kRecWords, rows, p->head, p->gemm_ws, p->gemm_ws_bytes, st));
+        FI_TRY(launch_zero2(p->d_losses, 4 * sizeof(double), nullptr, 0, st));
+        FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
+                                       c.baseline_cost, c.entropy_cost, p->dhead, nullptr, nullptr, p->d_losses, st));
+        return dense_backward_plain(l, s, FI_GEMM_SIMT, p->params, batch, kRecWords, p->dhead, rows, p->grads, nullptr, p->gemm_ws,
+                                    p->gemm_ws_bytes, p->colsum_ws, p->colsum_ws_bytes, st);
     }
-    return FI_OK;
-}
-
-// ---------------------------------------------------------------- tensor-core path -----------
-static int ac_forward_backward_tc(fi_learner* l, Player* p, const float* batch, int m, int t) {
-    const auto& T = l->tensors;
-    const auto& c = l->cfg;
-    AcTc* tc = static_cast<AcTc*>(p->ac_tc);
-    const int rows = m * t;
-    cudaStream_t st = p->stream;
-    float* g = p->grads;
     // pre-passes: weights (4.6 MB) and observations -> hi/lo pairs
-    const bool H = tc->half;
-    HScale* hs = tc->hs;
-    auto HS = [&](int slot) -> HScale* { return H ? hs + slot : nullptr; };
-    auto off = [&](void* base, size_t elems) -> void* { return static_cast<char*>(base) + elems * tc->esz; };
-    if (H) {
+    if (s->half) {
         // one scale for the whole parameter arena (weights and biases), one for the observations; every activation and
         // back-propagated gradient gets its scale from the producing GEMM (bound k * amax_a * amax_b, gemm_tc.cu)
-        FI_TRY(launch_zero2(hs, kHsCount * sizeof(HScale), p->d_losses, 4 * sizeof(double), st));
-        // parameters: max |p|, the split of the arena and dense1.w's re-laid-out copy in one cooperative launch
-        const int arena_ld = (int)((l->arena_elems + 7) & ~(size_t)7);
-        FI_TRY(launch_amax_split_params(p->params, (int)l->arena_elems, arena_ld, tc->w_hi, tc->w_lo, p->params + T[0].offset, kHid, kZDim,
-                                        tc->obs_ld, tc->w1_hi, tc->w1_lo, hs + kHsW, st));
+        FI_TRY(launch_zero2(s->hs, kHsCount * sizeof(HScale), p->d_losses, 4 * sizeof(double), st));
+        FI_TRY(dense_split_params(l, s, p->params, st));
         // observations: max |x| and the split in one cooperative launch (the second pass reads the batch out of L2)
-        FI_TRY(launch_amax_split_h(batch, kRecWords, (size_t)rows, kZDim, tc->obs_ld, tc->obs_hi, tc->obs_lo, hs + kHsObs, st));
+        FI_TRY(launch_amax_split_h(batch, kRecWords, (size_t)rows, kZDim, kObsLdH, s->in_hi, s->in_lo, s->hs + kHsIn, st));
     } else {
-        FI_TRY(launch_split_tf32(p->params, (int)l->arena_elems, 1, (int)l->arena_elems, (int)l->arena_elems, (float*)tc->w_hi, (float*)tc->w_lo, st));
-        FI_TRY(launch_split_tf32(p->params + T[0].offset, kZDim, kHid, kZDim, kObsLd, (float*)tc->w1_hi, (float*)tc->w1_lo, st));
-        FI_TRY(launch_split_tf32(batch, kRecWords, (size_t)rows, kZDim, kObsLd, (float*)tc->obs_hi, (float*)tc->obs_lo, st));
+        FI_TRY(dense_split_params(l, s, p->params, st));
+        FI_TRY(launch_split_tf32(batch, kRecWords, (size_t)rows, kZDim, kObsLd, (float*)s->in_hi, (float*)s->in_lo, st));
     }
-    auto W = [&](int tensor, int ld) { return SplitMat{off(tc->w_hi, T[tensor].offset), off(tc->w_lo, T[tensor].offset), ld, HS(kHsW)}; };
-    auto ACT = [&](int layer) { return SplitMat{tc->act_hi[layer], tc->act_lo[layer], kHid, HS(kHsAct0 + layer)}; };
-    const SplitMat obs{tc->obs_hi, tc->obs_lo, tc->obs_ld, HS(kHsObs)}, w1{tc->w1_hi, tc->w1_lo, tc->obs_ld, HS(kHsW)};
-    // forward: x_l = relu(x_{l-1} W_l^T + b_l), written as hi/lo pairs by the GEMM epilogue
-    for (int layer = 0; layer < 5; layer++) {
-        const SplitMat x = layer == 0 ? obs : ACT(layer - 1);
-        const SplitMat w = layer == 0 ? w1 : W(2 * layer, kHid);
-        const TcOut out{nullptr, 0, tc->act_hi[layer], tc->act_lo[layer], kHid, 0, nullptr, tc->relu_bits[layer], kHid / 32, nullptr,
-                        HS(kHsAct0 + layer), HS(kHsW)};
-        FI_TRY(launch_gemm_tc_split(0, rows, kHid, layer == 0 ? kZDim : kHid, x, w, out, p->params + T[2 * layer + 1].offset, 1,
-                                    nullptr, 0, nullptr, 0, st));
-    }
-    FI_TRY(launch_gemm_tc_split(0, rows, kHead, kHid, ACT(4), W(10, kHid), TcOut{p->head, kHead, nullptr, nullptr, 0, 0, nullptr, nullptr, 0, nullptr},
-                                p->params + T[11].offset, 0, nullptr, 0, nullptr, 0, st));
-    if (!H) FI_TRY(launch_zero2(p->d_losses, 4 * sizeof(double), nullptr, 0, st));
-    if (H) {  // the loss head writes plain fp32 rows and their max |x|; the fp16 split follows (13 MB)
+    FI_TRY(dense_forward_split(l, s, p->params, rows, p->head, st));
+    if (s->half) {  // the loss head writes plain fp32 rows and their max |x|; the fp16 split follows (13 MB)
         FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
-                                       c.baseline_cost, c.entropy_cost, tc->dhead, nullptr, nullptr, p->d_losses, st, nullptr, nullptr, 0,
-                                       hs + kHsDhead));
-        FI_TRY(launch_split_h(tc->dhead, kHead, (size_t)rows, kHead, kDheadLd, tc->dhead_hi, tc->dhead_lo, hs + kHsDhead, 1, st));
+                                       c.baseline_cost, c.entropy_cost, p->dhead, nullptr, nullptr, p->d_losses, st, nullptr, nullptr, 0,
+                                       s->hs + kHsDout));
+        FI_TRY(launch_split_h(p->dhead, kHead, (size_t)rows, kHead, kDoutLd, s->dout_hi, s->dout_lo, s->hs + kHsDout, 1, st));
     } else {
+        FI_TRY(launch_zero2(p->d_losses, 4 * sizeof(double), nullptr, 0, st));
         FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
-                                       c.baseline_cost, c.entropy_cost, nullptr, nullptr, nullptr, p->d_losses, st, (float*)tc->dhead_hi,
-                                       (float*)tc->dhead_lo, kDheadLd));
+                                       c.baseline_cost, c.entropy_cost, nullptr, nullptr, nullptr, p->d_losses, st, (float*)s->dout_hi,
+                                       (float*)s->dout_lo, kDoutLd));
     }
-    const SplitMat dhead{tc->dhead_hi, tc->dhead_lo, kDheadLd, HS(kHsDhead)};
-    // head: db = colsum(dhead); dWh^T [512,17] = act4^T dhead, stored transposed as dWh [17,512];
-    // d4 = (dhead Wh) * relu'(act4). Bias column sums and split-K slab sums are deferred to launch_grad_finalize below.
-    GradSegTable segs;
-    int splits = 1;
-    const int part_rows = 4 * ((rows + 127) / 128);
-    if (H) FI_TRY(grad_table_add_colsum(&segs, tc->dhead, kHead, rows, kHead, g + T[11].offset, tc->colsum_scratch[5]));
-    else FI_TRY(launch_colsum2((float*)tc->dhead_hi, (float*)tc->dhead_lo, kDheadLd, rows, kHead, g + T[11].offset, p->colsum_ws, p->colsum_ws_bytes, st));
-    {
-        TcOut o{g + T[10].offset, kHid, nullptr, nullptr, 0, 1, nullptr, nullptr, 0, nullptr};
-        o.deferred_splits = &splits;
-        FI_TRY(launch_gemm_tc_split(2, kHid, kHead, rows, ACT(4), dhead, o, nullptr, 0, nullptr, 0, tc->ws[5], tc->ws_bytes[5], st));
-        if (splits > 1) FI_TRY(grad_table_add_slabs(&segs, (const float*)tc->ws[5], splits, (size_t)kHid * kHead, kHid * kHead, g + T[10].offset));
-    }
-    int cur = 0, dslot = kHsD0;
-    FI_TRY(launch_gemm_tc_split(1, rows, kHid, kHead, dhead, W(10, kHid),
-                                TcOut{nullptr, 0, tc->d_hi[cur], tc->d_lo[cur], kHid, 0, tc->relu_bits[4], nullptr, kHid / 32, tc->colsum_part[4],
-                                      HS(dslot), nullptr},
-                                nullptr, 0, nullptr, 0, nullptr, 0, st));
-    for (int layer = 4; layer >= 0; layer--) {
-        const SplitMat d{tc->d_hi[cur], tc->d_lo[cur], kHid, HS(dslot)};
-        const SplitMat x = layer == 0 ? obs : ACT(layer - 1);
-        const int k = layer == 0 ? kZDim : kHid;
-        // bias gradient: the dgrad epilogue that produced d left per-32-row column sums (6.5 MB instead of re-reading 420 MB)
-        FI_TRY(grad_table_add_colsum(&segs, tc->colsum_part[layer], kHid, part_rows, kHid, g + T[2 * layer + 1].offset, tc->colsum_scratch[layer]));
-        {
-            TcOut o{g + T[2 * layer].offset, k, nullptr, nullptr, 0, 0, nullptr, nullptr, 0, nullptr};
-            o.deferred_splits = &splits;
-            FI_TRY(launch_gemm_tc_split(2, kHid, k, rows, d, x, o, nullptr, 0, nullptr, 0, tc->ws[layer], tc->ws_bytes[layer], st));
-            if (splits > 1) FI_TRY(grad_table_add_slabs(&segs, (const float*)tc->ws[layer], splits, (size_t)kHid * k, kHid * k, g + T[2 * layer].offset));
-        }
-        if (layer > 0) {
-            FI_TRY(launch_gemm_tc_split(1, rows, kHid, kHid, d, W(2 * layer, kHid),
-                                        TcOut{nullptr, 0, tc->d_hi[cur ^ 1], tc->d_lo[cur ^ 1], kHid, 0, tc->relu_bits[layer - 1], nullptr,
-                                              kHid / 32, tc->colsum_part[layer - 1], HS(dslot + 1), nullptr},
-                                        nullptr, 0, nullptr, 0, nullptr, 0, st));
-            cur ^= 1;
-            dslot++;
-        }
-    }
-    return launch_grad_finalize(&segs, st);
-}
-
-int ac_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int t, int /*global_m*/) {
-    return p->ac_tc ? ac_forward_backward_tc(l, p, batch, m, t) : ac_forward_backward_simt(l, p, batch, m, t);
+    return dense_backward_split(l, s, p->dhead, rows, p->grads, nullptr, 0, p->colsum_ws, p->colsum_ws_bytes, st);
 }
 
 // ---------------------------------------------------------------- batched actor inference -----
 // (SURVEY.md 8f rank 2) the forward kernels of the learner step on the published device snapshot of the weights:
 // obs_dev [rows,162] -> out_dev [rows,17]. Small batches (a few actors x a few rows) run the fp32 FFMA kernels; from
 // kInferTcRows rows on, the tensor-core forward of the step: 3xFP16 operand pairs, the same tcgen05 kernel and epilogue,
-// with two ping-pong activation buffers instead of five (nothing is kept for a backward pass).
+// with two alternating activation buffers instead of five (nothing is kept for a backward pass).
 constexpr size_t kInferTcRows = 256;
 
-struct AcInfTc {
-    size_t rows_cap = 0;
-    HScale* hs = nullptr;                                // [kHsCount]
-    void *w_hi = nullptr, *w_lo = nullptr, *w1_hi = nullptr, *w1_lo = nullptr;
-    void *obs_hi = nullptr, *obs_lo = nullptr;           // [rows, 168]
-    void* act_hi[2] = {nullptr, nullptr};
-    void* act_lo[2] = {nullptr, nullptr};                // [rows, 512]
-};
-
-static void ac_inf_tc_free(AcInfTc* t) {
-    if (!t) return;
-    void* f[] = {t->hs, t->w_hi, t->w_lo, t->w1_hi, t->w1_lo, t->obs_hi, t->obs_lo, t->act_hi[0], t->act_hi[1], t->act_lo[0], t->act_lo[1]};
-    for (void* x : f) if (x) cudaFree(x);
-    delete t;
-}
-
-void ac_infer_free(Player* p) {
-    ac_inf_tc_free(static_cast<AcInfTc*>(p->inf_model_ws));
-    p->inf_model_ws = nullptr;
-}
-
 int ac_infer_alloc(fi_learner* l, Player* p, size_t rows) {
-    for (auto a : p->inf_act) if (a) cudaFree(a);
-    p->inf_act.assign(5, nullptr);
-    for (int i = 0; i < 5; i++) FI_CUDA_OK(cudaMalloc((void**)&p->inf_act[i], rows * kHid * sizeof(float)));
-    ac_infer_free(p);
-    if (use_tc(l) && l->cfg.gemm_mode != FI_GEMM_TCGEN05 && rows >= kInferTcRows) {
-        AcInfTc* t = new AcInfTc();
-        p->inf_model_ws = t;
-        t->rows_cap = rows;
-        const size_t ab = ((l->arena_elems + 7) & ~(size_t)7) * 2, rb = rows * kHid * 2;
-        FI_CUDA_OK(cudaMalloc((void**)&t->hs, kHsCount * sizeof(HScale)));
-        FI_CUDA_OK(cudaMalloc((void**)&t->w_hi, ab));
-        FI_CUDA_OK(cudaMalloc((void**)&t->w_lo, ab));
-        FI_CUDA_OK(cudaMalloc((void**)&t->w1_hi, (size_t)kHid * kObsLdH * 2));
-        FI_CUDA_OK(cudaMalloc((void**)&t->w1_lo, (size_t)kHid * kObsLdH * 2));
-        FI_CUDA_OK(cudaMalloc((void**)&t->obs_hi, rows * kObsLdH * 2));
-        FI_CUDA_OK(cudaMalloc((void**)&t->obs_lo, rows * kObsLdH * 2));
-        for (int i = 0; i < 2; i++) {
-            FI_CUDA_OK(cudaMalloc((void**)&t->act_hi[i], rb));
-            FI_CUDA_OK(cudaMalloc((void**)&t->act_lo[i], rb));
-        }
-    }
-    return FI_OK;
-}
-
-static int ac_infer_tc(fi_learner* l, AcInfTc* t, const float* params, const float* obs_dev, int rows, float* out_dev, cudaStream_t st) {
-    const auto& T = l->tensors;
-    HScale* hs = t->hs;
-    const int arena_ld = (int)((l->arena_elems + 7) & ~(size_t)7);
-    auto off = [&](void* base, size_t elems) -> void* { return static_cast<char*>(base) + elems * 2; };
-    FI_TRY(launch_zero2(hs, kHsCount * sizeof(HScale), nullptr, 0, st));
-    FI_TRY(launch_amax(params, (int)l->arena_elems, 1, (int)l->arena_elems, hs + kHsW, st));
-    FI_TRY(launch_amax(obs_dev, kZDim, (size_t)rows, kZDim, hs + kHsObs, st));
-    FI_TRY(launch_split_h(params, (int)l->arena_elems, 1, (int)l->arena_elems, arena_ld, t->w_hi, t->w_lo, hs + kHsW, 1, st));
-    FI_TRY(launch_split_h(params + T[0].offset, kZDim, kHid, kZDim, kObsLdH, t->w1_hi, t->w1_lo, hs + kHsW, 0, st));
-    FI_TRY(launch_split_h(obs_dev, kZDim, (size_t)rows, kZDim, kObsLdH, t->obs_hi, t->obs_lo, hs + kHsObs, 1, st));
-    SplitMat x{t->obs_hi, t->obs_lo, kObsLdH, hs + kHsObs};
-    for (int layer = 0; layer < 5; layer++) {
-        const SplitMat w = layer == 0 ? SplitMat{t->w1_hi, t->w1_lo, kObsLdH, hs + kHsW}
-                                      : SplitMat{off(t->w_hi, T[2 * layer].offset), off(t->w_lo, T[2 * layer].offset), kHid, hs + kHsW};
-        const int cur = layer & 1;
-        const TcOut out{nullptr, 0, t->act_hi[cur], t->act_lo[cur], kHid, 0, nullptr, nullptr, kHid / 32, nullptr, hs + kHsAct0 + layer, hs + kHsW};
-        FI_TRY(launch_gemm_tc_split(0, rows, kHid, layer == 0 ? kZDim : kHid, x, w, out, params + T[2 * layer + 1].offset, 1, nullptr, 0, nullptr, 0, st));
-        x = SplitMat{t->act_hi[cur], t->act_lo[cur], kHid, hs + kHsAct0 + layer};
-    }
-    const SplitMat wh{off(t->w_hi, T[10].offset), off(t->w_lo, T[10].offset), kHid, hs + kHsW};
-    return launch_gemm_tc_split(0, rows, kHead, kHid, x, wh, TcOut{out_dev, kHead, nullptr, nullptr, 0, 0, nullptr, nullptr, 0, nullptr},
-                                params + T[11].offset, 0, nullptr, 0, nullptr, 0, st);
+    dense_free(&p->inf_dense);
+    const DenseUse split = use_tc(l) && l->cfg.gemm_mode != FI_GEMM_TCGEN05 && rows >= kInferTcRows ? kDenseForward : kDenseNone;
+    return dense_alloc(&p->inf_dense, DenseShape{kZDim, kObsLdH, kHead, 0}, rows, l->arena_elems, split, true, kDenseForward);
 }
 
 int ac_infer(fi_learner* l, Player* p, const float* params, const float* obs_dev, size_t rows, float* out_dev,
              cudaStream_t stream) {
-    AcInfTc* t = static_cast<AcInfTc*>(p->inf_model_ws);
-    if (t && rows >= kInferTcRows && rows <= t->rows_cap) return ac_infer_tc(l, t, params, obs_dev, (int)rows, out_dev, stream);
-    return ac_forward_simt(l, params, obs_dev, kZDim, (int)rows, p->inf_act.data(), out_dev, nullptr, 0, stream);
+    DenseStack* s = &p->inf_dense;
+    if (!s->split || rows < kInferTcRows || rows > s->rows)
+        return dense_forward_plain(l, s, FI_GEMM_SIMT, params, obs_dev, kZDim, (int)rows, out_dev, nullptr, 0, stream);
+    const int n = (int)l->arena_elems;
+    FI_TRY(launch_zero2(s->hs, kHsCount * sizeof(HScale), nullptr, 0, stream));
+    FI_TRY(launch_amax(params, n, 1, n, s->hs + kHsW, stream));
+    FI_TRY(launch_amax(obs_dev, kZDim, rows, kZDim, s->hs + kHsIn, stream));
+    FI_TRY(launch_split_h(params, n, 1, n, (int)((l->arena_elems + 7) & ~(size_t)7), s->w_hi, s->w_lo, s->hs + kHsW, 1, stream));
+    FI_TRY(launch_split_h(params + l->tensors[0].offset, kZDim, kHid, kZDim, kObsLdH, s->w1_hi, s->w1_lo, s->hs + kHsW, 0, stream));
+    FI_TRY(launch_split_h(obs_dev, kZDim, rows, kZDim, kObsLdH, s->in_hi, s->in_lo, s->hs + kHsIn, 1, stream));
+    return dense_forward_split(l, s, params, (int)rows, out_dev, stream);
 }
 
 }  // namespace fi

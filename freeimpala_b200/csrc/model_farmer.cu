@@ -30,8 +30,6 @@ struct FarmerWs {
     float* y = nullptr;       // [rows]
     float* dy = nullptr;      // [rows]
     float* target = nullptr;  // [rows]
-    float* act[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};  // [rows, 512]
-    float *d_a = nullptr, *d_b = nullptr;  // [rows, 612]
     void* gemm_ws = nullptr; size_t gemm_ws_bytes = 0;
     void* colsum_ws = nullptr; size_t colsum_ws_bytes = 0;
     size_t rows = 0, t = 0;
@@ -40,37 +38,17 @@ struct FarmerWs {
     // W_ih gradient, the gate gradients serve both weight gradients
     bool half = false;
     HScale* hs = nullptr;                          // [4]: observations, W_ih, gate gradients, h_prev
-    void *obs_hi = nullptr, *obs_lo = nullptr;     // [rows*T, 168] fp16
-    void *wih_hi = nullptr, *wih_lo = nullptr;     // [512, 168]
+    void *obs_hi = nullptr, *obs_lo = nullptr;     // [rows*T, 192] fp16
+    void *wih_hi = nullptr, *wih_lo = nullptr;     // [512, 192]
     void *dg_hi = nullptr, *dg_lo = nullptr;       // [rows*T, 512]
     void *hp_hi = nullptr, *hp_lo = nullptr;       // [rows*T, 128]
     void* split_ws = nullptr; size_t split_ws_bytes = 0;
     float* bias_part = nullptr;                    // [CTAs of the BPTT kernel, 512]: their column sums of dG (the LSTM bias gradient)
-    // Dense stack on the tensor cores, as model_ac.cu runs its trunk: the parameter arena split once per step, every
-    // activation and back-propagated gradient written as fp16 pairs by the GEMM that produces it (with its ReLU bit mask /
-    // the per-32-row column sums for the bias gradient), split-K slabs and column sums reduced by two launches at the end.
-    HScale* dhs = nullptr;                         // [kDhCount]
-    void *w_hi = nullptr, *w_lo = nullptr;         // split parameter arena (same element offsets as params)
-    void *w1_hi = nullptr, *w1_lo = nullptr;       // dense1.w re-laid out as [512, 640]
-    void *feat_hi = nullptr, *feat_lo = nullptr;   // [rows, 640]
-    void* act_hi[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    void* act_lo[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    uint32_t* relu_bits[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    void* dd_hi[2] = {nullptr, nullptr};
-    void* dd_lo[2] = {nullptr, nullptr};
-    void *dy_hi = nullptr, *dy_lo = nullptr;       // [rows, 32], columns 1..31 stay zero
-    float* dfeat = nullptr;                        // [rows, 128]: dL/dh_{T-1} (the x part of the feature row needs no gradient)
-    float* colsum_part[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-    float* colsum_scratch[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    void* slab_ws[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    size_t slab_bytes[6] = {0, 0, 0, 0, 0, 0};
-    bool last_dense_tc = false;                    // the last step's dense stack ran here (relu_bits), not on fp32 act[]
+    float* dfeat = nullptr;                        // [rows, 128]: dL/dh_{T-1} from the split-operand dense stack (the x part of the
+                                                   // feature row needs no gradient)
 };
 constexpr int kFeatLdH = 640;   // 612 feature columns padded to whole 128-byte lines of fp16
-constexpr int kDyLd = 32;
-enum { kDhW = 0, kDhFeat = 1, kDhDy = 2, kDhAct0 = 3, kDhD0 = 8, kDhCount = 14 };
-constexpr int kObsLdH = 192;   // 162 observation words padded to three whole 128-byte lines of fp16 (see model_ac.cu)
-enum { kHsObs = 0, kHsWih = 1, kHsDg = 2, kHsHp = 3 };
+enum { kLstmHsObs = 0, kLstmHsWih = 1, kLstmHsDg = 2, kLstmHsHp = 3 };   // FarmerWs::hs slots
 
 // Branch-free gate functions for the recurrent kernels. The library expf / tanhf / IEEE division carry range checks and
 // (tanhf) a data-dependent branch that a warp of 32 different pre-activations takes both ways; the element-wise part of a
@@ -485,27 +463,19 @@ __global__ void regression_loss_kernel(const float* __restrict__ y, const float*
 // ------------------------------------------------------------------------------------------
 static void ws_release(FarmerWs* w) {
     if (!w) return;
-    float* f[] = {w->gates, w->hprev, w->cst, w->whh_t, w->feat, w->y, w->dy, w->target, w->act[0], w->act[1], w->act[2],
-                  w->act[3], w->act[4], w->d_a, w->d_b};
+    float* f[] = {w->gates, w->hprev, w->cst, w->whh_t, w->feat, w->y, w->dy, w->target, w->dfeat};
     for (float* p : f)
         if (p) cudaFree(p);
     if (w->gemm_ws) cudaFree(w->gemm_ws);
     if (w->colsum_ws) cudaFree(w->colsum_ws);
-    void* h[] = {w->hs, w->obs_hi, w->obs_lo, w->wih_hi, w->wih_lo, w->dg_hi, w->dg_lo, w->hp_hi, w->hp_lo, w->split_ws, w->bias_part,
-                 w->dhs, w->w_hi, w->w_lo, w->w1_hi, w->w1_lo, w->feat_hi, w->feat_lo, w->dd_hi[0], w->dd_hi[1], w->dd_lo[0], w->dd_lo[1],
-                 w->dy_hi, w->dy_lo, w->dfeat};
+    void* h[] = {w->hs, w->obs_hi, w->obs_lo, w->wih_hi, w->wih_lo, w->dg_hi, w->dg_lo, w->hp_hi, w->hp_lo, w->split_ws, w->bias_part};
     for (void* p : h)
         if (p) cudaFree(p);
-    for (int i = 0; i < 6; i++) {
-        void* q[] = {i < 5 ? w->act_hi[i] : nullptr, i < 5 ? w->act_lo[i] : nullptr, i < 5 ? (void*)w->relu_bits[i] : nullptr,
-                     i < 5 ? (void*)w->colsum_part[i] : nullptr, w->colsum_scratch[i], w->slab_ws[i]};
-        for (void* p : q)
-            if (p) cudaFree(p);
-    }
     delete w;
 }
 
-static int ws_create(fi_learner* l, size_t rows, size_t t, bool training, FarmerWs** out) {
+// The workspaces of a step (training) or of batched inference, and the dense stack `ds` they run with.
+static int ws_create(fi_learner* l, size_t rows, size_t t, bool training, FarmerWs** out, DenseStack* ds) {
     FarmerWs* w = new FarmerWs();
     *out = w;
     w->rows = rows;
@@ -519,7 +489,6 @@ static int ws_create(fi_learner* l, size_t rows, size_t t, bool training, Farmer
     FI_CUDA_OK(cudaMalloc((void**)&w->whh_t, (size_t)kG4 * kLstmH * sizeof(float)));
     FI_CUDA_OK(cudaMalloc((void**)&w->feat, rows * kFeat * sizeof(float)));
     FI_CUDA_OK(cudaMalloc((void**)&w->y, rows * sizeof(float)));
-    for (int i = 0; i < 5; i++) FI_CUDA_OK(cudaMalloc((void**)&w->act[i], rows * kHid * sizeof(float)));
     if (training) {
         FI_CUDA_OK(cudaMalloc((void**)&w->hprev, rt * kLstmH * sizeof(float)));
         FI_CUDA_OK(cudaMalloc((void**)&w->cst, rt_pad * kLstmH * sizeof(float)));
@@ -527,8 +496,6 @@ static int ws_create(fi_learner* l, size_t rows, size_t t, bool training, Farmer
         FI_CUDA_OK(cudaMalloc((void**)&w->dy, rows * sizeof(float)));
         FI_CUDA_OK(cudaMalloc((void**)&w->bias_part, ((rows + kLstmRows - 1) / kLstmRows) * kG4 * sizeof(float)));   // one row per CTA of the BPTT kernel
         FI_CUDA_OK(cudaMalloc((void**)&w->target, rows * sizeof(float)));
-        FI_CUDA_OK(cudaMalloc((void**)&w->d_a, rows * kFeat * sizeof(float)));
-        FI_CUDA_OK(cudaMalloc((void**)&w->d_b, rows * kFeat * sizeof(float)));
         const int mode = l->cfg.gemm_mode;
         size_t ws = 0;
         auto upd = [&](size_t b) { if (b > ws) ws = b; };
@@ -566,51 +533,24 @@ static int ws_create(fi_learner* l, size_t rows, size_t t, bool training, Farmer
             if (sw2 > sw) sw = sw2;
             w->split_ws_bytes = sw;
             if (sw) FI_CUDA_OK(cudaMalloc(&w->split_ws, sw));
-            // dense stack
-            const size_t ab = ((l->arena_elems + 7) & ~(size_t)7) * 2, rb = rows * kHid * 2;
-            FI_CUDA_OK(cudaMalloc((void**)&w->dhs, kDhCount * sizeof(HScale)));
-            FI_CUDA_OK(cudaMalloc(&w->w_hi, ab));
-            FI_CUDA_OK(cudaMalloc(&w->w_lo, ab));
-            FI_CUDA_OK(cudaMalloc(&w->w1_hi, (size_t)kHid * kFeatLdH * 2));
-            FI_CUDA_OK(cudaMalloc(&w->w1_lo, (size_t)kHid * kFeatLdH * 2));
-            FI_CUDA_OK(cudaMalloc(&w->feat_hi, rows * kFeatLdH * 2));
-            FI_CUDA_OK(cudaMalloc(&w->feat_lo, rows * kFeatLdH * 2));
-            FI_CUDA_OK(cudaMalloc(&w->dy_hi, rows * kDyLd * 2));
-            FI_CUDA_OK(cudaMalloc(&w->dy_lo, rows * kDyLd * 2));
             FI_CUDA_OK(cudaMalloc((void**)&w->dfeat, rows * kLstmH * sizeof(float)));
-            const int part_rows = 4 * (int)((rows + 127) / 128);
-            for (int i = 0; i < 5; i++) {
-                FI_CUDA_OK(cudaMalloc(&w->act_hi[i], rb));
-                FI_CUDA_OK(cudaMalloc(&w->act_lo[i], rb));
-                FI_CUDA_OK(cudaMalloc((void**)&w->relu_bits[i], rows * (kHid / 32) * sizeof(uint32_t)));
-                FI_CUDA_OK(cudaMalloc((void**)&w->colsum_part[i], (size_t)part_rows * kHid * sizeof(float)));
-                FI_CUDA_OK(cudaMalloc((void**)&w->colsum_scratch[i], grad_colsum_scratch_bytes(part_rows, kHid)));
-                w->slab_bytes[i] = gemm_tc_split_workspace_bytes(2, kHid, i == 0 ? kFeat : kHid, (int)rows);
-            }
-            for (int i = 0; i < 2; i++) {
-                FI_CUDA_OK(cudaMalloc(&w->dd_hi[i], rb));
-                FI_CUDA_OK(cudaMalloc(&w->dd_lo[i], rb));
-            }
-            FI_CUDA_OK(cudaMalloc((void**)&w->colsum_scratch[5], grad_colsum_scratch_bytes((int)rows, 1)));
-            w->slab_bytes[5] = gemm_tc_split_workspace_bytes(2, kHid, 1, (int)rows);
-            for (int i = 0; i < 6; i++)
-                if (w->slab_bytes[i]) FI_CUDA_OK(cudaMalloc(&w->slab_ws[i], w->slab_bytes[i]));
         }
     }
-    return FI_OK;
+    // split-operand buffers wherever the 3xFP16 path is available; farmer_dense_tc picks the path per step
+    return dense_alloc(ds, DenseShape{kFeat, kFeatLdH, 1, 4}, rows, l->arena_elems, w->half ? kDenseTrain : kDenseNone, true,
+                       training ? kDenseTrain : kDenseForward);
 }
 
 int farmer_alloc(fi_learner* l, Player* p) {
     FarmerWs* w = nullptr;
-    const int rc = ws_create(l, l->cfg.batch_size, l->cfg.entry_size, true, &w);
-    p->model_ws = nullptr;
+    const int rc = ws_create(l, l->cfg.batch_size, l->cfg.entry_size, true, &w, &p->dense);
     p->farmer_ws = w;
     return rc;
 }
 
 void farmer_free(Player* p) {
-    ws_release(static_cast<FarmerWs*>(p->farmer_ws));
-    ws_release(static_cast<FarmerWs*>(p->farmer_inf_ws));
+    ws_release(p->farmer_ws);
+    ws_release(p->farmer_inf_ws);
     p->farmer_ws = p->farmer_inf_ws = nullptr;
 }
 
@@ -622,12 +562,12 @@ static bool farmer_use_half(const fi_learner* l, const FarmerWs* w, int rt) {
 
 // The dense stack runs on the tensor cores (3xFP16, fused epilogues) when that format is required, and under AUTO from 128
 // batch rows up (below that the fp32 FFMA kernels win: every product is launch-latency bound).
-static bool farmer_dense_tc(const fi_learner* l, const FarmerWs* w, int m) {
-    return w->half && w->dhs && (l->cfg.gemm_mode == FI_GEMM_TCGEN05_F16 || m >= 128);
+static bool farmer_dense_tc(const fi_learner* l, const DenseStack* ds, int m) {
+    return ds->split && (l->cfg.gemm_mode == FI_GEMM_TCGEN05_F16 || m >= 128);
 }
 
-// z rows: (b,t) at z + (b*t + s) * ldz. Leaves y[m], feat, act (and the BPTT state when training).
-static int farmer_forward(fi_learner* l, FarmerWs* w, const float* params, const float* z, int ldz, int m, int t,
+// z rows: (b,t) at z + (b*t + s) * ldz. Leaves y[m], feat, the dense stack's activations (and the BPTT state when training).
+static int farmer_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const float* params, const float* z, int ldz, int m, int t,
                           cudaStream_t st) {
     const auto& T = l->tensors;
     // inference workspaces carry no GEMM workspace: actor batches are small and run on the fp32 FFMA kernels
@@ -640,21 +580,17 @@ static int farmer_forward(fi_learner* l, FarmerWs* w, const float* params, const
         transpose_whh_kernel<<<(kG4 * kLstmH + 255) / 256, 256, 0, st>>>(params + T[1].offset, w->whh_t);
         FI_TRY(ls.done());
     }
-    const bool half_proj = farmer_use_half(l, w, rt), dense_tc = farmer_dense_tc(l, w, m);
-    if (half_proj || dense_tc) FI_TRY(launch_zero2(w->hs, 4 * sizeof(HScale), w->dhs, w->dhs ? kDhCount * sizeof(HScale) : 0, st));
-    if (dense_tc) {
-        // parameters: max |p|, the split of the whole arena and dense1.w's copy with padded rows, one launch
-        const int arena_ld = (int)((l->arena_elems + 7) & ~(size_t)7);
-        FI_TRY(launch_amax_split_params(params, (int)l->arena_elems, arena_ld, w->w_hi, w->w_lo, params + T[4].offset, kHid, kFeat, kFeatLdH,
-                                        w->w1_hi, w->w1_lo, w->dhs + kDhW, st));
-    }
+    const bool half_proj = farmer_use_half(l, w, rt), dense_tc = farmer_dense_tc(l, ds, m);
+    if (half_proj || dense_tc) FI_TRY(launch_zero2(w->hs, 4 * sizeof(HScale), ds->hs, ds->hs ? kHsCount * sizeof(HScale) : 0, st));
+    // parameters: max |p|, the split of the whole arena and dense1.w's copy with padded rows, one launch
+    if (dense_tc) FI_TRY(dense_split_params(l, ds, params, st));
     // gates = z W_ih^T + b_ih for all B*T rows at once
     if (half_proj) {
-        FI_TRY(launch_amax_split_h(z, ldz, (size_t)rt, kZDim, kObsLdH, w->obs_hi, w->obs_lo, w->hs + kHsObs, st));
-        HScale* wih_hs = dense_tc ? w->dhs + kDhW : w->hs + kHsWih;   // the arena's scale bounds W_ih as well
+        FI_TRY(launch_amax_split_h(z, ldz, (size_t)rt, kZDim, kObsLdH, w->obs_hi, w->obs_lo, w->hs + kLstmHsObs, st));
+        HScale* wih_hs = dense_tc ? ds->hs + kHsW : w->hs + kLstmHsWih;   // the arena's scale bounds W_ih as well
         if (!dense_tc) FI_TRY(launch_amax(params + T[0].offset, kZDim, kG4, kZDim, wih_hs, st));
         FI_TRY(launch_split_h(params + T[0].offset, kZDim, kG4, kZDim, kObsLdH, w->wih_hi, w->wih_lo, wih_hs, dense_tc ? 0 : 1, st));
-        const SplitMat a{w->obs_hi, w->obs_lo, kObsLdH, w->hs + kHsObs}, b{w->wih_hi, w->wih_lo, kObsLdH, wih_hs};
+        const SplitMat a{w->obs_hi, w->obs_lo, kObsLdH, w->hs + kLstmHsObs}, b{w->wih_hi, w->wih_lo, kObsLdH, wih_hs};
         TcOut out{w->gates, kG4, nullptr, nullptr, 0, 0, nullptr, nullptr, 0, nullptr};
         if (lstm_tc) {   // straight into the blocked layout the recurrent kernels move with one bulk copy per CTA and step
             out.step_t = t;
@@ -667,7 +603,7 @@ static int farmer_forward(fi_learner* l, FarmerWs* w, const float* params, const
     }
     if (lstm_tc) {
         // h_{s-1} leaves the kernel as the fp16 pairs the W_hh gradient product reads (scale 2^13: |h| <= 1)
-        FI_TRY(launch_lstm_forward_tc(w->gates, params + T[1].offset, params + T[3].offset, m, t, w->hp_hi, w->hp_lo, w->hs + kHsHp, w->cst,
+        FI_TRY(launch_lstm_forward_tc(w->gates, params + T[1].offset, params + T[3].offset, m, t, w->hp_hi, w->hp_lo, w->hs + kLstmHsHp, w->cst,
                                       w->feat, kFeat, st));
     } else {
         // recurrent flops: 2 * 128 * 512 per (row, step)
@@ -679,47 +615,23 @@ static int farmer_forward(fi_learner* l, FarmerWs* w, const float* params, const
         launch_pdl(lstm_forward_kernel, dim3((m + kLstmRows - 1) / kLstmRows), dim3(kLstmThreads), kLstmFwdSmem, st, w->gates, w->whh_t,
                    params + T[3].offset, m, t, hp_pairs ? nullptr : w->hprev, w->cst, w->feat,
                    hp_pairs ? static_cast<__half*>(w->hp_hi) : nullptr, hp_pairs ? static_cast<__half*>(w->hp_lo) : nullptr,
-                   hp_pairs ? w->hs + kHsHp : nullptr, lstm_trace_buffer());
+                   hp_pairs ? w->hs + kLstmHsHp : nullptr, lstm_trace_buffer());
         FI_TRY(ls.done());
         lstm_trace_report("forward (FFMA)", lstm_trace_buffer(), t, st);
     }
     if (dense_tc) {
-        // x_l = relu(x_{l-1} W_l^T + b_l), written as fp16 pairs (and ReLU bit masks) by the GEMM epilogue; y = x_5 w_6 + b_6
-        HScale* dhs = w->dhs;
-        FI_TRY(launch_amax_split_h(w->feat, kFeat, (size_t)m, kFeat, kFeatLdH, w->feat_hi, w->feat_lo, dhs + kDhFeat, st));
-        auto W = [&](int tensor, int ld) {
-            return SplitMat{static_cast<char*>(w->w_hi) + T[tensor].offset * 2, static_cast<char*>(w->w_lo) + T[tensor].offset * 2, ld, dhs + kDhW};
-        };
-        for (int layer = 0; layer < 5; layer++) {
-            const SplitMat x = layer == 0 ? SplitMat{w->feat_hi, w->feat_lo, kFeatLdH, dhs + kDhFeat}
-                                          : SplitMat{w->act_hi[layer - 1], w->act_lo[layer - 1], kHid, dhs + kDhAct0 + layer - 1};
-            const SplitMat wm = layer == 0 ? SplitMat{w->w1_hi, w->w1_lo, kFeatLdH, dhs + kDhW} : W(4 + 2 * layer, kHid);
-            const TcOut out{nullptr, 0, w->act_hi[layer], w->act_lo[layer], kHid, 0, nullptr, w->relu_bits[layer], kHid / 32, nullptr,
-                            dhs + kDhAct0 + layer, dhs + kDhW};
-            FI_TRY(launch_gemm_tc_split(0, m, kHid, layer == 0 ? kFeat : kHid, x, wm, out, params + T[5 + 2 * layer].offset, 1, nullptr, 0,
-                                        nullptr, 0, st));
-        }
-        return launch_gemm_tc_split(0, m, 1, kHid, SplitMat{w->act_hi[4], w->act_lo[4], kHid, dhs + kDhAct0 + 4}, W(14, kHid),
-                                    TcOut{w->y, 1, nullptr, nullptr, 0, 0, nullptr, nullptr, 0, nullptr}, params + T[15].offset, 0, nullptr, 0,
-                                    nullptr, 0, st);
+        FI_TRY(launch_amax_split_h(w->feat, kFeat, (size_t)m, kFeat, kFeatLdH, ds->in_hi, ds->in_lo, ds->hs + kHsIn, st));
+        return dense_forward_split(l, ds, params, m, w->y, st);
     }
-    const float* x = w->feat;
-    int k = kFeat;
-    for (int layer = 0; layer < 5; layer++) {
-        FI_TRY(launch_gemm(mode, 0, m, kHid, k, x, k, params + T[4 + 2 * layer].offset, k, w->act[layer], kHid,
-                           params + T[5 + 2 * layer].offset, 1, nullptr, 0, w->gemm_ws, w->gemm_ws_bytes, st));
-        x = w->act[layer];
-        k = kHid;
-    }
-    return launch_gemm(mode, 0, m, 1, kHid, x, kHid, params + T[14].offset, kHid, w->y, 1, params + T[15].offset, 0,
-                       nullptr, 0, w->gemm_ws, w->gemm_ws_bytes, st);
+    return dense_forward_plain(l, ds, mode, params, w->feat, kFeat, m, w->y, w->gemm_ws, w->gemm_ws_bytes, st);
 }
 
 int farmer_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int t, int global_m) {
-    FarmerWs* w = static_cast<FarmerWs*>(p->farmer_ws);
+    FarmerWs* w = p->farmer_ws;
     if (!w) return set_error(FI_ERR_STATE, "farmer workspaces missing");
     const auto& T = l->tensors;
     const int mode = l->cfg.gemm_mode;
+    DenseStack* ds = &p->dense;
     cudaStream_t st = p->stream;
     float* g = p->grads;
     {
@@ -727,99 +639,34 @@ int farmer_forward_backward(fi_learner* l, Player* p, const float* batch, int m,
         launch_pdl(farmer_assemble_kernel, dim3(m), dim3(128), 0, st, batch, m, t, w->feat, w->target);
         FI_TRY(ls.done());
     }
-    FI_TRY(farmer_forward(l, w, p->params, batch, kRecWords, m, t, st));
+    FI_TRY(farmer_forward(l, w, ds, p->params, batch, kRecWords, m, t, st));
     FI_TRY(launch_zero2(p->d_losses, 4 * sizeof(double), nullptr, 0, st));
+    const bool dense_tc = farmer_dense_tc(l, ds, m);
     {
         LaunchScope ls("regression_loss_kernel", st, 12.0 * m, kWorkBytes);
         launch_pdl(regression_loss_kernel, dim3((m + 255) / 256), dim3(256), 0, st, w->y, w->target, m, l->cfg.loss, 1.0 / (double)global_m,
-                   w->dy, p->d_losses, farmer_dense_tc(l, w, m) ? w->dhs + kDhDy : nullptr);
+                   w->dy, p->d_losses, dense_tc ? ds->hs + kHsDout : nullptr);
         FI_TRY(ls.done());
     }
-    float* d = w->d_a;
-    int ldd = kHid;
-    const bool dense_tc = farmer_dense_tc(l, w, m);
-    w->last_dense_tc = dense_tc;
+    const float* d;   // dL/dfeat [m, ldd]
+    int ldd;
     if (dense_tc) {
-        // As model_ac.cu's backward: every dgrad epilogue applies the ReLU bit mask, writes the next gradient as fp16 pairs and
-        // leaves per-32-row column sums (the bias gradient); wgrad split-K slabs and those sums are reduced by two launches.
-        HScale* dhs = w->dhs;
-        auto W = [&](int tensor, int ld) {
-            return SplitMat{static_cast<char*>(w->w_hi) + T[tensor].offset * 2, static_cast<char*>(w->w_lo) + T[tensor].offset * 2, ld, dhs + kDhW};
-        };
-        auto ACT = [&](int layer) { return SplitMat{w->act_hi[layer], w->act_lo[layer], kHid, dhs + kDhAct0 + layer}; };
-        FI_TRY(launch_split_h(w->dy, 1, (size_t)m, 1, kDyLd, w->dy_hi, w->dy_lo, dhs + kDhDy, 1, st));   // max |dy| came with the loss
-        const SplitMat dy{w->dy_hi, w->dy_lo, kDyLd, dhs + kDhDy};
-        GradSegTable segs;
-        int splits = 1;
-        const int part_rows = 4 * ((m + 127) / 128);
-        FI_TRY(grad_table_add_colsum(&segs, w->dy, 1, m, 1, g + T[15].offset, w->colsum_scratch[5]));
-        {
-            TcOut o{g + T[14].offset, kHid, nullptr, nullptr, 0, 1, nullptr, nullptr, 0, nullptr};
-            o.deferred_splits = &splits;
-            FI_TRY(launch_gemm_tc_split(2, kHid, 1, m, ACT(4), dy, o, nullptr, 0, nullptr, 0, w->slab_ws[5], w->slab_bytes[5], st));
-            if (splits > 1) FI_TRY(grad_table_add_slabs(&segs, (const float*)w->slab_ws[5], splits, (size_t)kHid, kHid, g + T[14].offset));
-        }
-        int cur = 0, dslot = kDhD0;
-        FI_TRY(launch_gemm_tc_split(1, m, kHid, 1, dy, W(14, kHid),
-                                    TcOut{nullptr, 0, w->dd_hi[cur], w->dd_lo[cur], kHid, 0, w->relu_bits[4], nullptr, kHid / 32,
-                                          w->colsum_part[4], dhs + dslot, nullptr},
-                                    nullptr, 0, nullptr, 0, nullptr, 0, st));
-        for (int layer = 4; layer >= 0; layer--) {
-            const SplitMat dl{w->dd_hi[cur], w->dd_lo[cur], kHid, dhs + dslot};
-            const SplitMat x = layer == 0 ? SplitMat{w->feat_hi, w->feat_lo, kFeatLdH, dhs + kDhFeat} : ACT(layer - 1);
-            const int k = layer == 0 ? kFeat : kHid;
-            FI_TRY(grad_table_add_colsum(&segs, w->colsum_part[layer], kHid, part_rows, kHid, g + T[5 + 2 * layer].offset, w->colsum_scratch[layer]));
-            {
-                TcOut o{g + T[4 + 2 * layer].offset, k, nullptr, nullptr, 0, 0, nullptr, nullptr, 0, nullptr};
-                o.deferred_splits = &splits;
-                FI_TRY(launch_gemm_tc_split(2, kHid, k, m, dl, x, o, nullptr, 0, nullptr, 0, w->slab_ws[layer], w->slab_bytes[layer], st));
-                if (splits > 1)
-                    FI_TRY(grad_table_add_slabs(&segs, (const float*)w->slab_ws[layer], splits, (size_t)kHid * k, kHid * k, g + T[4 + 2 * layer].offset));
-            }
-            if (layer > 0) {
-                FI_TRY(launch_gemm_tc_split(1, m, kHid, kHid, dl, W(4 + 2 * layer, kHid),
-                                            TcOut{nullptr, 0, w->dd_hi[cur ^ 1], w->dd_lo[cur ^ 1], kHid, 0, w->relu_bits[layer - 1], nullptr,
-                                                  kHid / 32, w->colsum_part[layer - 1], dhs + dslot + 1, nullptr},
-                                            nullptr, 0, nullptr, 0, nullptr, 0, st));
-                cur ^= 1;
-                dslot++;
-            } else {
-                // dL/dh_{T-1} = the first 128 columns of d0 W_1 (the x part of the feature row takes no gradient)
-                FI_TRY(launch_gemm_tc_split(1, m, kLstmH, kHid, dl, SplitMat{w->w1_hi, w->w1_lo, kFeatLdH, dhs + kDhW},
-                                            TcOut{w->dfeat, kLstmH, nullptr, nullptr, 0, 0, nullptr, nullptr, 0, nullptr}, nullptr, 0, nullptr,
-                                            0, nullptr, 0, st));
-            }
-        }
-        FI_TRY(launch_grad_finalize(&segs, st));
+        FI_TRY(launch_split_h(w->dy, 1, (size_t)m, 1, kDoutLd, ds->dout_hi, ds->dout_lo, ds->hs + kHsDout, 1, st));   // max |dy| came with the loss
+        // dL/dh_{T-1} = the first 128 columns of dL/dfeat (the x part of the feature row takes no gradient)
+        FI_TRY(dense_backward_split(l, ds, w->dy, m, g, w->dfeat, kLstmH, nullptr, 0, st));
         d = w->dfeat;
         ldd = kLstmH;
     } else {
-    // dense6: dW = dy^T act4, db = sum dy, d4 = (dy W6) * relu'(act4)
-    FI_TRY(launch_colsum(w->dy, 1, m, 1, g + T[15].offset, w->colsum_ws, w->colsum_ws_bytes, st));
-    FI_TRY(launch_gemm(mode, 2, 1, kHid, m, w->dy, 1, w->act[4], kHid, g + T[14].offset, kHid, nullptr, 0, nullptr, 0,
-                       w->gemm_ws, w->gemm_ws_bytes, st));
-    float* d_next = w->d_b;
-    FI_TRY(launch_gemm(mode, 1, m, kHid, 1, w->dy, 1, p->params + T[14].offset, kHid, d, kHid, nullptr, 0, w->act[4], kHid,
-                       w->gemm_ws, w->gemm_ws_bytes, st));
-    for (int layer = 4; layer >= 0; layer--) {
-        const float* in = layer == 0 ? w->feat : w->act[layer - 1];
-        const int k = layer == 0 ? kFeat : kHid;
-        FI_TRY(launch_colsum(d, ldd, m, kHid, g + T[5 + 2 * layer].offset, w->colsum_ws, w->colsum_ws_bytes, st));
-        FI_TRY(launch_gemm(mode, 2, kHid, k, m, d, ldd, in, k, g + T[4 + 2 * layer].offset, k, nullptr, 0, nullptr, 0,
-                           w->gemm_ws, w->gemm_ws_bytes, st));
-        // dgrad: into [m, k]; the ReLU mask of the producing layer, none for the feature row
-        FI_TRY(launch_gemm(mode, 1, m, k, kHid, d, ldd, p->params + T[4 + 2 * layer].offset, k, d_next, k, nullptr, 0,
-                           layer == 0 ? nullptr : w->act[layer - 1], kHid, w->gemm_ws, w->gemm_ws_bytes, st));
-        float* tmp = d; d = d_next; d_next = tmp;
-        ldd = k;
+        FI_TRY(dense_backward_plain(l, ds, mode, p->params, w->feat, kFeat, w->dy, m, g, &d, w->gemm_ws, w->gemm_ws_bytes, w->colsum_ws,
+                                    w->colsum_ws_bytes, st));
+        ldd = kFeat;
     }
-    }   // !dense_tc
     // d = dfeat [m, ldd]: its first 128 columns are dL/dh_{T-1}; BPTT turns the stored gates into pre-activation gate gradients
     const int rt = m * t;
     const bool lstm_tc = farmer_use_half(l, w, rt) && lstm_tc_enabled();
     if (lstm_tc) {
         // also leaves db_ih = db_hh (the column sums of dG) and max |dG|
-        FI_TRY(launch_lstm_backward_tc(w->gates, p->params + T[1].offset, w->cst, d, ldd, m, t, w->hs + kHsDg, w->bias_part,
+        FI_TRY(launch_lstm_backward_tc(w->gates, p->params + T[1].offset, w->cst, d, ldd, m, t, w->hs + kLstmHsDg, w->bias_part,
                                        g + T[2].offset, g + T[3].offset, st));
     } else {
         LaunchScope ls("lstm_backward_kernel", st, 2.0 * kLstmH * kG4 * (double)m * t, kWorkFlops);
@@ -827,7 +674,7 @@ int farmer_forward_backward(fi_learner* l, Player* p, const float* batch, int m,
         FI_TRY(ensure_dynamic_smem(bwd_attr, (const void*)lstm_backward_kernel, (int)kLstmBwdSmem));
         const int ctas = (m + kLstmRows - 1) / kLstmRows;
         launch_pdl(lstm_backward_kernel, dim3(ctas), dim3(kLstmThreads), kLstmBwdSmem, st, w->gates, p->params + T[1].offset, w->cst, d, ldd, m,
-                   t, farmer_use_half(l, w, rt) ? w->hs + kHsDg : nullptr, w->bias_part, lstm_trace_buffer());
+                   t, farmer_use_half(l, w, rt) ? w->hs + kLstmHsDg : nullptr, w->bias_part, lstm_trace_buffer());
         FI_TRY(ls.done());
         lstm_trace_report("backward (FFMA)", lstm_trace_buffer(), t, st);
         // db_ih = db_hh = the CTAs' column sums of dG, added in CTA order
@@ -837,10 +684,10 @@ int farmer_forward_backward(fi_learner* l, Player* p, const float* batch, int m,
         // dW_ih = dgates^T z, dW_hh = dgates^T h_prev: the gate gradients are split once and read MN-major by both. The
         // tensor-core recurrence has already left max |dG| and h_prev as fp16 pairs.
         // (both recurrent kernels have left max |dG| and h_prev as fp16 pairs)
-        if (lstm_tc) FI_TRY(launch_lstm_split_gates(w->gates, m, t, w->dg_hi, w->dg_lo, w->hs + kHsDg, st));
-        else FI_TRY(launch_split_h(w->gates, kG4, (size_t)rt, kG4, kG4, w->dg_hi, w->dg_lo, w->hs + kHsDg, 1, st));
-        const SplitMat dg{w->dg_hi, w->dg_lo, kG4, w->hs + kHsDg};
-        const SplitMat obs{w->obs_hi, w->obs_lo, kObsLdH, w->hs + kHsObs}, hp{w->hp_hi, w->hp_lo, kLstmH, w->hs + kHsHp};
+        if (lstm_tc) FI_TRY(launch_lstm_split_gates(w->gates, m, t, w->dg_hi, w->dg_lo, w->hs + kLstmHsDg, st));
+        else FI_TRY(launch_split_h(w->gates, kG4, (size_t)rt, kG4, kG4, w->dg_hi, w->dg_lo, w->hs + kLstmHsDg, 1, st));
+        const SplitMat dg{w->dg_hi, w->dg_lo, kG4, w->hs + kLstmHsDg};
+        const SplitMat obs{w->obs_hi, w->obs_lo, kObsLdH, w->hs + kLstmHsObs}, hp{w->hp_hi, w->hp_lo, kLstmH, w->hs + kLstmHsHp};
         FI_TRY(launch_gemm_tc_split(2, kG4, kZDim, rt, dg, obs, TcOut{g + T[0].offset, kZDim, nullptr, nullptr, 0, 0, nullptr, nullptr, 0, nullptr},
                                     nullptr, 0, nullptr, 0, w->split_ws, w->split_ws_bytes, st));
         FI_TRY(launch_gemm_tc_split(2, kG4, kLstmH, rt, dg, hp, TcOut{g + T[1].offset, kLstmH, nullptr, nullptr, 0, 0, nullptr, nullptr, 0, nullptr},
@@ -854,40 +701,25 @@ int farmer_forward_backward(fi_learner* l, Player* p, const float* batch, int m,
     return FI_OK;
 }
 
-// Bit-packed ReLU decisions of hidden layer `layer` ([rows, 16] words) when the last step ran the dense stack on the tensor
-// cores (they are what its backward pass used), else null: the fp32 activations of farmer_activation hold them.
-const uint32_t* farmer_relu_bits(Player* p, int layer) {
-    const FarmerWs* w = static_cast<const FarmerWs*>(p->farmer_ws);
-    return (w && w->last_dense_tc && layer >= 0 && layer < 5) ? w->relu_bits[layer] : nullptr;
-}
-
-int farmer_activation(Player* p, int layer, const float** a, const float** lo) {
-    FarmerWs* w = static_cast<FarmerWs*>(p->farmer_ws);
-    if (!w || layer < 0 || layer >= 5) return set_error(FI_ERR_ARG, "no such hidden layer %d", layer);
-    if (w->last_dense_tc) return set_error(FI_ERR_STATE, "the dense stack ran on fp16 pairs: no fp32 activations to read back");
-    *a = w->act[layer];
-    *lo = nullptr;
-    return FI_OK;
-}
-
 int farmer_infer_alloc(fi_learner* l, Player* p, size_t rows, size_t t) {
-    ws_release(static_cast<FarmerWs*>(p->farmer_inf_ws));
+    ws_release(p->farmer_inf_ws);
+    dense_free(&p->inf_dense);
     FarmerWs* w = nullptr;
-    const int rc = ws_create(l, rows, t, false, &w);
+    const int rc = ws_create(l, rows, t, false, &w, &p->inf_dense);
     p->farmer_inf_ws = w;
     return rc;
 }
 
 int farmer_infer(fi_learner* l, Player* p, const float* params, const float* z_dev, const float* x_dev, size_t rows,
                  size_t t, float* out_dev, cudaStream_t stream) {
-    FarmerWs* w = static_cast<FarmerWs*>(p->farmer_inf_ws);
+    FarmerWs* w = p->farmer_inf_ws;
     if (!w || rows > w->rows || t > w->t) return set_error(FI_ERR_STATE, "farmer inference workspaces too small");
     {
         LaunchScope ls("farmer_assemble_dense_kernel", stream, 2.0 * 4 * kXDim * (double)rows, kWorkBytes);
         farmer_assemble_dense_kernel<<<(unsigned)rows, 128, 0, stream>>>(x_dev, (int)rows, w->feat);
         FI_TRY(ls.done());
     }
-    FI_TRY(farmer_forward(l, w, params, z_dev, kZDim, (int)rows, (int)t, stream));
+    FI_TRY(farmer_forward(l, w, &p->inf_dense, params, z_dev, kZDim, (int)rows, (int)t, stream));
     FI_CUDA_OK(cudaMemcpyAsync(out_dev, w->y, rows * sizeof(float), cudaMemcpyDeviceToDevice, stream));
     return FI_OK;
 }
