@@ -375,6 +375,21 @@ fi_learner* fi_learner_create(const fi_learner_config* cfg) {
                               "(got %g, %g, %g)", cfg->rmsprop_alpha, cfg->rmsprop_eps, cfg->rmsprop_momentum);
         return nullptr;
     }
+    if (!farmer) {   // V-trace constants: a NaN or out-of-range value would otherwise surface as NaN or meaningless losses
+        const struct { const char* name; float v; bool ok; const char* range; } vt[] = {
+            {"rho_bar", cfg->rho_bar, cfg->rho_bar > 0.f, "> 0 (+inf = no clipping)"},
+            {"c_bar", cfg->c_bar, cfg->c_bar > 0.f, "> 0 (+inf = no clipping)"},
+            {"pg_rho_bar", cfg->pg_rho_bar, cfg->pg_rho_bar > 0.f, "> 0 (+inf = no clipping)"},
+            {"lambda_", cfg->lambda_, cfg->lambda_ >= 0.f && cfg->lambda_ <= 1.f, "in [0, 1]"},
+            {"baseline_cost", cfg->baseline_cost, cfg->baseline_cost >= 0.f && std::isfinite(cfg->baseline_cost), "finite and >= 0"},
+            {"entropy_cost", cfg->entropy_cost, cfg->entropy_cost >= 0.f && std::isfinite(cfg->entropy_cost), "finite and >= 0"},
+        };
+        for (const auto& f : vt)
+            if (!f.ok) {
+                set_error(FI_ERR_ARG, "fi_learner_create: V-trace %s must be %s, got %g", f.name, f.range, (double)f.v);
+                return nullptr;
+            }
+    }
     if (farmer && cfg->entry_size < fi::kFarmerMinEntry) {   // a shorter trajectory would train on a truncated x
         set_error(FI_ERR_ARG, "fi_learner_create: the FarmerLstm model needs entry_size >= %d (x[484] spans records 0..%d), got %zu",
                   fi::kFarmerMinEntry, fi::kFarmerMinEntry - 1, cfg->entry_size);

@@ -168,7 +168,9 @@ typedef struct fi_learner_config {
     int optimizer;            /* fi_opt_kind */
     double lr;                /* --learning-rate (main.cpp:157-159); README shape uses 5e-4 */
     uint64_t seed;            /* weight init seed (U(+-1/sqrt(fan_in)) like torch::nn defaults) */
-    /* V-trace constants (Espeholt et al. 2018); ignored unless loss == FI_LOSS_VTRACE */
+    /* V-trace constants (Espeholt et al. 2018); ignored unless loss == FI_LOSS_VTRACE. Accepted ranges (checked by
+       fi_learner_create for the actor-critic model): rho_bar, c_bar, pg_rho_bar > 0, +inf meaning no clipping;
+       0 <= lambda_ <= 1; baseline_cost, entropy_cost finite and >= 0. */
     float rho_bar, c_bar, pg_rho_bar, lambda_, baseline_cost, entropy_cost;
     int gemm_mode;            /* fi_gemm_mode */
     int publish_every;        /* D2H the weights into the model store every k steps (>=1) */
@@ -187,7 +189,8 @@ FI_API void fi_learner_config_default(fi_learner_config* cfg);
 /* Learner ctor (learner.h:100-140): creates p rings, p models (random init), optimiser
  * state and all step workspaces in HBM. Returns NULL on failure (see fi_last_error). An unknown
  * optimiser, max_grad_norm < 0 or not finite, rmsprop_alpha outside (0, 1), rmsprop_eps <= 0 or
- * rmsprop_momentum outside [0, 1) is rejected (FI_ERR_ARG) before any device is looked for. */
+ * rmsprop_momentum outside [0, 1), and, for the actor-critic model, a V-trace constant outside the range
+ * fi_learner_config states, is rejected (FI_ERR_ARG) before any device is looked for. */
 FI_API fi_learner* fi_learner_create(const fi_learner_config* cfg);
 FI_API void fi_learner_destroy(fi_learner* l);
 /* getSharedBuffers (learner.h:200-202): ring of one player, owned by the learner. */

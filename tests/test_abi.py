@@ -67,6 +67,34 @@ def test_farmer_learner_rejects_trajectories_too_short_for_x(fi, s):
         fi.Learner(1, 4, s, 2, model="farmer_lstm")
 
 
+NAN, INF = float("nan"), float("inf")
+VTRACE_REJECTED = ([(f, v) for f in ("rho_bar", "c_bar", "pg_rho_bar") for v in (NAN, 0.0, -0.5, -INF)] +
+                   [("lambda_", v) for v in (NAN, -0.01, 1.01, INF, -INF)] +
+                   [(f, v) for f in ("baseline_cost", "entropy_cost") for v in (NAN, -1e-3, INF, -INF)])
+
+
+@pytest.mark.parametrize("field,value", VTRACE_REJECTED, ids=[f"{f}={v}" for f, v in VTRACE_REJECTED])
+def test_actor_critic_learner_rejects_bad_vtrace_constants(fi, field, value):
+    """A NaN clipping threshold would otherwise give NaN losses, and lambda outside [0, 1] or a negative loss weight a step
+    that is not V-trace. Creation refuses with a message naming the field, before it looks for a device."""
+    with pytest.raises(fi.FiError, match=rf"V-trace {field} must be .*, got"):
+        fi.Learner(1, 4, 5, 2, model="mlp_actor_critic", **{field: value})
+
+
+def test_unclipped_vtrace_constants_are_accepted(fi):
+    """rho_bar = c_bar = pg_rho_bar = +inf means no clipping, with lambda and both costs at the ends of their ranges: creation
+    gets past the configuration checks (without a device it then stops at the device lookup)."""
+    import torch
+    kw = dict(rho_bar=INF, c_bar=INF, pg_rho_bar=INF, lambda_=0.0, baseline_cost=0.0, entropy_cost=0.0)
+    if torch.cuda.is_available():
+        fi.Learner(1, 4, 5, 2, model="mlp_actor_critic", **kw).close()
+        fi.Learner(1, 4, 5, 2, model="mlp_actor_critic", lambda_=1.0).close()
+        return
+    for k in (kw, dict(lambda_=1.0)):
+        with pytest.raises(fi.FiError, match="no CUDA device"):
+            fi.Learner(1, 4, 5, 2, model="mlp_actor_critic", **k)
+
+
 def test_defaults_follow_the_reference_cli(fi):
     from freeimpala_b200 import _lib
     cfg = _lib.FiLearnerConfig()

@@ -330,30 +330,74 @@ def test_vtrace_on_policy_reduces_to_nstep_returns(fi, torch_cuda):
 
 
 # ------------------------------------------------------------------------------- fused loss head
-@pytest.mark.parametrize("m,t", [(4, 7), (64, 100), (3, 65)])
-def test_vtrace_loss_head_vs_oracle(fi, oracle, torch_cuda, m, t):
+LH_BASE = dict(rho_bar=1.0, c_bar=1.0, pg_rho_bar=1.0, lambda_=0.97, baseline_cost=0.5, entropy_cost=0.01)
+# the V-trace constant sets of tests/test_gpu_ac_paths.py (distinct values, lambda = 0, c_bar > rho_bar, no clipping)
+LH_C1 = dict(rho_bar=2.0, c_bar=0.7, pg_rho_bar=1.5, lambda_=0.95, baseline_cost=0.25, entropy_cost=0.05)
+LH_SETS = {"c1-distinct": LH_C1, "c2-lambda0": dict(LH_BASE, lambda_=0.0, entropy_cost=0.0),
+           "c3-cbar-gt-rhobar": dict(LH_BASE, rho_bar=0.5, c_bar=3.0, pg_rho_bar=0.35, lambda_=1.0, baseline_cost=1.0),
+           "c4-unclipped": dict(LH_BASE, rho_bar=float("inf"), c_bar=float("inf"), pg_rho_bar=float("inf"), lambda_=1.0)}
+# (m, t, constants, ldh, behaviour-logit scale, learner-logit scale)
+LOSS_HEAD_CASES = (
+    [pytest.param(4, 7, LH_BASE, 17, 1, 1, id="4-7"), pytest.param(64, 100, LH_BASE, 17, 1, 1, id="64-100"),
+     pytest.param(3, 65, LH_BASE, 17, 1, 1, id="3-65")] +
+    # 32-step chunks: one partial / exact / exact + 1-step chunk, two exact, two + 1 step, a 4-step last chunk
+    [pytest.param(5, t, LH_C1, 17, 1, 1, id=f"chunks-t{t}") for t in (1, 31, 32, 33, 64, 65, 100)] +
+    [pytest.param(6, 65, c, 17, 1, 1, id=f"vtrace-{k}") for k, c in LH_SETS.items()] +
+    [pytest.param(5, 40, LH_C1, 20, 1, 1, id="padded-ldh20"),          # head rows of 20 floats, 3 of them padding
+     # |log rho| up to ~15: every threshold clips. (Not unclipped: the trace products c_s c_{s+1} ... then reach 1e70, far
+     # beyond fp32, and the targets themselves overflow.)
+     pytest.param(6, 65, LH_C1, 17, 4, 1, id="mu-x4"),
+     pytest.param(6, 65, LH_C1, 17, 1, 50, id="logits-x50")])          # fp32 softmax probabilities underflow to 0
+
+
+@pytest.mark.parametrize("m,t,cfg,ldh,mu_scale,logit_scale", LOSS_HEAD_CASES)
+def test_vtrace_loss_head_vs_oracle(fi, oracle, torch_cuda, m, t, cfg, ldh, mu_scale, logit_scale):
     from oracle import pyoracle as po
     torch = torch_cuda
     rng = np.random.default_rng(m + t)
     obs, mu, act, rew, disc, boot = U.vtrace_batch(5, m, t, done_p=0.05)
+    mu = mu * np.float32(mu_scale)
     batch = po.pack_vtrace_slots(obs, mu, act, rew, disc, boot)
-    head = rng.standard_normal((m * t, 17)).astype(np.float32)
-    cfg = dict(rho_bar=1.0, c_bar=1.0, pg_rho_bar=1.0, lambda_=0.97, baseline_cost=0.5, entropy_cost=0.01)
-    want = oracle.vtrace_losses(head[:, :16].reshape(m, t, 16), head[:, 16].reshape(m, t), mu, act, rew, disc, boot, **cfg)
+    head = np.full((m * t, ldh), np.nan, np.float32)     # padding columns are NaN: a kernel that reads them shows it
+    head[:, :17] = rng.standard_normal((m * t, 17)).astype(np.float32)
+    head[:, :16] *= np.float32(logit_scale)
+    want = oracle.vtrace_losses(head[:, :16].reshape(m, t, 16), head[:, 16].reshape(m, t), mu, act, rew, disc, boot,
+                                **{k: float(np.float32(v)) for k, v in cfg.items()})
     d_batch, d_head = _dev(torch, batch), _dev(torch, head)
-    dhead = torch.zeros((m * t, 17), device="cuda")
+    dhead = torch.full((m * t, ldh), 7.0, device="cuda")  # padding columns must keep this
     vs = torch.zeros(m * t, device="cuda")
     adv = torch.zeros(m * t, device="cuda")
     losses = torch.zeros(4, dtype=torch.float64, device="cuda")
-    fi.ops.vtrace_loss_head(d_batch.data_ptr(), m, t, d_head.data_ptr(), 17, dhead.data_ptr(), losses.data_ptr(),
+    fi.ops.vtrace_loss_head(d_batch.data_ptr(), m, t, d_head.data_ptr(), ldh, dhead.data_ptr(), losses.data_ptr(),
                             vs.data_ptr(), adv.data_ptr(), stream=torch.cuda.current_stream().cuda_stream, **cfg)
     torch.cuda.synchronize()
     got = dhead.cpu().numpy()
-    np.testing.assert_allclose(losses.cpu().numpy(), want["losses"], rtol=1e-5)
-    assert U.rel_max(vs.cpu().numpy(), want["vs"]) < 1e-5
-    assert U.rel_max(adv.cpu().numpy(), want["pg_adv"]) < 1e-5
-    assert U.rel_max(got[:, :16], want["dlogits"].reshape(-1, 16)) < 1e-5
-    assert U.rel_max(got[:, 16], want["dvalue"].reshape(-1)) < 1e-5
+    got_losses, got_vs, got_adv = losses.cpu().numpy(), vs.cpu().numpy(), adv.cpu().numpy()
+    for name, a in (("losses", got_losses), ("dhead", got[:, :17]), ("vs", got_vs), ("pg_adv", got_adv)):
+        assert np.all(np.isfinite(a)), name
+    assert np.all(got[:, 17:] == 7.0)
+    # Each loss is a sum over transitions. The baseline and entropy terms have one sign; the policy-gradient terms
+    # -log pi(a) * adv do not, and their sum (and the total's) can cancel: 515-fold for vtrace-c1-distinct (36.7-fold at most
+    # in the first three cases). fp32 terms cannot give that sum 1e-5 of itself, so a loss is held to 1e-5 relative but never
+    # to less than 1e-7 of the summed term magnitudes, which is looser only where a sum cancels more than 100-fold.
+    z = head[:, :16].astype(np.float64)
+    z = z - z.max(axis=1, keepdims=True)
+    logp = z - np.log(np.exp(z).sum(axis=1, keepdims=True))
+    pg_abs = np.abs(np.take_along_axis(logp, act.reshape(-1, 1), 1)[:, 0] * want["pg_adv"].reshape(-1)).sum()
+    bl_sum = 0.5 * ((want["vs"] - head[:, 16].reshape(m, t)) ** 2).sum()
+    ent_abs = np.abs((np.exp(logp) * logp).sum(axis=1)).sum()
+    magnitude = np.array([pg_abs + cfg["baseline_cost"] * bl_sum + cfg["entropy_cost"] * ent_abs, pg_abs, bl_sum, ent_abs])
+    loss_tol = 1e-5 * np.maximum(np.abs(want["losses"]), magnitude / 100)
+    errs = dict(losses=float(np.max(np.abs(got_losses - want["losses"]) / np.abs(want["losses"]))),
+                vs=U.rel_max(got_vs, want["vs"]), pg_adv=U.rel_max(got_adv, want["pg_adv"]),
+                dlogits=U.rel_max(got[:, :16], want["dlogits"].reshape(-1, 16)),
+                dvalue=U.rel_max(got[:, 16], want["dvalue"].reshape(-1)))
+    print(f"loss head m={m} t={t} ldh={ldh} mu x{mu_scale} logits x{logit_scale}: " +
+          ", ".join(f"{k} {v:.2e}" for k, v in errs.items()) +
+          f" (pg sum cancels {magnitude[1] / abs(want['losses'][1]):.0f}-fold)")
+    assert np.all(np.abs(got_losses - want["losses"]) <= loss_tol), (got_losses, want["losses"], loss_tol)
+    assert errs["vs"] < 1e-5 and errs["pg_adv"] < 1e-5
+    assert errs["dlogits"] < 1e-5 and errs["dvalue"] < 1e-5
 
 
 # ------------------------------------------------------------------------------- GEMM
