@@ -35,7 +35,7 @@ class FiLearnerConfig(C.Structure):
                 ("baseline_cost", c_float), ("entropy_cost", c_float),
                 ("gemm_mode", c_int), ("publish_every", c_int), ("checkpoint_location", c_char_p),
                 ("max_grad_norm", c_double), ("rmsprop_alpha", c_double), ("rmsprop_eps", c_double),
-                ("rmsprop_momentum", c_double)]
+                ("rmsprop_momentum", c_double), ("legal_action_mask", c_int)]
 
 
 class FiProfEntry(C.Structure):
@@ -111,6 +111,7 @@ SIGNATURES = {
     "fi_op_gather": (c_int, [_P, c_size_t, c_size_t, c_size_t, c_size_t, _P, _P]),
     "fi_op_vtrace": (c_int, [c_int, c_int] + [_P] * 5 + [c_float] * 4 + [_P, _P, _P]),
     "fi_op_vtrace_loss_head": (c_int, [_P, c_int, c_int, _P, c_int] + [c_float] * 6 + [_P] * 5),
+    "fi_op_vtrace_loss_head_legal": (c_int, [_P, c_int, c_int, _P, c_int] + [c_float] * 6 + [_P] * 5),
     "fi_op_adam": (c_int, [c_int, c_double, c_i64, c_size_t, _P, _P, _P, _P, c_float, _P]),
     "fi_op_grad_norm_clip": (c_int, [c_size_t, _P, c_double, _P, _P, _P]),
     "fi_op_rmsprop": (c_int, [c_double] * 4 + [c_size_t] + [_P] * 6),

@@ -202,6 +202,7 @@ constexpr int kWAction = 178;
 constexpr int kWReward = 179;
 constexpr int kWDiscount = 180;
 constexpr int kWAux = 181;
+constexpr int kWLegal = 182;   // uint32 legal-action word (bit j = action j legal); read only with legal_action_mask on
 constexpr int kWX = 192;
 constexpr int kXPerRec = 64;
 constexpr int kFarmerMinEntry = (kXDim + kXPerRec - 1) / kXPerRec;   // 8 records carry x: the shortest FarmerLstm trajectory

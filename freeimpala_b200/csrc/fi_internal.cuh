@@ -41,7 +41,7 @@ int launch_vtrace_scan(int m, int t, const float* log_rho, const float* discount
                        const float* value, const float* bootstrap, float rho_bar, float c_bar, float pg_rho_bar,
                        float lambda_, float* vs, float* pg_adv, cudaStream_t stream);
 int launch_vtrace_loss_head(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar,
-                            float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, float* dhead,
+                            float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, bool legal, float* dhead,
                             float* vs, float* pg_adv, double* losses, cudaStream_t stream,
                             float* dhead_hi = nullptr, float* dhead_lo = nullptr, int ld_split = 0, struct HScale* dhead_hs = nullptr);
 

@@ -347,6 +347,7 @@ void fi_learner_config_default(fi_learner_config* c) {
     c->rmsprop_alpha = 0.99;     // torch.optim.RMSprop defaults
     c->rmsprop_eps = 1e-8;
     c->rmsprop_momentum = 0.0;
+    c->legal_action_mask = 0;    // every action legal; record word 182 is not read
 }
 
 fi_learner* fi_learner_create(const fi_learner_config* cfg) {
@@ -373,6 +374,14 @@ fi_learner* fi_learner_create(const fi_learner_config* cfg) {
         !(cfg->rmsprop_momentum >= 0.0 && cfg->rmsprop_momentum < 1.0)) {
         set_error(FI_ERR_ARG, "fi_learner_create: RMSProp options need 0 < rmsprop_alpha < 1, rmsprop_eps > 0 and 0 <= rmsprop_momentum < 1 "
                               "(got %g, %g, %g)", cfg->rmsprop_alpha, cfg->rmsprop_eps, cfg->rmsprop_momentum);
+        return nullptr;
+    }
+    if (cfg->legal_action_mask != 0 && cfg->legal_action_mask != 1) {
+        set_error(FI_ERR_ARG, "fi_learner_create: legal_action_mask must be 0 or 1, got %d", cfg->legal_action_mask);
+        return nullptr;
+    }
+    if (farmer && cfg->legal_action_mask) {
+        set_error(FI_ERR_ARG, "fi_learner_create: legal_action_mask needs a policy; the FarmerLstm model has none");
         return nullptr;
     }
     if (!farmer) {   // V-trace constants: a NaN or out-of-range value would otherwise surface as NaN or meaningless losses

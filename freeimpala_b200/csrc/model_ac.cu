@@ -51,7 +51,8 @@ int ac_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int
         FI_TRY(dense_forward_plain(l, s, FI_GEMM_SIMT, p->params, batch, kRecWords, rows, p->head, p->gemm_ws, p->gemm_ws_bytes, st));
         FI_TRY(launch_zero2(p->d_losses, 4 * sizeof(double), nullptr, 0, st));
         FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
-                                       c.baseline_cost, c.entropy_cost, p->dhead, nullptr, nullptr, p->d_losses, st));
+                                       c.baseline_cost, c.entropy_cost, c.legal_action_mask != 0, p->dhead, nullptr, nullptr,
+                                       p->d_losses, st));
         return dense_backward_plain(l, s, FI_GEMM_SIMT, p->params, batch, kRecWords, p->dhead, rows, p->grads, nullptr, p->gemm_ws,
                                     p->gemm_ws_bytes, p->colsum_ws, p->colsum_ws_bytes, st);
     }
@@ -70,14 +71,14 @@ int ac_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int
     FI_TRY(dense_forward_split(l, s, p->params, rows, p->head, st));
     if (s->half) {  // the loss head writes plain fp32 rows and their max |x|; the fp16 split follows (13 MB)
         FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
-                                       c.baseline_cost, c.entropy_cost, p->dhead, nullptr, nullptr, p->d_losses, st, nullptr, nullptr, 0,
-                                       s->hs + kHsDout));
+                                       c.baseline_cost, c.entropy_cost, c.legal_action_mask != 0, p->dhead, nullptr, nullptr,
+                                       p->d_losses, st, nullptr, nullptr, 0, s->hs + kHsDout));
         FI_TRY(launch_split_h(p->dhead, kHead, (size_t)rows, kHead, kDoutLd, s->dout_hi, s->dout_lo, s->hs + kHsDout, 1, st));
     } else {
         FI_TRY(launch_zero2(p->d_losses, 4 * sizeof(double), nullptr, 0, st));
         FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
-                                       c.baseline_cost, c.entropy_cost, nullptr, nullptr, nullptr, p->d_losses, st, (float*)s->dout_hi,
-                                       (float*)s->dout_lo, kDoutLd));
+                                       c.baseline_cost, c.entropy_cost, c.legal_action_mask != 0, nullptr, nullptr, nullptr,
+                                       p->d_losses, st, (float*)s->dout_hi, (float*)s->dout_lo, kDoutLd));
     }
     return dense_backward_split(l, s, p->dhead, rows, p->grads, nullptr, 0, p->colsum_ws, p->colsum_ws_bytes, st);
 }

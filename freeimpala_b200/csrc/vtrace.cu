@@ -190,7 +190,13 @@ int launch_vtrace_scan(int m, int t, const float* log_rho, const float* discount
 // record fields are six 16-byte loads per lane (words 160..183 of the 1024-byte record); the gradient rows
 // go through padded tiles and leave as 128-byte coalesced stores. (The first version read and wrote every
 // row element by element from its own lane: 36 us for 22 MB, 0.09 of the HBM roofline.)
+// kLegal (fi_learner_config.legal_action_mask): both softmaxes, the entropy and d(head) run over the support
+// legal word (record word 182) | bit of the taken action. Outside the support every per-action operand is replaced before
+// use (-inf into fmaxf and expf, 0 as log pi), so logits there (-inf or NaN included) never reach the arithmetic, p = 0
+// and d(head) is exactly 0; the replacements are selects, not branches. The word sits in the record fields already
+// loaded, so the masked head reads no extra bytes.
 constexpr int kLossWarps = 4;
+template <bool kLegal>
 __global__ void __launch_bounds__(32 * kLossWarps)
 vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const float* __restrict__ head, int ldh,
                         float rho_bar, float c_bar, float pg_rho_bar, float lambda_, float baseline_cost,
@@ -239,10 +245,17 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
         const float* h = hs + (valid ? lane : nvalid - 1) * kHead;
         float z[kNumActions], p[kNumActions];
         float mx = -INFINITY, mmx = -INFINITY;
+        uint32_t sup = ~0u;   // support: bit j set = action j enters the softmaxes
+        if constexpr (kLegal) {
+            int a = __float_as_int(rf[kWAction - 160]);
+            a = a < 0 ? 0 : (a >= kNumActions ? kNumActions - 1 : a);
+            sup = __float_as_uint(rf[kWLegal - 160]) | (1u << a);
+        }
+        auto on = [&](int j) { return !kLegal || ((sup >> j) & 1u); };
 #pragma unroll
         for (int j = 0; j < kNumActions; j++) {
             z[j] = h[j];
-            mx = fmaxf(mx, z[j]);
+            mx = fmaxf(mx, on(j) ? z[j] : -INFINITY);
         }
         const float v = h[kNumActions];
         int act = __float_as_int(rf[kWAction - 160]);
@@ -252,20 +265,20 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
         for (int j = 0; j < kNumActions; j++) {
             const float mu = rf[kWMu - 160 + j];
             p[j] = mu;  // parked until the behaviour max is known
-            mmx = fmaxf(mmx, mu);
-            se += expf(z[j] - mx);
+            mmx = fmaxf(mmx, on(j) ? mu : -INFINITY);
+            se += expf(on(j) ? z[j] - mx : -INFINITY);
             if (j == act) { mu_a = mu; z_a = z[j]; }
         }
 #pragma unroll
-        for (int j = 0; j < kNumActions; j++) mu_se += expf(p[j] - mmx);
+        for (int j = 0; j < kNumActions; j++) mu_se += expf(on(j) ? p[j] - mmx : -INFINITY);
         const float lse = mx + logf(se);
         const float logp_a = z_a - lse;
         const float log_mu_a = mu_a - (mmx + logf(mu_se));
         float plogp = 0.f;
 #pragma unroll
         for (int j = 0; j < kNumActions; j++) {
-            const float lp = z[j] - lse;
-            p[j] = expf(lp);
+            const float lp = on(j) ? z[j] - lse : 0.f;   // outside the support: p = 0 and a finite log pi
+            p[j] = expf(on(j) ? lp : -INFINITY);
             z[j] = lp;  // z now holds log pi
             plogp = fmaf(p[j], lp, plogp);
         }
@@ -289,7 +302,7 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
         for (int j = 0; j < kNumActions; j++) {
             const float d_pg = adv * (p[j] - (j == act ? 1.f : 0.f));
             const float d_ent = p[j] * (z[j] - plogp);
-            dv[j] = fmaf(entropy_cost, d_ent, d_pg);
+            dv[j] = fmaf(entropy_cost, d_ent, d_pg);   // 0 outside the support: p = 0 and j != act
         }
         dv[kNumActions] = -baseline_cost * (vs - v);
         if (valid) {
@@ -358,7 +371,7 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
 
 int launch_vtrace_loss_head(const void* batch, int m, int t, const float* head, int ldh, float rho_bar,
                             float c_bar, float pg_rho_bar, float lambda_, float baseline_cost,
-                            float entropy_cost, float* dhead, float* vs, float* pg_adv, double* losses,
+                            float entropy_cost, bool legal, float* dhead, float* vs, float* pg_adv, double* losses,
                             cudaStream_t stream, float* dhead_hi, float* dhead_lo, int ld_split, HScale* dhead_hs) {
     if (m <= 0 || t <= 0) return FI_OK;
     if (!batch || !head || (!dhead && !dhead_hi) || !losses || ldh < kHead || (dhead_hi && (!dhead_lo || ld_split < kHead)))
@@ -367,10 +380,12 @@ int launch_vtrace_loss_head(const void* batch, int m, int t, const float* head, 
     if ((reinterpret_cast<uintptr_t>(batch) & 15) != 0) return set_error(FI_ERR_ARG, "vtrace loss head: batch must be 16-byte aligned");
     // algorithmic traffic per transition: head row in (17 x 4 B) + dhead row out (17 x 4 B) + the record's
     // behaviour logits, action, reward, discount (19 x 4 B) = 212 B (+ 8 B when vs / pg_adv are written)
-    LaunchScope ls("vtrace_loss_head_kernel", stream,
+    // (the masked head's legal word lies in the same 16-byte load as the discount and aux words: no extra traffic)
+    LaunchScope ls(legal ? "vtrace_loss_head_kernel_legal" : "vtrace_loss_head_kernel", stream,
                    (212.0 + (vs ? 4.0 : 0.0) + (pg_adv ? 4.0 : 0.0)) * (double)m * t, kWorkBytes);
-    launch_pdl(vtrace_loss_head_kernel, dim3((m + warps - 1) / warps), dim3(32 * warps), 0, stream, (const float*)batch, m, t, head, ldh, rho_bar,
-               c_bar, pg_rho_bar, lambda_, baseline_cost, entropy_cost, dhead, vs, pg_adv, losses, dhead_hi, dhead_lo, ld_split, dhead_hs);
+    launch_pdl(legal ? vtrace_loss_head_kernel<true> : vtrace_loss_head_kernel<false>, dim3((m + warps - 1) / warps),
+               dim3(32 * warps), 0, stream, (const float*)batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_,
+               baseline_cost, entropy_cost, dhead, vs, pg_adv, losses, dhead_hi, dhead_lo, ld_split, dhead_hs);
     return ls.done();
 }
 
@@ -389,6 +404,13 @@ int fi_op_vtrace_loss_head(const void* batch, int m, int t, const float* head, i
                            float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, float* dhead,
                            float* vs, float* pg_adv, double* losses, void* stream) {
     return fi::launch_vtrace_loss_head(batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_, baseline_cost,
-                                       entropy_cost, dhead, vs, pg_adv, losses, (cudaStream_t)stream);
+                                       entropy_cost, false, dhead, vs, pg_adv, losses, (cudaStream_t)stream);
+}
+
+int fi_op_vtrace_loss_head_legal(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar,
+                                 float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, float* dhead,
+                                 float* vs, float* pg_adv, double* losses, void* stream) {
+    return fi::launch_vtrace_loss_head(batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_, baseline_cost,
+                                       entropy_cost, true, dhead, vs, pg_adv, losses, (cudaStream_t)stream);
 }
 }

@@ -139,8 +139,9 @@ struct StepMetrics {
 class Learner {
 public:
     // Same order as learner.h:100-110. `r` (simulated training time) is ignored: the step is real work.
+    // legal_action_mask: fi_learner_config.legal_action_mask (actor-critic only; records carry the legal word, fi_learner.h).
     Learner(size_t p, size_t B, size_t S, size_t M, size_t /*r*/, size_t c, const std::string& l, const std::string& m,
-            size_t T, int device = 0, int model = FI_MODEL_MLP_ACTOR_CRITIC)
+            size_t T, int device = 0, int model = FI_MODEL_MLP_ACTOR_CRITIC, bool legal_action_mask = false)
         : num_players_(p), batch_size_(M), checkpoint_frequency_(c), checkpoint_location_(l), total_iterations_(T) {
         fi_learner_config cfg;
         fi_learner_config_default(&cfg);
@@ -152,6 +153,7 @@ public:
         cfg.model = model;
         cfg.loss = model == FI_MODEL_FARMER_LSTM ? FI_LOSS_MSE : FI_LOSS_VTRACE;
         cfg.checkpoint_location = l.empty() ? nullptr : l.c_str();
+        cfg.legal_action_mask = legal_action_mask ? 1 : 0;
         h_ = fi_learner_create(&cfg);
         if (!h_) throw std::runtime_error(std::string("fi_learner_create: ") + fi_last_error());
         model_manager_ = std::make_shared<ModelManager>(h_, p);

@@ -80,7 +80,7 @@ class Learner:
                  publish_every: int = 1, rho_bar: float = 1.0, c_bar: float = 1.0, pg_rho_bar: float = 1.0,
                  lambda_: float = 1.0, baseline_cost: float = 0.5, entropy_cost: float = 0.01,
                  max_grad_norm: float = 0.0, rmsprop_alpha: float = 0.99, rmsprop_eps: float = 1e-8,
-                 rmsprop_momentum: float = 0.0):
+                 rmsprop_momentum: float = 0.0, legal_action_mask: bool = False):
         self._lib = _lib.load()
         self.num_players, self.buffer_capacity, self.entry_size, self.batch_size = p, B, S, M
         self.train_time_ms, self.checkpoint_frequency = r, c
@@ -96,6 +96,7 @@ class Learner:
         cfg.gemm_mode, cfg.publish_every = _lib.GEMM[gemm_mode], publish_every
         cfg.max_grad_norm = max_grad_norm   # global-norm gradient clipping; 0 = off
         cfg.rmsprop_alpha, cfg.rmsprop_eps, cfg.rmsprop_momentum = rmsprop_alpha, rmsprop_eps, rmsprop_momentum
+        cfg.legal_action_mask = int(legal_action_mask)   # records carry the legal-action word (fi_learner.h)
         self._ckpt = l.encode() if l else None
         cfg.checkpoint_location = self._ckpt
         self._h = self._lib.fi_learner_create(C.byref(cfg))

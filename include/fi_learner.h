@@ -181,7 +181,30 @@ typedef struct fi_learner_config {
     double rmsprop_alpha;     /* FI_OPT_RMSPROP: square-average decay, 0 < alpha < 1 */
     double rmsprop_eps;       /* FI_OPT_RMSPROP: added to sqrt(square average), > 0 */
     double rmsprop_momentum;  /* FI_OPT_RMSPROP: 0 <= momentum < 1 (0 = no momentum buffer) */
+    /* Appended after rmsprop_momentum; fi_learner_config_default sets 0. Actor-critic model only: 1 = the V-trace loss
+       head reads each record's legal-action word (FI_REC_WORD_LEGAL) and computes log pi, log mu, the entropy and the
+       policy gradient over the legal set; 0 = all 16 actions, word 182 is not read. */
+    int legal_action_mask;
 } fi_learner_config;
+
+/* Trajectory record (FI_ELEMENT_SIZE bytes = 256 32-bit words) of the actor-critic model, the words the loss head reads
+ * (DESIGN.md section 1 has the whole layout): 0..161 observation, 162..177 behaviour logits mu (fp32), 178 action (int32,
+ * clamped to [0, 15]), 179 reward, 180 discount, 181 bootstrap value (last record of a trajectory), 182 legal-action word.
+ *
+ * Legal-action masking (legal_action_mask = 1). Word 182 is a uint32 in which bit j set means action j was legal at this
+ * step; bits 16..31 are ignored. The support is word | (1 << action): the action taken was legal by definition, so a word
+ * of 0 describes a forced move (pi(a) = 1, log pi(a) = 0, no entropy and no policy gradient for that transition). Then
+ *   log pi(a) = z_a - logsumexp of the learner's logits over the support
+ *   log mu(a) = mu_a - logsumexp of words 162..177 over the support
+ *   entropy term = sum over the support of pi log pi
+ * and d(loss)/d(logit j) is exactly 0 for every j outside it. The value path, the V-trace recurrence and the clipping
+ * constants are unchanged. Logits outside the support (learner or behaviour) never enter the arithmetic: -inf or NaN
+ * there changes nothing.
+ *
+ * What the actor does: fi_learner_infer returns the raw logits of all 16 actions. The actor samples from the
+ * softmax of those logits over its legal set, stores the logits it got (raw or already set to -inf outside the legal set)
+ * in words 162..177, the action in 178 and the legal word in 182. */
+#define FI_REC_WORD_LEGAL 182
 
 typedef struct fi_learner fi_learner;
 
@@ -189,7 +212,8 @@ FI_API void fi_learner_config_default(fi_learner_config* cfg);
 /* Learner ctor (learner.h:100-140): creates p rings, p models (random init), optimiser
  * state and all step workspaces in HBM. Returns NULL on failure (see fi_last_error). An unknown
  * optimiser, max_grad_norm < 0 or not finite, rmsprop_alpha outside (0, 1), rmsprop_eps <= 0 or
- * rmsprop_momentum outside [0, 1), and, for the actor-critic model, a V-trace constant outside the range
+ * rmsprop_momentum outside [0, 1), legal_action_mask other than 0 or 1 or set to 1 for the FarmerLstm model (which has
+ * no policy), and, for the actor-critic model, a V-trace constant outside the range
  * fi_learner_config states, is rejected (FI_ERR_ARG) before any device is looked for. */
 FI_API fi_learner* fi_learner_create(const fi_learner_config* cfg);
 FI_API void fi_learner_destroy(fi_learner* l);
@@ -309,6 +333,9 @@ FI_API int fi_op_vtrace(int m, int t, const float* log_rho, const float* discoun
  * discount / bootstrap; writes dhead (same layout), optionally vs / pg_adv [m*t], and ADDS
  * {total, pg, baseline, entropy} into losses[4] (double, zeroed by the caller). */
 FI_API int fi_op_vtrace_loss_head(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar, float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, float* dhead, float* vs, float* pg_adv, double* losses, void* stream);
+/* Same, with legal-action masking: the softmaxes, entropy and d(head) run over each record's legal word | the action's bit
+ * (see FI_REC_WORD_LEGAL); d(head) is 0 in every column outside that support. */
+FI_API int fi_op_vtrace_loss_head_legal(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar, float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, float* dhead, float* vs, float* pg_adv, double* losses, void* stream);
 
 /* One fused optimiser update over n contiguous fp32 values (28 B/param for Adam).
  * step counts from 1; grad_scale multiplies g first (1/world for averaged gradients). */
