@@ -97,6 +97,7 @@ SIGNATURES = {
     "fi_learner_param_ptr": (_P, [_P, c_int]),
     "fi_learner_infer": (c_int, [_P, c_int, _P, _P, c_size_t, c_size_t, _P, _P]),
     "fi_learner_infer_stats": (c_int, [_P, c_int, C.POINTER(c_u64), C.POINTER(c_u64), C.POINTER(c_u64)]),
+    "fi_learner_infer_grouped": (c_int, [_P, c_int, _P, c_size_t, c_size_t, _P, _P, _P, _P]),
     "fi_model_bytes": (c_size_t, [_P]),
     "fi_model_version": (c_u64, [_P, c_int]),
     "fi_model_get": (c_int, [_P, c_int, _P, c_size_t, C.POINTER(c_u64)]),

@@ -220,10 +220,10 @@ void free_player(fi_learner* l, Player* p) {
         if (d) cudaFree(d);
     for (float* d : p->store.dev_snap)
         if (d) cudaFree(d);
-    void* devv[] = {p->d_losses, p->gemm_ws, p->colsum_ws, p->stage_dev, p->clip_coef, p->norm_ws};
+    void* devv[] = {p->d_losses, p->gemm_ws, p->colsum_ws, p->stage_dev, p->clip_coef, p->norm_ws, p->inf_idx};
     for (void* d : devv)
         if (d) cudaFree(d);
-    void* pinned[] = {p->h_losses, p->stage_host, p->inf_host_in, p->inf_host_x, p->inf_host_out,
+    void* pinned[] = {p->h_losses, p->stage_host, p->inf_host_in, p->inf_host_x, p->inf_host_out, p->inf_host_idx,
                       p->store.host_buf[0], p->store.host_buf[1], p->store.host_buf[2]};
     for (void* h : pinned)
         if (h) cudaFreeHost(h);
@@ -872,62 +872,102 @@ constexpr size_t kInferMaxRows = 16384;
 int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& batch, size_t rows, size_t t) {
     const bool farmer = l->cfg.model == FI_MODEL_FARMER_LSTM;
     FI_CUDA_OK(cudaSetDevice(l->cfg.device));
+    size_t states = 0;
+    bool want_best = false;
+    for (const fi::InferReq* q : batch) {
+        states += q->states;
+        want_best |= q->best != nullptr;
+    }
+    // the farmer model uploads z once per state, the actor-critic one observation per row
     const size_t row_in = farmer ? t * fi::kZDim : fi::kZDim;
-    const size_t in_elems = rows * row_in;
-    const size_t out_cols = farmer ? 1 : fi::kHead;
-    if (rows > p->inf_rows_cap || (farmer && t > p->inf_t_cap)) {  // grow the inference workspaces (with head-room)
-        size_t cap = p->inf_rows_cap ? p->inf_rows_cap : 64;
-        while (cap < rows) cap *= 2;
+    const size_t in_elems = (farmer ? states : rows) * row_in;
+    if (rows > p->inf_rows_cap || (farmer && (states > p->inf_states_cap || t > p->inf_t_cap))) {  // grow (with head-room)
+        auto grow = [](size_t cap, size_t need) {
+            cap = cap ? cap : 64;
+            while (cap < need) cap *= 2;
+            return cap;
+        };
+        const size_t cap = grow(p->inf_rows_cap, rows);
+        const size_t scap = farmer ? grow(p->inf_states_cap, states) : 0;
         const size_t tcap = farmer ? (t > p->inf_t_cap ? t : p->inf_t_cap) : 0;
-        const size_t cap_in = cap * (farmer ? tcap * fi::kZDim : fi::kZDim);
+        const size_t cap_in = farmer ? scap * tcap * fi::kZDim : cap * fi::kZDim;
+        const size_t cap_out = farmer ? cap + scap : cap * fi::kHead;   // farmer: values, then best
         FI_CUDA_OK(cudaStreamSynchronize(p->infer_stream));
         if (p->inf_in) cudaFree(p->inf_in);
         if (p->inf_x) cudaFree(p->inf_x);
         if (p->inf_out) cudaFree(p->inf_out);
+        if (p->inf_idx) cudaFree(p->inf_idx);
         if (p->inf_host_in) cudaFreeHost(p->inf_host_in);
         if (p->inf_host_x) cudaFreeHost(p->inf_host_x);
         if (p->inf_host_out) cudaFreeHost(p->inf_host_out);
+        if (p->inf_host_idx) cudaFreeHost(p->inf_host_idx);
         p->inf_in = p->inf_x = p->inf_out = p->inf_host_in = p->inf_host_x = p->inf_host_out = nullptr;
-        p->inf_rows_cap = 0;
+        p->inf_idx = p->inf_host_idx = nullptr;
+        p->inf_rows_cap = p->inf_states_cap = 0;
         FI_CUDA_OK(cudaMalloc((void**)&p->inf_in, cap_in * sizeof(float)));
         FI_CUDA_OK(cudaHostAlloc((void**)&p->inf_host_in, cap_in * sizeof(float), cudaHostAllocPortable));
-        FI_CUDA_OK(cudaMalloc((void**)&p->inf_out, cap * out_cols * sizeof(float)));
-        FI_CUDA_OK(cudaHostAlloc((void**)&p->inf_host_out, cap * out_cols * sizeof(float), cudaHostAllocPortable));
+        FI_CUDA_OK(cudaMalloc((void**)&p->inf_out, cap_out * sizeof(float)));
+        FI_CUDA_OK(cudaHostAlloc((void**)&p->inf_host_out, cap_out * sizeof(float), cudaHostAllocPortable));
         if (farmer) {
+            const size_t cap_idx = scap + 1 + cap;
             FI_CUDA_OK(cudaMalloc((void**)&p->inf_x, cap * fi::kXDim * sizeof(float)));
             FI_CUDA_OK(cudaHostAlloc((void**)&p->inf_host_x, cap * fi::kXDim * sizeof(float), cudaHostAllocPortable));
-            FI_TRY(fi::farmer_infer_alloc(l, p, cap, tcap));
+            FI_CUDA_OK(cudaMalloc((void**)&p->inf_idx, cap_idx * sizeof(uint32_t)));
+            FI_CUDA_OK(cudaHostAlloc((void**)&p->inf_host_idx, cap_idx * sizeof(uint32_t), cudaHostAllocPortable));
+            FI_TRY(fi::farmer_infer_alloc(l, p, scap, cap, tcap));
         } else {
             FI_TRY(fi::ac_infer_alloc(l, p, cap));
         }
         p->inf_rows_cap = cap;
+        p->inf_states_cap = scap;
         p->inf_t_cap = tcap;
     }
     cudaStream_t st = p->infer_stream;
-    size_t r0 = 0;
-    for (const fi::InferReq* q : batch) {   // pack the callers' rows back to back
-        memcpy(p->inf_host_in + r0 * row_in, q->obs, q->rows * row_in * sizeof(float));
-        if (farmer) memcpy(p->inf_host_x + r0 * fi::kXDim, q->x, q->rows * fi::kXDim * sizeof(float));
+    uint32_t* const off = p->inf_host_idx;              // farmer: the batch's offsets [states + 1] ...
+    uint32_t* const row_state = off ? off + states + 1 : nullptr;   // ... then the state of each candidate row [rows]
+    size_t r0 = 0, s0 = 0;
+    for (const fi::InferReq* q : batch) {   // pack the callers' states and rows back to back, their offsets rebased
+        memcpy(p->inf_host_in + (farmer ? s0 : r0) * row_in, q->obs, (farmer ? q->states : q->rows) * row_in * sizeof(float));
+        if (farmer) {
+            memcpy(p->inf_host_x + r0 * fi::kXDim, q->x, q->rows * fi::kXDim * sizeof(float));
+            for (size_t s = 0; s < q->states; s++) {
+                const size_t b = q->offsets ? q->offsets[s] : s, e = q->offsets ? q->offsets[s + 1] : s + 1;
+                off[s0 + s] = (uint32_t)(r0 + b);
+                for (size_t r = b; r < e; r++) row_state[r0 + r] = (uint32_t)(s0 + s);
+            }
+        }
         r0 += q->rows;
+        s0 += q->states;
     }
     FI_CUDA_OK(cudaMemcpyAsync(p->inf_in, p->inf_host_in, in_elems * sizeof(float), cudaMemcpyHostToDevice, st));
-    if (farmer) FI_CUDA_OK(cudaMemcpyAsync(p->inf_x, p->inf_host_x, rows * fi::kXDim * sizeof(float), cudaMemcpyHostToDevice, st));
+    if (farmer) {
+        off[states] = (uint32_t)rows;
+        FI_CUDA_OK(cudaMemcpyAsync(p->inf_x, p->inf_host_x, rows * fi::kXDim * sizeof(float), cudaMemcpyHostToDevice, st));
+        FI_CUDA_OK(cudaMemcpyAsync(p->inf_idx, off, (states + 1 + rows) * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    }
+    int32_t* const best_dev = want_best ? reinterpret_cast<int32_t*>(p->inf_out + rows) : nullptr;
     {
         ModelStore& s = p->store;
         std::lock_guard<std::mutex> g(s.mu);  // pins the newest snapshot against the learner's next write into it
         const int sn = s.newest_snap;
         FI_CUDA_OK(cudaStreamWaitEvent(st, s.snap_ready[sn], 0));
-        if (farmer) FI_TRY(fi::farmer_infer(l, p, s.dev_snap[sn], p->inf_in, p->inf_x, rows, t, p->inf_out, st));
-        else FI_TRY(fi::ac_infer(l, p, s.dev_snap[sn], p->inf_in, rows, p->inf_out, st));
+        if (farmer)
+            FI_TRY(fi::farmer_infer(l, p, s.dev_snap[sn], p->inf_in, p->inf_x, p->inf_idx, p->inf_idx + states + 1, states, rows, t,
+                                    p->inf_out, best_dev, st));
+        else
+            FI_TRY(fi::ac_infer(l, p, s.dev_snap[sn], p->inf_in, rows, p->inf_out, st));
         FI_CUDA_OK(cudaEventRecord(s.infer_done[sn], st));
         s.infer_recorded[sn] = true;
     }
-    FI_CUDA_OK(cudaMemcpyAsync(p->inf_host_out, p->inf_out, rows * out_cols * sizeof(float), cudaMemcpyDeviceToHost, st));
+    const size_t out_elems = farmer ? rows + (want_best ? states : 0) : rows * fi::kHead;
+    FI_CUDA_OK(cudaMemcpyAsync(p->inf_host_out, p->inf_out, out_elems * sizeof(float), cudaMemcpyDeviceToHost, st));
     FI_CUDA_OK(cudaStreamSynchronize(st));   // one synchronisation per BATCH: the callers need their rows on the host
-    r0 = 0;
+    const int32_t* const best_host = reinterpret_cast<const int32_t*>(p->inf_host_out + rows);
+    r0 = s0 = 0;
     for (const fi::InferReq* q : batch) {
         if (farmer) {
-            memcpy(q->values, p->inf_host_out + r0, q->rows * sizeof(float));
+            if (q->values) memcpy(q->values, p->inf_host_out + r0, q->rows * sizeof(float));
+            if (q->best) memcpy(q->best, best_host + s0, q->states * sizeof(int32_t));
         } else {
             for (size_t r = 0; r < q->rows; r++) {
                 const float* o = p->inf_host_out + (r0 + r) * fi::kHead;
@@ -936,19 +976,14 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
             }
         }
         r0 += q->rows;
+        s0 += q->states;
     }
     return FI_OK;
 }
-}  // namespace
 
-int fi_learner_infer(fi_learner* l, int player, const float* obs_or_z, const float* x, size_t rows, size_t t,
-                     float* logits, float* values) {
-    Player* p = get_player(l, player);
-    if (!p || !obs_or_z || rows == 0) return set_error(FI_ERR_ARG, "fi_learner_infer: null argument");
-    const bool farmer = l->cfg.model == FI_MODEL_FARMER_LSTM;
-    if (farmer && (!x || t == 0 || !values)) return set_error(FI_ERR_ARG, "fi_learner_infer: the farmer model needs z, x, t and values");
-    if (rows > kInferMaxRows) return set_error(FI_ERR_ARG, "fi_learner_infer: at most %zu rows per call", kInferMaxRows);
-    fi::InferReq req{obs_or_z, x, rows, farmer ? t : 0, logits, values, FI_OK, false};
+// Queues `req` on its player and waits for it: the first caller that finds no forward in flight becomes the leader and runs
+// everything pending that fits one forward (the farmer model batches equal sequence lengths).
+int submit_infer(fi_learner* l, Player* p, fi::InferReq& req) {
     std::unique_lock<std::mutex> lk(p->infer_mu);
     p->infer_pending.push_back(&req);
     p->infer_calls++;
@@ -957,7 +992,6 @@ int fi_learner_infer(fi_learner* l, int player, const float* obs_or_z, const flo
             p->infer_cv.wait(lk);
             continue;
         }
-        // become the leader: everything pending that fits one forward (the farmer model batches equal sequence lengths)
         p->infer_busy = true;
         std::vector<fi::InferReq*> batch;
         size_t total = 0;
@@ -984,6 +1018,37 @@ int fi_learner_infer(fi_learner* l, int player, const float* obs_or_z, const flo
         p->infer_cv.notify_all();
     }
     return req.status;
+}
+}  // namespace
+
+int fi_learner_infer(fi_learner* l, int player, const float* obs_or_z, const float* x, size_t rows, size_t t,
+                     float* logits, float* values) {
+    Player* p = get_player(l, player);
+    if (!p || !obs_or_z || rows == 0) return set_error(FI_ERR_ARG, "fi_learner_infer: null argument");
+    const bool farmer = l->cfg.model == FI_MODEL_FARMER_LSTM;
+    if (farmer && (!x || t == 0 || !values)) return set_error(FI_ERR_ARG, "fi_learner_infer: the farmer model needs z, x, t and values");
+    if (rows > kInferMaxRows) return set_error(FI_ERR_ARG, "fi_learner_infer: at most %zu rows per call", kInferMaxRows);
+    fi::InferReq req{obs_or_z, x, rows, farmer ? t : 0, rows, nullptr, logits, values, nullptr, FI_OK, false};
+    return submit_infer(l, p, req);
+}
+
+int fi_learner_infer_grouped(fi_learner* l, int player, const float* z, size_t states, size_t t, const float* x,
+                             const uint32_t* offsets, float* values, int32_t* best) {
+    Player* p = get_player(l, player);
+    if (!p) return set_error(FI_ERR_ARG, "fi_learner_infer_grouped: no player %d", player);
+    if (l->cfg.model != FI_MODEL_FARMER_LSTM) return set_error(FI_ERR_ARG, "fi_learner_infer_grouped: FarmerLstm model only");
+    if (!z || !x || !offsets || (!values && !best))
+        return set_error(FI_ERR_ARG, "fi_learner_infer_grouped: z, x, offsets and one of values / best are required");
+    if (states == 0 || t == 0) return set_error(FI_ERR_ARG, "fi_learner_infer_grouped: states and t must be positive");
+    if (states > kInferMaxRows) return set_error(FI_ERR_ARG, "fi_learner_infer_grouped: at most %zu rows per call", kInferMaxRows);
+    if (offsets[0] != 0) return set_error(FI_ERR_ARG, "fi_learner_infer_grouped: offsets[0] must be 0");
+    for (size_t s = 0; s < states; s++)
+        if (offsets[s + 1] <= offsets[s])
+            return set_error(FI_ERR_ARG, "fi_learner_infer_grouped: offsets must increase strictly (state %zu has no candidate)", s);
+    const size_t rows = offsets[states];
+    if (rows > kInferMaxRows) return set_error(FI_ERR_ARG, "fi_learner_infer_grouped: %zu rows, at most %zu per call", rows, kInferMaxRows);
+    fi::InferReq req{z, x, rows, t, states, offsets, nullptr, values, best, FI_OK, false};
+    return submit_infer(l, p, req);
 }
 
 int fi_learner_infer_stats(fi_learner* l, int player, uint64_t* calls, uint64_t* batches, uint64_t* rows) {

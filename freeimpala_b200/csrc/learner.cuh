@@ -105,12 +105,17 @@ struct DenseStack {
 
 struct FarmerWs;   // model_farmer.cu
 
-struct InferReq {   // one caller of fi_learner_infer waiting for its rows
-    const float* obs;
+// One caller of fi_learner_infer / fi_learner_infer_grouped waiting for its rows. A FarmerLstm request is `states` histories z
+// [states, t, 162] and `rows` candidate rows x [rows, 484], rows offsets[s] .. offsets[s+1]-1 belonging to state s; a plain
+// fi_learner_infer request is `rows` states of one candidate each (offsets null).
+struct InferReq {
+    const float* obs;   // actor-critic: observations [rows, 162]; FarmerLstm: z
     const float* x;
-    size_t rows, t;
+    size_t rows, t, states;
+    const uint32_t* offsets;   // [states + 1], or null: candidate r belongs to state r
     float* logits;
     float* values;
+    int32_t* best;             // FarmerLstm, may be null: [states], each state's argmax within its group
     int status;
     bool done;
 };
@@ -153,10 +158,14 @@ struct Player {
     bool infer_busy = false;
     uint64_t infer_calls = 0, infer_batches = 0, infer_rows = 0;
     cudaStream_t infer_stream = nullptr;
+    // FarmerLstm: inf_in holds z per state, inf_x the candidate rows, inf_idx the batch's offsets [states + 1] followed by the
+    // state of each candidate row [rows], inf_out the values [rows] followed by best [states] (int32)
     float *inf_in = nullptr, *inf_x = nullptr, *inf_out = nullptr;
+    uint32_t* inf_idx = nullptr;
     float *inf_host_in = nullptr, *inf_host_x = nullptr, *inf_host_out = nullptr;  // pinned
+    uint32_t* inf_host_idx = nullptr;                                              // pinned
     DenseStack inf_dense;       // the dense stack of batched inference (forward only)
-    size_t inf_rows_cap = 0, inf_t_cap = 0;
+    size_t inf_rows_cap = 0, inf_states_cap = 0, inf_t_cap = 0;
     // the step as one CUDA graph (learner.cu step_with_graph)
     void* graph_exec = nullptr;       // cudaGraphExec_t
     void* graph = nullptr;            // cudaGraph_t it was instantiated from
@@ -219,7 +228,10 @@ int ac_infer(fi_learner* l, Player* p, const float* params, const float* obs_dev
 int farmer_alloc(fi_learner* l, Player* p);
 void farmer_free(Player* p);
 int farmer_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int t, int global_m);
-int farmer_infer_alloc(fi_learner* l, Player* p, size_t rows, size_t t);
-int farmer_infer(fi_learner* l, Player* p, const float* params, const float* z_dev, const float* x_dev, size_t rows,
-                 size_t t, float* out_dev, cudaStream_t stream);
+int farmer_infer_alloc(fi_learner* l, Player* p, size_t states, size_t rows, size_t t);
+// The recurrence once per state, the dense stack once per candidate row: values_dev [rows]; best_dev (may be null) [states], the
+// index within each group of its largest value (lowest on ties). offsets_dev [states + 1], state_dev [rows]: the groups.
+int farmer_infer(fi_learner* l, Player* p, const float* params, const float* z_dev, const float* x_dev, const uint32_t* offsets_dev,
+                 const uint32_t* state_dev, size_t states, size_t rows, size_t t, float* values_dev, int32_t* best_dev,
+                 cudaStream_t stream);
 }  // namespace fi

@@ -27,12 +27,13 @@ struct FarmerWs {
     float* cst = nullptr;     // [rows*T, 128]: c_t
     float* whh_t = nullptr;   // [128, 512]: W_hh transposed (coalesced reads in the forward recurrence)
     float* feat = nullptr;    // [rows, 612]
+    float* h_last = nullptr;  // inference: [states, 612], h_{T-1} of each state in columns 0..127 (the recurrence writes kFeat-wide rows)
     float* y = nullptr;       // [rows]
     float* dy = nullptr;      // [rows]
     float* target = nullptr;  // [rows]
     void* gemm_ws = nullptr; size_t gemm_ws_bytes = 0;
     void* colsum_ws = nullptr; size_t colsum_ws_bytes = 0;
-    size_t rows = 0, t = 0;
+    size_t states = 0, rows = 0, t = 0;   // rows of the recurrence, rows of the dense stack (equal when training), steps
     // tensor-core path of the three [rows*T]-sized products (input projection and the two LSTM weight gradients): 3xFP16
     // operand pairs (gemm_tc.cu), each big operand split ONCE per step — the observations serve the projection and the
     // W_ih gradient, the gate gradients serve both weight gradients
@@ -114,10 +115,46 @@ __global__ void farmer_assemble_kernel(const float* __restrict__ batch, int m, i
     }
     if (threadIdx.x == 0) target[b] = __ldg(slot + kWAux);
 }
-// inference variant: x is a dense [rows, 484] array
-__global__ void farmer_assemble_dense_kernel(const float* __restrict__ x, int m, float* __restrict__ feat) {
-    const int b = blockIdx.x;
-    for (int j = threadIdx.x; j < kXDim; j += blockDim.x) feat[(size_t)b * kFeat + kLstmH + j] = __ldg(x + (size_t)b * kXDim + j);
+// Inference: feat[r] = h_last[state[r], 0..127] ‖ x[r] for candidate rows r < rows. A feature row is 153 float4 (32 of h, 121
+// of x; every row of the three arrays starts on a 16-byte boundary), one float4 per thread.
+constexpr int kFeat4 = kFeat / 4, kH4 = kLstmH / 4, kX4 = kXDim / 4;
+static_assert(kFeat % 4 == 0 && kLstmH % 4 == 0 && kXDim % 4 == 0, "16-byte rows");
+
+__global__ void farmer_assemble_grouped_kernel(const float4* __restrict__ h_last, const float4* __restrict__ x,
+                                               const uint32_t* __restrict__ state, int rows, float4* __restrict__ feat) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= rows * kFeat4) return;
+    const int r = i / kFeat4, c = i - r * kFeat4;
+    feat[i] = c < kH4 ? __ldg(h_last + (size_t)__ldg(state + r) * kFeat4 + c) : __ldg(x + (size_t)r * kX4 + (c - kH4));
+}
+
+// best[s] = the index within group s (rows offsets[s] .. offsets[s+1]-1 of y) of its largest value, in numpy's argmax order:
+// NaN above every number, then the larger value, then the lower index. One warp per group: each lane scans every 32nd row in
+// ascending order, then a butterfly reduction on (value, index); the result does not depend on the group's size or on timing.
+__device__ __forceinline__ bool argmax_before(float v, int i, float bv, int bi) {
+    const bool vn = v != v, bn = bv != bv;
+    if (vn != bn) return vn;
+    return (!vn && v > bv) || ((vn || v == bv) && i < bi);
+}
+
+__global__ void segment_argmax_kernel(const float* __restrict__ y, const uint32_t* __restrict__ offsets, int states,
+                                      int32_t* __restrict__ best) {
+    const int s = blockIdx.x * (blockDim.x / 32) + threadIdx.x / 32, lane = threadIdx.x & 31;
+    if (s >= states) return;
+    const int r0 = (int)__ldg(offsets + s), n = (int)__ldg(offsets + s + 1) - r0;
+    float bv = -INFINITY;
+    int bi = INT_MAX;   // a lane without rows loses to any row (every group has one)
+    for (int i = lane; i < n; i += 32) {
+        const float v = __ldg(y + r0 + i);
+        if (argmax_before(v, i, bv, bi)) { bv = v; bi = i; }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        if (argmax_before(ov, oi, bv, bi)) { bv = ov; bi = oi; }
+    }
+    if (lane == 0) best[s] = bi;
 }
 
 // Forward recurrence. gates[(b,t), 512] holds W_ih z + b_ih on entry and the post-activation gates i,f,g,o on
@@ -463,7 +500,7 @@ __global__ void regression_loss_kernel(const float* __restrict__ y, const float*
 // ------------------------------------------------------------------------------------------
 static void ws_release(FarmerWs* w) {
     if (!w) return;
-    float* f[] = {w->gates, w->hprev, w->cst, w->whh_t, w->feat, w->y, w->dy, w->target, w->dfeat};
+    float* f[] = {w->gates, w->hprev, w->cst, w->whh_t, w->feat, w->h_last, w->y, w->dy, w->target, w->dfeat};
     for (float* p : f)
         if (p) cudaFree(p);
     if (w->gemm_ws) cudaFree(w->gemm_ws);
@@ -474,22 +511,25 @@ static void ws_release(FarmerWs* w) {
     delete w;
 }
 
-// The workspaces of a step (training) or of batched inference, and the dense stack `ds` they run with.
-static int ws_create(fi_learner* l, size_t rows, size_t t, bool training, FarmerWs** out, DenseStack* ds) {
+// The workspaces of a step (training: states == rows) or of batched inference (the recurrence runs on `states` rows, the
+// dense stack on `rows` candidate rows), and the dense stack `ds` they run with.
+static int ws_create(fi_learner* l, size_t states, size_t rows, size_t t, bool training, FarmerWs** out, DenseStack* ds) {
     FarmerWs* w = new FarmerWs();
     *out = w;
+    w->states = states;
     w->rows = rows;
     w->t = t;
-    const size_t rt = rows * t;
+    const size_t rt = states * t;
     // the tensor-core recurrence keeps gates and c in 64-row blocks (fi_internal.cuh): room for the padded rows, zeroed once so
     // that what the padding rows carry stays finite
-    const size_t rt_pad = ((rows + kStepBlockRows - 1) / kStepBlockRows) * kStepBlockRows * t;
+    const size_t rt_pad = ((states + kStepBlockRows - 1) / kStepBlockRows) * kStepBlockRows * t;
     FI_CUDA_OK(cudaMalloc((void**)&w->gates, rt_pad * kG4 * sizeof(float)));
     FI_CUDA_OK(cudaMemset(w->gates, 0, rt_pad * kG4 * sizeof(float)));
     FI_CUDA_OK(cudaMalloc((void**)&w->whh_t, (size_t)kG4 * kLstmH * sizeof(float)));
     FI_CUDA_OK(cudaMalloc((void**)&w->feat, rows * kFeat * sizeof(float)));
-    FI_CUDA_OK(cudaMalloc((void**)&w->y, rows * sizeof(float)));
+    if (!training) FI_CUDA_OK(cudaMalloc((void**)&w->h_last, states * kFeat * sizeof(float)));
     if (training) {
+        FI_CUDA_OK(cudaMalloc((void**)&w->y, rows * sizeof(float)));
         FI_CUDA_OK(cudaMalloc((void**)&w->hprev, rt * kLstmH * sizeof(float)));
         FI_CUDA_OK(cudaMalloc((void**)&w->cst, rt_pad * kLstmH * sizeof(float)));
         FI_CUDA_OK(cudaMemset(w->cst, 0, rt_pad * kLstmH * sizeof(float)));
@@ -543,7 +583,7 @@ static int ws_create(fi_learner* l, size_t rows, size_t t, bool training, Farmer
 
 int farmer_alloc(fi_learner* l, Player* p) {
     FarmerWs* w = nullptr;
-    const int rc = ws_create(l, l->cfg.batch_size, l->cfg.entry_size, true, &w, &p->dense);
+    const int rc = ws_create(l, l->cfg.batch_size, l->cfg.batch_size, l->cfg.entry_size, true, &w, &p->dense);
     p->farmer_ws = w;
     return rc;
 }
@@ -566,9 +606,12 @@ static bool farmer_dense_tc(const fi_learner* l, const DenseStack* ds, int m) {
     return ds->split && (l->cfg.gemm_mode == FI_GEMM_TCGEN05_F16 || m >= 128);
 }
 
-// z rows: (b,t) at z + (b*t + s) * ldz. Leaves y[m], feat, the dense stack's activations (and the BPTT state when training).
-static int farmer_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const float* params, const float* z, int ldz, int m, int t,
-                          cudaStream_t st) {
+// The LSTM half of the forward over m rows of z (row (b,t) at z + (b*t + s) * ldz): the input projection and the recurrence,
+// leaving h_{T-1} of row b in columns 0..127 of h [m, kFeat] (and the BPTT state when training). dense_tc: the dense stack
+// that follows runs on split operands; its scales are zeroed and its parameters split here, before W_ih's split that shares
+// the arena's scale.
+static int farmer_lstm_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const float* params, const float* z, int ldz, int m, int t,
+                               bool dense_tc, float* h, cudaStream_t st) {
     const auto& T = l->tensors;
     // inference workspaces carry no GEMM workspace: actor batches are small and run on the fp32 FFMA kernels
     const int mode = w->gemm_ws ? l->cfg.gemm_mode : FI_GEMM_SIMT;
@@ -580,7 +623,7 @@ static int farmer_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const floa
         transpose_whh_kernel<<<(kG4 * kLstmH + 255) / 256, 256, 0, st>>>(params + T[1].offset, w->whh_t);
         FI_TRY(ls.done());
     }
-    const bool half_proj = farmer_use_half(l, w, rt), dense_tc = farmer_dense_tc(l, ds, m);
+    const bool half_proj = farmer_use_half(l, w, rt);
     if (half_proj || dense_tc) FI_TRY(launch_zero2(w->hs, 4 * sizeof(HScale), ds->hs, ds->hs ? kHsCount * sizeof(HScale) : 0, st));
     // parameters: max |p|, the split of the whole arena and dense1.w's copy with padded rows, one launch
     if (dense_tc) FI_TRY(dense_split_params(l, ds, params, st));
@@ -604,7 +647,7 @@ static int farmer_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const floa
     if (lstm_tc) {
         // h_{s-1} leaves the kernel as the fp16 pairs the W_hh gradient product reads (scale 2^13: |h| <= 1)
         FI_TRY(launch_lstm_forward_tc(w->gates, params + T[1].offset, params + T[3].offset, m, t, w->hp_hi, w->hp_lo, w->hs + kLstmHsHp, w->cst,
-                                      w->feat, kFeat, st));
+                                      h, kFeat, st));
     } else {
         // recurrent flops: 2 * 128 * 512 per (row, step)
         LaunchScope ls("lstm_forward_kernel", st, 2.0 * kLstmH * kG4 * (double)rt, kWorkFlops);
@@ -613,16 +656,25 @@ static int farmer_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const floa
         // training on the 3xFP16 path: h_prev leaves the kernel as the fp16 pairs the W_hh gradient product reads
         const bool hp_pairs = half_proj && w->hp_hi;
         launch_pdl(lstm_forward_kernel, dim3((m + kLstmRows - 1) / kLstmRows), dim3(kLstmThreads), kLstmFwdSmem, st, w->gates, w->whh_t,
-                   params + T[3].offset, m, t, hp_pairs ? nullptr : w->hprev, w->cst, w->feat,
+                   params + T[3].offset, m, t, hp_pairs ? nullptr : w->hprev, w->cst, h,
                    hp_pairs ? static_cast<__half*>(w->hp_hi) : nullptr, hp_pairs ? static_cast<__half*>(w->hp_lo) : nullptr,
                    hp_pairs ? w->hs + kLstmHsHp : nullptr, lstm_trace_buffer());
         FI_TRY(ls.done());
         lstm_trace_report("forward (FFMA)", lstm_trace_buffer(), t, st);
     }
+    return FI_OK;
+}
+
+// The step's forward. Leaves y[m], feat, the dense stack's activations and the BPTT state.
+static int farmer_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const float* params, const float* z, int ldz, int m, int t,
+                          cudaStream_t st) {
+    const bool dense_tc = farmer_dense_tc(l, ds, m);
+    FI_TRY(farmer_lstm_forward(l, w, ds, params, z, ldz, m, t, dense_tc, w->feat, st));
     if (dense_tc) {
         FI_TRY(launch_amax_split_h(w->feat, kFeat, (size_t)m, kFeat, kFeatLdH, ds->in_hi, ds->in_lo, ds->hs + kHsIn, st));
         return dense_forward_split(l, ds, params, m, w->y, st);
     }
+    const int mode = w->gemm_ws ? l->cfg.gemm_mode : FI_GEMM_SIMT;
     return dense_forward_plain(l, ds, mode, params, w->feat, kFeat, m, w->y, w->gemm_ws, w->gemm_ws_bytes, st);
 }
 
@@ -701,26 +753,38 @@ int farmer_forward_backward(fi_learner* l, Player* p, const float* batch, int m,
     return FI_OK;
 }
 
-int farmer_infer_alloc(fi_learner* l, Player* p, size_t rows, size_t t) {
+int farmer_infer_alloc(fi_learner* l, Player* p, size_t states, size_t rows, size_t t) {
     ws_release(p->farmer_inf_ws);
     dense_free(&p->inf_dense);
     FarmerWs* w = nullptr;
-    const int rc = ws_create(l, rows, t, false, &w, &p->inf_dense);
+    const int rc = ws_create(l, states, rows, t, false, &w, &p->inf_dense);
     p->farmer_inf_ws = w;
     return rc;
 }
 
-int farmer_infer(fi_learner* l, Player* p, const float* params, const float* z_dev, const float* x_dev, size_t rows,
-                 size_t t, float* out_dev, cudaStream_t stream) {
+int farmer_infer(fi_learner* l, Player* p, const float* params, const float* z_dev, const float* x_dev, const uint32_t* offsets_dev,
+                 const uint32_t* state_dev, size_t states, size_t rows, size_t t, float* values_dev, int32_t* best_dev,
+                 cudaStream_t stream) {
     FarmerWs* w = p->farmer_inf_ws;
-    if (!w || rows > w->rows || t > w->t) return set_error(FI_ERR_STATE, "farmer inference workspaces too small");
+    if (!w || states > w->states || rows > w->rows || t > w->t) return set_error(FI_ERR_STATE, "farmer inference workspaces too small");
+    // inference runs every product on the fp32 FFMA kernels: each row's value is then independent of the batch around it
+    FI_TRY(farmer_lstm_forward(l, w, &p->inf_dense, params, z_dev, kZDim, (int)states, (int)t, false, w->h_last, stream));
     {
-        LaunchScope ls("farmer_assemble_dense_kernel", stream, 2.0 * 4 * kXDim * (double)rows, kWorkBytes);
-        farmer_assemble_dense_kernel<<<(unsigned)rows, 128, 0, stream>>>(x_dev, (int)rows, w->feat);
+        const int n4 = (int)rows * kFeat4;
+        LaunchScope ls("farmer_assemble_grouped_kernel", stream, 2.0 * 4 * kFeat * (double)rows, kWorkBytes);
+        farmer_assemble_grouped_kernel<<<(n4 + 255) / 256, 256, 0, stream>>>(reinterpret_cast<const float4*>(w->h_last),
+                                                                            reinterpret_cast<const float4*>(x_dev), state_dev, (int)rows,
+                                                                            reinterpret_cast<float4*>(w->feat));
         FI_TRY(ls.done());
     }
-    FI_TRY(farmer_forward(l, w, &p->inf_dense, params, z_dev, kZDim, (int)rows, (int)t, stream));
-    FI_CUDA_OK(cudaMemcpyAsync(out_dev, w->y, rows * sizeof(float), cudaMemcpyDeviceToDevice, stream));
+    FI_TRY(dense_forward_plain(l, &p->inf_dense, FI_GEMM_SIMT, params, w->feat, kFeat, (int)rows, values_dev, nullptr, 0, stream));
+    if (best_dev) {
+        constexpr int kWarps = 8;
+        LaunchScope ls("segment_argmax_kernel", stream, 4.0 * (double)rows + 12.0 * (double)states, kWorkBytes);
+        segment_argmax_kernel<<<(unsigned)((states + kWarps - 1) / kWarps), kWarps * 32, 0, stream>>>(values_dev, offsets_dev, (int)states,
+                                                                                                        best_dev);
+        FI_TRY(ls.done());
+    }
     return FI_OK;
 }
 

@@ -302,6 +302,26 @@ class Learner:
                                          values.ctypes.data), "fi_learner_infer")
         return values
 
+    def infer_grouped(self, player_index: int, z: np.ndarray, x: np.ndarray, offsets: np.ndarray):
+        """FarmerLstm inference of candidate actions grouped by state: z [S,T,162] is each state's history, x [R,484] the
+        candidate rows, rows offsets[s] .. offsets[s+1]-1 belonging to state s (offsets [S+1], offsets[0] = 0, R = offsets[S]).
+        Returns (values [R], best [S]): best[s] is the index within state s's group of its largest value, lowest on ties."""
+        zz = np.ascontiguousarray(z, dtype=np.float32)
+        xx = np.ascontiguousarray(x, dtype=np.float32)
+        off = np.ascontiguousarray(offsets, dtype=np.uint32)
+        if zz.ndim != 3 or zz.shape[2] != 162 or xx.ndim != 2 or xx.shape[1] != 484 or off.shape != (zz.shape[0] + 1,):
+            raise ValueError(f"infer_grouped: z {zz.shape}, x {xx.shape}, offsets {off.shape}: "
+                             "expected z [S,T,162], x [R,484], offsets [S+1]")
+        if off[-1] > xx.shape[0]:
+            raise ValueError(f"infer_grouped: offsets[-1] = {off[-1]} but x has {xx.shape[0]} rows")
+        states, t = zz.shape[0], zz.shape[1]
+        values = np.empty(int(off[-1]), np.float32)
+        best = np.empty(states, np.int32)
+        check(self._lib.fi_learner_infer_grouped(self._h, player_index, zz.ctypes.data, states, t, xx.ctypes.data,
+                                                 off.ctypes.data, values.ctypes.data, best.ctypes.data),
+              "fi_learner_infer_grouped")
+        return values, best
+
     # ---- data parallelism (SURVEY.md 8e) ------------------------------------------------------------
     def infer_stats(self, player_index: int) -> dict:
         """Counters of the combining inference path: calls made, forwards run, rows served."""

@@ -281,6 +281,22 @@ FI_API int fi_learner_infer(fi_learner* l, int player, const float* obs_or_z, co
  * host->device copy, one forward on the newest published weights and one device->host copy per batch. Counters since creation:
  * calls made, forwards run, rows served (any may be NULL). No counterpart in the reference (the hook is a comment, agent.h:52-56). */
 FI_API int fi_learner_infer_stats(fi_learner* l, int player, uint64_t* calls, uint64_t* batches, uint64_t* rows);
+/* FarmerLstm model only. States s = 0..states-1 with history z[s] ([t,162], row-major [states,t,162]); candidate rows
+ * offsets[s] .. offsets[s+1]-1 of x ([rows,484], rows = offsets[states]) belong to state s. Runs the recurrence once per
+ * state and the dense stack once per candidate, on the newest published weights, combined with concurrent callers like
+ * fi_learner_infer. values[r] (may be NULL) = the value of candidate r, bit-identical to fi_learner_infer on a z repeated per
+ * candidate; best[s] (may be NULL, not both) = index WITHIN state s's group of its largest value, the lowest index on ties
+ * (NaN counts as largest, as in numpy's argmax).
+ * FI_ERR_ARG, with the learner still usable, for an actor-critic learner, a NULL z / x / offsets, values and best both NULL,
+ * states or t of 0, offsets[0] != 0, offsets not strictly increasing (every state needs a candidate), or more than 16384
+ * candidate rows. fi_learner_infer_stats counts the candidate rows.
+ *
+ * What a DouZero-style actor does with it: for each decision it sends the state's move history once as z and one x row per
+ * legal action (state and action features), and plays legal action best[s]; with many environments per actor thread it sends
+ * one state per environment in one call. This replaces repeating z once per legal action for fi_learner_infer and taking the
+ * argmax of the returned values on the host. Exploration (epsilon-greedy) stays with the actor: it needs no value. */
+FI_API int fi_learner_infer_grouped(fi_learner* l, int player, const float* z, size_t states, size_t t, const float* x,
+                                    const uint32_t* offsets /* states + 1 */, float* values, int32_t* best);
 
 /* ---- model store: Model / ModelManager (data_structures.h:43-157, 310-481) ---- */
 FI_API size_t fi_model_bytes(const fi_learner* l);                                  /* blob size, fixed */
