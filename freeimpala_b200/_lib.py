@@ -98,6 +98,7 @@ SIGNATURES = {
     "fi_learner_infer": (c_int, [_P, c_int, _P, _P, c_size_t, c_size_t, _P, _P]),
     "fi_learner_infer_stats": (c_int, [_P, c_int, C.POINTER(c_u64), C.POINTER(c_u64), C.POINTER(c_u64)]),
     "fi_learner_infer_grouped": (c_int, [_P, c_int, _P, c_size_t, c_size_t, _P, _P, _P, _P]),
+    "fi_learner_infer_sample": (c_int, [_P, c_int, _P, _P, c_size_t, c_u64, c_int, _P, _P, _P]),
     "fi_model_bytes": (c_size_t, [_P]),
     "fi_model_version": (c_u64, [_P, c_int]),
     "fi_model_get": (c_int, [_P, c_int, _P, c_size_t, C.POINTER(c_u64)]),
@@ -113,6 +114,7 @@ SIGNATURES = {
     "fi_op_vtrace": (c_int, [c_int, c_int] + [_P] * 5 + [c_float] * 4 + [_P, _P, _P]),
     "fi_op_vtrace_loss_head": (c_int, [_P, c_int, c_int, _P, c_int] + [c_float] * 6 + [_P] * 5),
     "fi_op_vtrace_loss_head_legal": (c_int, [_P, c_int, c_int, _P, c_int] + [c_float] * 6 + [_P] * 5),
+    "fi_op_policy_sample": (c_int, [_P, c_int, c_size_t, _P, c_u64, c_int, _P, _P]),
     "fi_op_adam": (c_int, [c_int, c_double, c_i64, c_size_t, _P, _P, _P, _P, c_float, _P]),
     "fi_op_grad_norm_clip": (c_int, [c_size_t, _P, c_double, _P, _P, _P]),
     "fi_op_rmsprop": (c_int, [c_double] * 4 + [c_size_t] + [_P] * 6),

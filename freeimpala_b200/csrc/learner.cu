@@ -873,10 +873,11 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
     const bool farmer = l->cfg.model == FI_MODEL_FARMER_LSTM;
     FI_CUDA_OK(cudaSetDevice(l->cfg.device));
     size_t states = 0;
-    bool want_best = false;
+    bool want_best = false, want_actions = false;
     for (const fi::InferReq* q : batch) {
         states += q->states;
         want_best |= q->best != nullptr;
+        want_actions |= q->actions != nullptr;
     }
     // the farmer model uploads z once per state, the actor-critic one observation per row
     const size_t row_in = farmer ? t * fi::kZDim : fi::kZDim;
@@ -891,7 +892,7 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
         const size_t scap = farmer ? grow(p->inf_states_cap, states) : 0;
         const size_t tcap = farmer ? (t > p->inf_t_cap ? t : p->inf_t_cap) : 0;
         const size_t cap_in = farmer ? scap * tcap * fi::kZDim : cap * fi::kZDim;
-        const size_t cap_out = farmer ? cap + scap : cap * fi::kHead;   // farmer: values, then best
+        const size_t cap_out = farmer ? cap + scap : cap * (fi::kHead + 1);   // farmer: values, then best; ac: head, then actions
         FI_CUDA_OK(cudaStreamSynchronize(p->infer_stream));
         if (p->inf_in) cudaFree(p->inf_in);
         if (p->inf_x) cudaFree(p->inf_x);
@@ -916,6 +917,8 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
             FI_CUDA_OK(cudaHostAlloc((void**)&p->inf_host_idx, cap_idx * sizeof(uint32_t), cudaHostAllocPortable));
             FI_TRY(fi::farmer_infer_alloc(l, p, scap, cap, tcap));
         } else {
+            FI_CUDA_OK(cudaMalloc((void**)&p->inf_idx, cap * sizeof(uint4)));
+            FI_CUDA_OK(cudaHostAlloc((void**)&p->inf_host_idx, cap * sizeof(uint4), cudaHostAllocPortable));
             FI_TRY(fi::ac_infer_alloc(l, p, cap));
         }
         p->inf_rows_cap = cap;
@@ -936,6 +939,13 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
                 for (size_t r = b; r < e; r++) row_state[r0 + r] = (uint32_t)(s0 + s);
             }
         }
+        if (want_actions) {   // actor-critic sampling descriptors; rows of plain requests get an empty support (action -1, dropped)
+            uint4* const desc = reinterpret_cast<uint4*>(p->inf_host_idx) + r0;
+            for (size_t r = 0; r < q->rows; r++) {
+                const uint32_t sup = q->actions ? (q->legal ? q->legal[r] & 0xFFFFu : 0xFFFFu) : 0u;
+                desc[r] = make_uint4(sup | ((uint32_t)q->greedy << 31), (uint32_t)r, (uint32_t)q->seed, (uint32_t)(q->seed >> 32));
+            }
+        }
         r0 += q->rows;
         s0 += q->states;
     }
@@ -945,7 +955,10 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
         FI_CUDA_OK(cudaMemcpyAsync(p->inf_x, p->inf_host_x, rows * fi::kXDim * sizeof(float), cudaMemcpyHostToDevice, st));
         FI_CUDA_OK(cudaMemcpyAsync(p->inf_idx, off, (states + 1 + rows) * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
     }
+    if (want_actions)
+        FI_CUDA_OK(cudaMemcpyAsync(p->inf_idx, p->inf_host_idx, rows * sizeof(uint4), cudaMemcpyHostToDevice, st));
     int32_t* const best_dev = want_best ? reinterpret_cast<int32_t*>(p->inf_out + rows) : nullptr;
+    int32_t* const actions_dev = reinterpret_cast<int32_t*>(p->inf_out + rows * fi::kHead);
     {
         ModelStore& s = p->store;
         std::lock_guard<std::mutex> g(s.mu);  // pins the newest snapshot against the learner's next write into it
@@ -956,13 +969,17 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
                                     p->inf_out, best_dev, st));
         else
             FI_TRY(fi::ac_infer(l, p, s.dev_snap[sn], p->inf_in, rows, p->inf_out, st));
+        if (want_actions)
+            FI_TRY(fi::launch_policy_sample(p->inf_out, fi::kHead, rows, reinterpret_cast<const uint4*>(p->inf_idx), nullptr, 0, 0,
+                                            actions_dev, st));
         FI_CUDA_OK(cudaEventRecord(s.infer_done[sn], st));
         s.infer_recorded[sn] = true;
     }
-    const size_t out_elems = farmer ? rows + (want_best ? states : 0) : rows * fi::kHead;
+    const size_t out_elems = farmer ? rows + (want_best ? states : 0) : rows * fi::kHead + (want_actions ? rows : 0);
     FI_CUDA_OK(cudaMemcpyAsync(p->inf_host_out, p->inf_out, out_elems * sizeof(float), cudaMemcpyDeviceToHost, st));
     FI_CUDA_OK(cudaStreamSynchronize(st));   // one synchronisation per BATCH: the callers need their rows on the host
     const int32_t* const best_host = reinterpret_cast<const int32_t*>(p->inf_host_out + rows);
+    const int32_t* const actions_host = reinterpret_cast<const int32_t*>(p->inf_host_out + rows * fi::kHead);
     r0 = s0 = 0;
     for (const fi::InferReq* q : batch) {
         if (farmer) {
@@ -974,6 +991,7 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
                 if (q->logits) memcpy(q->logits + r * fi::kNumActions, o, fi::kNumActions * sizeof(float));
                 if (q->values) q->values[r] = o[fi::kNumActions];
             }
+            if (q->actions) memcpy(q->actions, actions_host + r0, q->rows * sizeof(int32_t));
         }
         r0 += q->rows;
         s0 += q->states;
@@ -1048,6 +1066,23 @@ int fi_learner_infer_grouped(fi_learner* l, int player, const float* z, size_t s
     const size_t rows = offsets[states];
     if (rows > kInferMaxRows) return set_error(FI_ERR_ARG, "fi_learner_infer_grouped: %zu rows, at most %zu per call", rows, kInferMaxRows);
     fi::InferReq req{z, x, rows, t, states, offsets, nullptr, values, best, FI_OK, false};
+    return submit_infer(l, p, req);
+}
+
+int fi_learner_infer_sample(fi_learner* l, int player, const float* obs, const uint32_t* legal, size_t rows, uint64_t seed,
+                            int greedy, int32_t* actions, float* logits, float* values) {
+    Player* p = get_player(l, player);
+    if (!p) return set_error(FI_ERR_ARG, "fi_learner_infer_sample: no player %d", player);
+    if (l->cfg.model != FI_MODEL_MLP_ACTOR_CRITIC) return set_error(FI_ERR_ARG, "fi_learner_infer_sample: actor-critic model only");
+    if (!obs || !actions) return set_error(FI_ERR_ARG, "fi_learner_infer_sample: obs and actions are required");
+    if (rows == 0 || rows > kInferMaxRows)
+        return set_error(FI_ERR_ARG, "fi_learner_infer_sample: %zu rows, 1 to %zu per call", rows, kInferMaxRows);
+    if (greedy != 0 && greedy != 1) return set_error(FI_ERR_ARG, "fi_learner_infer_sample: greedy must be 0 or 1, got %d", greedy);
+    if (legal)
+        for (size_t r = 0; r < rows; r++)
+            if ((legal[r] & 0xFFFFu) == 0)
+                return set_error(FI_ERR_ARG, "fi_learner_infer_sample: row %zu has no legal action (word 0x%08x)", r, legal[r]);
+    fi::InferReq req{obs, nullptr, rows, 0, rows, nullptr, logits, values, nullptr, FI_OK, false, actions, legal, seed, greedy};
     return submit_infer(l, p, req);
 }
 

@@ -105,9 +105,10 @@ struct DenseStack {
 
 struct FarmerWs;   // model_farmer.cu
 
-// One caller of fi_learner_infer / fi_learner_infer_grouped waiting for its rows. A FarmerLstm request is `states` histories z
-// [states, t, 162] and `rows` candidate rows x [rows, 484], rows offsets[s] .. offsets[s+1]-1 belonging to state s; a plain
-// fi_learner_infer request is `rows` states of one candidate each (offsets null).
+// One caller of fi_learner_infer / fi_learner_infer_grouped / fi_learner_infer_sample waiting for its rows. A FarmerLstm
+// request is `states` histories z [states, t, 162] and `rows` candidate rows x [rows, 484], rows offsets[s] .. offsets[s+1]-1
+// belonging to state s; a plain fi_learner_infer request is `rows` states of one candidate each (offsets null). An
+// actor-critic request with `actions` set also has each row's action drawn on the device (fi_learner_infer_sample).
 struct InferReq {
     const float* obs;   // actor-critic: observations [rows, 162]; FarmerLstm: z
     const float* x;
@@ -118,6 +119,10 @@ struct InferReq {
     int32_t* best;             // FarmerLstm, may be null: [states], each state's argmax within its group
     int status;
     bool done;
+    int32_t* actions = nullptr;         // actor-critic sampling request: [rows]; null for every other request
+    const uint32_t* legal = nullptr;    // [rows] legal words, or null = all 16 legal
+    uint64_t seed = 0;
+    int greedy = 0;
 };
 
 struct Player {
@@ -159,7 +164,9 @@ struct Player {
     uint64_t infer_calls = 0, infer_batches = 0, infer_rows = 0;
     cudaStream_t infer_stream = nullptr;
     // FarmerLstm: inf_in holds z per state, inf_x the candidate rows, inf_idx the batch's offsets [states + 1] followed by the
-    // state of each candidate row [rows], inf_out the values [rows] followed by best [states] (int32)
+    // state of each candidate row [rows], inf_out the values [rows] followed by best [states] (int32).
+    // Actor-critic: inf_in holds the observations, inf_out the head rows [rows, 17] followed by the actions [rows] (int32) of
+    // a batch with a sampling request, inf_idx that batch's sampling descriptors [rows] x 4 words (policy_sample_kernel)
     float *inf_in = nullptr, *inf_x = nullptr, *inf_out = nullptr;
     uint32_t* inf_idx = nullptr;
     float *inf_host_in = nullptr, *inf_host_x = nullptr, *inf_host_out = nullptr;  // pinned
@@ -224,6 +231,11 @@ int ac_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int
 int ac_infer_alloc(fi_learner* l, Player* p, size_t rows);
 int ac_infer(fi_learner* l, Player* p, const float* params, const float* obs_dev, size_t rows, float* out_dev,
              cudaStream_t stream);
+// actions[r] drawn from head row r (columns 0..15, row stride ldh) over its legal set (the rule: fi_learner.h). desc (may be
+// null): per row {legal word | greedy << 31, RNG counter, seed low, seed high}; without it every row uses legal[r] (null = all
+// 16 legal), seed, greedy and counter r.
+int launch_policy_sample(const float* head, int ldh, size_t rows, const uint4* desc, const uint32_t* legal, uint64_t seed,
+                         int greedy, int32_t* actions, cudaStream_t stream);
 // model_farmer.cu
 int farmer_alloc(fi_learner* l, Player* p);
 void farmer_free(Player* p);

@@ -111,4 +111,110 @@ int ac_infer(fi_learner* l, Player* p, const float* params, const float* obs_dev
     return dense_forward_split(l, s, params, (int)rows, out_dev, stream);
 }
 
+// ---------------------------------------------------------------- policy sampling -----
+// The actor's action drawn from the softmax of a head row over its legal set (the rule is stated in fi_learner.h, at
+// fi_learner_infer_sample, and restated in float64 by tests/sampling_reference.py). One thread per row. The uniform comes from
+// Philox4x32-10 (Salmon et al., "Parallel random numbers: as easy as 1, 2, 3", SC 2011), counter (r, 0, 0, 0), key = the
+// seed: stateless, so a row's draw depends only on (seed, r) and a call can be replayed.
+__device__ __forceinline__ uint32_t philox4x32_10_word0(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1) {
+#pragma unroll
+    for (int round = 0; round < 10; round++) {
+        if (round) {
+            k0 += 0x9E3779B9u;
+            k1 += 0xBB67AE85u;
+        }
+        const uint32_t lo0 = 0xD2511F53u * c0, hi0 = __umulhi(0xD2511F53u, c0);
+        const uint32_t lo1 = 0xCD9E8D57u * c2, hi1 = __umulhi(0xCD9E8D57u, c2);
+        c0 = hi1 ^ c1 ^ k0;
+        c1 = lo1;
+        c2 = hi0 ^ c3 ^ k1;
+        c3 = lo0;
+    }
+    return c0;
+}
+
+// desc (learner path, may be null): per row {support | greedy << 31, row index within its call, seed low, seed high}.
+// Without desc (operator path) every row uses `legal` (null = all 16 legal), `seed`, `greedy` and its own row number.
+// Head rows are staged through shared memory: a row of 17 floats is not 16-byte aligned, and with ldh == 17 the block's rows
+// are one contiguous span, read with coalesced loads and read back one row per thread (odd stride: no bank conflict).
+constexpr int kSampleThreads = 128;
+__global__ void __launch_bounds__(kSampleThreads)
+policy_sample_kernel(const float* __restrict__ head, int ldh, size_t rows, const uint4* __restrict__ desc,
+                     const uint32_t* __restrict__ legal, uint32_t seed_lo, uint32_t seed_hi, int greedy_all,
+                     int32_t* __restrict__ actions) {
+    __shared__ float s_z[kSampleThreads * kNumActions];
+    const size_t r0 = (size_t)blockIdx.x * kSampleThreads;
+    const int n = (int)min((size_t)kSampleThreads, rows - r0);
+    for (int i = threadIdx.x; i < n * kNumActions; i += kSampleThreads)
+        s_z[i] = __ldg(head + (r0 + i / kNumActions) * ldh + i % kNumActions);
+    __syncthreads();
+    if ((int)threadIdx.x >= n) return;
+    const size_t row = r0 + threadIdx.x;
+    uint32_t sup, ctr, k0 = seed_lo, k1 = seed_hi;
+    bool greedy = greedy_all != 0;
+    if (desc) {
+        const uint4 d = __ldg(desc + row);
+        sup = d.x;
+        greedy = (d.x >> 31) != 0;
+        ctr = d.y;
+        k0 = d.z;
+        k1 = d.w;
+    } else {
+        sup = legal ? __ldg(legal + row) : 0xFFFFu;
+        ctr = (uint32_t)row;
+    }
+    sup &= 0xFFFFu;
+    const float* z = s_z + threadIdx.x * kNumActions;
+    // greedy action: the largest logit in the support, NaN counting as largest, the lowest index on ties (numpy's argmax)
+    int g = -1;
+    float zg = 0.f;
+#pragma unroll
+    for (int j = 0; j < kNumActions; j++) {
+        const float zj = z[j];
+        if (((sup >> j) & 1u) && (g < 0 || (!isnan(zg) && (isnan(zj) || zj > zg)))) {
+            g = j;
+            zg = zj;
+        }
+    }
+    int a = g;
+    if (g >= 0 && !greedy && isfinite(zg)) {
+        const uint32_t x0 = philox4x32_10_word0(ctr, 0u, 0u, 0u, k0, k1);
+        const float u = (float)(x0 >> 8) * 0x1p-24f;
+        float w[kNumActions], p[kNumActions], acc = 0.f;
+#pragma unroll
+        for (int j = 0; j < kNumActions; j++) {
+            w[j] = ((sup >> j) & 1u) ? expf(z[j] - zg) : 0.f;
+            acc += w[j];
+            p[j] = acc;
+        }
+        const float thr = u * acc;
+        int pick = -1, last = -1;
+#pragma unroll
+        for (int j = kNumActions - 1; j >= 0; j--) {   // the smallest j with P_j > u W (w_j = 0 outside the support)
+            if (p[j] > thr && w[j] > 0.f) pick = j;
+            if (last < 0 && w[j] > 0.f) last = j;
+        }
+        a = pick >= 0 ? pick : last;   // rounding left no P_j above u W: the largest j with a positive weight
+    }
+    actions[row] = a;
+}
+
+int launch_policy_sample(const float* head, int ldh, size_t rows, const uint4* desc, const uint32_t* legal, uint64_t seed,
+                         int greedy, int32_t* actions, cudaStream_t stream) {
+    if (ldh < kNumActions || (greedy != 0 && greedy != 1)) return set_error(FI_ERR_ARG, "policy sample: ldh >= 16 and greedy 0 or 1");
+    if (rows == 0) return FI_OK;
+    if (!head || !actions) return set_error(FI_ERR_ARG, "policy sample: null head or actions");
+    if (rows > 0xFFFFFFFFull) return set_error(FI_ERR_ARG, "policy sample: the row counter is 32 bits, %zu rows", rows);
+    // algorithmic traffic per row: 16 logits in, the legal word or the 16-byte descriptor in, the action out
+    LaunchScope ls("policy_sample_kernel", stream, (64.0 + (desc ? 16.0 : legal ? 4.0 : 0.0) + 4.0) * (double)rows, kWorkBytes);
+    policy_sample_kernel<<<(unsigned)((rows + kSampleThreads - 1) / kSampleThreads), kSampleThreads, 0, stream>>>(
+        head, ldh, rows, desc, legal, (uint32_t)seed, (uint32_t)(seed >> 32), greedy, actions);
+    return ls.done();
+}
+
 }  // namespace fi
+
+extern "C" int fi_op_policy_sample(const float* head, int ldh, size_t rows, const uint32_t* legal, uint64_t seed, int greedy,
+                                   int32_t* actions, void* stream) {
+    return fi::launch_policy_sample(head, ldh, rows, nullptr, legal, seed, greedy, actions, (cudaStream_t)stream);
+}

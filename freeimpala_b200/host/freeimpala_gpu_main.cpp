@@ -5,6 +5,10 @@
 // (agent.h:96) and then refresh their model copy when a newer version is published (agent.h:155-165).
 // BASELINE.json configs[2]: --players 2 --buffer-capacity 32 --batch-size 32 --agents 64.
 // Prints one JSON line: learner updates, updates/s, transitions/s (= updates * M * S / wall).
+// --sample-actions: on-policy records through the library's own inference. The learner masks illegal actions, and for each
+// trajectory an actor draws a random non-empty legal word per record, makes one fi_learner_infer_sample call on the S
+// observations, and stores the returned logits (words 162..177), action (178) and legal word (182). The JSON line then also
+// reports the rows sampled and how many returned actions fell outside their legal word (always 0).
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -21,6 +25,7 @@ struct Params {  // ProgramParams, cmd/freeimpala/main.cpp:18-35 (defaults :38-1
     std::string checkpoint_location = "", starting_model = "";
     unsigned seed = 0;
     int infer_every = 0;  // >0: every k-th iteration an actor asks for batched policy inference on its observations
+    bool sample_actions = false;
 };
 
 static bool parse(int argc, char** argv, Params& p) {
@@ -31,6 +36,7 @@ static bool parse(int argc, char** argv, Params& p) {
         {"-a", &p.agents}, {"--agents", &p.agents}, {"--game-steps", &p.game_steps}, {"--agent-time", &p.agent_time}};
     for (int i = 1; i < argc; i++) {
         std::string a = argv[i];
+        if (a == "--sample-actions") { p.sample_actions = true; continue; }
         if (i + 1 >= argc) return false;
         if (num.count(a)) *num[a] = strtoull(argv[++i], nullptr, 10);
         else if (a == "-l" || a == "--checkpoint-location") p.checkpoint_location = argv[++i];
@@ -46,7 +52,12 @@ static bool parse(int argc, char** argv, Params& p) {
     return true;
 }
 
-static void actor(size_t id, const Params& P, Learner& learner, std::atomic<uint64_t>& inferences) {
+struct SampleCounts {
+    std::atomic<uint64_t> rows{0}, illegal{0};
+    std::atomic<bool> failed{false};
+};
+
+static void actor(size_t id, const Params& P, Learner& learner, std::atomic<uint64_t>& inferences, SampleCounts& sampled) {
     auto buffers = learner.getSharedBuffers();
     auto models = learner.getModelManager();
     std::vector<uint64_t> versions(P.players, 0);
@@ -72,6 +83,30 @@ static void actor(size_t id, const Params& P, Learner& learner, std::atomic<uint
                 rec[180] = (next() % 100) ? 0.99f : 0.f;                 // discount = 0.99 (1 - done)
                 rec[181] = s + 1 == P.entry_size ? unif() : 0.f;         // bootstrap value in the last record
             }
+            if (P.sample_actions) {   // the policy's own logits and actions over a random legal set per record
+                std::vector<float> obs(P.entry_size * 162), logits(P.entry_size * 16);
+                std::vector<uint32_t> legal(P.entry_size);
+                std::vector<int32_t> acts(P.entry_size);
+                for (size_t s = 0; s < P.entry_size; s++) {
+                    memcpy(&obs[s * 162], &slot[s * 256], 162 * 4);
+                    do legal[s] = (uint32_t)(next() & 0xFFFF); while (legal[s] == 0);
+                }
+                const uint64_t seed = ((uint64_t)id << 40) ^ ((uint64_t)it << 8) ^ p;
+                if (fi_learner_infer_sample(learner.handle(), (int)p, obs.data(), legal.data(), P.entry_size, seed, 0, acts.data(),
+                                            logits.data(), nullptr) != FI_OK) {
+                    fprintf(stderr, "freeimpala_gpu: fi_learner_infer_sample: %s\n", fi_last_error());
+                    sampled.failed.store(true);
+                } else {
+                    sampled.rows.fetch_add(P.entry_size);
+                    for (size_t s = 0; s < P.entry_size; s++) {
+                        float* rec = slot.data() + s * 256;
+                        if (acts[s] < 0 || acts[s] >= 16 || !((legal[s] >> acts[s]) & 1u)) sampled.illegal.fetch_add(1);
+                        memcpy(rec + 162, &logits[s * 16], 16 * 4);
+                        memcpy(rec + 178, &acts[s], 4);
+                        memcpy(rec + FI_REC_WORD_LEGAL, &legal[s], 4);
+                    }
+                }
+            }
             if (P.infer_every && it % P.infer_every == 0) {              // batched actor policy inference
                 std::vector<float> obs(P.entry_size * 162), logits(P.entry_size * 16), values(P.entry_size);
                 for (size_t s = 0; s < P.entry_size; s++) memcpy(&obs[s * 162], &slot[s * 256], 162 * 4);
@@ -94,18 +129,20 @@ int main(int argc, char** argv) {
     Params P;
     if (!parse(argc, argv, P)) {
         fprintf(stderr, "usage: freeimpala_gpu [-p N] [-T N] [-S N] [-B N] [-M N] [-a N] [--game-steps N] [--agent-time ms] "
-                        "[-c N] [-l DIR] [-m DIR] [--seed N] [--infer-every K]\n");
+                        "[-c N] [-l DIR] [-m DIR] [--seed N] [--infer-every K] [--sample-actions]\n");
         return 2;
     }
     const size_t learner_iterations = (P.agents * P.iterations) / P.batch_size;  // main.cpp:179 (integer division)
     try {
         Learner learner(P.players, P.buffer_capacity, P.entry_size, P.batch_size, P.learner_time, P.checkpoint_freq,
-                        P.checkpoint_location, P.starting_model, learner_iterations);
+                        P.checkpoint_location, P.starting_model, learner_iterations, 0, FI_MODEL_MLP_ACTOR_CRITIC,
+                        P.sample_actions);
         const auto t0 = std::chrono::steady_clock::now();
         learner.start();
         std::atomic<uint64_t> inferences{0};
+        SampleCounts sampled;
         std::vector<std::thread> threads;
-        for (size_t a = 0; a < P.agents; a++) threads.emplace_back([&, a] { actor(a, P, learner, inferences); });
+        for (size_t a = 0; a < P.agents; a++) threads.emplace_back([&, a] { actor(a, P, learner, inferences, sampled); });
         for (auto& t : threads) t.join();
         // The reference stops the learner as soon as the agents have joined (main.cpp:239-246), which drops whatever
         // the workers have not consumed yet. Every trajectory needed for learner_iterations updates has been written
@@ -130,11 +167,16 @@ int main(int argc, char** argv) {
         printf("{\"harness\": \"freeimpala_gpu\", \"players\": %zu, \"agents\": %zu, \"batch_size\": %zu, \"entry_size\": %zu, "
                "\"learner_updates\": %zu, \"expected_updates\": %zu, \"seconds\": %.4f, \"updates_per_s\": %.2f, "
                "\"transitions_per_s\": %.1f, \"min_model_version\": %llu, \"actor_inference_rows\": %llu, "
-               "\"actor_inference_calls\": %llu, \"actor_inference_forwards\": %llu, \"kernel_launches\": %llu}\n",
+               "\"actor_inference_calls\": %llu, \"actor_inference_forwards\": %llu, \"kernel_launches\": %llu",
                P.players, P.agents, P.batch_size, P.entry_size, updates, learner_iterations * P.players, sec, updates / sec,
                updates * (double)P.batch_size * P.entry_size / sec, (unsigned long long)vmin,
                (unsigned long long)inferences.load(), (unsigned long long)inf_calls, (unsigned long long)inf_batches,
                (unsigned long long)fi_kernel_launch_count());
+        if (P.sample_actions)
+            printf(", \"actor_sampled_rows\": %llu, \"illegal_actions\": %llu", (unsigned long long)sampled.rows.load(),
+                   (unsigned long long)sampled.illegal.load());
+        printf("}\n");
+        if (sampled.failed.load() || sampled.illegal.load()) return 1;
         return updates == learner_iterations * P.players ? 0 : 1;
     } catch (const std::exception& e) {
         fprintf(stderr, "freeimpala_gpu: %s\n", e.what());

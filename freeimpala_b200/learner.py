@@ -322,6 +322,29 @@ class Learner:
               "fi_learner_infer_grouped")
         return values, best
 
+    def infer_sample(self, player_index: int, obs: np.ndarray, legal: np.ndarray | None = None, seed: int = 0,
+                     greedy: bool = False):
+        """Actor-critic inference with each row's action drawn on the device from the softmax of its logits over its legal
+        set (fi_learner_infer_sample: the rule, Philox4x32-10 at counter = row index, key = seed). obs [rows,162], legal
+        [rows] uint32 words (bit j = action j legal; None = all 16). Returns (actions [rows] int32, logits [rows,16],
+        values [rows])."""
+        a = np.ascontiguousarray(obs, dtype=np.float32)
+        rows = a.size // 162
+        if a.size != rows * 162 or rows == 0:
+            raise ValueError(f"infer_sample: obs {a.shape}: expected [rows,162]")
+        lg = None
+        if legal is not None:
+            lg = np.ascontiguousarray(legal, dtype=np.uint32)
+            if lg.shape != (rows,):
+                raise ValueError(f"infer_sample: legal {lg.shape}: expected [{rows}]")
+        actions = np.empty(rows, np.int32)
+        logits = np.empty((rows, 16), np.float32)
+        values = np.empty(rows, np.float32)
+        check(self._lib.fi_learner_infer_sample(self._h, player_index, a.ctypes.data, None if lg is None else lg.ctypes.data,
+                                                rows, seed, int(greedy), actions.ctypes.data, logits.ctypes.data,
+                                                values.ctypes.data), "fi_learner_infer_sample")
+        return actions, logits, values
+
     # ---- data parallelism (SURVEY.md 8e) ------------------------------------------------------------
     def infer_stats(self, player_index: int) -> dict:
         """Counters of the combining inference path: calls made, forwards run, rows served."""

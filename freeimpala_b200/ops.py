@@ -27,6 +27,12 @@ def vtrace_loss_head(batch: int, m: int, t: int, head: int, ldh: int, dhead: int
                                      baseline_cost, entropy_cost, dhead, vs, pg_adv, losses, stream), name)
 
 
+def policy_sample(head: int, ldh: int, rows: int, actions: int, legal: int = None, seed=0, greedy=False, stream=None) -> None:
+    """actions[r] (int32) drawn from head row r (columns 0..15 of [rows, ldh]) over legal[r] (uint32 words; None = all 16),
+    RNG counter r (fi_op_policy_sample); an empty support gives -1."""
+    check(_lib.load().fi_op_policy_sample(head, ldh, rows, legal, seed, int(greedy), actions, stream), "fi_op_policy_sample")
+
+
 def adam(kind: str, lr: float, step: int, n: int, p: int, g: int, m: int, v: int, grad_scale=1.0, stream=None) -> None:
     check(_lib.load().fi_op_adam(_lib.OPT[kind], lr, step, n, p, g, m, v, grad_scale, stream), "fi_op_adam")
 

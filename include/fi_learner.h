@@ -201,9 +201,10 @@ typedef struct fi_learner_config {
  * constants are unchanged. Logits outside the support (learner or behaviour) never enter the arithmetic: -inf or NaN
  * there changes nothing.
  *
- * What the actor does: fi_learner_infer returns the raw logits of all 16 actions. The actor samples from the
- * softmax of those logits over its legal set, stores the logits it got (raw or already set to -inf outside the legal set)
- * in words 162..177, the action in 178 and the legal word in 182. */
+ * What the actor does: it calls fi_learner_infer_sample with its observations and their legal words, which draws each
+ * action on the device from the softmax of the returned logits over the legal set, then stores the returned logits in
+ * words 162..177, the action in 178 and the legal word in 182. The learner's log mu(a) is then exactly the log-probability
+ * the action was drawn with. */
 #define FI_REC_WORD_LEGAL 182
 
 typedef struct fi_learner fi_learner;
@@ -297,6 +298,29 @@ FI_API int fi_learner_infer_stats(fi_learner* l, int player, uint64_t* calls, ui
  * argmax of the returned values on the host. Exploration (epsilon-greedy) stays with the actor: it needs no value. */
 FI_API int fi_learner_infer_grouped(fi_learner* l, int player, const float* z, size_t states, size_t t, const float* x,
                                     const uint32_t* offsets /* states + 1 */, float* values, int32_t* best);
+/* Actor-critic model only. Runs the same forward as fi_learner_infer on obs [rows,162] and, for every row r, draws
+ * actions[r] from the policy over that row's legal set. legal (may be NULL = all 16 legal) holds one word per row with
+ * the FI_REC_WORD_LEGAL meaning: bit j set = action j legal, bits 16..31 ignored. greedy = 1 takes the arg-max instead.
+ * logits [rows,16] and values [rows] may be NULL; they are the raw outputs the actor stores in words 162..177.
+ * Combined with concurrent fi_learner_infer / fi_learner_infer_sample callers into one forward; logits and values are the
+ * ones fi_learner_infer returns for the same batch.
+ *
+ * The sampling rule, for row r with S = legal[r] & 0xFFFF and z = its 16 logits:
+ *   greedy action g = the action in S with the largest z_j, NaN counting as largest, ties to the lowest index (numpy's
+ *     argmax over S; all -inf in S gives the lowest action in S). greedy = 1: a = g.
+ *   greedy = 0: if z_g is not finite (NaN or +inf in S, or all -inf), a = g. Otherwise, in fp32, w_j = expf(z_j - z_g) for
+ *     j in S (0 outside), prefix sums P_j in ascending j, W = P_15, u = (x0 >> 8) * 2^-24 with x0 word 0 of Philox4x32-10
+ *     (Random123) at counter (r, 0, 0, 0) and key (seed & 0xFFFFFFFF, seed >> 32); a = the smallest j in S with P_j > u W,
+ *     or, if rounding leaves none, the largest j in S with w_j > 0. An action of fp32 weight 0 is never drawn, and no action
+ *     outside S ever is.
+ *   r is the row's index within this call (0..rows-1), whatever other requests shared the forward: an action depends only
+ *   on the returned logits, the legal word, the seed and r. A reused seed reuses the uniforms, so an actor derives one per
+ *   call (e.g. from its id and step).
+ * FI_ERR_ARG, with the learner still usable, for a FarmerLstm learner, a NULL obs or actions, rows of 0 or more than 16384,
+ * greedy other than 0 or 1, or a legal word with no bit in 0..15 (checked on the host before the request is queued).
+ * fi_learner_infer_stats counts these calls and rows like any other inference. */
+FI_API int fi_learner_infer_sample(fi_learner* l, int player, const float* obs, const uint32_t* legal, size_t rows,
+                                   uint64_t seed, int greedy, int32_t* actions, float* logits, float* values);
 
 /* ---- model store: Model / ModelManager (data_structures.h:43-157, 310-481) ---- */
 FI_API size_t fi_model_bytes(const fi_learner* l);                                  /* blob size, fixed */
@@ -352,6 +376,13 @@ FI_API int fi_op_vtrace_loss_head(const void* batch, int m, int t, const float* 
 /* Same, with legal-action masking: the softmaxes, entropy and d(head) run over each record's legal word | the action's bit
  * (see FI_REC_WORD_LEGAL); d(head) is 0 in every column outside that support. */
 FI_API int fi_op_vtrace_loss_head_legal(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar, float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, float* dhead, float* vs, float* pg_adv, double* losses, void* stream);
+
+/* The sampling kernel of fi_learner_infer_sample on caller-owned device pointers. head [rows, ldh], ldh >= 16: only columns
+ * 0..15 are read. legal [rows] (may be NULL = all 16 legal), actions [rows] int32. Row r uses RNG counter r, the seed and
+ * greedy flag apply to every row; the rule is fi_learner_infer_sample's. A row whose support is empty gets action -1.
+ * ldh < 16 and greedy other than 0 or 1 are refused (FI_ERR_ARG) before the device is touched. */
+FI_API int fi_op_policy_sample(const float* head, int ldh, size_t rows, const uint32_t* legal, uint64_t seed, int greedy,
+                               int32_t* actions, void* stream);
 
 /* One fused optimiser update over n contiguous fp32 values (28 B/param for Adam).
  * step counts from 1; grad_scale multiplies g first (1/world for averaged gradients). */
