@@ -35,7 +35,8 @@ class FiLearnerConfig(C.Structure):
                 ("baseline_cost", c_float), ("entropy_cost", c_float),
                 ("gemm_mode", c_int), ("publish_every", c_int), ("checkpoint_location", c_char_p),
                 ("max_grad_norm", c_double), ("rmsprop_alpha", c_double), ("rmsprop_eps", c_double),
-                ("rmsprop_momentum", c_double), ("legal_action_mask", c_int)]
+                ("rmsprop_momentum", c_double), ("legal_action_mask", c_int),
+                ("variable_length", c_int)]
 
 
 class FiProfEntry(C.Structure):
@@ -114,6 +115,7 @@ SIGNATURES = {
     "fi_op_vtrace": (c_int, [c_int, c_int] + [_P] * 5 + [c_float] * 4 + [_P, _P, _P]),
     "fi_op_vtrace_loss_head": (c_int, [_P, c_int, c_int, _P, c_int] + [c_float] * 6 + [_P] * 5),
     "fi_op_vtrace_loss_head_legal": (c_int, [_P, c_int, c_int, _P, c_int] + [c_float] * 6 + [_P] * 5),
+    "fi_op_vtrace_loss_head_opts": (c_int, [_P, c_int, c_int, _P, c_int] + [c_float] * 6 + [c_int, c_int] + [_P] * 5),
     "fi_op_policy_sample": (c_int, [_P, c_int, c_size_t, _P, c_u64, c_int, _P, _P]),
     "fi_op_adam": (c_int, [c_int, c_double, c_i64, c_size_t, _P, _P, _P, _P, c_float, _P]),
     "fi_op_grad_norm_clip": (c_int, [c_size_t, _P, c_double, _P, _P, _P]),

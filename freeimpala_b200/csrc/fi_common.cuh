@@ -203,6 +203,9 @@ constexpr int kWReward = 179;
 constexpr int kWDiscount = 180;
 constexpr int kWAux = 181;
 constexpr int kWLegal = 182;   // uint32 legal-action word (bit j = action j legal); read only with legal_action_mask on
+constexpr int kWLength = 183;  // uint32 trajectory length, record 0 only; read only with variable_length on
+// L = (W == 0 || W > t) ? t : W for the length word W of a t-record trajectory (fi_learner.h, FI_REC_WORD_LENGTH)
+__host__ __device__ __forceinline__ int traj_length(uint32_t w, int t) { return (w == 0u || w > (uint32_t)t) ? t : (int)w; }
 constexpr int kWX = 192;
 constexpr int kXPerRec = 64;
 constexpr int kFarmerMinEntry = (kXDim + kXPerRec - 1) / kXPerRec;   // 8 records carry x: the shortest FarmerLstm trajectory

@@ -40,9 +40,10 @@ int launch_grad_norm_clip(size_t n, const float* g, double max_norm, double* nor
 int launch_vtrace_scan(int m, int t, const float* log_rho, const float* discount, const float* reward,
                        const float* value, const float* bootstrap, float rho_bar, float c_bar, float pg_rho_bar,
                        float lambda_, float* vs, float* pg_adv, cudaStream_t stream);
+// legal: legal-action masking (record word 182); lengths: each trajectory's length from word 183 of its record 0
 int launch_vtrace_loss_head(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar,
-                            float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, bool legal, float* dhead,
-                            float* vs, float* pg_adv, double* losses, cudaStream_t stream,
+                            float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, bool legal, bool lengths,
+                            float* dhead, float* vs, float* pg_adv, double* losses, cudaStream_t stream,
                             float* dhead_hi = nullptr, float* dhead_lo = nullptr, int ld_split = 0, struct HScale* dhead_hs = nullptr);
 
 // trans: 0 "NT" C = A[m,k] B[n,k]^T; 1 "NN" C = A[m,k] B[k,n]; 2 "TN" C = A[k,m]^T B[k,n].
@@ -139,14 +140,19 @@ __host__ __device__ __forceinline__ size_t step_block_offset(int s, int b, int c
 __host__ __device__ __forceinline__ size_t step_cell_offset(int s, int b, int unit, int nblk) {
     return step_block_index(s, b, unit, nblk) * kStepCellBlock + step_row_offset(b, unit);
 }
-int launch_split_tf32(const float* x, int ld_in, size_t rows, int cols, int ld_out, float* hi, float* lo, cudaStream_t st);
+// len_t > 0: x is a gathered batch of len_t-record trajectories (ld_in = 256 words) and the rows of records at or past their
+// trajectory's length (word 183 of its record 0, fi_learner.h) are split as zeros without being read
+int launch_split_tf32(const float* x, int ld_in, size_t rows, int cols, int ld_out, float* hi, float* lo, cudaStream_t st,
+                      int len_t = 0);
 // fp16 format pre-passes: amax accumulates max |x| into hs->amax; split derives the scale from hs->amax (which must
 // bound the matrix) and writes hi / lo' with columns [cols, ld_out) zero-filled. write_scale: publish scale/inv in *hs.
 int launch_amax(const float* x, int ld_in, size_t rows, int cols, HScale* hs, cudaStream_t st);
 int launch_split_h(const float* x, int ld_in, size_t rows, int cols, int ld_out, void* hi, void* lo, HScale* hs, int write_scale,
                    cudaStream_t st);
-// amax + split in one cooperative launch (row matrices; hs->amax must be zero on entry; publishes scale / inv / bound)
-int launch_amax_split_h(const float* x, int ld_in, size_t rows, int cols, int ld_out, void* hi, void* lo, HScale* hs, cudaStream_t st);
+// amax + split in one cooperative launch (row matrices; hs->amax must be zero on entry; publishes scale / inv / bound).
+// len_t > 0: as launch_split_tf32, padding rows are left out of the max and split as zeros (always the cooperative launch)
+int launch_amax_split_h(const float* x, int ld_in, size_t rows, int cols, int ld_out, void* hi, void* lo, HScale* hs, cudaStream_t st,
+                        int len_t = 0);
 // lstm_tc.cu: the FarmerLstm recurrence on tcgen05 (clusters of 8 CTAs per 128 batch rows, exchange through DSMEM)
 bool lstm_tc_enabled();   // FI_LSTM_TC=0 keeps the fp32 FFMA kernels of model_farmer.cu
 int launch_lstm_forward_tc(float* gates, const float* whh, const float* b_hh, int m, int t, void* hp_hi, void* hp_lo, HScale* hp_hs,

@@ -822,16 +822,27 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_consta
     }
 }
 
+// Length-aware pre-passes (kLength, fi_learner_config.variable_length): x is a gathered batch of len_t-record trajectories
+// and row r is record r % len_t of its trajectory; it is a valid step when that index is below the length in word 183 of the
+// trajectory's record 0 (rows < 2^32, checked by the launchers). Padding rows are never read: they count as zero rows.
+__device__ __forceinline__ bool row_in_length(const float* x, int ld_in, size_t r, int len_t) {
+    const uint32_t rr = (uint32_t)r, s = rr % (uint32_t)len_t;
+    return (int)s < traj_length(__ldg(reinterpret_cast<const uint32_t*>(x + (size_t)(rr - s) * ld_in) + kWLength), len_t);
+}
+
 // fp32 -> (hi, lo) split of a [rows, cols] matrix (row stride ld_in) into two dense [rows, ld_out] arrays;
 // columns [cols, ld_out) are zero-filled. Algorithmic traffic 12 B per element.
+template <bool kLength>
 __global__ void split_tf32_kernel(const float* __restrict__ x, int ld_in, size_t rows, int cols, int ld_out,
-                                  float* __restrict__ hi, float* __restrict__ lo) {
+                                  float* __restrict__ hi, float* __restrict__ lo, int len_t) {
     const size_t total = rows * (size_t)ld_out;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         const size_t r = i / ld_out;
         const int c = (int)(i - r * ld_out);
         float v = 0.f;
-        if (c < cols) v = __ldg(x + r * ld_in + c);
+        bool in = c < cols;
+        if constexpr (kLength) in = in && row_in_length(x, ld_in, r, len_t);
+        if (in) v = __ldg(x + r * ld_in + c);
         const float h = __uint_as_float(__float_as_uint(v) & 0xFFFFE000u);
         hi[i] = h;
         lo[i] = v - h;
@@ -844,13 +855,24 @@ static bool coop_prepass() {
     return on;
 }
 
-int launch_split_tf32(const float* x, int ld_in, size_t rows, int cols, int ld_out, float* hi, float* lo, cudaStream_t st) {
+static int check_len_t(int len_t, int ld_in, size_t rows, const char* what) {
+    if (len_t < 0 || (len_t > 0 && (ld_in < kWLength + 1 || rows > 0xFFFFFFFFull)))
+        return set_error(FI_ERR_ARG, "%s: a length-aware split needs record rows (ld_in > %d) and rows < 2^32", what, kWLength);
+    return FI_OK;
+}
+
+int launch_split_tf32(const float* x, int ld_in, size_t rows, int cols, int ld_out, float* hi, float* lo, cudaStream_t st,
+                      int len_t) {
     if (rows == 0 || ld_out == 0) return FI_OK;
+    FI_TRY(check_len_t(len_t, ld_in, rows, "split_tf32"));
     const size_t total = rows * (size_t)ld_out;
     size_t blocks = (total + 255) / 256;
     if (blocks > (size_t)kNumSMs * 16) blocks = (size_t)kNumSMs * 16;
-    LaunchScope ls("split_tf32_kernel", st, 4.0 * (double)rows * cols + 8.0 * (double)total, kWorkBytes);
-    split_tf32_kernel<<<(unsigned)blocks, 256, 0, st>>>(x, ld_in, rows, cols, ld_out, hi, lo);
+    // the length-aware split also reads each row's length word (4 B per row)
+    LaunchScope ls(len_t ? "split_tf32_kernel_length" : "split_tf32_kernel", st,
+                   4.0 * (double)rows * cols + 8.0 * (double)total + (len_t ? 4.0 * (double)rows : 0.0), kWorkBytes);
+    (len_t ? split_tf32_kernel<true> : split_tf32_kernel<false>)<<<(unsigned)blocks, 256, 0, st>>>(x, ld_in, rows, cols, ld_out, hi,
+                                                                                                 lo, len_t);
     return ls.done();
 }
 
@@ -942,10 +964,11 @@ int launch_split_h(const float* x, int ld_in, size_t rows, int cols, int ld_out,
 // max |x| AND the fp16 (hi, lo') split of a [rows, cols] matrix in ONE cooperative launch: every warp takes the maximum over its
 // rows, the grid synchronises, every warp splits the same rows again (they come out of L2 the second time). Replaces an amax
 // launch + a split launch on the step's critical path (observations: 25 + 30 us as two launches that read 66 MB from HBM twice;
-// the head gradient: 13 + 14 us). hs->amax must be zero on entry.
+// the head gradient: 13 + 14 us). hs->amax must be zero on entry. kLength: padding rows (row_in_length) are zero rows.
+template <bool kLength>
 __global__ void __launch_bounds__(256)
 amax_split_h_kernel(const float* __restrict__ x, int ld_in, size_t rows, int cols, int ld_out, __half2* __restrict__ hi,
-                    __half2* __restrict__ lo, HScale* hs) {
+                    __half2* __restrict__ lo, HScale* hs, int len_t) {
     const size_t warp = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = ((size_t)gridDim.x * blockDim.x) >> 5;
     const int lane = threadIdx.x & 31;
     // Four rows per warp and trip, 8-byte loads where the layout allows: one row at a time with scalar loads left the pass
@@ -953,13 +976,25 @@ amax_split_h_kernel(const float* __restrict__ x, int ld_in, size_t rows, int col
     const bool vec2 = (ld_in & 1) == 0 && (cols & 1) == 0 && (reinterpret_cast<uintptr_t>(x) & 7) == 0;
     constexpr int kRowsPerTrip = 4;
     float m = 0.f;
+    bool ok[kRowsPerTrip];   // kLength: row r0 + j exists and is a valid step
+    auto live = [&](size_t r0, int j) {
+        if constexpr (kLength) return ok[j];
+        else return r0 + j < rows;
+    };
+    auto set_live = [&](size_t r0) {
+        if constexpr (kLength) {
+#pragma unroll
+            for (int j = 0; j < kRowsPerTrip; j++) ok[j] = r0 + j < rows && row_in_length(x, ld_in, r0 + j, len_t);
+        }
+    };
     for (size_t r0 = warp * kRowsPerTrip; r0 < rows; r0 += nwarps * kRowsPerTrip) {
+        set_live(r0);
         if (vec2) {
             for (int c = 2 * lane; c < cols; c += 64) {
                 float2 v[kRowsPerTrip];
 #pragma unroll
                 for (int j = 0; j < kRowsPerTrip; j++)
-                    v[j] = r0 + j < rows ? __ldg(reinterpret_cast<const float2*>(x + (r0 + j) * ld_in + c)) : make_float2(0.f, 0.f);
+                    v[j] = live(r0, j) ? __ldg(reinterpret_cast<const float2*>(x + (r0 + j) * ld_in + c)) : make_float2(0.f, 0.f);
 #pragma unroll
                 for (int j = 0; j < kRowsPerTrip; j++) m = fmaxf(m, fmaxf(fabsf(v[j].x), fabsf(v[j].y)));
             }
@@ -967,7 +1002,7 @@ amax_split_h_kernel(const float* __restrict__ x, int ld_in, size_t rows, int col
             for (int c = lane; c < cols; c += 32) {
                 float v[kRowsPerTrip];
 #pragma unroll
-                for (int j = 0; j < kRowsPerTrip; j++) v[j] = r0 + j < rows ? __ldg(x + (r0 + j) * ld_in + c) : 0.f;
+                for (int j = 0; j < kRowsPerTrip; j++) v[j] = live(r0, j) ? __ldg(x + (r0 + j) * ld_in + c) : 0.f;
 #pragma unroll
                 for (int j = 0; j < kRowsPerTrip; j++) m = fmaxf(m, fabsf(v[j]));
             }
@@ -985,13 +1020,14 @@ amax_split_h_kernel(const float* __restrict__ x, int ld_in, size_t rows, int col
     }
     const int ldp = ld_out >> 1;
     for (size_t r0 = warp * kRowsPerTrip; r0 < rows; r0 += nwarps * kRowsPerTrip) {
+        set_live(r0);
         for (int p = lane; p < ldp; p += 32) {
             const int c = 2 * p;
             float2 v[kRowsPerTrip];
 #pragma unroll
             for (int j = 0; j < kRowsPerTrip; j++) {
                 v[j] = make_float2(0.f, 0.f);
-                if (r0 + j < rows) {
+                if (live(r0, j)) {
                     const float* xr = x + (r0 + j) * ld_in;
                     if (vec2) {
                         if (c < cols) v[j] = __ldg(reinterpret_cast<const float2*>(xr + c));
@@ -1013,8 +1049,10 @@ amax_split_h_kernel(const float* __restrict__ x, int ld_in, size_t rows, int col
     }
 }
 
-int launch_amax_split_h(const float* x, int ld_in, size_t rows, int cols, int ld_out, void* hi, void* lo, HScale* hs, cudaStream_t st) {
-    if (!coop_prepass()) {   // FI_COOP=0: two ordinary launches
+int launch_amax_split_h(const float* x, int ld_in, size_t rows, int cols, int ld_out, void* hi, void* lo, HScale* hs, cudaStream_t st,
+                        int len_t) {
+    FI_TRY(check_len_t(len_t, ld_in, rows, "amax_split_h"));
+    if (!coop_prepass() && !len_t) {   // FI_COOP=0: two ordinary launches
         FI_TRY(launch_amax(x, ld_in, rows, cols, hs, st));
         return launch_split_h(x, ld_in, rows, cols, ld_out, hi, lo, hs, 1, st);
     }
@@ -1022,27 +1060,32 @@ int launch_amax_split_h(const float* x, int ld_in, size_t rows, int cols, int ld
     if (ld_out & 1) return set_error(FI_ERR_ARG, "split_h: ld_out must be even");
     // every block must be resident for the grid barrier: as many blocks as fit (queried once per device), capped by the work
     static std::mutex mu;
-    static int blocks_per_sm[64] = {};
+    static int blocks_per_sm[2][64] = {};
+    const void* kernel = len_t ? (const void*)amax_split_h_kernel<true> : (const void*)amax_split_h_kernel<false>;
     int dev = 0;
     cudaGetDevice(&dev);
     int bps;
     {
         std::lock_guard<std::mutex> g(mu);
-        if (!blocks_per_sm[dev & 63]) {
+        int& cached = blocks_per_sm[len_t ? 1 : 0][dev & 63];
+        if (!cached) {
             int n = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, amax_split_h_kernel, 256, 0) != cudaSuccess || n < 1) n = 1;
-            blocks_per_sm[dev & 63] = n > 4 ? 4 : n;
+            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kernel, 256, 0) != cudaSuccess || n < 1) n = 1;
+            cached = n > 4 ? 4 : n;
         }
-        bps = blocks_per_sm[dev & 63];
+        bps = cached;
     }
     size_t blocks = (rows + 31) / 32;   // 8 warps x 4 rows per trip
     if (blocks < 1) blocks = 1;
     if (blocks > (size_t)kNumSMs * bps) blocks = (size_t)kNumSMs * bps;
     __half2* hi2 = static_cast<__half2*>(hi);
     __half2* lo2 = static_cast<__half2*>(lo);
-    void* args[] = {(void*)&x, (void*)&ld_in, (void*)&rows, (void*)&cols, (void*)&ld_out, (void*)&hi2, (void*)&lo2, (void*)&hs};
-    LaunchScope ls("amax_split_h_kernel", st, 8.0 * (double)rows * cols + 4.0 * (double)rows * ld_out, kWorkBytes);
-    const cudaError_t e = cudaLaunchCooperativeKernel((const void*)amax_split_h_kernel, dim3((unsigned)blocks), dim3(256), args, 0, st);
+    void* args[] = {(void*)&x, (void*)&ld_in, (void*)&rows, (void*)&cols, (void*)&ld_out, (void*)&hi2, (void*)&lo2, (void*)&hs,
+                    (void*)&len_t};
+    // the length-aware pass also reads each row's length word, once per pass (8 B per row)
+    LaunchScope ls(len_t ? "amax_split_h_kernel_length" : "amax_split_h_kernel", st,
+                   8.0 * (double)rows * cols + 4.0 * (double)rows * ld_out + (len_t ? 8.0 * (double)rows : 0.0), kWorkBytes);
+    const cudaError_t e = cudaLaunchCooperativeKernel(kernel, dim3((unsigned)blocks), dim3(256), args, 0, st);
     if (e != cudaSuccess) return set_error(FI_ERR_CUDA, "cooperative launch of amax_split_h_kernel failed: %s", cudaGetErrorString(e));
     return ls.done();
 }

@@ -215,7 +215,7 @@ void free_player(fi_learner* l, Player* p) {
     if (l->cfg.model == FI_MODEL_FARMER_LSTM) fi::farmer_free(p);
     fi::dense_free(&p->dense);
     fi::dense_free(&p->inf_dense);
-    float* dev[] = {p->params, p->grads, p->adam_m, p->adam_v, p->head, p->dhead, p->inf_in, p->inf_x, p->inf_out};
+    float* dev[] = {p->params, p->grads, p->adam_m, p->adam_v, p->head, p->dhead, p->obs, p->inf_in, p->inf_x, p->inf_out};
     for (float* d : dev)
         if (d) cudaFree(d);
     for (float* d : p->store.dev_snap)
@@ -348,6 +348,7 @@ void fi_learner_config_default(fi_learner_config* c) {
     c->rmsprop_eps = 1e-8;
     c->rmsprop_momentum = 0.0;
     c->legal_action_mask = 0;    // every action legal; record word 182 is not read
+    c->variable_length = 0;      // every trajectory entry_size records long; record word 183 is not read
 }
 
 fi_learner* fi_learner_create(const fi_learner_config* cfg) {
@@ -382,6 +383,14 @@ fi_learner* fi_learner_create(const fi_learner_config* cfg) {
     }
     if (farmer && cfg->legal_action_mask) {
         set_error(FI_ERR_ARG, "fi_learner_create: legal_action_mask needs a policy; the FarmerLstm model has none");
+        return nullptr;
+    }
+    if (cfg->variable_length != 0 && cfg->variable_length != 1) {
+        set_error(FI_ERR_ARG, "fi_learner_create: variable_length must be 0 or 1, got %d", cfg->variable_length);
+        return nullptr;
+    }
+    if (farmer && cfg->variable_length) {
+        set_error(FI_ERR_ARG, "fi_learner_create: variable_length is for the actor-critic model, not the FarmerLstm model");
         return nullptr;
     }
     if (!farmer) {   // V-trace constants: a NaN or out-of-range value would otherwise surface as NaN or meaningless losses

@@ -149,6 +149,7 @@ struct Player {
     // step workspaces (sized for the step's rows: batch_size x entry_size for the actor-critic, batch_size for FarmerLstm)
     DenseStack dense;               // the step's dense stack
     float *head = nullptr, *dhead = nullptr;   // actor-critic: head output [rows, 17] and the loss head's fp32 gradient of it
+    float* obs = nullptr;       // actor-critic, simt path with variable_length: the observations [rows, 164], padding rows zero
     void* gemm_ws = nullptr; size_t gemm_ws_bytes = 0;       // actor-critic FFMA path
     void* colsum_ws = nullptr; size_t colsum_ws_bytes = 0;   // actor-critic
     FarmerWs* farmer_ws = nullptr;      // FarmerLstm training workspaces

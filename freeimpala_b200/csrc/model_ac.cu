@@ -8,7 +8,12 @@
 //    3xTF32 for gemm_mode tcgen05 (and auto with FI_AC_FORMAT=tf32). The observations are split out of the gathered batch
 //    (row stride 256 words) by a pre-pass here.
 //  * plain fp32 (gemm_mode simt): FFMA GEMMs (gemm_simt.cu); the first GEMM reads the observations straight out of the
-//    gathered batch.
+//    gathered batch, or, with variable_length, out of a copy whose padding rows are zero (obs_length_kernel).
+// variable_length: every observation pre-pass writes the rows past a trajectory's length (fi_learner.h, FI_REC_WORD_LENGTH)
+// as zero rows without reading them, and the loss head gives them zero d(head) rows. The padding rows still run through the
+// trunk and the head (fixed shapes: one captured graph), on zero inputs, so every later activation and gradient scale stays
+// finite and independent of them (the scales are bounded from the input and weight maxima, gemm_tc.cu), and they add exact
+// zeros to every weight and bias gradient.
 #include "learner.cuh"
 
 namespace fi {
@@ -16,6 +21,28 @@ namespace fi {
 constexpr int kObsLd = 164;     // 162 observation words padded to a 16-byte multiple (TMA row stride), 3xTF32 format
 
 static bool use_tc(const fi_learner* l) { return l->cfg.gemm_mode != FI_GEMM_SIMT && gemm_tc_available(); }
+
+// out [rows, kObsLd] = the observations (words 0..161) of a gathered batch of t-record trajectories; rows past their
+// trajectory's length, and columns 162..163, are zero. One warp per row: the length word is one broadcast load per row.
+__global__ void obs_length_kernel(const float* __restrict__ batch, int rows, int t, float* __restrict__ out) {
+    const int warp = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), nwarps = (int)((gridDim.x * blockDim.x) >> 5);
+    const int lane = threadIdx.x & 31;
+    for (int r = warp; r < rows; r += nwarps) {
+        const int s = r % t;
+        const float* rec = batch + (size_t)r * kRecWords;
+        const bool in = s < traj_length(__ldg(reinterpret_cast<const uint32_t*>(rec - (size_t)s * kRecWords) + kWLength), t);
+        for (int c = lane; c < kObsLd; c += 32) out[(size_t)r * kObsLd + c] = in && c < kZDim ? __ldg(rec + c) : 0.f;
+    }
+}
+
+static int launch_obs_length(const float* batch, int rows, int t, float* out, cudaStream_t st) {
+    int blocks = (rows + 7) / 8;
+    if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
+    // algorithmic traffic per row: 162 words in, 164 out, the length word
+    LaunchScope ls("obs_length_kernel", st, (4.0 * (kZDim + kObsLd) + 4.0) * rows, kWorkBytes);
+    obs_length_kernel<<<blocks, 256, 0, st>>>(batch, rows, t, out);
+    return ls.done();
+}
 
 int ac_alloc(fi_learner* l, Player* p) {
     const size_t rows = l->cfg.batch_size * l->cfg.entry_size;
@@ -37,6 +64,7 @@ int ac_alloc(fi_learner* l, Player* p) {
     }
     FI_TRY(dense_alloc(&p->dense, DenseShape{kZDim, 0, kHead, 0}, rows, l->arena_elems, kDenseNone, false, kDenseTrain));
     FI_CUDA_OK(cudaMalloc((void**)&p->dhead, rows * kHead * sizeof(float)));
+    if (l->cfg.variable_length) FI_CUDA_OK(cudaMalloc((void**)&p->obs, rows * kObsLd * sizeof(float)));
     p->gemm_ws_bytes = gemm_simt_workspace_bytes(2, kHid, kHid, (int)rows);
     if (p->gemm_ws_bytes) FI_CUDA_OK(cudaMalloc(&p->gemm_ws, p->gemm_ws_bytes));
     return FI_OK;
@@ -47,13 +75,20 @@ int ac_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int
     DenseStack* s = &p->dense;
     const int rows = m * t;
     cudaStream_t st = p->stream;
+    const bool legal = c.legal_action_mask != 0, lengths = c.variable_length != 0;
     if (!s->split) {
-        FI_TRY(dense_forward_plain(l, s, FI_GEMM_SIMT, p->params, batch, kRecWords, rows, p->head, p->gemm_ws, p->gemm_ws_bytes, st));
+        const float* x = batch;   // the first GEMM's input: the batch itself (row stride 256 words) or its length-aware copy
+        int ldx = kRecWords;
+        if (lengths) {
+            FI_TRY(launch_obs_length(batch, rows, t, p->obs, st));
+            x = p->obs;
+            ldx = kObsLd;
+        }
+        FI_TRY(dense_forward_plain(l, s, FI_GEMM_SIMT, p->params, x, ldx, rows, p->head, p->gemm_ws, p->gemm_ws_bytes, st));
         FI_TRY(launch_zero2(p->d_losses, 4 * sizeof(double), nullptr, 0, st));
         FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
-                                       c.baseline_cost, c.entropy_cost, c.legal_action_mask != 0, p->dhead, nullptr, nullptr,
-                                       p->d_losses, st));
-        return dense_backward_plain(l, s, FI_GEMM_SIMT, p->params, batch, kRecWords, p->dhead, rows, p->grads, nullptr, p->gemm_ws,
+                                       c.baseline_cost, c.entropy_cost, legal, lengths, p->dhead, nullptr, nullptr, p->d_losses, st));
+        return dense_backward_plain(l, s, FI_GEMM_SIMT, p->params, x, ldx, p->dhead, rows, p->grads, nullptr, p->gemm_ws,
                                     p->gemm_ws_bytes, p->colsum_ws, p->colsum_ws_bytes, st);
     }
     // pre-passes: weights (4.6 MB) and observations -> hi/lo pairs
@@ -63,22 +98,24 @@ int ac_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int
         FI_TRY(launch_zero2(s->hs, kHsCount * sizeof(HScale), p->d_losses, 4 * sizeof(double), st));
         FI_TRY(dense_split_params(l, s, p->params, st));
         // observations: max |x| and the split in one cooperative launch (the second pass reads the batch out of L2)
-        FI_TRY(launch_amax_split_h(batch, kRecWords, (size_t)rows, kZDim, kObsLdH, s->in_hi, s->in_lo, s->hs + kHsIn, st));
+        FI_TRY(launch_amax_split_h(batch, kRecWords, (size_t)rows, kZDim, kObsLdH, s->in_hi, s->in_lo, s->hs + kHsIn, st,
+                                   lengths ? t : 0));
     } else {
         FI_TRY(dense_split_params(l, s, p->params, st));
-        FI_TRY(launch_split_tf32(batch, kRecWords, (size_t)rows, kZDim, kObsLd, (float*)s->in_hi, (float*)s->in_lo, st));
+        FI_TRY(launch_split_tf32(batch, kRecWords, (size_t)rows, kZDim, kObsLd, (float*)s->in_hi, (float*)s->in_lo, st,
+                                 lengths ? t : 0));
     }
     FI_TRY(dense_forward_split(l, s, p->params, rows, p->head, st));
     if (s->half) {  // the loss head writes plain fp32 rows and their max |x|; the fp16 split follows (13 MB)
         FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
-                                       c.baseline_cost, c.entropy_cost, c.legal_action_mask != 0, p->dhead, nullptr, nullptr,
-                                       p->d_losses, st, nullptr, nullptr, 0, s->hs + kHsDout));
+                                       c.baseline_cost, c.entropy_cost, legal, lengths, p->dhead, nullptr, nullptr, p->d_losses, st,
+                                       nullptr, nullptr, 0, s->hs + kHsDout));
         FI_TRY(launch_split_h(p->dhead, kHead, (size_t)rows, kHead, kDoutLd, s->dout_hi, s->dout_lo, s->hs + kHsDout, 1, st));
     } else {
         FI_TRY(launch_zero2(p->d_losses, 4 * sizeof(double), nullptr, 0, st));
         FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
-                                       c.baseline_cost, c.entropy_cost, c.legal_action_mask != 0, nullptr, nullptr, nullptr,
-                                       p->d_losses, st, (float*)s->dout_hi, (float*)s->dout_lo, kDoutLd));
+                                       c.baseline_cost, c.entropy_cost, legal, lengths, nullptr, nullptr, nullptr, p->d_losses, st,
+                                       (float*)s->dout_hi, (float*)s->dout_lo, kDoutLd));
     }
     return dense_backward_split(l, s, p->dhead, rows, p->grads, nullptr, 0, p->colsum_ws, p->colsum_ws_bytes, st);
 }

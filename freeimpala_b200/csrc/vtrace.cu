@@ -195,8 +195,14 @@ int launch_vtrace_scan(int m, int t, const float* log_rho, const float* discount
 // use (-inf into fmaxf and expf, 0 as log pi), so logits there (-inf or NaN included) never reach the arithmetic, p = 0
 // and d(head) is exactly 0; the replacements are selects, not branches. The word sits in the record fields already
 // loaded, so the masked head reads no extra bytes.
+// kLength (fi_learner_config.variable_length): the warp reads the trajectory's length L from word 183 of record 0 (one 4-byte
+// load) and the step is that of the trajectory cut to its first L records: the bootstrap is word 181 of record L - 1, the scan
+// starts there, and the lanes at s >= L contribute a = b = 0 and no loss, leave dmax alone and store zero d(head), vs and
+// pg_adv rows (the buffers are reused across steps, so those rows are written). Lanes past L read the head row and the record
+// of step L - 1, as the lanes past t read those of step t - 1, and their d(head) row is replaced by a select: no byte of a
+// padding record or head row reaches the arithmetic. A chunk wholly past L only stores its zero rows.
 constexpr int kLossWarps = 4;
-template <bool kLegal>
+template <bool kLegal, bool kLength>
 __global__ void __launch_bounds__(32 * kLossWarps)
 vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const float* __restrict__ head, int ldh,
                         float rho_bar, float c_bar, float pg_rho_bar, float lambda_, float baseline_cost,
@@ -213,18 +219,41 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
     float* o_a = s_out[wib][0];   // plain / hi tile, [32][33]
     float* o_b = s_out[wib][1];   // lo tile
     const float* slot = batch + (size_t)traj * t * kRecWords;
-    const float boot = __ldg(slot + (size_t)(t - 1) * kRecWords + kWAux);
+    int tl = t;   // valid records of this trajectory
+    if constexpr (kLength) tl = traj_length(__ldg(reinterpret_cast<const uint32_t*>(slot) + kWLength), t);
+    const float boot = __ldg(slot + (size_t)(tl - 1) * kRecWords + kWAux);
     float carry = 0.f, vs_next_chunk = boot, v_next_chunk = boot;
     double l_pg = 0.0, l_bl = 0.0, l_ent = 0.0;
     float dmax = 0.f;
     for (int c0 = ((t - 1) >> 5) << 5; c0 >= 0; c0 -= 32) {
         const int s = c0 + lane;
-        const bool valid = s < t;
-        const size_t row = (size_t)traj * t + (valid ? s : t - 1);
-        const float* rec = slot + (size_t)(valid ? s : t - 1) * kRecWords;
-        // stage the chunk's head rows: rows base_row .. base_row + nvalid - 1
-        const int nvalid = min(32, t - c0);
+        // rows base_row .. base_row + nrows - 1 get d(head) rows; the first nvalid of them are valid steps
+        const int nrows = min(32, t - c0);
         const size_t base_row = (size_t)traj * t + c0;
+        if constexpr (kLength) {
+            if (c0 >= tl) {   // every step of the chunk is padding: zero rows out, nothing read
+                if (lane < nrows) {
+                    if (vs_out) vs_out[base_row + lane] = 0.f;
+                    if (adv_out) adv_out[base_row + lane] = 0.f;
+                }
+                if (dhead)
+                    for (int i = lane; i < nrows * kHead; i += 32) dhead[(base_row + i / kHead) * ldh + i % kHead] = 0.f;
+                if (dhead_hi) {   // as the stores below: all 32 columns of a 32-float row, else the 17 head columns
+                    const int w = ld_split == 32 ? 32 : kHead;
+                    for (int i = lane; i < nrows * w; i += 32) {
+                        const size_t o = (base_row + i / w) * ld_split + i % w;
+                        dhead_hi[o] = 0.f;
+                        dhead_lo[o] = 0.f;
+                    }
+                }
+                continue;
+            }
+        }
+        const bool valid = s < tl;
+        const size_t row = (size_t)traj * t + (valid ? s : tl - 1);
+        const float* rec = slot + (size_t)(valid ? s : tl - 1) * kRecWords;
+        // stage the chunk's valid head rows: rows base_row .. base_row + nvalid - 1
+        const int nvalid = min(32, tl - c0);
         __syncwarp();
         if (ldh == kHead) {
             for (int i = lane; i < nvalid * kHead; i += 32) hs[i] = __ldg(head + base_row * kHead + i);
@@ -285,7 +314,7 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
         const float r = rf[kWReward - 160], g = rf[kWDiscount - 160];
         const float is = expf(logp_a - log_mu_a);
         float v_next = __shfl_down_sync(0xffffffffu, v, 1);
-        if (lane == 31 || s >= t - 1) v_next = v_next_chunk;
+        if (lane == 31 || s >= tl - 1) v_next = v_next_chunk;
         float a = 0.f, b = 0.f;
         if (valid) {
             b = fminf(rho_bar, is) * (r + g * v_next - v);
@@ -295,7 +324,7 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
         const float acc = fmaf(a, carry, b);
         const float vs = v + acc;
         float vs_next = __shfl_down_sync(0xffffffffu, vs, 1);
-        if (lane == 31 || s >= t - 1) vs_next = vs_next_chunk;
+        if (lane == 31 || s >= tl - 1) vs_next = vs_next_chunk;
         const float adv = fminf(pg_rho_bar, is) * (r + g * vs_next - v);
         float dv[kHead];
 #pragma unroll
@@ -305,6 +334,14 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
             dv[j] = fmaf(entropy_cost, d_ent, d_pg);   // 0 outside the support: p = 0 and j != act
         }
         dv[kNumActions] = -baseline_cost * (vs - v);
+        if constexpr (kLength) {
+#pragma unroll
+            for (int j = 0; j < kHead; j++) dv[j] = valid ? dv[j] : 0.f;   // padding step: a zero row
+            if (!valid && s < t) {
+                if (vs_out) vs_out[(size_t)traj * t + s] = 0.f;
+                if (adv_out) adv_out[(size_t)traj * t + s] = 0.f;
+            }
+        }
         if (valid) {
 #pragma unroll
             for (int j = 0; j < kHead; j++) dmax = fmaxf(dmax, fabsf(dv[j]));
@@ -319,7 +356,7 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
 #pragma unroll
             for (int j = 0; j < kHead; j++) o_a[lane * 33 + j] = dv[j];
             __syncwarp();
-            for (int i = lane; i < nvalid * kHead; i += 32) {
+            for (int i = lane; i < nrows * kHead; i += 32) {
                 const int rr = i / kHead, j = i % kHead;
                 dhead[(base_row + rr) * ldh + j] = o_a[rr * 33 + j];
             }
@@ -338,12 +375,12 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
             }
             __syncwarp();
             if (ld_split == 32) {  // 128 contiguous bytes per row: one coalesced store per row and array
-                for (int rr = 0; rr < nvalid; rr++) {
+                for (int rr = 0; rr < nrows; rr++) {
                     dhead_hi[(base_row + rr) * 32 + lane] = o_a[rr * 33 + lane];
                     dhead_lo[(base_row + rr) * 32 + lane] = o_b[rr * 33 + lane];
                 }
             } else {
-                for (int i = lane; i < nvalid * kHead; i += 32) {
+                for (int i = lane; i < nrows * kHead; i += 32) {
                     const int rr = i / kHead, j = i % kHead;
                     dhead_hi[(base_row + rr) * ld_split + j] = o_a[rr * 33 + j];
                     dhead_lo[(base_row + rr) * ld_split + j] = o_b[rr * 33 + j];
@@ -371,8 +408,9 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
 
 int launch_vtrace_loss_head(const void* batch, int m, int t, const float* head, int ldh, float rho_bar,
                             float c_bar, float pg_rho_bar, float lambda_, float baseline_cost,
-                            float entropy_cost, bool legal, float* dhead, float* vs, float* pg_adv, double* losses,
-                            cudaStream_t stream, float* dhead_hi, float* dhead_lo, int ld_split, HScale* dhead_hs) {
+                            float entropy_cost, bool legal, bool lengths, float* dhead, float* vs, float* pg_adv,
+                            double* losses, cudaStream_t stream, float* dhead_hi, float* dhead_lo, int ld_split,
+                            HScale* dhead_hs) {
     if (m <= 0 || t <= 0) return FI_OK;
     if (!batch || !head || (!dhead && !dhead_hi) || !losses || ldh < kHead || (dhead_hi && (!dhead_lo || ld_split < kHead)))
         return set_error(FI_ERR_ARG, "vtrace loss head: bad argument");
@@ -380,12 +418,17 @@ int launch_vtrace_loss_head(const void* batch, int m, int t, const float* head, 
     if ((reinterpret_cast<uintptr_t>(batch) & 15) != 0) return set_error(FI_ERR_ARG, "vtrace loss head: batch must be 16-byte aligned");
     // algorithmic traffic per transition: head row in (17 x 4 B) + dhead row out (17 x 4 B) + the record's
     // behaviour logits, action, reward, discount (19 x 4 B) = 212 B (+ 8 B when vs / pg_adv are written)
-    // (the masked head's legal word lies in the same 16-byte load as the discount and aux words: no extra traffic)
-    LaunchScope ls(legal ? "vtrace_loss_head_kernel_legal" : "vtrace_loss_head_kernel", stream,
-                   (212.0 + (vs ? 4.0 : 0.0) + (pg_adv ? 4.0 : 0.0)) * (double)m * t, kWorkBytes);
-    launch_pdl(legal ? vtrace_loss_head_kernel<true> : vtrace_loss_head_kernel<false>, dim3((m + warps - 1) / warps),
-               dim3(32 * warps), 0, stream, (const float*)batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_,
-               baseline_cost, entropy_cost, dhead, vs, pg_adv, losses, dhead_hi, dhead_lo, ld_split, dhead_hs);
+    // (the masked head's legal word lies in the same 16-byte load as the discount and aux words: no extra traffic;
+    // the length-aware head adds the 4-byte length word per trajectory)
+    static const char* const names[2][2] = {{"vtrace_loss_head_kernel", "vtrace_loss_head_kernel_length"},
+                                            {"vtrace_loss_head_kernel_legal", "vtrace_loss_head_kernel_legal_length"}};
+    LaunchScope ls(names[legal][lengths], stream,
+                   (212.0 + (vs ? 4.0 : 0.0) + (pg_adv ? 4.0 : 0.0)) * (double)m * t + (lengths ? 4.0 * m : 0.0), kWorkBytes);
+    auto kernel = legal ? (lengths ? vtrace_loss_head_kernel<true, true> : vtrace_loss_head_kernel<true, false>)
+                        : (lengths ? vtrace_loss_head_kernel<false, true> : vtrace_loss_head_kernel<false, false>);
+    launch_pdl(kernel, dim3((m + warps - 1) / warps), dim3(32 * warps), 0, stream, (const float*)batch, m, t, head, ldh, rho_bar,
+               c_bar, pg_rho_bar, lambda_, baseline_cost, entropy_cost, dhead, vs, pg_adv, losses, dhead_hi, dhead_lo, ld_split,
+               dhead_hs);
     return ls.done();
 }
 
@@ -404,13 +447,22 @@ int fi_op_vtrace_loss_head(const void* batch, int m, int t, const float* head, i
                            float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, float* dhead,
                            float* vs, float* pg_adv, double* losses, void* stream) {
     return fi::launch_vtrace_loss_head(batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_, baseline_cost,
-                                       entropy_cost, false, dhead, vs, pg_adv, losses, (cudaStream_t)stream);
+                                       entropy_cost, false, false, dhead, vs, pg_adv, losses, (cudaStream_t)stream);
 }
 
 int fi_op_vtrace_loss_head_legal(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar,
                                  float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, float* dhead,
                                  float* vs, float* pg_adv, double* losses, void* stream) {
     return fi::launch_vtrace_loss_head(batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_, baseline_cost,
-                                       entropy_cost, true, dhead, vs, pg_adv, losses, (cudaStream_t)stream);
+                                       entropy_cost, true, false, dhead, vs, pg_adv, losses, (cudaStream_t)stream);
+}
+
+int fi_op_vtrace_loss_head_opts(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar,
+                                float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, int legal, int lengths,
+                                float* dhead, float* vs, float* pg_adv, double* losses, void* stream) {
+    if ((legal != 0 && legal != 1) || (lengths != 0 && lengths != 1))
+        return fi::set_error(FI_ERR_ARG, "fi_op_vtrace_loss_head_opts: legal and lengths must be 0 or 1 (got %d, %d)", legal, lengths);
+    return fi::launch_vtrace_loss_head(batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_, baseline_cost,
+                                       entropy_cost, legal != 0, lengths != 0, dhead, vs, pg_adv, losses, (cudaStream_t)stream);
 }
 }

@@ -9,6 +9,10 @@
 // trajectory an actor draws a random non-empty legal word per record, makes one fi_learner_infer_sample call on the S
 // observations, and stores the returned logits (words 162..177), action (178) and legal word (182). The JSON line then also
 // reports the rows sampled and how many returned actions fell outside their legal word (always 0).
+// --variable-length: games of varying length. The learner trains on each trajectory's own length (variable_length), and an
+// actor draws L uniform in 1..game_steps per trajectory, makes and writes only L records (the slot keeps the tail of whatever
+// trajectory used it before), with L in word 183 of record 0 and the bootstrap value in record L - 1; with --sample-actions
+// it samples those L rows. The JSON line then also reports valid_transitions, the sum of the lengths written.
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -26,6 +30,7 @@ struct Params {  // ProgramParams, cmd/freeimpala/main.cpp:18-35 (defaults :38-1
     unsigned seed = 0;
     int infer_every = 0;  // >0: every k-th iteration an actor asks for batched policy inference on its observations
     bool sample_actions = false;
+    bool variable_length = false;
 };
 
 static bool parse(int argc, char** argv, Params& p) {
@@ -37,6 +42,7 @@ static bool parse(int argc, char** argv, Params& p) {
     for (int i = 1; i < argc; i++) {
         std::string a = argv[i];
         if (a == "--sample-actions") { p.sample_actions = true; continue; }
+        if (a == "--variable-length") { p.variable_length = true; continue; }
         if (i + 1 >= argc) return false;
         if (num.count(a)) *num[a] = strtoull(argv[++i], nullptr, 10);
         else if (a == "-l" || a == "--checkpoint-location") p.checkpoint_location = argv[++i];
@@ -49,11 +55,12 @@ static bool parse(int argc, char** argv, Params& p) {
     // validateParameters, main.cpp:160-172
     if (p.batch_size > p.buffer_capacity) { fprintf(stderr, "Batch size (M) must be <= buffer capacity (B)\n"); return false; }
     if (p.game_steps > p.entry_size) { fprintf(stderr, "Game steps must be <= entry size (S)\n"); return false; }
+    if (p.variable_length && p.game_steps == 0) { fprintf(stderr, "--variable-length needs game steps >= 1\n"); return false; }
     return true;
 }
 
 struct SampleCounts {
-    std::atomic<uint64_t> rows{0}, illegal{0};
+    std::atomic<uint64_t> rows{0}, illegal{0}, valid_transitions{0};
     std::atomic<bool> failed{false};
 };
 
@@ -73,32 +80,39 @@ static void actor(size_t id, const Params& P, Learner& learner, std::atomic<uint
     for (size_t it = 0; it < P.iterations; it++) {
         if (P.agent_time) std::this_thread::sleep_for(std::chrono::milliseconds(P.agent_time));  // agent.h:41
         for (size_t p = 0; p < P.players; p++) {
+            // the game's length: entry_size records, or (--variable-length) L uniform in 1..game_steps
+            const size_t len = P.variable_length ? 1 + next() % P.game_steps : P.entry_size;
             // simulateGame (agent.h:34-75): game_steps records, here with a well-formed transition in each
-            for (size_t s = 0; s < P.entry_size; s++) {
+            for (size_t s = 0; s < len; s++) {
                 float* rec = slot.data() + s * 256;
                 for (int j = 0; j < 178; j++) rec[j] = unif();           // observation + behaviour logits
                 int32_t act = (int32_t)(next() % 16);
                 memcpy(rec + 178, &act, 4);
                 rec[179] = unif();                                       // reward
                 rec[180] = (next() % 100) ? 0.99f : 0.f;                 // discount = 0.99 (1 - done)
-                rec[181] = s + 1 == P.entry_size ? unif() : 0.f;         // bootstrap value in the last record
+                rec[181] = s + 1 == len ? unif() : 0.f;                  // bootstrap value in the last record
+            }
+            if (P.variable_length) {
+                const uint32_t w = (uint32_t)len;
+                memcpy(slot.data() + FI_REC_WORD_LENGTH, &w, 4);         // the length, in record 0
+                sampled.valid_transitions.fetch_add(len);
             }
             if (P.sample_actions) {   // the policy's own logits and actions over a random legal set per record
-                std::vector<float> obs(P.entry_size * 162), logits(P.entry_size * 16);
-                std::vector<uint32_t> legal(P.entry_size);
-                std::vector<int32_t> acts(P.entry_size);
-                for (size_t s = 0; s < P.entry_size; s++) {
+                std::vector<float> obs(len * 162), logits(len * 16);
+                std::vector<uint32_t> legal(len);
+                std::vector<int32_t> acts(len);
+                for (size_t s = 0; s < len; s++) {
                     memcpy(&obs[s * 162], &slot[s * 256], 162 * 4);
                     do legal[s] = (uint32_t)(next() & 0xFFFF); while (legal[s] == 0);
                 }
                 const uint64_t seed = ((uint64_t)id << 40) ^ ((uint64_t)it << 8) ^ p;
-                if (fi_learner_infer_sample(learner.handle(), (int)p, obs.data(), legal.data(), P.entry_size, seed, 0, acts.data(),
+                if (fi_learner_infer_sample(learner.handle(), (int)p, obs.data(), legal.data(), len, seed, 0, acts.data(),
                                             logits.data(), nullptr) != FI_OK) {
                     fprintf(stderr, "freeimpala_gpu: fi_learner_infer_sample: %s\n", fi_last_error());
                     sampled.failed.store(true);
                 } else {
-                    sampled.rows.fetch_add(P.entry_size);
-                    for (size_t s = 0; s < P.entry_size; s++) {
+                    sampled.rows.fetch_add(len);
+                    for (size_t s = 0; s < len; s++) {
                         float* rec = slot.data() + s * 256;
                         if (acts[s] < 0 || acts[s] >= 16 || !((legal[s] >> acts[s]) & 1u)) sampled.illegal.fetch_add(1);
                         memcpy(rec + 162, &logits[s * 16], 16 * 4);
@@ -113,7 +127,7 @@ static void actor(size_t id, const Params& P, Learner& learner, std::atomic<uint
                 if (fi_learner_infer(learner.handle(), (int)p, obs.data(), nullptr, P.entry_size, 0, logits.data(), values.data()) == FI_OK)
                     inferences.fetch_add(P.entry_size);
             }
-            buffers[p]->write(slot.data(), slot.size() * sizeof(float));  // transferThread, agent.h:96
+            buffers[p]->write(slot.data(), len * 256 * sizeof(float));     // transferThread, agent.h:96
         }
         for (size_t p = 0; p < P.players; p++) {                          // modelUpdateThread, agent.h:155-165
             const uint64_t latest = models->getLatestVersion(p);
@@ -129,14 +143,14 @@ int main(int argc, char** argv) {
     Params P;
     if (!parse(argc, argv, P)) {
         fprintf(stderr, "usage: freeimpala_gpu [-p N] [-T N] [-S N] [-B N] [-M N] [-a N] [--game-steps N] [--agent-time ms] "
-                        "[-c N] [-l DIR] [-m DIR] [--seed N] [--infer-every K] [--sample-actions]\n");
+                        "[-c N] [-l DIR] [-m DIR] [--seed N] [--infer-every K] [--sample-actions] [--variable-length]\n");
         return 2;
     }
     const size_t learner_iterations = (P.agents * P.iterations) / P.batch_size;  // main.cpp:179 (integer division)
     try {
         Learner learner(P.players, P.buffer_capacity, P.entry_size, P.batch_size, P.learner_time, P.checkpoint_freq,
                         P.checkpoint_location, P.starting_model, learner_iterations, 0, FI_MODEL_MLP_ACTOR_CRITIC,
-                        P.sample_actions);
+                        P.sample_actions, P.variable_length);
         const auto t0 = std::chrono::steady_clock::now();
         learner.start();
         std::atomic<uint64_t> inferences{0};
@@ -175,6 +189,7 @@ int main(int argc, char** argv) {
         if (P.sample_actions)
             printf(", \"actor_sampled_rows\": %llu, \"illegal_actions\": %llu", (unsigned long long)sampled.rows.load(),
                    (unsigned long long)sampled.illegal.load());
+        if (P.variable_length) printf(", \"valid_transitions\": %llu", (unsigned long long)sampled.valid_transitions.load());
         printf("}\n");
         if (sampled.failed.load() || sampled.illegal.load()) return 1;
         return updates == learner_iterations * P.players ? 0 : 1;

@@ -20,8 +20,15 @@ def vtrace(m: int, t: int, log_rho: int, discount: int, reward: int, value: int,
 
 def vtrace_loss_head(batch: int, m: int, t: int, head: int, ldh: int, dhead: int, losses: int, vs: int = None,
                      pg_adv: int = None, rho_bar=1.0, c_bar=1.0, pg_rho_bar=1.0, lambda_=1.0, baseline_cost=0.5,
-                     entropy_cost=0.01, stream=None, legal_mask=False) -> None:
-    """legal_mask: the softmaxes, entropy and d(head) run over each record's legal-action word (fi_learner.h)."""
+                     entropy_cost=0.01, stream=None, legal_mask=False, lengths=False) -> None:
+    """legal_mask: the softmaxes, entropy and d(head) run over each record's legal-action word (fi_learner.h).
+    lengths: each trajectory holds as many steps as word 183 of its record 0 says; the rows past them get zero d(head),
+    vs and pg_adv."""
+    if lengths:
+        check(_lib.load().fi_op_vtrace_loss_head_opts(batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_, baseline_cost,
+                                                      entropy_cost, int(legal_mask), 1, dhead, vs, pg_adv, losses, stream),
+              "fi_op_vtrace_loss_head_opts")
+        return
     name = "fi_op_vtrace_loss_head_legal" if legal_mask else "fi_op_vtrace_loss_head"
     check(getattr(_lib.load(), name)(batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_,
                                      baseline_cost, entropy_cost, dhead, vs, pg_adv, losses, stream), name)

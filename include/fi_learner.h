@@ -185,6 +185,10 @@ typedef struct fi_learner_config {
        head reads each record's legal-action word (FI_REC_WORD_LEGAL) and computes log pi, log mu, the entropy and the
        policy gradient over the legal set; 0 = all 16 actions, word 182 is not read. */
     int legal_action_mask;
+    /* Appended after legal_action_mask; fi_learner_config_default sets 0. Actor-critic model only: 1 = each trajectory
+       carries its length in word 183 of its record 0 (FI_REC_WORD_LENGTH) and the step trains on exactly those records;
+       0 = every trajectory is entry_size records long, word 183 is not read. */
+    int variable_length;
 } fi_learner_config;
 
 /* Trajectory record (FI_ELEMENT_SIZE bytes = 256 32-bit words) of the actor-critic model, the words the loss head reads
@@ -207,6 +211,20 @@ typedef struct fi_learner_config {
  * the action was drawn with. */
 #define FI_REC_WORD_LEGAL 182
 
+/* Variable-length trajectories (variable_length = 1). Games end after a varying number of moves; a trajectory of T =
+ * entry_size records holds L <= T of them. Word 183 of record 0 (the one record every write covers; word 183 of every other
+ * record is not read) is a uint32 W, and L = (W == 0 || W > T) ? T : W, so a zero-filled word means full length. The step
+ * on a batch is then the step on the same trajectories cut to their first L records:
+ *   - the bootstrap value is word 181 of record L - 1 (record T - 1 when L = T);
+ *   - records L..T-1 add nothing to any loss, their rows of d(head) are exactly 0, and no byte of them (observation, mu,
+ *     action, reward, discount, legal word) is read into anything that reaches a loss, a gradient or a per-tensor scale,
+ *     so they may hold anything, NaN included: the tail of an older trajectory, say. They still run through the network
+ *     (as zero observations), which keeps the step's shapes fixed.
+ * What the actor does: it writes records 0..L-1 with L in word 183 of record 0, puts the bootstrap value in word 181 of
+ * record L - 1 (any value if the episode ended there, because its discount is 0), and may hand fi_ring_write only those
+ * L x FI_ELEMENT_SIZE bytes: the slot's older tail is then ignored. A learner with variable_length = 0 never reads word 183. */
+#define FI_REC_WORD_LENGTH 183
+
 typedef struct fi_learner fi_learner;
 
 FI_API void fi_learner_config_default(fi_learner_config* cfg);
@@ -214,7 +232,7 @@ FI_API void fi_learner_config_default(fi_learner_config* cfg);
  * state and all step workspaces in HBM. Returns NULL on failure (see fi_last_error). An unknown
  * optimiser, max_grad_norm < 0 or not finite, rmsprop_alpha outside (0, 1), rmsprop_eps <= 0 or
  * rmsprop_momentum outside [0, 1), legal_action_mask other than 0 or 1 or set to 1 for the FarmerLstm model (which has
- * no policy), and, for the actor-critic model, a V-trace constant outside the range
+ * no policy), variable_length other than 0 or 1 or set to 1 for the FarmerLstm model, and, for the actor-critic model, a V-trace constant outside the range
  * fi_learner_config states, is rejected (FI_ERR_ARG) before any device is looked for. */
 FI_API fi_learner* fi_learner_create(const fi_learner_config* cfg);
 FI_API void fi_learner_destroy(fi_learner* l);
@@ -376,6 +394,10 @@ FI_API int fi_op_vtrace_loss_head(const void* batch, int m, int t, const float* 
 /* Same, with legal-action masking: the softmaxes, entropy and d(head) run over each record's legal word | the action's bit
  * (see FI_REC_WORD_LEGAL); d(head) is 0 in every column outside that support. */
 FI_API int fi_op_vtrace_loss_head_legal(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar, float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, float* dhead, float* vs, float* pg_adv, double* losses, void* stream);
+/* Same, with either option: legal = 1 masks as fi_op_vtrace_loss_head_legal; lengths = 1 reads each trajectory's length
+ * from word 183 of its record 0 (see FI_REC_WORD_LENGTH) and writes zero d(head), vs and pg_adv rows for the steps past it.
+ * legal and lengths must be 0 or 1. */
+FI_API int fi_op_vtrace_loss_head_opts(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar, float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, int legal, int lengths, float* dhead, float* vs, float* pg_adv, double* losses, void* stream);
 
 /* The sampling kernel of fi_learner_infer_sample on caller-owned device pointers. head [rows, ldh], ldh >= 16: only columns
  * 0..15 are read. legal [rows] (may be NULL = all 16 legal), actions [rows] int32. Row r uses RNG counter r, the seed and
