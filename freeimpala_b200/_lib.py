@@ -36,7 +36,7 @@ class FiLearnerConfig(C.Structure):
                 ("gemm_mode", c_int), ("publish_every", c_int), ("checkpoint_location", c_char_p),
                 ("max_grad_norm", c_double), ("rmsprop_alpha", c_double), ("rmsprop_eps", c_double),
                 ("rmsprop_momentum", c_double), ("legal_action_mask", c_int),
-                ("variable_length", c_int)]
+                ("variable_length", c_int), ("history_length", c_int)]
 
 
 class FiProfEntry(C.Structure):
@@ -99,6 +99,7 @@ SIGNATURES = {
     "fi_learner_infer": (c_int, [_P, c_int, _P, _P, c_size_t, c_size_t, _P, _P]),
     "fi_learner_infer_stats": (c_int, [_P, c_int, C.POINTER(c_u64), C.POINTER(c_u64), C.POINTER(c_u64)]),
     "fi_learner_infer_grouped": (c_int, [_P, c_int, _P, c_size_t, c_size_t, _P, _P, _P, _P]),
+    "fi_learner_infer_grouped_lengths": (c_int, [_P, c_int, _P, c_size_t, c_size_t, _P, _P, _P, _P, _P]),
     "fi_learner_infer_sample": (c_int, [_P, c_int, _P, _P, c_size_t, c_u64, c_int, _P, _P, _P]),
     "fi_model_bytes": (c_size_t, [_P]),
     "fi_model_version": (c_u64, [_P, c_int]),

@@ -144,6 +144,10 @@ __host__ __device__ __forceinline__ size_t step_cell_offset(int s, int b, int un
 // trajectory's length (word 183 of its record 0, fi_learner.h) are split as zeros without being read
 int launch_split_tf32(const float* x, int ld_in, size_t rows, int cols, int ld_out, float* hi, float* lo, cudaStream_t st,
                       int len_t = 0);
+constexpr int kObsLd = 164;     // 162 observation words padded to a 16-byte multiple (TMA row stride), 3xTF32 format
+// out [rows, kObsLd]: the observations of a gathered batch of t-record trajectories (rows = trajectories x t), zero rows at
+// and past each trajectory's length (word 183 of its record 0) and zero in columns 162..163; the batch's padding is not read
+int launch_obs_length(const float* batch, int rows, int t, float* out, cudaStream_t st);
 // fp16 format pre-passes: amax accumulates max |x| into hs->amax; split derives the scale from hs->amax (which must
 // bound the matrix) and writes hi / lo' with columns [cols, ld_out) zero-filled. write_scale: publish scale/inv in *hs.
 int launch_amax(const float* x, int ld_in, size_t rows, int cols, HScale* hs, cudaStream_t st);

@@ -876,6 +876,29 @@ int launch_split_tf32(const float* x, int ld_in, size_t rows, int cols, int ld_o
     return ls.done();
 }
 
+// The plain-fp32 paths' length-aware copy (the actor-critic's simt trunk, the FarmerLstm projection and W_ih gradient off the
+// 3xFP16 path): out [rows, kObsLd] = the observations (words 0..161) of a gathered batch of t-record trajectories; rows past
+// their trajectory's length, and columns 162..163, are zero. One warp per row: the length word is one broadcast load per row.
+__global__ void obs_length_kernel(const float* __restrict__ batch, int rows, int t, float* __restrict__ out) {
+    const int warp = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), nwarps = (int)((gridDim.x * blockDim.x) >> 5);
+    const int lane = threadIdx.x & 31;
+    for (int r = warp; r < rows; r += nwarps) {
+        const int s = r % t;
+        const float* rec = batch + (size_t)r * kRecWords;
+        const bool in = s < traj_length(__ldg(reinterpret_cast<const uint32_t*>(rec - (size_t)s * kRecWords) + kWLength), t);
+        for (int c = lane; c < kObsLd; c += 32) out[(size_t)r * kObsLd + c] = in && c < kZDim ? __ldg(rec + c) : 0.f;
+    }
+}
+
+int launch_obs_length(const float* batch, int rows, int t, float* out, cudaStream_t st) {
+    int blocks = (rows + 7) / 8;
+    if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
+    // algorithmic traffic per row: 162 words in, 164 out, the length word
+    LaunchScope ls("obs_length_kernel", st, (4.0 * (kZDim + kObsLd) + 4.0) * rows, kWorkBytes);
+    obs_length_kernel<<<blocks, 256, 0, st>>>(batch, rows, t, out);
+    return ls.done();
+}
+
 // ---- 3xFP16 pre-passes ---------------------------------------------------------------------------------------
 // max |x| over a [rows, cols] matrix (row stride ld_in) into hs->amax. Non-negative floats order like their bit patterns.
 __global__ void amax_kernel(const float* __restrict__ x, int ld_in, size_t rows, int cols, HScale* hs) {

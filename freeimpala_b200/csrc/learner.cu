@@ -349,6 +349,7 @@ void fi_learner_config_default(fi_learner_config* c) {
     c->rmsprop_momentum = 0.0;
     c->legal_action_mask = 0;    // every action legal; record word 182 is not read
     c->variable_length = 0;      // every trajectory entry_size records long; record word 183 is not read
+    c->history_length = 0;       // every FarmerLstm history entry_size records long; record word 183 is not read
 }
 
 fi_learner* fi_learner_create(const fi_learner_config* cfg) {
@@ -391,6 +392,14 @@ fi_learner* fi_learner_create(const fi_learner_config* cfg) {
     }
     if (farmer && cfg->variable_length) {
         set_error(FI_ERR_ARG, "fi_learner_create: variable_length is for the actor-critic model, not the FarmerLstm model");
+        return nullptr;
+    }
+    if (cfg->history_length != 0 && cfg->history_length != 1) {
+        set_error(FI_ERR_ARG, "fi_learner_create: history_length must be 0 or 1, got %d", cfg->history_length);
+        return nullptr;
+    }
+    if (!farmer && cfg->history_length) {
+        set_error(FI_ERR_ARG, "fi_learner_create: history_length is for the FarmerLstm model; the actor-critic has variable_length");
         return nullptr;
     }
     if (!farmer) {   // V-trace constants: a NaN or out-of-range value would otherwise surface as NaN or meaningless losses
@@ -882,11 +891,12 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
     const bool farmer = l->cfg.model == FI_MODEL_FARMER_LSTM;
     FI_CUDA_OK(cudaSetDevice(l->cfg.device));
     size_t states = 0;
-    bool want_best = false, want_actions = false;
+    bool want_best = false, want_actions = false, want_lengths = false;
     for (const fi::InferReq* q : batch) {
         states += q->states;
         want_best |= q->best != nullptr;
         want_actions |= q->actions != nullptr;
+        want_lengths |= q->lengths != nullptr;
     }
     // the farmer model uploads z once per state, the actor-critic one observation per row
     const size_t row_in = farmer ? t * fi::kZDim : fi::kZDim;
@@ -919,7 +929,7 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
         FI_CUDA_OK(cudaMalloc((void**)&p->inf_out, cap_out * sizeof(float)));
         FI_CUDA_OK(cudaHostAlloc((void**)&p->inf_host_out, cap_out * sizeof(float), cudaHostAllocPortable));
         if (farmer) {
-            const size_t cap_idx = scap + 1 + cap;
+            const size_t cap_idx = scap + 1 + cap + scap;   // offsets, row states, history lengths
             FI_CUDA_OK(cudaMalloc((void**)&p->inf_x, cap * fi::kXDim * sizeof(float)));
             FI_CUDA_OK(cudaHostAlloc((void**)&p->inf_host_x, cap * fi::kXDim * sizeof(float), cudaHostAllocPortable));
             FI_CUDA_OK(cudaMalloc((void**)&p->inf_idx, cap_idx * sizeof(uint32_t)));
@@ -936,10 +946,20 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
     }
     cudaStream_t st = p->infer_stream;
     uint32_t* const off = p->inf_host_idx;              // farmer: the batch's offsets [states + 1] ...
-    uint32_t* const row_state = off ? off + states + 1 : nullptr;   // ... then the state of each candidate row [rows]
+    uint32_t* const row_state = off ? off + states + 1 : nullptr;   // ... then the state of each candidate row [rows] ...
+    uint32_t* const lengths = row_state ? row_state + rows : nullptr;   // ... then (want_lengths) each state's history length
     size_t r0 = 0, s0 = 0;
     for (const fi::InferReq* q : batch) {   // pack the callers' states and rows back to back, their offsets rebased
-        memcpy(p->inf_host_in + (farmer ? s0 : r0) * row_in, q->obs, (farmer ? q->states : q->rows) * row_in * sizeof(float));
+        if (q->lengths) {   // only each state's history: z[s, L..t-1] is never read
+            for (size_t s = 0; s < q->states; s++) {
+                memcpy(p->inf_host_in + (s0 + s) * row_in, q->obs + s * row_in, q->lengths[s] * fi::kZDim * sizeof(float));
+                lengths[s0 + s] = q->lengths[s];
+            }
+        } else {
+            memcpy(p->inf_host_in + (farmer ? s0 : r0) * row_in, q->obs, (farmer ? q->states : q->rows) * row_in * sizeof(float));
+            if (want_lengths)
+                for (size_t s = 0; s < q->states; s++) lengths[s0 + s] = (uint32_t)t;
+        }
         if (farmer) {
             memcpy(p->inf_host_x + r0 * fi::kXDim, q->x, q->rows * fi::kXDim * sizeof(float));
             for (size_t s = 0; s < q->states; s++) {
@@ -962,7 +982,8 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
     if (farmer) {
         off[states] = (uint32_t)rows;
         FI_CUDA_OK(cudaMemcpyAsync(p->inf_x, p->inf_host_x, rows * fi::kXDim * sizeof(float), cudaMemcpyHostToDevice, st));
-        FI_CUDA_OK(cudaMemcpyAsync(p->inf_idx, off, (states + 1 + rows) * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+        FI_CUDA_OK(cudaMemcpyAsync(p->inf_idx, off, (states + 1 + rows + (want_lengths ? states : 0)) * sizeof(uint32_t),
+                                   cudaMemcpyHostToDevice, st));
     }
     if (want_actions)
         FI_CUDA_OK(cudaMemcpyAsync(p->inf_idx, p->inf_host_idx, rows * sizeof(uint4), cudaMemcpyHostToDevice, st));
@@ -974,8 +995,8 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
         const int sn = s.newest_snap;
         FI_CUDA_OK(cudaStreamWaitEvent(st, s.snap_ready[sn], 0));
         if (farmer)
-            FI_TRY(fi::farmer_infer(l, p, s.dev_snap[sn], p->inf_in, p->inf_x, p->inf_idx, p->inf_idx + states + 1, states, rows, t,
-                                    p->inf_out, best_dev, st));
+            FI_TRY(fi::farmer_infer(l, p, s.dev_snap[sn], p->inf_in, p->inf_x, p->inf_idx, p->inf_idx + states + 1,
+                                    want_lengths ? p->inf_idx + states + 1 + rows : nullptr, states, rows, t, p->inf_out, best_dev, st));
         else
             FI_TRY(fi::ac_infer(l, p, s.dev_snap[sn], p->inf_in, rows, p->inf_out, st));
         if (want_actions)
@@ -1009,7 +1030,8 @@ int run_infer_batch(fi_learner* l, Player* p, const std::vector<fi::InferReq*>& 
 }
 
 // Queues `req` on its player and waits for it: the first caller that finds no forward in flight becomes the leader and runs
-// everything pending that fits one forward (the farmer model batches equal sequence lengths).
+// everything pending that fits one forward (the farmer model batches equal sequence lengths t, with or without per-state
+// history lengths).
 int submit_infer(fi_learner* l, Player* p, fi::InferReq& req) {
     std::unique_lock<std::mutex> lk(p->infer_mu);
     p->infer_pending.push_back(&req);
@@ -1075,6 +1097,31 @@ int fi_learner_infer_grouped(fi_learner* l, int player, const float* z, size_t s
     const size_t rows = offsets[states];
     if (rows > kInferMaxRows) return set_error(FI_ERR_ARG, "fi_learner_infer_grouped: %zu rows, at most %zu per call", rows, kInferMaxRows);
     fi::InferReq req{z, x, rows, t, states, offsets, nullptr, values, best, FI_OK, false};
+    return submit_infer(l, p, req);
+}
+
+int fi_learner_infer_grouped_lengths(fi_learner* l, int player, const float* z, size_t states, size_t t, const uint32_t* lengths,
+                                     const float* x, const uint32_t* offsets, float* values, int32_t* best) {
+    Player* p = get_player(l, player);
+    if (!p) return set_error(FI_ERR_ARG, "fi_learner_infer_grouped_lengths: no player %d", player);
+    if (l->cfg.model != FI_MODEL_FARMER_LSTM) return set_error(FI_ERR_ARG, "fi_learner_infer_grouped_lengths: FarmerLstm model only");
+    if (!z || !x || !offsets || !lengths || (!values && !best))
+        return set_error(FI_ERR_ARG, "fi_learner_infer_grouped_lengths: z, x, offsets, lengths and one of values / best are required");
+    if (states == 0 || t == 0) return set_error(FI_ERR_ARG, "fi_learner_infer_grouped_lengths: states and t must be positive");
+    if (states > kInferMaxRows)
+        return set_error(FI_ERR_ARG, "fi_learner_infer_grouped_lengths: at most %zu rows per call", kInferMaxRows);
+    for (size_t s = 0; s < states; s++)
+        if (lengths[s] < 1 || lengths[s] > t)
+            return set_error(FI_ERR_ARG, "fi_learner_infer_grouped_lengths: lengths[%zu] = %u, must be in 1..t = %zu", s, lengths[s], t);
+    if (offsets[0] != 0) return set_error(FI_ERR_ARG, "fi_learner_infer_grouped_lengths: offsets[0] must be 0");
+    for (size_t s = 0; s < states; s++)
+        if (offsets[s + 1] <= offsets[s])
+            return set_error(FI_ERR_ARG, "fi_learner_infer_grouped_lengths: offsets must increase strictly (state %zu has no candidate)", s);
+    const size_t rows = offsets[states];
+    if (rows > kInferMaxRows)
+        return set_error(FI_ERR_ARG, "fi_learner_infer_grouped_lengths: %zu rows, at most %zu per call", rows, kInferMaxRows);
+    fi::InferReq req{z, x, rows, t, states, offsets, nullptr, values, best, FI_OK, false};
+    req.lengths = lengths;
     return submit_infer(l, p, req);
 }
 

@@ -123,6 +123,7 @@ struct InferReq {
     const uint32_t* legal = nullptr;    // [rows] legal words, or null = all 16 legal
     uint64_t seed = 0;
     int greedy = 0;
+    const uint32_t* lengths = nullptr;  // FarmerLstm, may be null (= t): [states], the history length of each state
 };
 
 struct Player {
@@ -165,7 +166,8 @@ struct Player {
     uint64_t infer_calls = 0, infer_batches = 0, infer_rows = 0;
     cudaStream_t infer_stream = nullptr;
     // FarmerLstm: inf_in holds z per state, inf_x the candidate rows, inf_idx the batch's offsets [states + 1] followed by the
-    // state of each candidate row [rows], inf_out the values [rows] followed by best [states] (int32).
+    // state of each candidate row [rows] and, in a batch with a fi_learner_infer_grouped_lengths request, each state's history
+    // length [states]; inf_out the values [rows] followed by best [states] (int32).
     // Actor-critic: inf_in holds the observations, inf_out the head rows [rows, 17] followed by the actions [rows] (int32) of
     // a batch with a sampling request, inf_idx that batch's sampling descriptors [rows] x 4 words (policy_sample_kernel)
     float *inf_in = nullptr, *inf_x = nullptr, *inf_out = nullptr;
@@ -244,7 +246,8 @@ int farmer_forward_backward(fi_learner* l, Player* p, const float* batch, int m,
 int farmer_infer_alloc(fi_learner* l, Player* p, size_t states, size_t rows, size_t t);
 // The recurrence once per state, the dense stack once per candidate row: values_dev [rows]; best_dev (may be null) [states], the
 // index within each group of its largest value (lowest on ties). offsets_dev [states + 1], state_dev [rows]: the groups.
+// lengths_dev (may be null = every history t steps): [states], state s's history is z[s, 0..lengths[s]-1], 1 <= lengths[s] <= t.
 int farmer_infer(fi_learner* l, Player* p, const float* params, const float* z_dev, const float* x_dev, const uint32_t* offsets_dev,
-                 const uint32_t* state_dev, size_t states, size_t rows, size_t t, float* values_dev, int32_t* best_dev,
-                 cudaStream_t stream);
+                 const uint32_t* state_dev, const uint32_t* lengths_dev, size_t states, size_t rows, size_t t, float* values_dev,
+                 int32_t* best_dev, cudaStream_t stream);
 }  // namespace fi

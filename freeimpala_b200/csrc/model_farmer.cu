@@ -47,6 +47,11 @@ struct FarmerWs {
     float* bias_part = nullptr;                    // [CTAs of the BPTT kernel, 512]: their column sums of dG (the LSTM bias gradient)
     float* dfeat = nullptr;                        // [rows, 128]: dL/dh_{T-1} from the split-operand dense stack (the x part of the
                                                    // feature row needs no gradient)
+    // history_length (training): each slot's history is its first L records (word 183 of record 0). The plain-fp32 projection
+    // and W_ih gradient read z from this zero-padded copy [rows*T, kObsLd] instead of the batch (allocated when the learner's
+    // GEMM mode can take that path); the 3xFP16 path splits padding rows as zeros itself.
+    bool history = false;
+    float* zpad = nullptr;
 };
 constexpr int kFeatLdH = 640;   // 612 feature columns padded to whole 128-byte lines of fp16
 enum { kLstmHsObs = 0, kLstmHsWih = 1, kLstmHsDg = 2, kLstmHsHp = 3 };   // FarmerWs::hs slots
@@ -169,10 +174,18 @@ constexpr int kLstmSmemK = 64;  // k-rows of W_hh^T kept in shared memory
 constexpr float kHprevScale = 8192.f;   // hscale_from_bound(1)
 constexpr size_t kLstmFwdSmem = ((size_t)kLstmSmemK * kG4 + kLstmRows * kG4 + kLstmH * kLstmRows + kLstmRows * kLstmH) * sizeof(float);
 
+//
+// kLength (history_length, and inference with per-state lengths): row b's history is its first L_b = traj_length(len[b *
+// len_stride], t) steps. The CTA runs the steps below the largest L of its rows; a row at s >= L keeps h and c by select (no
+// arithmetic on a padding gate reaches them), takes feat from h_{L-1}, and gets a zero h_prev row (fp32 or fp16 pair) at every
+// s >= L, the steps past the CTA's loop included: the W_hh gradient product reads all m*T rows. Its gate and c rows are not
+// written (the backward pass does not read them).
+template <bool kLength>
 __global__ void __launch_bounds__(kLstmThreads, 1)
 lstm_forward_kernel(float* __restrict__ gates, const float* __restrict__ whh_t, const float* __restrict__ b_hh,
                     int m, int t, float* __restrict__ hprev, float* __restrict__ cst, float* __restrict__ feat,
-                    __half* __restrict__ hp_hi, __half* __restrict__ hp_lo, HScale* __restrict__ hp_hs, unsigned long long* trace) {
+                    __half* __restrict__ hp_hi, __half* __restrict__ hp_lo, HScale* __restrict__ hp_hs, unsigned long long* trace,
+                    const uint32_t* __restrict__ len, int len_stride) {
     extern __shared__ __align__(16) float lstm_smem[];
     float* Ws = lstm_smem;                          // [64][512]   W_hh^T rows k < 64
     float* ps = Ws + kLstmSmemK * kG4;              // [8][512]    pre-activations of this step
@@ -201,8 +214,21 @@ lstm_forward_kernel(float* __restrict__ gates, const float* __restrict__ whh_t, 
         hp_hs->amax = 1.f;
         hp_hs->bound = 1.f;
     }
+    constexpr int kPairs = kLstmRows * kLstmH / kLstmThreads;
+    const int u = tid & (kLstmH - 1), r4 = (tid >> 7) * kPairs;   // this thread's unit and first row in the element-wise part
+    int steps = t;            // steps this CTA runs
+    int lrow[kPairs];         // kLength: the lengths of this thread's rows (0 past the batch)
+    if constexpr (kLength) {
+        steps = 0;
+#pragma unroll
+        for (int r = 0; r < kLstmRows; r++)
+            if (r < nrows) steps = max(steps, traj_length(__ldg(len + (size_t)(b0 + r) * len_stride), t));
+#pragma unroll
+        for (int k = 0; k < kPairs; k++)
+            lrow[k] = r4 + k < nrows ? traj_length(__ldg(len + (size_t)(b0 + r4 + k) * len_stride), t) : 0;
+    }
     unsigned long long* tr = (blockIdx.x == 0 && tid == 0) ? trace : nullptr;
-    for (int s = 0; s < t; s++) {
+    for (int s = 0; s < steps; s++) {
         lstm_trace_ev(tr, s, 0);
         float2 acc2[kLstmRows / 2][2];   // [row pair][column]: .x = row 2 rp, .y = row 2 rp + 1
         float2 gx[kLstmRows];
@@ -247,10 +273,8 @@ lstm_forward_kernel(float* __restrict__ gates, const float* __restrict__ whh_t, 
         // first, then the four gate chains side by side, then the stores: written pair by pair the shared-memory stores of one
         // pair ordered the loads of the next behind them and the phase took 3200 clocks of exposed latency per step. A pair's
         // h_{s-1} entry in hs is read by its own thread only (the product is done), so h_s goes straight back into it.
-        constexpr int kPairs = kLstmRows * kLstmH / kLstmThreads;
         float pin[kPairs][4], cin[kPairs], hin[kPairs];
 #pragma unroll
-        const int u = tid & (kLstmH - 1), r4 = (tid >> 7) * kPairs;   // this thread's unit and first row
         for (int k = 0; k < kPairs; k++) {
             const int r = r4 + k;
 #pragma unroll
@@ -271,10 +295,27 @@ lstm_forward_kernel(float* __restrict__ gates, const float* __restrict__ whh_t, 
             cv[k] = fmaf(gv[k][1], cin[k], gv[k][0] * gv[k][2]);
             hv[k] = gv[k][3] * fast_tanh(cv[k]);
         }
+        if constexpr (kLength) {
+#pragma unroll
+            for (int k = 0; k < kPairs; k++) {   // past its length a row keeps h and c (selects: the gates there may be anything)
+                cv[k] = s < lrow[k] ? cv[k] : cin[k];
+                hv[k] = s < lrow[k] ? hv[k] : hin[k];
+            }
+        }
 #pragma unroll
         for (int k = 0; k < kPairs; k++) {
             const int r = r4 + k;
-            if (r < nrows) {
+            if constexpr (kLength) {
+                if (r < nrows && s >= lrow[k]) {   // a padding step: only its zero h_prev row
+                    const size_t row = (size_t)(b0 + r) * t + s;
+                    if (hprev) hprev[row * kLstmH + u] = 0.f;
+                    if (hp_hi) {
+                        hp_hi[row * kLstmH + u] = __float2half_rn(0.f);
+                        hp_lo[row * kLstmH + u] = __float2half_rn(0.f);
+                    }
+                }
+            }
+            if (r < nrows && (!kLength || s < lrow[k])) {
                 const size_t row = (size_t)(b0 + r) * t + s;
                 float* g = gates + row * kG4;
                 g[u] = gv[k][0]; g[kLstmH + u] = gv[k][1]; g[2 * kLstmH + u] = gv[k][2]; g[3 * kLstmH + u] = gv[k][3];
@@ -286,7 +327,7 @@ lstm_forward_kernel(float* __restrict__ gates, const float* __restrict__ whh_t, 
                     hp_hi[row * kLstmH + u] = hh;
                     hp_lo[row * kLstmH + u] = __float2half_rn((x - __half2float(hh)) * 2048.f);
                 }
-                if (s == t - 1) feat[(size_t)(b0 + r) * kFeat + u] = hv[k];
+                if (s == (kLength ? lrow[k] : t) - 1) feat[(size_t)(b0 + r) * kFeat + u] = hv[k];
             }
             cs[r * kLstmH + u] = r < nrows ? cv[k] : 0.f;
             if (r >= nrows) hv[k] = 0.f;
@@ -296,6 +337,19 @@ lstm_forward_kernel(float* __restrict__ gates, const float* __restrict__ whh_t, 
         __syncthreads();
         lstm_trace_ev(tr, s, 6);
         lstm_trace_ev(tr, s, 7);
+    }
+    if constexpr (kLength) {   // the steps past the CTA's longest row: zero h_prev rows only
+        for (int s = steps; s < t; s++)
+#pragma unroll
+            for (int k = 0; k < kPairs; k++) {
+                const size_t row = (size_t)(b0 + r4 + k) * t + s;
+                if (r4 + k >= nrows) continue;
+                if (hprev) hprev[row * kLstmH + u] = 0.f;
+                if (hp_hi) {
+                    hp_hi[row * kLstmH + u] = __float2half_rn(0.f);
+                    hp_lo[row * kLstmH + u] = __float2half_rn(0.f);
+                }
+            }
     }
 }
 
@@ -309,10 +363,15 @@ constexpr int kLstmBwdPre = 6;   // per (row, unit) pair and step: gates i, f, g
 constexpr size_t kLstmBwdSmem =
     ((size_t)kLstmSmemJ * kLstmH + kG4 * kLstmRows + 4 * kLstmRows * kLstmH + kLstmBwdPre * kLstmRows * kLstmH) * sizeof(float);
 
+//
+// kLength: the loop starts at the CTA's largest L - 1. A row at s >= L gets dG = 0 and carries dL/dh and dL/dc to s - 1
+// unchanged (selects; its gate and c operands are not fetched), and every step past the loop gets zero dG rows: the weight
+// gradient products and their max |dG| read all m*T rows.
+template <bool kLength>
 __global__ void __launch_bounds__(kLstmThreads, 1)
 lstm_backward_kernel(float* __restrict__ gates, const float* __restrict__ whh, const float* __restrict__ cst,
                      const float* __restrict__ dfeat, int ldf, int m, int t, HScale* __restrict__ dg_hs, float* __restrict__ bias_part,
-                     unsigned long long* trace) {
+                     unsigned long long* trace, const uint32_t* __restrict__ len, int len_stride) {
     extern __shared__ __align__(16) float lstm_smem[];
     float* Wh = lstm_smem;                          // [4][64][128] W_hh rows 128q + jj, jj < 64
     float* dgs = Wh + kLstmSmemJ * kLstmH;          // [512][8]    dG of this step, j-major
@@ -325,11 +384,13 @@ lstm_backward_kernel(float* __restrict__ gates, const float* __restrict__ whh, c
     // they cost 4900 clocks of exposed latency per step (41 % of the step, clock64 trace). Each thread fetches ITS pairs'
     // operands of step s-1 with cp.async while the dh product of step s runs; it is also the only reader of those entries.
     const int u = tid & (kLstmH - 1), r4 = (tid >> 7) * (kLstmRows * kLstmH / kLstmThreads);   // this thread's unit and first of its 4 rows
+    int steps = t;                                               // steps this CTA runs
+    int lrow[kLstmRows * kLstmH / kLstmThreads];                 // kLength: the lengths of this thread's rows (0 past the batch)
     auto prefetch = [&](int s) {
 #pragma unroll
         for (int i = tid; i < kLstmRows * kLstmH; i += kLstmThreads) {   // i: the thread's private slots of `pre`
             const int r = r4 + i / kLstmThreads;
-            if (r < nrows) {
+            if (r < nrows && (!kLength || s < lrow[i / kLstmThreads])) {
                 const size_t row = (size_t)(b0 + r) * t + s;
                 const float* g = gates + row * kG4 + u;
                 const uint32_t dst = (uint32_t)__cvta_generic_to_shared(pre + i);
@@ -356,7 +417,16 @@ lstm_backward_kernel(float* __restrict__ gates, const float* __restrict__ whh, c
 #pragma unroll
     for (int jj = 0; jj < 64; jj++) wreg[jj] = __ldg(reinterpret_cast<const float2*>(whh + (size_t)(q * kLstmH + 64 + jj) * kLstmH + k0));
     pdl_wait();
-    prefetch(t - 1);
+    if constexpr (kLength) {
+        steps = 0;
+#pragma unroll
+        for (int r = 0; r < kLstmRows; r++)
+            if (r < nrows) steps = max(steps, traj_length(__ldg(len + (size_t)(b0 + r) * len_stride), t));
+#pragma unroll
+        for (int k = 0; k < kLstmRows * kLstmH / kLstmThreads; k++)
+            lrow[k] = r4 + k < nrows ? traj_length(__ldg(len + (size_t)(b0 + r4 + k) * len_stride), t) : 0;
+    }
+    prefetch(steps - 1);
     // dL/dh and dL/dc of this thread's 4 (row, unit) pairs (unit tid % 128, rows 4 (tid / 128) + k) live in registers
     constexpr int kPairs = kLstmRows * kLstmH / kLstmThreads;
     float dhr[kPairs], dcr[kPairs];
@@ -371,7 +441,7 @@ lstm_backward_kernel(float* __restrict__ gates, const float* __restrict__ whh, c
     // meets unit tid % 128 (rows 4 (tid / 128) + k)
     float run_max = 0.f, bs0 = 0.f, bs1 = 0.f, bs2 = 0.f, bs3 = 0.f;
     unsigned long long* tr = (blockIdx.x == 0 && tid == 0) ? trace : nullptr;
-    for (int s = t - 1; s >= 0; s--) {
+    for (int s = steps - 1; s >= 0; s--) {
         lstm_trace_ev(tr, t - 1 - s, 0);
         asm volatile("cp.async.wait_group 0;" ::: "memory");   // this thread's operands of step s have landed
         float pv[kLstmRows * kLstmH / kLstmThreads][kLstmBwdPre];
@@ -391,7 +461,14 @@ lstm_backward_kernel(float* __restrict__ gates, const float* __restrict__ whh, c
             dd[k][1] = dct * cp * fg * (1.f - fg);
             dd[k][2] = dct * ig * (1.f - gg * gg);
             dd[k][3] = dhr[k] * tc * og * (1.f - og);
-            dcr[k] = dct * fg;
+            if constexpr (kLength) {   // past its length a row has dG = 0 and keeps dL/dc (its operands were not fetched)
+                const bool live = s < lrow[k];
+#pragma unroll
+                for (int g = 0; g < 4; g++) dd[k][g] = live ? dd[k][g] : 0.f;
+                dcr[k] = live ? dct * fg : dcr[k];
+            } else {
+                dcr[k] = dct * fg;
+            }
         }
 #pragma unroll
         for (int k = 0; k < kPairs; k++) {
@@ -443,11 +520,22 @@ lstm_backward_kernel(float* __restrict__ gates, const float* __restrict__ whh, c
 #pragma unroll
             for (int k = 0; k < kPairs; k++) {
                 const int i = (r4 + k) * kLstmH + u;
-                dhr[k] = (part[i] + part[kLstmRows * kLstmH + i]) + (part[2 * kLstmRows * kLstmH + i] + part[3 * kLstmRows * kLstmH + i]);
+                const float dh = (part[i] + part[kLstmRows * kLstmH + i]) + (part[2 * kLstmRows * kLstmH + i] + part[3 * kLstmRows * kLstmH + i]);
+                if constexpr (kLength) dhr[k] = s < lrow[k] ? dh : dhr[k];   // past its length a row keeps dL/dh
+                else dhr[k] = dh;
             }
             // (no barrier here: `part` is next written after the barrier that follows the next step's element-wise part)
             lstm_trace_ev(tr, t - 1 - s, 7);
         }
+    }
+    if constexpr (kLength) {   // the steps past the CTA's longest row: zero dG rows only
+        for (int s = steps; s < t; s++)
+#pragma unroll
+            for (int k = 0; k < kPairs; k++) {
+                if (r4 + k >= nrows) continue;
+                float* g = gates + ((size_t)(b0 + r4 + k) * t + s) * kG4;
+                g[u] = 0.f; g[kLstmH + u] = 0.f; g[2 * kLstmH + u] = 0.f; g[3 * kLstmH + u] = 0.f;
+            }
     }
     if (dg_hs) {
         const uint32_t wm = __reduce_max_sync(0xFFFFFFFFu, __float_as_uint(run_max));
@@ -500,7 +588,7 @@ __global__ void regression_loss_kernel(const float* __restrict__ y, const float*
 // ------------------------------------------------------------------------------------------
 static void ws_release(FarmerWs* w) {
     if (!w) return;
-    float* f[] = {w->gates, w->hprev, w->cst, w->whh_t, w->feat, w->h_last, w->y, w->dy, w->target, w->dfeat};
+    float* f[] = {w->gates, w->hprev, w->cst, w->whh_t, w->feat, w->h_last, w->y, w->dy, w->target, w->dfeat, w->zpad};
     for (float* p : f)
         if (p) cudaFree(p);
     if (w->gemm_ws) cudaFree(w->gemm_ws);
@@ -575,6 +663,9 @@ static int ws_create(fi_learner* l, size_t states, size_t rows, size_t t, bool t
             if (sw) FI_CUDA_OK(cudaMalloc(&w->split_ws, sw));
             FI_CUDA_OK(cudaMalloc((void**)&w->dfeat, rows * kLstmH * sizeof(float)));
         }
+        w->history = l->cfg.history_length != 0;
+        // partial batches move AUTO below farmer_use_half's threshold: every mode but a 3xFP16-only learner can take the plain path
+        if (w->history && !(w->half && mode == FI_GEMM_TCGEN05_F16)) FI_CUDA_OK(cudaMalloc((void**)&w->zpad, rt * kObsLd * sizeof(float)));
     }
     // split-operand buffers wherever the 3xFP16 path is available; farmer_dense_tc picks the path per step
     return dense_alloc(ds, DenseShape{kFeat, kFeatLdH, 1, 4}, rows, l->arena_elems, w->half ? kDenseTrain : kDenseNone, true,
@@ -609,15 +700,16 @@ static bool farmer_dense_tc(const fi_learner* l, const DenseStack* ds, int m) {
 // The LSTM half of the forward over m rows of z (row (b,t) at z + (b*t + s) * ldz): the input projection and the recurrence,
 // leaving h_{T-1} of row b in columns 0..127 of h [m, kFeat] (and the BPTT state when training). dense_tc: the dense stack
 // that follows runs on split operands; its scales are zeroed and its parameters split here, before W_ih's split that shares
-// the arena's scale.
+// the arena's scale. len (may be null): row b's history is its first traj_length(len[b * len_stride], t) steps, and h is
+// h_{L-1}; a history learner's step passes the length words of the gathered batch (z is then that batch).
 static int farmer_lstm_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const float* params, const float* z, int ldz, int m, int t,
-                               bool dense_tc, float* h, cudaStream_t st) {
+                               bool dense_tc, float* h, cudaStream_t st, const uint32_t* len, int len_stride) {
     const auto& T = l->tensors;
     // inference workspaces carry no GEMM workspace: actor batches are small and run on the fp32 FFMA kernels
     const int mode = w->gemm_ws ? l->cfg.gemm_mode : FI_GEMM_SIMT;
     const int rt = m * t;
-    // the recurrence on the tensor cores (lstm_tc.cu) needs the BPTT state arrays of a training workspace
-    const bool lstm_tc = farmer_use_half(l, w, rt) && w->hp_hi && w->cst && lstm_tc_enabled();
+    // the recurrence on the tensor cores (lstm_tc.cu) needs the BPTT state arrays of a training workspace, and has no lengths
+    const bool lstm_tc = !len && farmer_use_half(l, w, rt) && w->hp_hi && w->cst && lstm_tc_enabled();
     if (!lstm_tc) {
         LaunchScope ls("transpose_whh_kernel", st, 2.0 * 4 * kG4 * kLstmH, kWorkBytes);
         transpose_whh_kernel<<<(kG4 * kLstmH + 255) / 256, 256, 0, st>>>(params + T[1].offset, w->whh_t);
@@ -629,7 +721,8 @@ static int farmer_lstm_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const
     if (dense_tc) FI_TRY(dense_split_params(l, ds, params, st));
     // gates = z W_ih^T + b_ih for all B*T rows at once
     if (half_proj) {
-        FI_TRY(launch_amax_split_h(z, ldz, (size_t)rt, kZDim, kObsLdH, w->obs_hi, w->obs_lo, w->hs + kLstmHsObs, st));
+        // a history learner's padding rows leave the max out and are split as zeros
+        FI_TRY(launch_amax_split_h(z, ldz, (size_t)rt, kZDim, kObsLdH, w->obs_hi, w->obs_lo, w->hs + kLstmHsObs, st, w->history ? t : 0));
         HScale* wih_hs = dense_tc ? ds->hs + kHsW : w->hs + kLstmHsWih;   // the arena's scale bounds W_ih as well
         if (!dense_tc) FI_TRY(launch_amax(params + T[0].offset, kZDim, kG4, kZDim, wih_hs, st));
         FI_TRY(launch_split_h(params + T[0].offset, kZDim, kG4, kZDim, kObsLdH, w->wih_hi, w->wih_lo, wih_hs, dense_tc ? 0 : 1, st));
@@ -641,6 +734,11 @@ static int farmer_lstm_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const
         }
         FI_TRY(launch_gemm_tc_split(0, rt, kG4, kZDim, a, b, out, params + T[2].offset, 0, nullptr, 0, nullptr, 0, st));
     } else {
+        if (w->history) {   // the zero-padded copy of z (also the W_ih gradient's operand)
+            FI_TRY(launch_obs_length(z, rt, t, w->zpad, st));
+            z = w->zpad;
+            ldz = kObsLd;
+        }
         FI_TRY(launch_gemm(mode, 0, rt, kG4, kZDim, z, ldz, params + T[0].offset, kZDim, w->gates, kG4, params + T[2].offset,
                            0, nullptr, 0, w->gemm_ws, w->gemm_ws_bytes, st));
     }
@@ -650,15 +748,17 @@ static int farmer_lstm_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const
                                       h, kFeat, st));
     } else {
         // recurrent flops: 2 * 128 * 512 per (row, step)
-        LaunchScope ls("lstm_forward_kernel", st, 2.0 * kLstmH * kG4 * (double)rt, kWorkFlops);
-        static std::atomic<uint64_t> fwd_attr{0};
-        FI_TRY(ensure_dynamic_smem(fwd_attr, (const void*)lstm_forward_kernel, (int)kLstmFwdSmem));
+        // (with lengths: nominal flops, as if every row ran all t steps)
+        LaunchScope ls(len ? "lstm_forward_kernel_length" : "lstm_forward_kernel", st, 2.0 * kLstmH * kG4 * (double)rt, kWorkFlops);
+        static std::atomic<uint64_t> fwd_attr[2] = {};
+        const auto kernel = len ? lstm_forward_kernel<true> : lstm_forward_kernel<false>;
+        FI_TRY(ensure_dynamic_smem(fwd_attr[len ? 1 : 0], (const void*)kernel, (int)kLstmFwdSmem));
         // training on the 3xFP16 path: h_prev leaves the kernel as the fp16 pairs the W_hh gradient product reads
         const bool hp_pairs = half_proj && w->hp_hi;
-        launch_pdl(lstm_forward_kernel, dim3((m + kLstmRows - 1) / kLstmRows), dim3(kLstmThreads), kLstmFwdSmem, st, w->gates, w->whh_t,
+        launch_pdl(kernel, dim3((m + kLstmRows - 1) / kLstmRows), dim3(kLstmThreads), kLstmFwdSmem, st, w->gates, w->whh_t,
                    params + T[3].offset, m, t, hp_pairs ? nullptr : w->hprev, w->cst, h,
                    hp_pairs ? static_cast<__half*>(w->hp_hi) : nullptr, hp_pairs ? static_cast<__half*>(w->hp_lo) : nullptr,
-                   hp_pairs ? w->hs + kLstmHsHp : nullptr, lstm_trace_buffer());
+                   hp_pairs ? w->hs + kLstmHsHp : nullptr, lstm_trace_buffer(), len, len_stride);
         FI_TRY(ls.done());
         lstm_trace_report("forward (FFMA)", lstm_trace_buffer(), t, st);
     }
@@ -669,7 +769,9 @@ static int farmer_lstm_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const
 static int farmer_forward(fi_learner* l, FarmerWs* w, DenseStack* ds, const float* params, const float* z, int ldz, int m, int t,
                           cudaStream_t st) {
     const bool dense_tc = farmer_dense_tc(l, ds, m);
-    FI_TRY(farmer_lstm_forward(l, w, ds, params, z, ldz, m, t, dense_tc, w->feat, st));
+    // a history learner: each slot's length word, word 183 of its record 0
+    const uint32_t* len = w->history ? reinterpret_cast<const uint32_t*>(z) + kWLength : nullptr;
+    FI_TRY(farmer_lstm_forward(l, w, ds, params, z, ldz, m, t, dense_tc, w->feat, st, len, t * kRecWords));
     if (dense_tc) {
         FI_TRY(launch_amax_split_h(w->feat, kFeat, (size_t)m, kFeat, kFeatLdH, ds->in_hi, ds->in_lo, ds->hs + kHsIn, st));
         return dense_forward_split(l, ds, params, m, w->y, st);
@@ -715,18 +817,21 @@ int farmer_forward_backward(fi_learner* l, Player* p, const float* batch, int m,
     }
     // d = dfeat [m, ldd]: its first 128 columns are dL/dh_{T-1}; BPTT turns the stored gates into pre-activation gate gradients
     const int rt = m * t;
-    const bool lstm_tc = farmer_use_half(l, w, rt) && lstm_tc_enabled();
+    const bool lstm_tc = !w->history && farmer_use_half(l, w, rt) && lstm_tc_enabled();
     if (lstm_tc) {
         // also leaves db_ih = db_hh (the column sums of dG) and max |dG|
         FI_TRY(launch_lstm_backward_tc(w->gates, p->params + T[1].offset, w->cst, d, ldd, m, t, w->hs + kLstmHsDg, w->bias_part,
                                        g + T[2].offset, g + T[3].offset, st));
     } else {
-        LaunchScope ls("lstm_backward_kernel", st, 2.0 * kLstmH * kG4 * (double)m * t, kWorkFlops);
-        static std::atomic<uint64_t> bwd_attr{0};
-        FI_TRY(ensure_dynamic_smem(bwd_attr, (const void*)lstm_backward_kernel, (int)kLstmBwdSmem));
+        const bool hist = w->history;
+        LaunchScope ls(hist ? "lstm_backward_kernel_length" : "lstm_backward_kernel", st, 2.0 * kLstmH * kG4 * (double)m * t, kWorkFlops);
+        static std::atomic<uint64_t> bwd_attr[2] = {};
+        const auto kernel = hist ? lstm_backward_kernel<true> : lstm_backward_kernel<false>;
+        FI_TRY(ensure_dynamic_smem(bwd_attr[hist ? 1 : 0], (const void*)kernel, (int)kLstmBwdSmem));
         const int ctas = (m + kLstmRows - 1) / kLstmRows;
-        launch_pdl(lstm_backward_kernel, dim3(ctas), dim3(kLstmThreads), kLstmBwdSmem, st, w->gates, p->params + T[1].offset, w->cst, d, ldd, m,
-                   t, farmer_use_half(l, w, rt) ? w->hs + kLstmHsDg : nullptr, w->bias_part, lstm_trace_buffer());
+        launch_pdl(kernel, dim3(ctas), dim3(kLstmThreads), kLstmBwdSmem, st, w->gates, p->params + T[1].offset, w->cst, d, ldd, m,
+                   t, farmer_use_half(l, w, rt) ? w->hs + kLstmHsDg : nullptr, w->bias_part, lstm_trace_buffer(),
+                   hist ? reinterpret_cast<const uint32_t*>(batch) + kWLength : nullptr, t * kRecWords);
         FI_TRY(ls.done());
         lstm_trace_report("backward (FFMA)", lstm_trace_buffer(), t, st);
         // db_ih = db_hh = the CTAs' column sums of dG, added in CTA order
@@ -745,7 +850,9 @@ int farmer_forward_backward(fi_learner* l, Player* p, const float* batch, int m,
         FI_TRY(launch_gemm_tc_split(2, kG4, kLstmH, rt, dg, hp, TcOut{g + T[1].offset, kLstmH, nullptr, nullptr, 0, 0, nullptr, nullptr, 0, nullptr},
                                     nullptr, 0, nullptr, 0, w->split_ws, w->split_ws_bytes, st));
     } else {
-        FI_TRY(launch_gemm(mode, 2, kG4, kZDim, rt, w->gates, kG4, batch, kRecWords, g + T[0].offset, kZDim, nullptr, 0, nullptr,
+        // a history learner's z is the zero-padded copy the projection read
+        FI_TRY(launch_gemm(mode, 2, kG4, kZDim, rt, w->gates, kG4, w->history ? w->zpad : batch, w->history ? kObsLd : kRecWords,
+                           g + T[0].offset, kZDim, nullptr, 0, nullptr,
                            0, w->gemm_ws, w->gemm_ws_bytes, st));
         FI_TRY(launch_gemm(mode, 2, kG4, kLstmH, rt, w->gates, kG4, w->hprev, kLstmH, g + T[1].offset, kLstmH, nullptr, 0,
                            nullptr, 0, w->gemm_ws, w->gemm_ws_bytes, st));
@@ -763,12 +870,12 @@ int farmer_infer_alloc(fi_learner* l, Player* p, size_t states, size_t rows, siz
 }
 
 int farmer_infer(fi_learner* l, Player* p, const float* params, const float* z_dev, const float* x_dev, const uint32_t* offsets_dev,
-                 const uint32_t* state_dev, size_t states, size_t rows, size_t t, float* values_dev, int32_t* best_dev,
-                 cudaStream_t stream) {
+                 const uint32_t* state_dev, const uint32_t* lengths_dev, size_t states, size_t rows, size_t t, float* values_dev,
+                 int32_t* best_dev, cudaStream_t stream) {
     FarmerWs* w = p->farmer_inf_ws;
     if (!w || states > w->states || rows > w->rows || t > w->t) return set_error(FI_ERR_STATE, "farmer inference workspaces too small");
     // inference runs every product on the fp32 FFMA kernels: each row's value is then independent of the batch around it
-    FI_TRY(farmer_lstm_forward(l, w, &p->inf_dense, params, z_dev, kZDim, (int)states, (int)t, false, w->h_last, stream));
+    FI_TRY(farmer_lstm_forward(l, w, &p->inf_dense, params, z_dev, kZDim, (int)states, (int)t, false, w->h_last, stream, lengths_dev, 1));
     {
         const int n4 = (int)rows * kFeat4;
         LaunchScope ls("farmer_assemble_grouped_kernel", stream, 2.0 * 4 * kFeat * (double)rows, kWorkBytes);

@@ -80,7 +80,8 @@ class Learner:
                  publish_every: int = 1, rho_bar: float = 1.0, c_bar: float = 1.0, pg_rho_bar: float = 1.0,
                  lambda_: float = 1.0, baseline_cost: float = 0.5, entropy_cost: float = 0.01,
                  max_grad_norm: float = 0.0, rmsprop_alpha: float = 0.99, rmsprop_eps: float = 1e-8,
-                 rmsprop_momentum: float = 0.0, legal_action_mask: bool = False, variable_length: bool = False):
+                 rmsprop_momentum: float = 0.0, legal_action_mask: bool = False, variable_length: bool = False,
+                 history_length: bool = False):
         self._lib = _lib.load()
         self.num_players, self.buffer_capacity, self.entry_size, self.batch_size = p, B, S, M
         self.train_time_ms, self.checkpoint_frequency = r, c
@@ -98,6 +99,7 @@ class Learner:
         cfg.rmsprop_alpha, cfg.rmsprop_eps, cfg.rmsprop_momentum = rmsprop_alpha, rmsprop_eps, rmsprop_momentum
         cfg.legal_action_mask = int(legal_action_mask)   # records carry the legal-action word (fi_learner.h)
         cfg.variable_length = int(variable_length)       # record 0 of a trajectory carries its length (fi_learner.h)
+        cfg.history_length = int(history_length)         # FarmerLstm: record 0 of a slot carries its history's length
         self._ckpt = l.encode() if l else None
         cfg.checkpoint_location = self._ckpt
         self._h = self._lib.fi_learner_create(C.byref(cfg))
@@ -303,9 +305,11 @@ class Learner:
                                          values.ctypes.data), "fi_learner_infer")
         return values
 
-    def infer_grouped(self, player_index: int, z: np.ndarray, x: np.ndarray, offsets: np.ndarray):
+    def infer_grouped(self, player_index: int, z: np.ndarray, x: np.ndarray, offsets: np.ndarray, lengths: np.ndarray | None = None):
         """FarmerLstm inference of candidate actions grouped by state: z [S,T,162] is each state's history, x [R,484] the
         candidate rows, rows offsets[s] .. offsets[s+1]-1 belonging to state s (offsets [S+1], offsets[0] = 0, R = offsets[S]).
+        lengths [S] (fi_learner_infer_grouped_lengths): state s's history is z[s, :lengths[s]], 1 <= lengths[s] <= T, and the
+        rest of z[s] is not read; None runs fi_learner_infer_grouped (every history T steps).
         Returns (values [R], best [S]): best[s] is the index within state s's group of its largest value, lowest on ties."""
         zz = np.ascontiguousarray(z, dtype=np.float32)
         xx = np.ascontiguousarray(x, dtype=np.float32)
@@ -318,9 +322,17 @@ class Learner:
         states, t = zz.shape[0], zz.shape[1]
         values = np.empty(int(off[-1]), np.float32)
         best = np.empty(states, np.int32)
-        check(self._lib.fi_learner_infer_grouped(self._h, player_index, zz.ctypes.data, states, t, xx.ctypes.data,
-                                                 off.ctypes.data, values.ctypes.data, best.ctypes.data),
-              "fi_learner_infer_grouped")
+        if lengths is None:
+            check(self._lib.fi_learner_infer_grouped(self._h, player_index, zz.ctypes.data, states, t, xx.ctypes.data,
+                                                     off.ctypes.data, values.ctypes.data, best.ctypes.data),
+                  "fi_learner_infer_grouped")
+            return values, best
+        ln = np.ascontiguousarray(lengths, dtype=np.uint32)
+        if ln.shape != (states,):
+            raise ValueError(f"infer_grouped: lengths {ln.shape}, expected [{states}]")
+        check(self._lib.fi_learner_infer_grouped_lengths(self._h, player_index, zz.ctypes.data, states, t, ln.ctypes.data,
+                                                         xx.ctypes.data, off.ctypes.data, values.ctypes.data, best.ctypes.data),
+              "fi_learner_infer_grouped_lengths")
         return values, best
 
     def infer_sample(self, player_index: int, obs: np.ndarray, legal: np.ndarray | None = None, seed: int = 0,

@@ -189,6 +189,10 @@ typedef struct fi_learner_config {
        carries its length in word 183 of its record 0 (FI_REC_WORD_LENGTH) and the step trains on exactly those records;
        0 = every trajectory is entry_size records long, word 183 is not read. */
     int variable_length;
+    /* Appended after variable_length; fi_learner_config_default sets 0. FarmerLstm model only: 1 = each slot is one sample
+       whose move history z is its first L records, L read from word 183 of its record 0 (FI_REC_WORD_LENGTH), and the step
+       runs the LSTM over exactly those records; 0 = every history is entry_size records long, word 183 is not read. */
+    int history_length;
 } fi_learner_config;
 
 /* Trajectory record (FI_ELEMENT_SIZE bytes = 256 32-bit words) of the actor-critic model, the words the loss head reads
@@ -222,7 +226,16 @@ typedef struct fi_learner_config {
  *     (as zero observations), which keeps the step's shapes fixed.
  * What the actor does: it writes records 0..L-1 with L in word 183 of record 0, puts the bootstrap value in word 181 of
  * record L - 1 (any value if the episode ended there, because its discount is 0), and may hand fi_ring_write only those
- * L x FI_ELEMENT_SIZE bytes: the slot's older tail is then ignored. A learner with variable_length = 0 never reads word 183. */
+ * L x FI_ELEMENT_SIZE bytes: the slot's older tail is then ignored. A learner with variable_length = 0 never reads word 183.
+ *
+ * FarmerLstm move histories (history_length = 1) read the same word with the same rule. A slot is one sample: its value is
+ * the reference model on z[0..L-1] (cat(h_{L-1}, x) -> dense stack -> y), with the same loss, optimiser and mean over the batch,
+ * so the step equals the reference's train_step on each sample cut to T = L. The step reads z from words 0..161 of records
+ * 0..L-1, x from words 192..255 of records 0..7 whatever L is, and the target from word 181 of record 0. Words 0..161 of
+ * records L..T-1, and every word of records max(L, 8)..T-1, are never read into anything that reaches a loss, a gradient or
+ * a per-tensor scale: they may hold anything, NaN included. The step's shapes stay fixed (padding rows still run through the
+ * input projection as zero rows). What the actor does: it writes records 0..max(L, 8)-1 with L in word 183 of record 0, and
+ * may hand fi_ring_write only those max(L, 8) x FI_ELEMENT_SIZE bytes. A learner with history_length = 0 never reads word 183. */
 #define FI_REC_WORD_LENGTH 183
 
 typedef struct fi_learner fi_learner;
@@ -232,7 +245,8 @@ FI_API void fi_learner_config_default(fi_learner_config* cfg);
  * state and all step workspaces in HBM. Returns NULL on failure (see fi_last_error). An unknown
  * optimiser, max_grad_norm < 0 or not finite, rmsprop_alpha outside (0, 1), rmsprop_eps <= 0 or
  * rmsprop_momentum outside [0, 1), legal_action_mask other than 0 or 1 or set to 1 for the FarmerLstm model (which has
- * no policy), variable_length other than 0 or 1 or set to 1 for the FarmerLstm model, and, for the actor-critic model, a V-trace constant outside the range
+ * no policy), variable_length other than 0 or 1 or set to 1 for the FarmerLstm model, history_length other than 0 or 1 or set
+ * to 1 for the actor-critic model, and, for the actor-critic model, a V-trace constant outside the range
  * fi_learner_config states, is rejected (FI_ERR_ARG) before any device is looked for. */
 FI_API fi_learner* fi_learner_create(const fi_learner_config* cfg);
 FI_API void fi_learner_destroy(fi_learner* l);
@@ -316,6 +330,16 @@ FI_API int fi_learner_infer_stats(fi_learner* l, int player, uint64_t* calls, ui
  * argmax of the returned values on the host. Exploration (epsilon-greedy) stays with the actor: it needs no value. */
 FI_API int fi_learner_infer_grouped(fi_learner* l, int player, const float* z, size_t states, size_t t, const float* x,
                                     const uint32_t* offsets /* states + 1 */, float* values, int32_t* best);
+/* fi_learner_infer_grouped for states at different points of their games: state s's history is z[s, 0..lengths[s]-1] of z
+ * [states, t, 162]; z[s, lengths[s]..t-1] is never read (it may hold anything, NaN included). lengths is required, with
+ * 1 <= lengths[s] <= t. Each candidate's value and best[s] are bit-identical to fi_learner_infer_grouped called on that state
+ * alone with z[s, :lengths[s]] and t = lengths[s]. Any FarmerLstm learner (history_length on or off: inference reads no
+ * records). Combined with concurrent fi_learner_infer / fi_learner_infer_grouped requests of the same t (those run with every
+ * length t). FI_ERR_ARG, with the learner still usable, for a NULL lengths, a length outside 1..t, and every argument
+ * fi_learner_infer_grouped refuses. fi_learner_infer_stats counts the candidate rows. */
+FI_API int fi_learner_infer_grouped_lengths(fi_learner* l, int player, const float* z, size_t states, size_t t,
+                                            const uint32_t* lengths, const float* x, const uint32_t* offsets, float* values,
+                                            int32_t* best);
 /* Actor-critic model only. Runs the same forward as fi_learner_infer on obs [rows,162] and, for every row r, draws
  * actions[r] from the policy over that row's legal set. legal (may be NULL = all 16 legal) holds one word per row with
  * the FI_REC_WORD_LEGAL meaning: bit j set = action j legal, bits 16..31 ignored. greedy = 1 takes the arg-max instead.
