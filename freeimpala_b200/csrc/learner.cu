@@ -1352,6 +1352,12 @@ int fi_learner_dp_init(fi_learner* l, const void* ids, int rank, int world_size)
         cudaFree(d);
         l->dp_global_batch = (size_t)(total + 0.5);
     }
+    // A step graph captured before joining holds no all-reduce and, for FarmerLstm, the local 1/m of the mean: replaying it
+    // would train every rank on its own shard. The next step re-captures with the collective inside.
+    for (Player* p : l->players) {
+        std::lock_guard<std::mutex> step_lock(p->step_mu);
+        drop_graph(p);
+    }
     return FI_OK;
 }
 int fi_learner_dp_world(const fi_learner* l) { return l ? l->dp_world : 0; }

@@ -131,13 +131,17 @@ def _f64_dense_preactivations(params, z, x):
     return np.stack(pre)
 
 
-def _kink_signature(L, m, params_before, z, x):
-    """(units decided differently by the CUDA step and the float64 forward, the largest |pre-activation| / rms among them)."""
-    pre = _f64_dense_preactivations(params_before, z, x)
-    cuda_on = L.debug_relu_masks(0, m).reshape(5, m, 512).astype(bool)
+def kink_signature(masks, pre):
+    """(units decided differently by the CUDA step's ReLU decisions `masks` (debug_relu_masks, [5, m*512]) and the float64
+    pre-activations `pre` [5, m, 512], the largest |pre-activation| / rms among them)."""
+    cuda_on = np.asarray(masks).reshape(pre.shape).astype(bool)
     flips = cuda_on != (pre > 0)
     rel = np.abs(pre) / np.sqrt(np.mean(pre * pre, axis=(1, 2)))[:, None, None]
     return int(flips.sum()), float(rel[flips].max()) if flips.any() else 0.0
+
+
+def _kink_signature(L, m, params_before, z, x):
+    return kink_signature(L.debug_relu_masks(0, m), _f64_dense_preactivations(params_before, z, x))
 
 
 def _steps(opt):

@@ -20,6 +20,7 @@ import pytest
 import _util as U
 import history_reference as H
 from oracle import pyoracle as po
+from test_gpu_farmer_paths import kink_signature
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-5
@@ -43,11 +44,7 @@ def _uniform_lengths(seed, m, t):
 
 
 def _kink_signature(L, m, params_before, z, x, lengths):
-    pre = H.dense_preactivations(params_before, z, x, lengths)
-    cuda_on = L.debug_relu_masks(0, m).reshape(5, m, 512).astype(bool)
-    flips = cuda_on != (pre > 0)
-    rel = np.abs(pre) / np.sqrt(np.mean(pre * pre, axis=(1, 2)))[:, None, None]
-    return int(flips.sum()), float(rel[flips].max()) if flips.any() else 0.0
+    return kink_signature(L.debug_relu_masks(0, m), H.dense_preactivations(params_before, z, x, lengths))
 
 
 def _check_history_steps(fi, oracle, case, t, ms, lengths_of, *, m_cfg=None, gemm_mode="auto", seed=0):
