@@ -36,7 +36,7 @@ class FiLearnerConfig(C.Structure):
                 ("gemm_mode", c_int), ("publish_every", c_int), ("checkpoint_location", c_char_p),
                 ("max_grad_norm", c_double), ("rmsprop_alpha", c_double), ("rmsprop_eps", c_double),
                 ("rmsprop_momentum", c_double), ("legal_action_mask", c_int),
-                ("variable_length", c_int), ("history_length", c_int)]
+                ("variable_length", c_int), ("history_length", c_int), ("popart_beta", c_double)]
 
 
 class FiProfEntry(C.Structure):
@@ -85,6 +85,7 @@ SIGNATURES = {
     "fi_learner_set_lr": (c_int, [_P, c_int, c_double]),
     "fi_learner_sync": (c_int, [_P, c_int]),
     "fi_learner_steps_done": (c_u64, [_P, c_int]),
+    "fi_learner_popart_stats": (c_int, [_P, c_int, C.POINTER(c_double)]),
     "fi_learner_debug_relu_masks": (c_int, [_P, c_int, _P, c_size_t]),
     "fi_learner_param_count": (c_size_t, [_P]),
     "fi_learner_num_tensors": (c_int, [_P]),
@@ -117,6 +118,8 @@ SIGNATURES = {
     "fi_op_vtrace_loss_head": (c_int, [_P, c_int, c_int, _P, c_int] + [c_float] * 6 + [_P] * 5),
     "fi_op_vtrace_loss_head_legal": (c_int, [_P, c_int, c_int, _P, c_int] + [c_float] * 6 + [_P] * 5),
     "fi_op_vtrace_loss_head_opts": (c_int, [_P, c_int, c_int, _P, c_int] + [c_float] * 6 + [c_int, c_int] + [_P] * 5),
+    "fi_op_vtrace_loss_head_popart": (c_int, [_P, c_int, c_int, _P, c_int] + [c_float] * 6 + [c_int, c_int] + [_P] * 4 +
+                                      [c_float, c_float, _P, _P]),
     "fi_op_policy_sample": (c_int, [_P, c_int, c_size_t, _P, c_u64, c_int, _P, _P]),
     "fi_op_adam": (c_int, [c_int, c_double, c_i64, c_size_t, _P, _P, _P, _P, c_float, _P]),
     "fi_op_grad_norm_clip": (c_int, [c_size_t, _P, c_double, _P, _P, _P]),

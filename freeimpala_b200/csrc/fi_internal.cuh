@@ -1,5 +1,7 @@
 // Internal (non-ABI) entry points shared between the translation units of the library.
 #pragma once
+#include <cmath>
+
 #include "fi_common.cuh"
 
 namespace fi {
@@ -12,6 +14,8 @@ int ring_note_consumed(const void* dev_ptr, cudaStream_t consumer);
 // The learner's device loss slots: {total, pg, baseline, entropy} of the step, then the pre-clip gradient norm that
 // grad_norm_clip_kernel writes. The optimiser kernel copies all of them into the pinned read-back ring.
 constexpr int kLossWords = 5;
+// PopArt's {S1, S2, N} follow them (popart_sums_kernel writes them; the data-parallel all-reduce then sums words 0..7)
+constexpr int kLossPopArt = 5, kLossAlloc = 8;
 struct OptConfig {       // what the fused optimiser kernel computes (adam.cu)
     int kind = FI_OPT_ADAM;  // fi_opt_kind
     double lr = 0.0;
@@ -40,11 +44,62 @@ int launch_grad_norm_clip(size_t n, const float* g, double max_norm, double* nor
 int launch_vtrace_scan(int m, int t, const float* log_rho, const float* discount, const float* reward,
                        const float* value, const float* bootstrap, float rho_bar, float c_bar, float pg_rho_bar,
                        float lambda_, float* vs, float* pg_adv, cudaStream_t stream);
+// PopArt value normalisation (popart.cu, fi_learner_config.popart_beta). Per player, on the device: the statistics (mu, nu) and
+// the fp32 copies of mu and sigma(mu, nu) that the loss head reads.
+struct PopArtState {
+    double mu, nu;
+    float mu_f, sigma_f;
+};
+// sigma(mu, nu) = clamp(sqrt(max(nu - mu^2, 0)), 1e-4, 1e6), every operation rounded once (host and device give the same bits)
+__host__ __device__ __forceinline__ double popart_sigma(double mu, double nu) {
+#ifdef __CUDA_ARCH__
+    const double var = __dsub_rn(nu, __dmul_rn(mu, mu));
+    const double s = var > 0.0 ? __dsqrt_rn(var) : 0.0;
+#else
+    const double var = nu - mu * mu;
+    const double s = var > 0.0 ? std::sqrt(var) : 0.0;
+#endif
+    return s < 1e-4 ? 1e-4 : (s > 1e6 ? 1e6 : s);
+}
+// The published (reward-unit) value row from the normalised one: w_pub = sigma w, b_pub = sigma b + mu, in double, rounded once
+__host__ __device__ __forceinline__ float popart_publish_w(double sigma, float w) {
+#ifdef __CUDA_ARCH__
+    return (float)__dmul_rn(sigma, (double)w);
+#else
+    return (float)(sigma * (double)w);
+#endif
+}
+__host__ __device__ __forceinline__ float popart_publish_b(double sigma, double mu, float b) {
+#ifdef __CUDA_ARCH__
+    return (float)__dadd_rn(__dmul_rn(sigma, (double)b), mu);
+#else
+    return (float)(sigma * (double)b + mu);
+#endif
+}
+struct PopArtArgs {        // the loss head's PopArt operands; part == null: PopArt off
+    const float* ms = nullptr;   // device {mu, sigma} (PopArtState::mu_f), or null: mu / sigma below
+    float mu = 0.f, sigma = 1.f;
+    double* part = nullptr;      // [m][3] per-trajectory {sum vs, sum vs^2, valid steps}
+};
+// sums[0..2] = the partials [m][3] summed over the trajectories in index order (one block)
+int launch_popart_sums(const double* part, int m, double* sums, cudaStream_t st);
+// The statistics update and value-row rescale after the optimiser (update = 1, sums = the reduced {S1, S2, N}), and the
+// published value row written into `snap` (may be null) from the arena and the (updated) statistics. update = 0 only publishes.
+struct PopArtLaunchDesc {  // by value, so that the step graph can re-parameterise the node (the snapshot changes per step)
+    const void* func;
+    PopArtState* st; const double* sums; double beta; float* params; float* snap; int w_off, b_off, update;
+    void* args[8];
+};
+void popart_launch_desc(PopArtState* st, const double* sums, double beta, float* params, float* snap, int w_off, int b_off, int update,
+                        PopArtLaunchDesc* d);
+int launch_popart_update(PopArtLaunchDesc* d, cudaStream_t stream);
+
 // legal: legal-action masking (record word 182); lengths: each trajectory's length from word 183 of its record 0
 int launch_vtrace_loss_head(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar,
                             float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, bool legal, bool lengths,
                             float* dhead, float* vs, float* pg_adv, double* losses, cudaStream_t stream,
-                            float* dhead_hi = nullptr, float* dhead_lo = nullptr, int ld_split = 0, struct HScale* dhead_hs = nullptr);
+                            float* dhead_hi = nullptr, float* dhead_lo = nullptr, int ld_split = 0, struct HScale* dhead_hs = nullptr,
+                            const PopArtArgs& pa = PopArtArgs{});
 
 // trans: 0 "NT" C = A[m,k] B[n,k]^T; 1 "NN" C = A[m,k] B[k,n]; 2 "TN" C = A[k,m]^T B[k,n].
 int launch_gemm_simt(int trans, int m, int n, int k, const float* a, int lda, const float* b, int ldb, float* c,

@@ -179,11 +179,17 @@ int publish_end(Player* p, uint64_t version, int sn) {
     return FI_OK;
 }
 
-// Enqueue the publication of the weights currently in p->params as `version` (snapshot by a device-to-device copy).
+// Enqueue the publication of the weights currently in p->params as `version` (snapshot by a device-to-device copy; with PopArt
+// the snapshot's value row is then rewritten in reward units by the update kernel's publish-only mode).
 int publish_async(Player* p, uint64_t version) {
     int sn = 0;
     FI_TRY(publish_begin(p, &sn));
     FI_CUDA_OK(cudaMemcpyAsync(p->store.dev_snap[sn], p->params, p->store.bytes, cudaMemcpyDeviceToDevice, p->stream));
+    if (p->popart) {
+        fi::PopArtLaunchDesc d;
+        fi::popart_launch_desc(p->popart, nullptr, 0.0, p->params, p->store.dev_snap[sn], p->popart_w_off, p->popart_b_off, 0, &d);
+        FI_TRY(fi::launch_popart_update(&d, p->stream));
+    }
     return publish_end(p, version, sn);
 }
 
@@ -216,6 +222,9 @@ void free_player(fi_learner* l, Player* p) {
     fi::dense_free(&p->dense);
     fi::dense_free(&p->inf_dense);
     float* dev[] = {p->params, p->grads, p->adam_m, p->adam_v, p->head, p->dhead, p->obs, p->inf_in, p->inf_x, p->inf_out};
+    void* pa[] = {p->popart, p->popart_part};
+    for (void* d : pa)
+        if (d) cudaFree(d);
     for (float* d : dev)
         if (d) cudaFree(d);
     for (float* d : p->store.dev_snap)
@@ -253,8 +262,17 @@ int create_player(fi_learner* l, int index) {
         FI_CUDA_OK(cudaMalloc((void**)a, abytes));
         FI_CUDA_OK(cudaMemset(*a, 0, abytes));
     }
-    FI_CUDA_OK(cudaMalloc((void**)&p->d_losses, fi::kLossWords * sizeof(double)));
-    FI_CUDA_OK(cudaMemset(p->d_losses, 0, fi::kLossWords * sizeof(double)));
+    FI_CUDA_OK(cudaMalloc((void**)&p->d_losses, fi::kLossAlloc * sizeof(double)));
+    FI_CUDA_OK(cudaMemset(p->d_losses, 0, fi::kLossAlloc * sizeof(double)));
+    if (l->cfg.popart_beta > 0.0) {
+        const fi::PopArtState init{0.0, 1.0, 0.f, 1.f};
+        FI_CUDA_OK(cudaMalloc((void**)&p->popart, sizeof(fi::PopArtState)));
+        FI_CUDA_OK(cudaMemcpy(p->popart, &init, sizeof(init), cudaMemcpyHostToDevice));
+        FI_CUDA_OK(cudaMalloc((void**)&p->popart_part, 3 * sizeof(double) * l->cfg.batch_size));
+        FI_CUDA_OK(cudaMemset(p->popart_part, 0, 3 * sizeof(double) * l->cfg.batch_size));
+        p->popart_w_off = (int)(l->tensors[10].offset + (size_t)fi::kNumActions * fi::kHid);   // head.w row 16
+        p->popart_b_off = (int)(l->tensors[11].offset + fi::kNumActions);                      // head.b[16]
+    }
     const size_t ring_bytes = (Player::kLossRing + 1) * fi::kLossWords * sizeof(double);
     FI_CUDA_OK(cudaHostAlloc((void**)&p->h_losses, ring_bytes, cudaHostAllocPortable | cudaHostAllocMapped));
     memset(p->h_losses, 0, ring_bytes);
@@ -316,6 +334,9 @@ bool file_exists(const std::string& path) {
 const char kOptMagic[8] = {'F', 'I', 'O', 'P', 'T', '0', '0', '1'};
 const char kRmsMagic[8] = {'F', 'I', 'R', 'M', 'S', '0', '0', '1'};
 const char* opt_magic(const fi_learner* l) { return l->cfg.optimizer == FI_OPT_RMSPROP ? kRmsMagic : kOptMagic; }
+// PopArt section, after the optimiser section: mu, nu (doubles), then the normalised value row (head.w row 16, head.b[16])
+const char kPopMagic[8] = {'F', 'I', 'P', 'O', 'P', '0', '0', '1'};
+constexpr size_t kPopRow = fi::kHid + 1;
 
 }  // namespace
 
@@ -350,6 +371,7 @@ void fi_learner_config_default(fi_learner_config* c) {
     c->legal_action_mask = 0;    // every action legal; record word 182 is not read
     c->variable_length = 0;      // every trajectory entry_size records long; record word 183 is not read
     c->history_length = 0;       // every FarmerLstm history entry_size records long; record word 183 is not read
+    c->popart_beta = 0.0;        // no PopArt: the value head regresses raw returns
 }
 
 fi_learner* fi_learner_create(const fi_learner_config* cfg) {
@@ -400,6 +422,14 @@ fi_learner* fi_learner_create(const fi_learner_config* cfg) {
     }
     if (!farmer && cfg->history_length) {
         set_error(FI_ERR_ARG, "fi_learner_create: history_length is for the FarmerLstm model; the actor-critic has variable_length");
+        return nullptr;
+    }
+    if (!(cfg->popart_beta >= 0.0 && cfg->popart_beta <= 1.0)) {
+        set_error(FI_ERR_ARG, "fi_learner_create: popart_beta must be finite and in [0, 1] (0 = off), got %g", cfg->popart_beta);
+        return nullptr;
+    }
+    if (farmer && cfg->popart_beta > 0.0) {
+        set_error(FI_ERR_ARG, "fi_learner_create: popart_beta is for the actor-critic model; the FarmerLstm step has no PopArt");
         return nullptr;
     }
     if (!farmer) {   // V-trace constants: a NaN or out-of-range value would otherwise surface as NaN or meaningless losses
@@ -520,7 +550,9 @@ int enqueue_allreduce(fi_learner* l, Player* p) {
                        2.0 * (l->dp_world - 1) / l->dp_world * 4.0 * (double)l->param_count, fi::kWorkBytes);
     FI_NCCL_OK(n.GroupStart());
     FI_NCCL_OK(n.AllReduce(p->grads, p->grads, l->param_count, ncclFloat, ncclSum, (ncclComm_t)p->nccl_comm, p->stream));
-    FI_NCCL_OK(n.AllReduce(p->d_losses, p->d_losses, 4, ncclDouble, ncclSum, (ncclComm_t)p->nccl_comm, p->stream));
+    // the loss sums, and with PopArt the statistics' sums S1, S2, N too (word 4, the gradient norm, is written after this)
+    FI_NCCL_OK(n.AllReduce(p->d_losses, p->d_losses, p->popart ? fi::kLossAlloc : 4, ncclDouble, ncclSum, (ncclComm_t)p->nccl_comm,
+                           p->stream));
     FI_NCCL_OK(n.GroupEnd());
     ls.done_external();
     return FI_OK;
@@ -569,6 +601,20 @@ int opt_desc_for(fi_learner* l, Player* p, const UpdateTicket& u, fi::OptLaunchD
 int enqueue_clip(fi_learner* l, Player* p) {
     if (!(l->cfg.max_grad_norm > 0.0)) return FI_OK;
     return fi::launch_grad_norm_clip(l->param_count, p->grads, l->cfg.max_grad_norm, p->d_losses + 4, p->clip_coef, p->norm_ws, p->stream);
+}
+
+// PopArt: the statistics update, the value-row rescale and (when the step publishes) the snapshot's reward-unit value row, right
+// after the optimiser. The snapshot changes per step, so the graph path re-parameterises this node like the optimiser's.
+void popart_desc_for(fi_learner* l, Player* p, const UpdateTicket& u, fi::PopArtLaunchDesc* d) {
+    fi::popart_launch_desc(p->popart, p->d_losses + fi::kLossPopArt, l->cfg.popart_beta, p->params, u.publish ? p->store.dev_snap[u.sn] : nullptr,
+                           p->popart_w_off, p->popart_b_off, 1, d);
+}
+
+int enqueue_popart(fi_learner* l, Player* p, const UpdateTicket& u) {
+    if (!p->popart) return FI_OK;
+    fi::PopArtLaunchDesc d;
+    popart_desc_for(l, p, u, &d);
+    return fi::launch_popart_update(&d, p->stream);
 }
 
 int finish_update(fi_learner* l, Player* p, const UpdateTicket& u) {
@@ -622,6 +668,7 @@ void drop_graph(Player* p) {
     p->graph_exec = nullptr;
     p->graph = nullptr;
     p->graph_opt_node = nullptr;
+    p->graph_popart_node = nullptr;
 }
 
 // The whole step -- forward, fused loss head, backward, gradient finalisation, (NCCL all-reduce,) optimiser -- as ONE CUDA
@@ -658,6 +705,7 @@ int step_with_graph(fi_learner* l, Player* p, const fi_batch* b, bool* used) {
             e = cudaLaunchKernel(d.func, dim3(d.grid), dim3(d.block), d.args, 0, p->stream);
             rc = e == cudaSuccess ? ls.done() : FI_ERR_CUDA;
         }
+        if (rc == FI_OK) rc = enqueue_popart(l, p, u);
         const cudaError_t e_end = cudaStreamEndCapture(p->stream, &graph);
         cudaGraphExec_t exec = nullptr;
         if (rc == FI_OK && e_end == cudaSuccess && graph) {
@@ -666,18 +714,23 @@ int step_with_graph(fi_learner* l, Player* p, const fi_batch* b, bool* used) {
             cudaGraphGetNodes(graph, nullptr, &nn);
             std::vector<cudaGraphNode_t> nodes(nn);
             cudaGraphGetNodes(graph, nodes.data(), &nn);
-            cudaGraphNode_t opt_node = nullptr;
+            cudaGraphNode_t opt_node = nullptr, popart_node = nullptr;
+            fi::PopArtLaunchDesc pd;
+            popart_desc_for(l, p, u, &pd);
             for (cudaGraphNode_t nd : nodes) {
                 cudaGraphNodeType ty;
                 if (cudaGraphNodeGetType(nd, &ty) != cudaSuccess || ty != cudaGraphNodeTypeKernel) continue;
                 cudaKernelNodeParams kp;
-                if (cudaGraphKernelNodeGetParams(nd, &kp) == cudaSuccess && kp.func == d.func) opt_node = nd;
+                if (cudaGraphKernelNodeGetParams(nd, &kp) != cudaSuccess) continue;
+                if (kp.func == d.func) opt_node = nd;
+                if (p->popart && kp.func == pd.func) popart_node = nd;
             }
-            if (opt_node && cudaGraphInstantiate(&exec, graph, 0) == cudaSuccess) {
+            if (opt_node && (popart_node || !p->popart) && cudaGraphInstantiate(&exec, graph, 0) == cudaSuccess) {
                 p->graph_exec = exec;
                 p->graph = graph;
                 graph = nullptr;
                 p->graph_opt_node = opt_node;
+                p->graph_popart_node = popart_node;
                 p->graph_batch_ptr = b->dev_ptr;
                 p->graph_batch_m = b->num_slots;
                 p->graph_kernels = fi::launch_counter().load() - n0;
@@ -698,6 +751,7 @@ int step_with_graph(fi_learner* l, Player* p, const fi_batch* b, bool* used) {
             if (cudaLaunchKernel(d.func, dim3(d.grid), dim3(d.block), d.args, 0, p->stream) != cudaSuccess)
                 return set_error(FI_ERR_CUDA, "launch of fused_opt_kernel failed");
             FI_TRY(ls.done());
+            FI_TRY(enqueue_popart(l, p, u));
             FI_TRY(fi::ring_note_consumed(b->dev_ptr, p->stream));
             *used = true;
             return finish_update(l, p, u);
@@ -711,6 +765,18 @@ int step_with_graph(fi_learner* l, Player* p, const fi_batch* b, bool* used) {
         kp.kernelParams = d.args;
         kp.extra = nullptr;
         FI_CUDA_OK(cudaGraphExecKernelNodeSetParams((cudaGraphExec_t)p->graph_exec, (cudaGraphNode_t)p->graph_opt_node, &kp));
+        if (p->popart) {
+            fi::PopArtLaunchDesc pd;
+            popart_desc_for(l, p, u, &pd);
+            cudaKernelNodeParams pk = {};
+            pk.func = const_cast<void*>(pd.func);
+            pk.gridDim = dim3(1);
+            pk.blockDim = dim3(fi::kHid);
+            pk.sharedMemBytes = 0;
+            pk.kernelParams = pd.args;
+            pk.extra = nullptr;
+            FI_CUDA_OK(cudaGraphExecKernelNodeSetParams((cudaGraphExec_t)p->graph_exec, (cudaGraphNode_t)p->graph_popart_node, &pk));
+        }
         p->last_rows = b->num_slots * l->cfg.entry_size;
         p->grads_valid = true;
     }
@@ -747,6 +813,7 @@ int fi_learner_apply_update(fi_learner* l, int player) {
     FI_TRY(fi::launch_opt(opt_config(l, p), p->opt_step, l->param_count, p->params, p->grads, p->adam_m, p->adam_v, 1.0f,
                           p->stream, p->clip_coef, u.publish ? p->store.dev_snap[u.sn] : nullptr, p->d_losses,
                           p->h_losses_dev + fi::kLossWords * u.slot));
+    FI_TRY(enqueue_popart(l, p, u));
     return finish_update(l, p, u);
 }
 
@@ -822,6 +889,20 @@ int fi_learner_set_lr(fi_learner* l, int player, double lr) {
     if (!(lr >= 0.0) || !std::isfinite(lr)) return set_error(FI_ERR_ARG, "fi_learner_set_lr: lr must be finite and >= 0, got %g", lr);
     std::lock_guard<std::mutex> step_lock(p->step_mu);   // the next update (graph or stream) reads it under the same lock
     p->lr = lr;
+    return FI_OK;
+}
+int fi_learner_popart_stats(fi_learner* l, int player, double out[3]) {
+    Player* p = get_player(l, player);
+    if (!p || !out) return set_error(FI_ERR_ARG, "fi_learner_popart_stats: null argument");
+    if (!p->popart) return set_error(FI_ERR_STATE, "fi_learner_popart_stats: the learner runs without PopArt (popart_beta = 0)");
+    FI_CUDA_OK(cudaSetDevice(l->cfg.device));
+    std::lock_guard<std::mutex> step_lock(p->step_mu);
+    FI_CUDA_OK(cudaStreamSynchronize(p->stream));
+    fi::PopArtState st;
+    FI_CUDA_OK(cudaMemcpy(&st, p->popart, sizeof(st), cudaMemcpyDeviceToHost));
+    out[0] = st.mu;
+    out[1] = st.nu;
+    out[2] = fi::popart_sigma(st.mu, st.nu);
     return FI_OK;
 }
 uint64_t fi_learner_steps_done(fi_learner* l, int player) {
@@ -1190,6 +1271,8 @@ int fi_model_save(fi_learner* l, int player, uint64_t iteration, int with_optimi
     std::vector<unsigned char> blob(s.bytes);
     std::vector<float> om, ov;
     uint64_t version = 0, opt_step = 0;
+    fi::PopArtState pst{};
+    float prow[kPopRow];   // PopArt: the arena's normalised value row
     if (with_optimizer_state) {  // consistent (weights, m, v, step): quiesce the player's stream
         std::lock_guard<std::mutex> step_lock(p->step_mu);
         FI_CUDA_OK(cudaStreamSynchronize(p->stream));
@@ -1198,6 +1281,17 @@ int fi_model_save(fi_learner* l, int player, uint64_t iteration, int with_optimi
         FI_CUDA_OK(cudaMemcpy(blob.data(), p->params, s.bytes, cudaMemcpyDeviceToHost));
         FI_CUDA_OK(cudaMemcpy(om.data(), p->adam_m, s.bytes, cudaMemcpyDeviceToHost));
         FI_CUDA_OK(cudaMemcpy(ov.data(), p->adam_v, s.bytes, cudaMemcpyDeviceToHost));
+        if (p->popart) {   // the blob is the published model: the value row in reward units, as the update kernel publishes it
+            FI_CUDA_OK(cudaMemcpy(&pst, p->popart, sizeof(pst), cudaMemcpyDeviceToHost));
+            float* w = reinterpret_cast<float*>(blob.data());
+            const double sig = fi::popart_sigma(pst.mu, pst.nu);
+            for (int i = 0; i < fi::kHid; i++) {
+                prow[i] = w[p->popart_w_off + i];
+                w[p->popart_w_off + i] = fi::popart_publish_w(sig, prow[i]);
+            }
+            prow[fi::kHid] = w[p->popart_b_off];
+            w[p->popart_b_off] = fi::popart_publish_b(sig, pst.mu, prow[fi::kHid]);
+        }
         version = p->version;
         opt_step = (uint64_t)p->opt_step;
     } else {  // the published model, as the reference's saveModel copies models[p] (:396)
@@ -1227,6 +1321,9 @@ int fi_model_save(fi_learner* l, int player, uint64_t iteration, int with_optimi
             const uint64_t n = l->param_count;
             ok = fwrite(opt_magic(l), 1, 8, f) == 8 && fwrite(&opt_step, 8, 1, f) == 1 && fwrite(&n, 8, 1, f) == 1 &&
                  fwrite(om.data(), 4, n, f) == n && fwrite(ov.data(), 4, n, f) == n;
+            if (ok && p->popart)
+                ok = fwrite(kPopMagic, 1, 8, f) == 8 && fwrite(&pst.mu, 8, 1, f) == 1 && fwrite(&pst.nu, 8, 1, f) == 1 &&
+                     fwrite(prow, 4, kPopRow, f) == kPopRow;
         }
         ok = (fclose(f) == 0) && ok;
         if (!ok) {
@@ -1295,6 +1392,21 @@ int fi_model_load(fi_learner* l, const char* dir) {
             ov.resize(n);
             have_opt = fread(om.data(), 4, n, f) == n && fread(ov.data(), 4, n, f) == n;
         }
+        // PopArt: the statistics and the normalised value row, if the file has them; otherwise mu = 0, nu = 1 (sigma = 1), which
+        // keeps the blob's reward-unit outputs. A learner without PopArt never reads past the optimiser section.
+        fi::PopArtState pst{0.0, 1.0, 0.f, 1.f};
+        float prow[kPopRow];
+        char pmagic[8];
+        const bool have_pop = p->popart && have_opt && fread(pmagic, 1, 8, f) == 8 && memcmp(pmagic, kPopMagic, 8) == 0 &&
+                              fread(&pst.mu, 8, 1, f) == 1 && fread(&pst.nu, 8, 1, f) == 1 && fread(prow, 4, kPopRow, f) == kPopRow;
+        if (have_pop) {
+            pst.mu_f = (float)pst.mu;
+            pst.sigma_f = (float)fi::popart_sigma(pst.mu, pst.nu);
+            memcpy(blob.data() + p->popart_w_off, prow, fi::kHid * sizeof(float));
+            blob[p->popart_b_off] = prow[fi::kHid];
+        } else {
+            pst = fi::PopArtState{0.0, 1.0, 0.f, 1.f};
+        }
         fclose(f);
         std::lock_guard<std::mutex> step_lock(p->step_mu);
         FI_CUDA_OK(cudaStreamSynchronize(p->stream));
@@ -1304,6 +1416,7 @@ int fi_model_load(fi_learner* l, const char* dir) {
             FI_CUDA_OK(cudaMemcpy(p->adam_v, ov.data(), n * 4, cudaMemcpyHostToDevice));
             p->opt_step = (int64_t)opt_step;
         }
+        if (p->popart) FI_CUDA_OK(cudaMemcpy(p->popart, &pst, sizeof(pst), cudaMemcpyHostToDevice));
         p->version = version;
         FI_TRY(publish_sync(p, version));
         loaded++;

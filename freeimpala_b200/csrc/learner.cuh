@@ -137,7 +137,7 @@ struct Player {
     void* norm_ws = nullptr;    // grad_norm_clip_kernel's block partials and ticket
     std::atomic<uint64_t> steps_done{0};  // written under step_mu (release), read without it by fi_learner_losses_at / steps_done
     uint64_t version = 1;       // version of the weights in `params` (Model ctor -> 1, :55-58,127)
-    double* d_losses = nullptr; // device double[kLossWords]: the four loss sums, then the step's pre-clip gradient norm
+    double* d_losses = nullptr; // device double[kLossAlloc]: the four loss sums, the step's pre-clip gradient norm, PopArt's S1, S2, N
     // loss read-back ring: step s (1-based) lands in slot s % kLossRing of the pinned array, so that a host loop can read
     // step s-1's losses while step s runs (fi_learner_losses_at) without stalling the stream
     static constexpr int kLossRing = 8;
@@ -184,6 +184,12 @@ struct Player {
     size_t graph_batch_m = 0;
     uint64_t graph_kernels = 0;       // launches inside the graph (fi_kernel_launch_count)
     bool graph_failed = false;
+    // PopArt (popart_beta > 0): the statistics, the loss head's per-trajectory partials [batch_size][3] and the update kernel's
+    // node in the step graph (re-parameterised every step with the snapshot it publishes into, like the optimiser's)
+    PopArtState* popart = nullptr;
+    double* popart_part = nullptr;
+    int popart_w_off = 0, popart_b_off = 0;   // head.w row 16 and head.b[16] in the arena
+    void* graph_popart_node = nullptr;
     ModelStore store;
     uint64_t checkpoint_counter = 0;
     std::mutex save_mu;         // one fi_model_save per player at a time

@@ -52,6 +52,12 @@ int ac_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int
     const int rows = m * t;
     cudaStream_t st = p->stream;
     const bool legal = c.legal_action_mask != 0, lengths = c.variable_length != 0;
+    PopArtArgs pa;   // PopArt: mu and sigma from the player's device slot, per-trajectory partials reduced right after the loss head
+    if (p->popart) {
+        pa.ms = &p->popart->mu_f;
+        pa.part = p->popart_part;
+    }
+    auto popart_sums = [&]() { return p->popart ? launch_popart_sums(p->popart_part, m, p->d_losses + kLossPopArt, st) : FI_OK; };
     if (!s->split) {
         const float* x = batch;   // the first GEMM's input: the batch itself (row stride 256 words) or its length-aware copy
         int ldx = kRecWords;
@@ -63,7 +69,9 @@ int ac_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int
         FI_TRY(dense_forward_plain(l, s, FI_GEMM_SIMT, p->params, x, ldx, rows, p->head, p->gemm_ws, p->gemm_ws_bytes, st));
         FI_TRY(launch_zero2(p->d_losses, 4 * sizeof(double), nullptr, 0, st));
         FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
-                                       c.baseline_cost, c.entropy_cost, legal, lengths, p->dhead, nullptr, nullptr, p->d_losses, st));
+                                       c.baseline_cost, c.entropy_cost, legal, lengths, p->dhead, nullptr, nullptr, p->d_losses, st,
+                                       nullptr, nullptr, 0, nullptr, pa));
+        FI_TRY(popart_sums());
         return dense_backward_plain(l, s, FI_GEMM_SIMT, p->params, x, ldx, p->dhead, rows, p->grads, nullptr, p->gemm_ws,
                                     p->gemm_ws_bytes, p->colsum_ws, p->colsum_ws_bytes, st);
     }
@@ -85,14 +93,15 @@ int ac_forward_backward(fi_learner* l, Player* p, const float* batch, int m, int
     if (s->half) {  // the loss head writes plain fp32 rows and their max |x|; the fp16 split follows (13 MB)
         FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
                                        c.baseline_cost, c.entropy_cost, legal, lengths, p->dhead, nullptr, nullptr, p->d_losses, st,
-                                       nullptr, nullptr, 0, s->hs + kHsDout));
+                                       nullptr, nullptr, 0, s->hs + kHsDout, pa));
         FI_TRY(launch_split_h(p->dhead, kHead, (size_t)rows, kHead, kDoutLd, s->dout_hi, s->dout_lo, s->hs + kHsDout, 1, st));
     } else {
         FI_TRY(launch_zero2(p->d_losses, 4 * sizeof(double), nullptr, 0, st));
         FI_TRY(launch_vtrace_loss_head(batch, m, t, p->head, kHead, c.rho_bar, c.c_bar, c.pg_rho_bar, c.lambda_,
                                        c.baseline_cost, c.entropy_cost, legal, lengths, nullptr, nullptr, nullptr, p->d_losses, st,
-                                       (float*)s->dout_hi, (float*)s->dout_lo, kDoutLd));
+                                       (float*)s->dout_hi, (float*)s->dout_lo, kDoutLd, nullptr, pa));
     }
+    FI_TRY(popart_sums());
     return dense_backward_split(l, s, p->dhead, rows, p->grads, nullptr, 0, p->colsum_ws, p->colsum_ws_bytes, st);
 }
 

@@ -9,6 +9,8 @@
 // The reverse-time first-order recurrence is associative under (a1,b1)o(a2,b2) =
 // (a1 a2, b1 + a1 b2), so each warp scans 32 time steps at once with shuffles and carries one
 // scalar across 32-step chunks (last chunk first).
+#include <cmath>
+
 #include "fi_internal.cuh"
 
 namespace fi {
@@ -201,14 +203,21 @@ int launch_vtrace_scan(int m, int t, const float* log_rho, const float* discount
 // pg_adv rows (the buffers are reused across steps, so those rows are written). Lanes past L read the head row and the record
 // of step L - 1, as the lanes past t read those of step t - 1, and their d(head) row is replaced by a select: no byte of a
 // padding record or head row reaches the arithmetic. A chunk wholly past L only stores its zero rows.
+// kPopArt (fi_learner_config.popart_beta > 0): head column 16 is the normalised value n and V = sigma n + mu feeds the scan (the
+// bootstrap stays in reward units); the policy gradient and its loss use A / sigma, the baseline regresses n on (vs - mu) / sigma.
+// mu and sigma come from pa_ms (the learner's device slot, so a replayed graph picks up each step's statistics) or, when that is
+// null, from pa_mu / pa_sigma. Each warp writes its trajectory's {sum vs, sum vs^2, valid steps} to pa_part[3 traj ..]: fixed-order
+// partials that popart_sums_kernel (popart.cu) reduces, so the statistics do not depend on the order blocks finish in. The
+// parameters are appended after the existing ones, so the <kLegal, kLength, false> instantiations keep the parent's SASS.
 constexpr int kLossWarps = 4;
-template <bool kLegal, bool kLength>
+template <bool kLegal, bool kLength, bool kPopArt>
 __global__ void __launch_bounds__(32 * kLossWarps)
 vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const float* __restrict__ head, int ldh,
                         float rho_bar, float c_bar, float pg_rho_bar, float lambda_, float baseline_cost,
                         float entropy_cost, float* __restrict__ dhead, float* __restrict__ vs_out,
                         float* __restrict__ adv_out, double* __restrict__ losses, float* __restrict__ dhead_hi,
-                        float* __restrict__ dhead_lo, int ld_split, HScale* __restrict__ dhead_hs) {
+                        float* __restrict__ dhead_lo, int ld_split, HScale* __restrict__ dhead_hs,
+                        const float* __restrict__ pa_ms, float pa_mu, float pa_sigma, double* __restrict__ pa_part) {
     __shared__ float s_head[kLossWarps][32 * kHead];
     __shared__ float s_out[kLossWarps][2][32 * 33];
     pdl_wait();
@@ -225,6 +234,12 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
     float carry = 0.f, vs_next_chunk = boot, v_next_chunk = boot;
     double l_pg = 0.0, l_bl = 0.0, l_ent = 0.0;
     float dmax = 0.f;
+    float pmu = 0.f, psig = 1.f;
+    double s1 = 0.0, s2 = 0.0;   // kPopArt: sum vs, sum vs^2 over the trajectory's valid steps
+    if constexpr (kPopArt) {
+        pmu = pa_ms ? __ldg(pa_ms) : pa_mu;
+        psig = pa_ms ? __ldg(pa_ms + 1) : pa_sigma;
+    }
     for (int c0 = ((t - 1) >> 5) << 5; c0 >= 0; c0 -= 32) {
         const int s = c0 + lane;
         // rows base_row .. base_row + nrows - 1 get d(head) rows; the first nvalid of them are valid steps
@@ -286,7 +301,8 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
             z[j] = h[j];
             mx = fmaxf(mx, on(j) ? z[j] : -INFINITY);
         }
-        const float v = h[kNumActions];
+        const float nv = h[kNumActions];   // kPopArt: the normalised value n
+        const float v = kPopArt ? fmaf(psig, nv, pmu) : nv;
         int act = __float_as_int(rf[kWAction - 160]);
         act = act < 0 ? 0 : (act >= kNumActions ? kNumActions - 1 : act);
         float se = 0.f, mu_se = 0.f, mu_a = 0.f, z_a = 0.f;
@@ -326,14 +342,16 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
         float vs_next = __shfl_down_sync(0xffffffffu, vs, 1);
         if (lane == 31 || s >= tl - 1) vs_next = vs_next_chunk;
         const float adv = fminf(pg_rho_bar, is) * (r + g * vs_next - v);
+        const float adv_n = kPopArt ? adv / psig : adv;               // the advantage in normalised units
+        const float verr = kPopArt ? (vs - pmu) / psig - nv : vs - v;  // baseline residual (normalised target - n)
         float dv[kHead];
 #pragma unroll
         for (int j = 0; j < kNumActions; j++) {
-            const float d_pg = adv * (p[j] - (j == act ? 1.f : 0.f));
+            const float d_pg = adv_n * (p[j] - (j == act ? 1.f : 0.f));
             const float d_ent = p[j] * (z[j] - plogp);
             dv[j] = fmaf(entropy_cost, d_ent, d_pg);   // 0 outside the support: p = 0 and j != act
         }
-        dv[kNumActions] = -baseline_cost * (vs - v);
+        dv[kNumActions] = -baseline_cost * verr;
         if constexpr (kLength) {
 #pragma unroll
             for (int j = 0; j < kHead; j++) dv[j] = valid ? dv[j] : 0.f;   // padding step: a zero row
@@ -347,9 +365,13 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
             for (int j = 0; j < kHead; j++) dmax = fmaxf(dmax, fabsf(dv[j]));
             if (vs_out) vs_out[row] = vs;
             if (adv_out) adv_out[row] = adv;
-            l_pg += (double)(-logp_a * adv);
-            l_bl += 0.5 * (double)(vs - v) * (double)(vs - v);
+            l_pg += (double)(-logp_a * adv_n);
+            l_bl += 0.5 * (double)verr * (double)verr;
             l_ent += (double)plogp;
+            if constexpr (kPopArt) {
+                s1 += (double)vs;
+                s2 += (double)vs * (double)vs;
+            }
         }
         if (dhead) {  // plain rows: the chunk is one contiguous span of nvalid * ldh floats when ldh == 17
             __syncwarp();
@@ -398,6 +420,15 @@ vtrace_loss_head_kernel(const float* __restrict__ batch, int m, int t, const flo
     l_pg = warp_sum(l_pg);
     l_bl = warp_sum(l_bl);
     l_ent = warp_sum(l_ent);
+    if constexpr (kPopArt) {
+        s1 = warp_sum(s1);
+        s2 = warp_sum(s2);
+        if (lane == 0) {
+            pa_part[3 * (size_t)traj] = s1;
+            pa_part[3 * (size_t)traj + 1] = s2;
+            pa_part[3 * (size_t)traj + 2] = (double)tl;
+        }
+    }
     if (lane == 0) {
         atomicAdd(losses + 1, l_pg);
         atomicAdd(losses + 2, l_bl);
@@ -410,25 +441,37 @@ int launch_vtrace_loss_head(const void* batch, int m, int t, const float* head, 
                             float c_bar, float pg_rho_bar, float lambda_, float baseline_cost,
                             float entropy_cost, bool legal, bool lengths, float* dhead, float* vs, float* pg_adv,
                             double* losses, cudaStream_t stream, float* dhead_hi, float* dhead_lo, int ld_split,
-                            HScale* dhead_hs) {
+                            HScale* dhead_hs, const PopArtArgs& pa) {
     if (m <= 0 || t <= 0) return FI_OK;
     if (!batch || !head || (!dhead && !dhead_hi) || !losses || ldh < kHead || (dhead_hi && (!dhead_lo || ld_split < kHead)))
         return set_error(FI_ERR_ARG, "vtrace loss head: bad argument");
+    const bool popart = pa.part != nullptr;
+    if (popart && !pa.ms && !(pa.sigma > 0.f && std::isfinite(pa.sigma) && std::isfinite(pa.mu)))
+        return set_error(FI_ERR_ARG, "vtrace loss head: PopArt needs a finite mu and a finite sigma > 0 (got %g, %g)", (double)pa.mu,
+                         (double)pa.sigma);
     const int warps = kLossWarps;
     if ((reinterpret_cast<uintptr_t>(batch) & 15) != 0) return set_error(FI_ERR_ARG, "vtrace loss head: batch must be 16-byte aligned");
     // algorithmic traffic per transition: head row in (17 x 4 B) + dhead row out (17 x 4 B) + the record's
     // behaviour logits, action, reward, discount (19 x 4 B) = 212 B (+ 8 B when vs / pg_adv are written)
     // (the masked head's legal word lies in the same 16-byte load as the discount and aux words: no extra traffic;
     // the length-aware head adds the 4-byte length word per trajectory)
-    static const char* const names[2][2] = {{"vtrace_loss_head_kernel", "vtrace_loss_head_kernel_length"},
-                                            {"vtrace_loss_head_kernel_legal", "vtrace_loss_head_kernel_legal_length"}};
-    LaunchScope ls(names[legal][lengths], stream,
-                   (212.0 + (vs ? 4.0 : 0.0) + (pg_adv ? 4.0 : 0.0)) * (double)m * t + (lengths ? 4.0 * m : 0.0), kWorkBytes);
-    auto kernel = legal ? (lengths ? vtrace_loss_head_kernel<true, true> : vtrace_loss_head_kernel<true, false>)
-                        : (lengths ? vtrace_loss_head_kernel<false, true> : vtrace_loss_head_kernel<false, false>);
-    launch_pdl(kernel, dim3((m + warps - 1) / warps), dim3(32 * warps), 0, stream, (const float*)batch, m, t, head, ldh, rho_bar,
-               c_bar, pg_rho_bar, lambda_, baseline_cost, entropy_cost, dhead, vs, pg_adv, losses, dhead_hi, dhead_lo, ld_split,
-               dhead_hs);
+    // (PopArt adds 24 B of partials per trajectory)
+    static const char* const names[2][2][2] = {
+        {{"vtrace_loss_head_kernel", "vtrace_loss_head_kernel_popart"}, {"vtrace_loss_head_kernel_length", "vtrace_loss_head_kernel_length_popart"}},
+        {{"vtrace_loss_head_kernel_legal", "vtrace_loss_head_kernel_legal_popart"},
+         {"vtrace_loss_head_kernel_legal_length", "vtrace_loss_head_kernel_legal_length_popart"}}};
+    LaunchScope ls(names[legal][lengths][popart], stream,
+                   (212.0 + (vs ? 4.0 : 0.0) + (pg_adv ? 4.0 : 0.0)) * (double)m * t + (lengths ? 4.0 * m : 0.0) + (popart ? 24.0 * m : 0.0),
+                   kWorkBytes);
+    using K = decltype(&vtrace_loss_head_kernel<false, false, false>);
+    static const K kernels[2][2][2] = {
+        {{vtrace_loss_head_kernel<false, false, false>, vtrace_loss_head_kernel<false, false, true>},
+         {vtrace_loss_head_kernel<false, true, false>, vtrace_loss_head_kernel<false, true, true>}},
+        {{vtrace_loss_head_kernel<true, false, false>, vtrace_loss_head_kernel<true, false, true>},
+         {vtrace_loss_head_kernel<true, true, false>, vtrace_loss_head_kernel<true, true, true>}}};
+    launch_pdl(kernels[legal][lengths][popart], dim3((m + warps - 1) / warps), dim3(32 * warps), 0, stream, (const float*)batch, m, t,
+               head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_, baseline_cost, entropy_cost, dhead, vs, pg_adv, losses, dhead_hi, dhead_lo,
+               ld_split, dhead_hs, pa.ms, pa.mu, pa.sigma, pa.part);
     return ls.done();
 }
 
@@ -464,5 +507,27 @@ int fi_op_vtrace_loss_head_opts(const void* batch, int m, int t, const float* he
         return fi::set_error(FI_ERR_ARG, "fi_op_vtrace_loss_head_opts: legal and lengths must be 0 or 1 (got %d, %d)", legal, lengths);
     return fi::launch_vtrace_loss_head(batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_, baseline_cost,
                                        entropy_cost, legal != 0, lengths != 0, dhead, vs, pg_adv, losses, (cudaStream_t)stream);
+}
+
+int fi_op_vtrace_loss_head_popart(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar,
+                                  float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, int legal, int lengths,
+                                  float* dhead, float* vs, float* pg_adv, double* losses, float mu, float sigma, double* sums,
+                                  void* stream) {
+    if ((legal != 0 && legal != 1) || (lengths != 0 && lengths != 1))
+        return fi::set_error(FI_ERR_ARG, "fi_op_vtrace_loss_head_popart: legal and lengths must be 0 or 1 (got %d, %d)", legal, lengths);
+    if (!sums) return fi::set_error(FI_ERR_ARG, "fi_op_vtrace_loss_head_popart: null sums");
+    if (!(sigma > 0.f) || !std::isfinite(sigma) || !std::isfinite(mu))
+        return fi::set_error(FI_ERR_ARG, "fi_op_vtrace_loss_head_popart: need a finite mu and a finite sigma > 0 (got %g, %g)", (double)mu,
+                             (double)sigma);
+    if (m <= 0 || t <= 0) return FI_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    double* part = nullptr;   // the per-trajectory partials, stream-ordered scratch
+    FI_CUDA_OK(cudaMallocAsync((void**)&part, 3 * sizeof(double) * (size_t)m, st));
+    int rc = fi::launch_vtrace_loss_head(batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_, baseline_cost, entropy_cost,
+                                         legal != 0, lengths != 0, dhead, vs, pg_adv, losses, st, nullptr, nullptr, 0, nullptr,
+                                         fi::PopArtArgs{nullptr, mu, sigma, part});
+    if (rc == FI_OK) rc = fi::launch_popart_sums(part, m, sums, st);
+    cudaFreeAsync(part, st);
+    return rc;
 }
 }

@@ -142,9 +142,10 @@ public:
     // legal_action_mask: fi_learner_config.legal_action_mask (actor-critic only; records carry the legal word, fi_learner.h).
     // variable_length: fi_learner_config.variable_length (actor-critic only; record 0 carries the trajectory's length).
     // history_length: fi_learner_config.history_length (FarmerLstm only; record 0 carries the move history's length).
+    // popart_beta: fi_learner_config.popart_beta (actor-critic only; 0 = off, > 0 = PopArt value normalisation).
     Learner(size_t p, size_t B, size_t S, size_t M, size_t /*r*/, size_t c, const std::string& l, const std::string& m,
             size_t T, int device = 0, int model = FI_MODEL_MLP_ACTOR_CRITIC, bool legal_action_mask = false,
-            bool variable_length = false, bool history_length = false)
+            bool variable_length = false, bool history_length = false, double popart_beta = 0.0)
         : num_players_(p), batch_size_(M), checkpoint_frequency_(c), checkpoint_location_(l), total_iterations_(T) {
         fi_learner_config cfg;
         fi_learner_config_default(&cfg);
@@ -159,6 +160,7 @@ public:
         cfg.legal_action_mask = legal_action_mask ? 1 : 0;
         cfg.variable_length = variable_length ? 1 : 0;
         cfg.history_length = history_length ? 1 : 0;
+        cfg.popart_beta = popart_beta;
         h_ = fi_learner_create(&cfg);
         if (!h_) throw std::runtime_error(std::string("fi_learner_create: ") + fi_last_error());
         model_manager_ = std::make_shared<ModelManager>(h_, p);

@@ -13,6 +13,8 @@
 // actor draws L uniform in 1..game_steps per trajectory, makes and writes only L records (the slot keeps the tail of whatever
 // trajectory used it before), with L in word 183 of record 0 and the bootstrap value in record L - 1; with --sample-actions
 // it samples those L rows. The JSON line then also reports valid_transitions, the sum of the lengths written.
+// --popart-beta B: the learner normalises its value head with PopArt (fi_learner_config.popart_beta); the JSON line then also
+// reports each player's final statistics, popart_mu and popart_sigma.
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -31,6 +33,7 @@ struct Params {  // ProgramParams, cmd/freeimpala/main.cpp:18-35 (defaults :38-1
     int infer_every = 0;  // >0: every k-th iteration an actor asks for batched policy inference on its observations
     bool sample_actions = false;
     bool variable_length = false;
+    double popart_beta = 0.0;  // --popart-beta B: PopArt value normalisation of the learner (0 = off)
 };
 
 static bool parse(int argc, char** argv, Params& p) {
@@ -49,6 +52,7 @@ static bool parse(int argc, char** argv, Params& p) {
         else if (a == "-m" || a == "--starting-model") p.starting_model = argv[++i];
         else if (a == "--seed") p.seed = (unsigned)strtoul(argv[++i], nullptr, 10);
         else if (a == "--infer-every") p.infer_every = atoi(argv[++i]);
+        else if (a == "--popart-beta") p.popart_beta = strtod(argv[++i], nullptr);
         else if (a == "--metrics-file" || a == "--log-level" || a == "--broker") ++i;  // accepted, unused here
         else return false;
     }
@@ -143,14 +147,14 @@ int main(int argc, char** argv) {
     Params P;
     if (!parse(argc, argv, P)) {
         fprintf(stderr, "usage: freeimpala_gpu [-p N] [-T N] [-S N] [-B N] [-M N] [-a N] [--game-steps N] [--agent-time ms] "
-                        "[-c N] [-l DIR] [-m DIR] [--seed N] [--infer-every K] [--sample-actions] [--variable-length]\n");
+                        "[-c N] [-l DIR] [-m DIR] [--seed N] [--infer-every K] [--sample-actions] [--variable-length] [--popart-beta B]\n");
         return 2;
     }
     const size_t learner_iterations = (P.agents * P.iterations) / P.batch_size;  // main.cpp:179 (integer division)
     try {
         Learner learner(P.players, P.buffer_capacity, P.entry_size, P.batch_size, P.learner_time, P.checkpoint_freq,
                         P.checkpoint_location, P.starting_model, learner_iterations, 0, FI_MODEL_MLP_ACTOR_CRITIC,
-                        P.sample_actions, P.variable_length);
+                        P.sample_actions, P.variable_length, false, P.popart_beta);
         const auto t0 = std::chrono::steady_clock::now();
         learner.start();
         std::atomic<uint64_t> inferences{0};
@@ -190,6 +194,22 @@ int main(int argc, char** argv) {
             printf(", \"actor_sampled_rows\": %llu, \"illegal_actions\": %llu", (unsigned long long)sampled.rows.load(),
                    (unsigned long long)sampled.illegal.load());
         if (P.variable_length) printf(", \"valid_transitions\": %llu", (unsigned long long)sampled.valid_transitions.load());
+        if (P.popart_beta > 0.0) {   // each player's final PopArt statistics
+            std::string mus, sigmas;
+            for (size_t p = 0; p < P.players; p++) {
+                double st[3] = {0.0, 0.0, 0.0};
+                if (fi_learner_popart_stats(learner.handle(), (int)p, st) != FI_OK) {
+                    fprintf(stderr, "freeimpala_gpu: fi_learner_popart_stats: %s\n", fi_last_error());
+                    return 1;
+                }
+                char buf[64];
+                snprintf(buf, sizeof(buf), "%s%.17g", p ? ", " : "", st[0]);
+                mus += buf;
+                snprintf(buf, sizeof(buf), "%s%.17g", p ? ", " : "", st[2]);
+                sigmas += buf;
+            }
+            printf(", \"popart_mu\": [%s], \"popart_sigma\": [%s]", mus.c_str(), sigmas.c_str());
+        }
         printf("}\n");
         if (sampled.failed.load() || sampled.illegal.load()) return 1;
         return updates == learner_iterations * P.players ? 0 : 1;

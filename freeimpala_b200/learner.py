@@ -81,7 +81,7 @@ class Learner:
                  lambda_: float = 1.0, baseline_cost: float = 0.5, entropy_cost: float = 0.01,
                  max_grad_norm: float = 0.0, rmsprop_alpha: float = 0.99, rmsprop_eps: float = 1e-8,
                  rmsprop_momentum: float = 0.0, legal_action_mask: bool = False, variable_length: bool = False,
-                 history_length: bool = False):
+                 history_length: bool = False, popart_beta: float = 0.0):
         self._lib = _lib.load()
         self.num_players, self.buffer_capacity, self.entry_size, self.batch_size = p, B, S, M
         self.train_time_ms, self.checkpoint_frequency = r, c
@@ -100,6 +100,7 @@ class Learner:
         cfg.legal_action_mask = int(legal_action_mask)   # records carry the legal-action word (fi_learner.h)
         cfg.variable_length = int(variable_length)       # record 0 of a trajectory carries its length (fi_learner.h)
         cfg.history_length = int(history_length)         # FarmerLstm: record 0 of a slot carries its history's length
+        cfg.popart_beta = popart_beta                     # PopArt value normalisation; 0 = off (fi_learner.h)
         self._ckpt = l.encode() if l else None
         cfg.checkpoint_location = self._ckpt
         self._h = self._lib.fi_learner_create(C.byref(cfg))
@@ -244,6 +245,12 @@ class Learner:
         check(self._lib.fi_learner_debug_relu_masks(self._h, player_index, out.ctypes.data, out.size),
               "fi_learner_debug_relu_masks")
         return out
+
+    def popart_stats(self, player_index: int) -> tuple[float, float, float]:
+        """PopArt statistics (mu, nu, sigma) after the updates enqueued so far (synchronises the player's stream)."""
+        out = (C.c_double * 3)()
+        check(self._lib.fi_learner_popart_stats(self._h, player_index, out), "fi_learner_popart_stats")
+        return out[0], out[1], out[2]
 
     def steps_done(self, player_index: int) -> int:
         return self._lib.fi_learner_steps_done(self._h, player_index)

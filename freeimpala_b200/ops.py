@@ -20,10 +20,20 @@ def vtrace(m: int, t: int, log_rho: int, discount: int, reward: int, value: int,
 
 def vtrace_loss_head(batch: int, m: int, t: int, head: int, ldh: int, dhead: int, losses: int, vs: int = None,
                      pg_adv: int = None, rho_bar=1.0, c_bar=1.0, pg_rho_bar=1.0, lambda_=1.0, baseline_cost=0.5,
-                     entropy_cost=0.01, stream=None, legal_mask=False, lengths=False) -> None:
+                     entropy_cost=0.01, stream=None, legal_mask=False, lengths=False, popart=None, sums: int = None) -> None:
     """legal_mask: the softmaxes, entropy and d(head) run over each record's legal-action word (fi_learner.h).
     lengths: each trajectory holds as many steps as word 183 of its record 0 says; the rows past them get zero d(head),
-    vs and pg_adv."""
+    vs and pg_adv.
+    popart: (mu, sigma) runs PopArt normalisation (fi_op_vtrace_loss_head_popart): head column 16 is the normalised value and
+    `sums` (device double[3]) receives {sum vs, sum vs^2, valid steps}."""
+    if popart is not None:
+        if sums is None:
+            raise ValueError("vtrace_loss_head: popart needs a sums pointer")
+        mu, sigma = popart
+        check(_lib.load().fi_op_vtrace_loss_head_popart(batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_, baseline_cost,
+                                                        entropy_cost, int(legal_mask), int(lengths), dhead, vs, pg_adv, losses, mu,
+                                                        sigma, sums, stream), "fi_op_vtrace_loss_head_popart")
+        return
     if lengths:
         check(_lib.load().fi_op_vtrace_loss_head_opts(batch, m, t, head, ldh, rho_bar, c_bar, pg_rho_bar, lambda_, baseline_cost,
                                                       entropy_cost, int(legal_mask), 1, dhead, vs, pg_adv, losses, stream),

@@ -193,6 +193,10 @@ typedef struct fi_learner_config {
        whose move history z is its first L records, L read from word 183 of its record 0 (FI_REC_WORD_LENGTH), and the step
        runs the LSTM over exactly those records; 0 = every history is entry_size records long, word 183 is not read. */
     int history_length;
+    /* Appended after history_length; fi_learner_config_default sets 0 (off). Actor-critic model only; finite, 0 <= beta <= 1
+       (a NaN, a value outside [0, 1] or beta > 0 on a FarmerLstm learner is rejected). beta > 0 turns on PopArt value
+       normalisation: see "PopArt" below. */
+    double popart_beta;
 } fi_learner_config;
 
 /* Trajectory record (FI_ELEMENT_SIZE bytes = 256 32-bit words) of the actor-critic model, the words the loss head reads
@@ -238,6 +242,38 @@ typedef struct fi_learner_config {
  * may hand fi_ring_write only those max(L, 8) x FI_ELEMENT_SIZE bytes. A learner with history_length = 0 never reads word 183. */
 #define FI_REC_WORD_LENGTH 183
 
+/* PopArt value normalisation (popart_beta = beta > 0; van Hasselt et al. 2016, Hessel et al. 2019). Each player keeps doubles
+ * mu and nu on the device, initially 0 and 1, and sigma(mu, nu) = clamp(sqrt(max(nu - mu^2, 0)), 1e-4, 1e6). Step s runs with
+ * the statistics mu_s, nu_s, sigma_s (the kernels use fp32 copies of mu_s and sigma_s). For every valid transition (every one,
+ * or the first L of each trajectory with variable_length) head column 16 is the normalised value n_t, and:
+ *   - V_t = sigma_s n_t + mu_s. V-trace runs on V_t and on the bootstrap value in word 181, which stays in reward units,
+ *     giving vs_t and A_t = rho_pg_t (r_t + gamma_t vs_{t+1} - V_t);
+ *   - policy-gradient loss: sum -log pi(a_t) A_t / sigma_s, and the policy gradient uses the same A_t / sigma_s; the entropy
+ *     and legal-action masking are unchanged;
+ *   - baseline loss: 1/2 sum ((vs_t - mu_s) / sigma_s - n_t)^2, gradient d/dn_t = -baseline_cost ((vs_t - mu_s) / sigma_s - n_t);
+ *   - losses[4] reports {total, pg, baseline, entropy} in these normalised units;
+ *   - S1 = sum vs_t, S2 = sum vs_t^2, N = the number of valid transitions, over every data-parallel rank, summed in a fixed
+ *     order (two identical runs give the same bits).
+ * The optimiser then updates the parameters as without PopArt (gradient clipping sees the normalised gradient), and after it
+ *   mu_{s+1} = (1 - beta) mu_s + beta S1 / N,  nu_{s+1} = (1 - beta) nu_s + beta S2 / N,  sigma_{s+1} = sigma(mu_{s+1}, nu_{s+1}),
+ * and the value row of the head (head.w row 16, 512 values, and head.b[16]) is rescaled so that sigma n + mu does not change:
+ *   w <- w sigma_s / sigma_{s+1},  b <- (sigma_s b + mu_s - mu_{s+1}) / sigma_{s+1}   (double, rounded to fp32 once).
+ * Optimiser moments are not rescaled. Batch s is normalised with the statistics of the batches before it (DESIGN.md says why).
+ *
+ * Publication: the published model is a plain actor-critic whose value output is in reward units. The model store (fi_model_get,
+ * inference, the snapshots) holds every parameter as the arena does except the value row: w_pub = sigma w, b_pub = sigma b + mu,
+ * with the current statistics, in double, rounded once. So fi_model_bytes and the blob format are unchanged, every inference
+ * entry point returns reward-unit values, and actors keep writing reward-unit bootstrap values. fi_learner_get_params /
+ * set_params read and write the arena itself (normalised value row).
+ *
+ * Checkpoints: fi_model_save writes the published blob. With with_optimizer_state = 1 it appends, after the optimiser section,
+ * "FIPOP001", mu and nu (doubles) and the 513 normalised value-row floats (w then b), so that a PopArt learner resumes bit-exact.
+ * A PopArt learner that loads a file without the section starts from mu = 0, nu = 1 (sigma = 1: the same outputs); a learner
+ * without PopArt ignores the section.
+ *
+ * Data parallelism: S1, S2 and N travel in the step's all-reduce, so every rank derives the same statistics. A host that runs
+ * its own collective on fi_learner_grad_ptr gets statistics from its own rank's batch only. */
+
 typedef struct fi_learner fi_learner;
 
 FI_API void fi_learner_config_default(fi_learner_config* cfg);
@@ -246,7 +282,7 @@ FI_API void fi_learner_config_default(fi_learner_config* cfg);
  * optimiser, max_grad_norm < 0 or not finite, rmsprop_alpha outside (0, 1), rmsprop_eps <= 0 or
  * rmsprop_momentum outside [0, 1), legal_action_mask other than 0 or 1 or set to 1 for the FarmerLstm model (which has
  * no policy), variable_length other than 0 or 1 or set to 1 for the FarmerLstm model, history_length other than 0 or 1 or set
- * to 1 for the actor-critic model, and, for the actor-critic model, a V-trace constant outside the range
+ * to 1 for the actor-critic model, popart_beta not finite or outside [0, 1] or above 0 for the FarmerLstm model, and, for the actor-critic model, a V-trace constant outside the range
  * fi_learner_config states, is rejected (FI_ERR_ARG) before any device is looked for. */
 FI_API fi_learner* fi_learner_create(const fi_learner_config* cfg);
 FI_API void fi_learner_destroy(fi_learner* l);
@@ -285,6 +321,9 @@ FI_API int fi_learner_set_lr(fi_learner* l, int player, double lr);
 /* Wait until everything enqueued for this player (step and weight publication) has finished. */
 FI_API int fi_learner_sync(fi_learner* l, int player);
 FI_API uint64_t fi_learner_steps_done(fi_learner* l, int player);
+/* PopArt statistics of this player after the updates enqueued so far: out = {mu, nu, sigma} (synchronises the player's
+ * stream). FI_ERR_STATE when the learner runs without PopArt (popart_beta = 0). */
+FI_API int fi_learner_popart_stats(fi_learner* l, int player, double out[3]);
 
 /* Inspection for parity tests: the ReLU decisions (1 = active) of the 5 hidden layers in the last
  * forward pass of this player, [5][rows * 512] bytes (rows = M*T for the actor-critic model, M for
@@ -422,6 +461,10 @@ FI_API int fi_op_vtrace_loss_head_legal(const void* batch, int m, int t, const f
  * from word 183 of its record 0 (see FI_REC_WORD_LENGTH) and writes zero d(head), vs and pg_adv rows for the steps past it.
  * legal and lengths must be 0 or 1. */
 FI_API int fi_op_vtrace_loss_head_opts(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar, float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, int legal, int lengths, float* dhead, float* vs, float* pg_adv, double* losses, void* stream);
+/* fi_op_vtrace_loss_head_opts with PopArt normalisation at statistics mu, sigma (finite, sigma > 0; see "PopArt" above): head
+ * column 16 is the normalised value, d(head) and the losses are in normalised units, vs and pg_adv (optional) are vs_t and A_t
+ * in reward units. sums (device double[3]) receives {S1, S2, N} over the valid transitions (written, not added). */
+FI_API int fi_op_vtrace_loss_head_popart(const void* batch, int m, int t, const float* head, int ldh, float rho_bar, float c_bar, float pg_rho_bar, float lambda_, float baseline_cost, float entropy_cost, int legal, int lengths, float* dhead, float* vs, float* pg_adv, double* losses, float mu, float sigma, double* sums, void* stream);
 
 /* The sampling kernel of fi_learner_infer_sample on caller-owned device pointers. head [rows, ldh], ldh >= 16: only columns
  * 0..15 are read. legal [rows] (may be NULL = all 16 legal), actions [rows] int32. Row r uses RNG counter r, the seed and
